@@ -6,7 +6,11 @@ atlas priors, full brain (speedup_segmentation=False: every voxel is a candidate
 one whole volume from "volume + atlas resident in HBM" to "label volume resident in HBM"
 (sc_segment_volume: dense dilated formulation of the three-branch CNN + atlas-fused FC head).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size 256] [--dump-outputs DIR]
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the label volume of its last step as DIR/labels.npy (float32
+labels at a fixed, seeded sample of at most DUMP_VOXELS voxels) and DIR/label_index.npy (their flat C-order indices,
+float64).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 N > 1 (launched by torchrun, one rank per GPU): every rank segments its own volume (configs[2]:
 volumes sharded across GPUs, no collective) -> weak scaling; value = N * voxels * K / max-over-ranks time.
@@ -54,6 +58,17 @@ FLOP_PATCHWISE = 35407800       # SURVEY.md 8(d): algorithmic forward FLOPs per 
 FLOP_DENSE = {"conv1": 3 * 2 * 180, "conv2": 3 * 2 * 3600, "conv3": 3 * 2 * 7200, "conv4": 3 * 2 * 14400,
               "conv5": 3 * 2 * 21600, "gemm_d1": 3 * 2 * 97200, "gemm_fc1": 2 * 291600, "gemm_fc2": 2 * 149850,
               "out_softmax": 2 * 4050}
+DUMP_VOXELS = 1 << 22           # 16 MB of float32 labels + 32 MB of float64 indices at most
+
+
+def dump_labels(lab, out_dir):
+    """a fixed, seeded sample of the uint8 label volume (all of it when it has <= DUMP_VOXELS voxels) -> out_dir/*.npy"""
+    n = lab.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_VOXELS), replace=False))
+    vals = lab.view(-1).cpu().numpy()[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "labels.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, "label_index.npy"), idx.astype(np.float64))
 
 
 def load_peaks():
@@ -389,7 +404,10 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=65536)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="headline + e2e only (skip train / sharded / 320^3 / dp_check sections)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the labels of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -457,6 +475,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * n_cand * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_labels(d_lab, args.dump_outputs)       # before the sections below overwrite d_lab
 
     # ---- end to end through the host-buffer C-ABI call: pinned host volume + atlas in, labels out ----
     h_vol = torch.from_numpy(norm).pin_memory()

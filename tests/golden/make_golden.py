@@ -1,10 +1,13 @@
 #!/usr/bin/env python
-"""Generate the committed golden fixtures.  Run HERE (build container) only:
+"""Generate the committed golden fixtures from a checkout of the original project:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py /path/to/original/project
 
-``/root/reference`` is read-only and does not exist on the GPU box; nothing in the
-test-suite reads it -- only this script does, once, and its outputs are committed.
+Nothing in the test-suite reads the original project -- only this script does, and its
+outputs are committed.  To keep each fixture under 1 MB, every voxel of a stored volume
+that no patch around a stored centre reads is set to zero (a patch is a copy of the
+voxels it reads, so the stored patches are still the original's output for the stored
+volume).
 
 gather_golden.npz  -- produced by EXECUTING the reference's own source text of
     ``get_patches`` (cnn_cort/base.py:272-308), ``get_mask_voxels`` (:310-331) and
@@ -15,6 +18,8 @@ gather_golden.npz  -- produced by EXECUTING the reference's own source text of
       2. ``map(add, ...)``               ->  ``list(map(...))`` (py2 map returns a list)
       3. ``new_image[idx]`` (list of slices) -> ``new_image[tuple(idx)]`` (numpy>=1.23)
       4. the two-line ``print "..."`` debug block in generate_training_set is dropped.
+    The patch arrays of generate_training_set's output are the B_x_* patches (unshuffled)
+    and those rows in the order T_shuf_perm (shuffled); tests/conftest.py rebuilds them.
 forward_golden.npz -- oracle/network.py (fp64 and fp32) on the committed weights and
     seeded inputs: a regression pin of the restatement (the Theano stack is absent, so
     this part is NOT reference output; see oracle/__init__.py "parity unpinned").
@@ -28,7 +33,39 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/cnn_cort/base.py"
+def read_mask(shape, centres):
+    """the voxels that the axial, coronal and saggital (32, 32) patches around ``centres`` read"""
+    m = np.zeros(shape, bool)
+    for x, y, z in np.asarray(centres).tolist():
+        sx, sy, sz = (slice(max(c - 16, 0), c + 16) for c in (x, y, z))
+        m[sx, sy, z] = m[sx, y, sz] = m[x, sy, sz] = True
+    return m
+
+
+def restrict(vol, centres):
+    vol = vol.copy()
+    vol[~read_mask(vol.shape, centres)] = 0
+    return vol
+
+
+def shrink_gather(out):
+    """zero the unread voxels, store the shuffle of generate_training_set as a permutation"""
+    out = dict(out)
+    out["A_vol"] = restrict(out["A_vol"], out["A_centers"])
+    out["B_vol"] = restrict(out["B_vol"], out["B_sel"])
+    rows = [r.tobytes() for r in out["T_plain_xa"]]
+    perm = np.array([rows.index(r.tobytes()) for r in out["T_shuf_xa"]], dtype=np.int64)
+    for k, mode in (("xa", "axial"), ("xc", "coronal"), ("xs", "saggital")):
+        plain, shuf = out.pop("T_plain_" + k), out.pop("T_shuf_" + k)
+        assert plain.dtype == out["B_x_" + mode].dtype and np.array_equal(plain, out["B_x_" + mode][:, None]), k
+        assert np.array_equal(shuf, plain[perm]), k
+    assert np.array_equal(out["T_shuf_at"], out["T_plain_at"][perm]) and np.array_equal(out["T_shuf_y"], out["T_plain_y"][perm])
+    out["T_shuf_perm"] = perm
+    return out
+
+
+def shrink_forward(out):
+    return dict(out, vol=restrict(out["vol"], out["centers"]))
 
 
 def _slice_def(src, name):
@@ -36,8 +73,8 @@ def _slice_def(src, name):
     return m.group(0)
 
 
-def reference_functions():
-    src = open(REF).read()
+def reference_functions(ref_root):
+    src = open(os.path.join(ref_root, "cnn_cort", "base.py")).read()
     gp = _slice_def(src, "get_patches")
     gp = gp.replace("idx/2", "idx//2")
     gp = gp.replace("[map(add, center, patch_half) for center in centers]",
@@ -53,8 +90,8 @@ def reference_functions():
     return ns["get_patches"], ns["get_mask_voxels"], ns["generate_training_set"]
 
 
-def make_gather():
-    get_patches, get_mask_voxels, generate_training_set = reference_functions()
+def make_gather(ref_root):
+    get_patches, get_mask_voxels, generate_training_set = reference_functions(ref_root)
     rng = np.random.RandomState(20121)
     out = {}
     # case A: non-cubic volume smaller than a patch in one axis, float64 (test-path dtype)
@@ -100,6 +137,7 @@ def make_gather():
     r = generate_training_set(xa, xc, xs, at, ya, {"debug": "False"}, randomize=True)
     for k, v in zip(("xa", "xc", "xs", "at", "y"), r):
         out["T_shuf_" + k] = v
+    out = shrink_gather(out)
     np.savez_compressed(os.path.join(HERE, "gather_golden.npz"), **out)
     print("gather_golden.npz:", {k: v.shape for k, v in out.items()})
 
@@ -124,11 +162,11 @@ def make_forward():
     at[5, 14] = 1
     p64 = net.forward(P, x1, x2, x3, at, dtype=torch.float64)
     p32 = net.forward(P, x1, x2, x3, at, dtype=torch.float32)
-    np.savez_compressed(os.path.join(HERE, "forward_golden.npz"), vol=vol, centers=cen.astype(np.int64),
-                        atlas=at, proba64=p64, proba32=p32)
+    np.savez_compressed(os.path.join(HERE, "forward_golden.npz"), **shrink_forward(dict(
+        vol=vol, centers=cen.astype(np.int64), atlas=at, proba64=p64, proba32=p32)))
     print("forward_golden.npz: max|p64-p32| =", np.abs(p64 - p32).max(), "labels", np.argmax(p64, 1)[:16])
 
 
 if __name__ == "__main__":
-    make_gather()
+    make_gather(sys.argv[1])
     make_forward()

@@ -1,6 +1,5 @@
 """K1 parity (bit-exact): CUDA gather / candidate indexing / scatter through the C-ABI vs the
 reference-generated golden vectors and the oracle."""
-import os
 
 import numpy as np
 import pytest
@@ -19,8 +18,8 @@ def ctx():
 
 
 @pytest.fixture(scope="module")
-def G(golden_dir):
-    return np.load(os.path.join(golden_dir, "gather_golden.npz"))
+def G(gather_golden):
+    return gather_golden
 
 
 def _gather(ctx, vol, cen, atlas=None, bg_fix=True):

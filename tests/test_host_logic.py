@@ -89,8 +89,8 @@ def test_train_split_is_first_stratified_fold():
     assert set(tr).isdisjoint(va)
 
 
-def test_generate_training_set_matches_reference(golden_dir):
-    G = np.load(os.path.join(golden_dir, "gather_golden.npz"))
+def test_generate_training_set_matches_reference(gather_golden):
+    G = gather_golden
     n0 = 10
     args = ([G["B_x_axial"][:n0], G["B_x_axial"][n0:]], [G["B_x_coronal"][:n0], G["B_x_coronal"][n0:]],
             [G["B_x_saggital"][:n0], G["B_x_saggital"][n0:]], [G["T_atlas0"], G["T_atlas1"]],

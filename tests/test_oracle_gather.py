@@ -1,6 +1,5 @@
 """Oracle gather vs. the golden vectors produced by executing the reference's own
 get_patches / get_mask_voxels / generate_training_set text (tests/golden/make_golden.py)."""
-import os
 
 import numpy as np
 import pytest
@@ -9,8 +8,8 @@ from oracle import gather
 
 
 @pytest.fixture(scope="module")
-def G(golden_dir):
-    return np.load(os.path.join(golden_dir, "gather_golden.npz"))
+def G(gather_golden):
+    return gather_golden
 
 
 @pytest.mark.parametrize("mode", gather.VIEWS)
