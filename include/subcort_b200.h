@@ -134,6 +134,27 @@ SC_API int sc_gather_patches(sc_ctx* ctx, const float* vol_dev, const int32_t di
 SC_API int sc_gather_center_labels(sc_ctx* ctx, const uint8_t* labels_dev, const int32_t dims[3],
                             const int32_t* xyz_dev, int64_t n, uint8_t* y_dev, void* stream);
 
+/* ---- training minibatch from device-resident scans -----------------------------------
+ * replaces: the patch arrays of load_patch_vectors / generate_training_set (base.py:53-184), i.e.
+ * 12 KB of materialised patches per training sample, by a per-minibatch gather from the scans.
+ * A training set is a table of N sample rows (scan, x, y, z) int32 [N][4] (16-byte aligned) over
+ * n_scans caller-owned float32 volumes [X][Y][Z] (C order, normalised), optionally with an atlas
+ * row float32 [N][15] and a label uint8 [N] per sample.  For i < n the call writes row
+ * r = idx_dev[i] (r = i when idx_dev is NULL) of the table: the axial / coronal / saggital
+ * patches [n][1][32][32] of scan `scan` around (x, y, z), exactly get_patches's windows and zero
+ * fill (base.py:272-308), atlas_out[i] = atlas_rows[r] and y_out[i] = labels[r].  Any output may be
+ * NULL; n == 0 is a no-op.  SC_ERR_ARG: negative counts, a NULL table or scan list (n > 0), an
+ * atlas / label output requested without its source.
+ * The table is device data and is not range-checked on the device: the caller guarantees
+ * 0 <= idx[i] < N, 0 <= scan < n_scans, and a centre inside its scan's dims (cnn_cort checks
+ * the table once, when the set is built).  A scan index outside [0, n_scans) yields zero
+ * patches rather than an out-of-bounds read. */
+typedef struct { const float* vol; int32_t dims[3]; int32_t reserved; } sc_scan;   /* 24 bytes; vol: caller-owned device array */
+SC_API int sc_gather_samples(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans, const int32_t* samples_dev,
+                      const float* atlas_rows_dev, const uint8_t* labels_dev, const int64_t* idx_dev, int64_t n,
+                      float* axial_dev, float* coronal_dev, float* saggital_dev, float* atlas_out_dev,
+                      uint8_t* y_out_dev, void* stream);
+
 /* ---- network forward (patchwise) -----------------------------------------------------
  * replaces: net.predict_proba / net.predict on {'in1','in2','in3','in4'}
  * (call sites base.py:425-428, 435-438).  proba_dev [n][15] and/or label_dev [n] may be

@@ -15,6 +15,10 @@ PARAM_FLOATS = 883455
 # sc_dtype codes of raw (un-normalised) volumes, include/subcort_b200.h
 DTYPE_CODES = {"u1": 1, "i1": 2, "u2": 3, "i2": 4, "u4": 5, "i4": 6, "f4": 7, "f8": 8}
 
+# sc_scan of include/subcort_b200.h: {const float* vol; int32_t dims[3]; int32_t reserved;}
+SCAN_DTYPE = np.dtype([("vol", "<u8"), ("dims", "<i4", (3,)), ("reserved", "<i4")])
+assert SCAN_DTYPE.itemsize == 24
+
 _lib = None
 
 
@@ -52,6 +56,7 @@ PROTOTYPES = {
     "sc_post_process": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _vp, _vp]),
     "sc_gather_patches": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, ctypes.c_int, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp]),
     "sc_gather_center_labels": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _c_i64, _vp, _vp]),
+    "sc_gather_samples": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sc_forward": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp]),
     "sc_forward_host": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp]),
     "sc_dense_layer": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _c_i64, _vp, ctypes.c_int, _vp]),
@@ -275,6 +280,33 @@ class Context(object):
         y = torch.empty((xyz.shape[0],), dtype=torch.uint8, device=labels.device)
         _check(self.lib.sc_gather_center_labels(self.h, _ptr(labels), _dims(labels.shape), _ptr(xyz), xyz.shape[0], _ptr(y), _stream()))
         return y
+
+    def scan_table(self, volumes):
+        """float32 CUDA volumes [X,Y,Z] -> the sc_scan array sc_gather_samples reads (uint8 CUDA tensor).  The table
+        holds raw pointers: the volumes must outlive it."""
+        import torch
+        t = np.zeros(len(volumes), SCAN_DTYPE)
+        for k, v in enumerate(volumes):
+            assert v.dtype == torch.float32 and v.dim() == 3 and v.is_contiguous()
+            t[k]["vol"], t[k]["dims"] = v.data_ptr(), tuple(v.shape)
+        return torch.from_numpy(t.view(np.uint8)).to("cuda:%d" % self.device)
+
+    def gather_samples(self, table, n_scans, samples, atlas_rows=None, labels=None, idx=None, n=None,
+                       views=(True, True, True), want_atlas=True, want_y=True):
+        """Rows idx (None: the first n rows) of a device sample table (int32 [N,4] scan, x, y, z) ->
+        (axial, coronal, saggital [n,1,32,32] float32, atlas [n,15] float32, y [n] uint8); outputs not asked for, or
+        whose source is None, are None (sc_gather_samples)."""
+        import torch
+        if n is None:
+            n = idx.shape[0] if idx is not None else samples.shape[0]
+        d = samples.device
+        outs = [torch.empty((n, 1, 32, 32), dtype=torch.float32, device=d) if v else None for v in views]
+        at = torch.empty((n, 15), dtype=torch.float32, device=d) if want_atlas and atlas_rows is not None else None
+        y = torch.empty((n,), dtype=torch.uint8, device=d) if want_y and labels is not None else None
+        _check(self.lib.sc_gather_samples(self.h, _ptr(table), int(n_scans), _ptr(samples), _ptr(atlas_rows), _ptr(labels),
+                                          _ptr(idx), int(n), _ptr(outs[0]), _ptr(outs[1]), _ptr(outs[2]), _ptr(at), _ptr(y),
+                                          _stream()))
+        return outs[0], outs[1], outs[2], at, y
 
     # -- network ------------------------------------------------------------------------------
     def forward(self, in1, in2, in3, in4, want_proba=True, want_label=True):

@@ -366,6 +366,31 @@ def load_patches(dir_name, mask_name, t1_name, size, seeds=None, balance_neg=Tru
     return x_axial, y_axial, x_cor, y_cor, x_sag, y_sag, x_atlas, t1_names
 
 
+def _train_normalise(im):
+    """float32 (im - mean_nz) / std_nz of the training path. [base.py:146]"""
+    nz = im[np.nonzero(im)]
+    # base.py:146 under the reference's numpy 1.12: a float32 array combined with float64 *scalars* stays float32
+    # (value-based casting), i.e. the mean and std are rounded to float32 first; NumPy 2 would promote to float64
+    return (im.astype(np.float32) - np.float32(nz.mean())) / np.float32(nz.std())
+
+
+def _training_centres(mask, device, balance_neg=True):
+    """int32 [n, 3]: every voxel with label 1..14 in np.nonzero order, then as many shuffled label-15 voxels (Python's
+    ``random``, consumed as get_mask_voxels(..., size=len(pos)) does). [base.py:153-181]"""
+    pos = get_mask_voxels(np.logical_and(mask > 0, mask < 15), device=device, as_array=True)
+    neg = get_mask_voxels(mask == 15, size=len(pos) if balance_neg else None, device=device, as_array=True)
+    return np.concatenate([pos, neg]).astype(np.int32)
+
+
+def _training_order(n, randomize):
+    """Row order of generate_training_set: None (concatenation order) or the permutation drawn from np.random. [base.py:98-110]"""
+    if not randomize:
+        return None
+    seed = np.random.randint(np.iinfo(np.int32).max)
+    # np.random.seed(seed); np.random.permutation(a) == a[RandomState(seed).permutation(len(a))]
+    return np.random.RandomState(seed).permutation(n)
+
+
 def load_patch_vectors(name, label_name, dir_name, size, random_state=42, balance_neg=True, device=None):
     """Boundary-restricted sampling per subject: every voxel with label 1..14 plus as many
     shuffled label-15 voxels; T1 patches of the three views and the label patches.
@@ -383,15 +408,9 @@ def load_patch_vectors(name, label_name, dir_name, size, random_state=42, balanc
     label_names = [os.path.join(dir_name, subject, label_name) for subject in subjects]
     x_axial, y_axial, x_cor, y_cor, x_sag, y_sag, vox_positions = [], [], [], [], [], [], []
     for image_name, lab_name in zip(image_names, label_names):
-        im = load_nii(image_name).get_data()
-        nz = im[np.nonzero(im)]
-        # base.py:146 under the reference's numpy 1.12: a float32 array combined with float64 *scalars* stays float32
-        # (value-based casting), i.e. the mean and std are rounded to float32 first; NumPy 2 would promote to float64
-        im_norm = (im.astype(np.float32) - np.float32(nz.mean())) / np.float32(nz.std())
+        im_norm = _train_normalise(load_nii(image_name).get_data())
         mask = load_nii(lab_name).get_data()
-        pos = get_mask_voxels(np.logical_and(mask > 0, mask < 15), device=ctx.device, as_array=True)
-        neg = get_mask_voxels(mask == 15, size=len(pos) if balance_neg else None, device=ctx.device, as_array=True)
-        cen = np.concatenate([pos, neg]).astype(np.int32)
+        cen = _training_centres(mask, ctx.device, balance_neg)
         vol = _dev(im_norm, ctx.device, np.float32)
         cdev = _centers_tensor(cen, ctx.device)
         ax, co, sa, _ = ctx.gather_patches(vol, cdev)
@@ -431,10 +450,8 @@ def generate_training_set(x_axial, x_coronal, x_saggital, x_atlas, y, options, r
     y_train = np.concatenate(y, axis=0).astype('uint8')
     y_train = np.squeeze(y_train[:, y_train.shape[1] // 2, y_train.shape[2] // 2])
     y_train[y_train == 15] = 0
-    if randomize:
-        seed = np.random.randint(np.iinfo(np.int32).max)
-        perm = np.random.RandomState(seed).permutation(len(y_train))
-        # np.random.seed(seed); np.random.permutation(a) == a[RandomState(seed).permutation(len(a))]
+    perm = _training_order(len(y_train), randomize)
+    if perm is not None:
         x_train_axial, x_train_cor, x_train_sag = x_train_axial[perm], x_train_cor[perm], x_train_sag[perm]
         y_train, x_train_atlas = y_train[perm], x_train_atlas[perm]
     x_train_axial = np.expand_dims(x_train_axial, axis=1)
@@ -445,3 +462,139 @@ def generate_training_set(x_axial, x_coronal, x_saggital, x_atlas, y, options, r
         print("    --> Y_TRAIN POS: ", y_train[y_train > 0].shape[0])
         print("    --> Y_TRAIN NEG: ", y_train[y_train == 0].shape[0])
     return x_train_axial, x_train_cor, x_train_sag, x_train_atlas, y_train
+
+
+# ---------------------------------------------------------------------------------------------
+# training data kept on the device: scans + sample table instead of patch arrays
+# ---------------------------------------------------------------------------------------------
+def check_sample_table(shapes, samples, atlas_rows, labels):
+    """Reject a malformed training table before anything reaches the device: sc_gather_samples trusts its table.
+    shapes: (X, Y, Z) per scan; samples: int [N, 4] (scan, x, y, z); atlas_rows: [N, 15]; labels: [N]."""
+    samples, atlas_rows, labels = np.asarray(samples), np.asarray(atlas_rows), np.asarray(labels)
+    if samples.ndim != 2 or samples.shape[1] != 4:
+        raise ValueError("sample table must be [N, 4] (scan, x, y, z), got shape %s" % (samples.shape,))
+    n = samples.shape[0]
+    if atlas_rows.shape != (n, 15):
+        raise ValueError("atlas rows must be [%d, 15] (one per sample), got shape %s" % (n, atlas_rows.shape))
+    if labels.shape != (n,):
+        raise ValueError("labels must be [%d] (one per sample), got shape %s" % (n, labels.shape))
+    dims = np.asarray([tuple(int(d) for d in s) for s in shapes], dtype=np.int64).reshape(-1, 3)
+    if n == 0:
+        return
+    scan = samples[:, 0].astype(np.int64)
+    bad = np.nonzero((scan < 0) | (scan >= len(dims)))[0]
+    if len(bad):
+        raise ValueError("sample %d: scan index %d out of range [0, %d)" % (bad[0], scan[bad[0]], len(dims)))
+    c = samples[:, 1:].astype(np.int64)
+    bad = np.nonzero(((c < 0) | (c >= dims[scan])).any(1))[0]
+    if len(bad):
+        i = bad[0]
+        raise ValueError("sample %d: centre %s outside scan %d of shape %s" % (i, tuple(c[i]), scan[i], tuple(dims[scan[i]])))
+
+
+class ScanTrainingSet(object):
+    """A training set held as its normalised scans plus one row per sample, all on the device: (scan, x, y, z), the
+    15 atlas priors at the centre and the class label (0..14).  About 80 B per sample instead of the 12 KB of patches
+    that generate_training_set materialises on the host; every minibatch is gathered from the scans by
+    sc_gather_samples.  Row i is row i of what load_data + generate_training_set return for the same seeds.
+
+        scans = load_scan_training_set(options)
+        net.fit(scans)
+        in1, in2, in3, in4, y = scans.gather(idx)       # CUDA tensors of rows idx
+    """
+
+    def __init__(self, volumes, samples, atlas_rows, labels, names=(), device=None):
+        """volumes: float32 [X, Y, Z] per scan (numpy or CUDA tensors); samples int [N, 4]; atlas_rows [N, 15];
+        labels [N].  The table is validated here, on the host, before any upload."""
+        samples = np.ascontiguousarray(samples, dtype=np.int32)
+        atlas_rows = np.ascontiguousarray(atlas_rows, dtype=np.float32)
+        labels = np.ascontiguousarray(labels, dtype=np.uint8)
+        for v in volumes:
+            if len(v.shape) != 3:
+                raise ValueError("scan volumes must be 3-D, got shape %s" % (tuple(v.shape),))
+        check_sample_table([tuple(v.shape) for v in volumes], samples, atlas_rows, labels)
+        import torch
+        from . import parallel
+        self.ctx = get_context(device)
+        d = self.ctx.device
+        self.volumes = [v.to('cuda:%d' % d, torch.float32).contiguous() if torch.is_tensor(v) else _dev(v, d, np.float32)
+                        for v in volumes]
+        self.table = self.ctx.scan_table(self.volumes)
+        self.samples, self.atlas, self.labels = _dev(samples, d), _dev(atlas_rows, d), _dev(labels, d)
+        self.y = labels                       # host copy: TrainSplit's stratified folds
+        self.names = list(names)
+        self.fingerprint = parallel.scan_set_fingerprint(samples, atlas_rows, labels, self.volumes)
+
+    def __len__(self):
+        return len(self.y)
+
+    def device_bytes(self):
+        """bytes of device memory the set holds"""
+        ts = self.volumes + [self.table, self.samples, self.atlas, self.labels]
+        return int(sum(t.numel() * t.element_size() for t in ts))
+
+    def gather(self, idx=None, ctx=None):
+        """-> (in1, in2, in3, in4, y): axial / coronal / saggital [n, 1, 32, 32] float32, atlas [n, 15] float32 and
+        labels [n] uint8 CUDA tensors of rows idx (host integer array, CUDA int64 tensor, or None for every row).  A host
+        idx is range-checked; a device idx is trusted.  ctx: the sc_ctx to launch on (default: the data layer's)."""
+        import torch
+        n = None
+        if idx is None:
+            n = len(self)
+        elif not torch.is_tensor(idx):
+            idx = np.ascontiguousarray(idx, dtype=np.int64).reshape(-1)
+            if idx.size and (idx.min() < 0 or idx.max() >= len(self)):
+                raise IndexError("row index out of range [0, %d)" % len(self))
+            idx = _dev(idx, self.ctx.device)
+        return (ctx or self.ctx).gather_samples(self.table, len(self.volumes), self.samples, self.atlas, self.labels,
+                                                idx=idx, n=n)
+
+    def to_arrays(self, chunk=32768):
+        """(x_axial, x_cor, x_sag, x_atlas, y) host arrays: what generate_training_set returns for the same seeds."""
+        n = len(self)
+        out = [np.empty((n, 1, 32, 32), np.float32) for _ in range(3)] + [np.empty((n, 15), np.float32), np.empty(n, np.uint8)]
+        for s in range(0, n, chunk):
+            for o, t in zip(out, self.gather(np.arange(s, min(n, s + chunk)))):
+                o[s:s + len(t)] = t.cpu().numpy()
+        return tuple(out)
+
+
+def load_scan_training_set(options, randomize=True, device=None):
+    """load_data followed by generate_training_set, kept on the device -> ScanTrainingSet.
+
+    Same semantics and the same random draws as the materialised path, so that the same ``random`` / ``np.random``
+    seeds give the same set in the same order: per subject (sorted sub-folders of train_folder) the train-path
+    normalised T1 (base.py:146), every voxel with label 1..14 in np.nonzero order and as many shuffled label-15 voxels
+    (base.py:153-181), the atlas rows without background fix (quirk Q4), labels with 15 -> 0; subjects concatenated,
+    then one permutation drawn as generate_training_set draws it.  Only the normalised T1 volumes stay on the device;
+    the atlas rows and labels are picked from the host arrays the NIfTI reader returns (an upload of the 15-channel
+    priors would move 60 B per voxel to read 60 B per sample)."""
+    if tuple(options['patch_size']) != (32, 32):
+        raise ValueError("only patch_size (32, 32) is implemented")
+    ctx = get_context(options.get('device') if device is None else device)
+    dir_name = options['train_folder']
+    subjects = [f for f in sorted(os.listdir(dir_name)) if os.path.isdir(os.path.join(dir_name, f))]
+    names, vols, samples, atlas_rows, labels = [], [], [], [], []
+    for k, subject in enumerate(subjects):
+        image_name = os.path.join(dir_name, subject, options['t1_name'])
+        atlas_name = os.path.join(dir_name, subject, 'tmp', 'MNI_sub_probabilities.nii.gz')
+        _require_registered(atlas_name)
+        vols.append(_dev(_train_normalise(load_nii(image_name).get_data()), ctx.device, np.float32))
+        mask = load_nii(os.path.join(dir_name, subject, options['roi_name'])).get_data()
+        cen = _training_centres(mask, ctx.device)
+        x, y, z = cen[:, 0], cen[:, 1], cen[:, 2]
+        lab = mask[x, y, z].astype(np.uint8)
+        lab[lab == 15] = 0
+        atlas_rows.append(np.asarray(load_nii(atlas_name).get_data()[x, y, z], dtype=np.float32))
+        samples.append(np.concatenate([np.full((len(cen), 1), k, np.int32), cen], axis=1))
+        labels.append(lab)
+        names.append(image_name)
+    samples = np.concatenate(samples) if samples else np.zeros((0, 4), np.int32)
+    atlas_rows = np.concatenate(atlas_rows) if atlas_rows else np.zeros((0, 15), np.float32)
+    labels = np.concatenate(labels) if labels else np.zeros(0, np.uint8)
+    perm = _training_order(len(labels), randomize)
+    if perm is not None:
+        samples, atlas_rows, labels = samples[perm], atlas_rows[perm], labels[perm]
+    if options.get('debug') == 'True':
+        print("    --> X_TRAIN: ", len(labels), "samples from", len(vols), "scans")
+    return ScanTrainingSet(vols, samples, atlas_rows, labels, names=names, device=ctx.device)

@@ -219,23 +219,35 @@ class Net(object):
         return self.ctx.forward_host(*xs, want_proba=False)[1].astype(np.int64)
 
     # -- training (nolearn epoch loop: nets.py:233-246) ---------------------------------------
-    def fit(self, X, y, epochs=None):
+    def fit(self, X, y=None, epochs=None):
+        """nolearn's fit on X = {'in1', 'in2', 'in3', 'in4'} arrays with labels y, or on a base.ScanTrainingSet (y
+        omitted), whose minibatches are gathered on the device from the scans.  Same epoch loop either way."""
         import torch
         import torch.distributed as dist
         ctx = self.ctx
         dev = torch.device('cuda', self.device)
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         rank = dist.get_rank() if world > 1 else 0
-        y = np.asarray(y).astype(np.uint8)
+        scans = hasattr(X, 'gather')
+        if scans:
+            if y is not None:
+                raise ValueError("fit: a ScanTrainingSet carries its own labels; call fit(scans) without y")
+            y = X.y
+        else:
+            y = np.asarray(y).astype(np.uint8)
         if y.size and int(y.max()) > 14:
             raise ValueError("fit: labels must be in 0..14 (generate_training_set maps the boundary label 15 to 0, base.py:89)")
         tr, va = self.train_split.indices(y)
-        xs = [np.ascontiguousarray(X[k], dtype=np.float32) for k in ('in1', 'in2', 'in3', 'in4')]
+        if not scans:
+            xs = [np.ascontiguousarray(X[k], dtype=np.float32) for k in ('in1', 'in2', 'in3', 'in4')]
         if world > 1:
             # data parallel: every rank must hold the SAME training set in the same order (shard_batch strides through the
             # global minibatch) and start from the SAME parameters; neither is true by construction (the reference's
             # negative sampling and its weight initialisation are unseeded), so check the first and enforce the second
-            parallel.assert_same_dataset(xs, y, dev)
+            if scans:
+                parallel.assert_same_fingerprint(X.fingerprint, dev)
+            else:
+                parallel.assert_same_dataset(xs, y, dev)
             p = ctx.param_tensor()
             dist.broadcast(p, 0)
             ctx.load_weights(p.cpu().numpy())          # re-derives the inference layouts from the broadcast parameters
@@ -248,7 +260,75 @@ class Net(object):
         fused = world > 1 and str(self.options.get('fused_adam', 'False')) == 'True'
         if fused:
             ctx.fused_attach()
+        batches = self._scan_batches(X, dev) if scans else self._array_batches(xs, y, dev)
 
+        best_valid, best_train = np.inf, np.inf
+        best_epoch, best_weights = 0, None
+        first = len(self.train_history_)
+        bs = self.batch_size
+        n_epochs = epochs or self.max_epochs
+        grads = ctx.grad_tensor()
+        rng = np.random.RandomState(self._seed)
+        loss_buf = torch.zeros(1, dtype=torch.float32, device=dev)
+        steps = [tr[s:s + bs] for s in range(0, len(tr), bs)]
+        local_steps = [parallel.shard_batch(gidx, rank, world) for gidx in steps]
+        valid_steps = [va[s:s + bs] for s in range(0, len(va), bs)]
+        for ep in range(first + 1, first + n_epochs + 1):
+            t0 = time.time()
+            losses, sizes = [], []
+            for gidx, b in zip(steps, batches(local_steps)):
+                if b is not None:
+                    ctx.train_forward_backward(*b, n_global=len(gidx), seed=int(rng.randint(1 << 62)) + rank, loss_out=loss_buf)
+                else:                      # a last partial batch smaller than the world size: contribute zeros
+                    grads.zero_()
+                    loss_buf.zero_()
+                if fused:
+                    ctx.allreduce_adam_step(lr=self.update_learning_rate)
+                    if world > 1:
+                        dist.all_reduce(loss_buf)
+                else:
+                    parallel.allreduce_gradients(grads, loss_buf)
+                    # the BN-statistics slots hold the SUM of the batch statistics of the ranks that had samples: rank r of
+                    # shard_batch has some iff r < len(gidx)
+                    ctx.adam_step(lr=self.update_learning_rate, stat_scale=1.0 / min(world, len(gidx)))
+                losses.append(loss_buf.clone())
+                sizes.append(len(gidx))
+            train_loss = float(np.average(torch.cat(losses).cpu().numpy(), weights=sizes)) if losses else float('nan')
+            vsum = torch.zeros(2, dtype=torch.float32, device=dev)
+            for b in batches(valid_steps):
+                vsum += ctx.eval_batch(*b)
+            vs = vsum.cpu().numpy()
+            valid_loss = float(vs[0] / max(1, len(va)))
+            valid_acc = float(vs[1] / max(1, len(va)))
+            info = {'epoch': ep, 'train_loss': train_loss, 'valid_loss': valid_loss, 'valid_accuracy': valid_acc,
+                    'train_loss_best': train_loss < best_train, 'valid_loss_best': valid_loss < best_valid,
+                    'dur': time.time() - t0}
+            best_train = min(best_train, train_loss)
+            self.train_history_.append(info)
+            if self.verbose:
+                print("  %4d  train %.5f  valid %.5f  acc %.5f  %.2fs" % (ep, train_loss, valid_loss, valid_acc, info['dur']))
+            # on_epoch_finished: SaveWeights(only_best), SaveTrainingHistory, EarlyStopping (nets.py:154-156)
+            if valid_loss < best_valid or len(va) == 0:
+                best_valid, best_epoch = valid_loss, ep
+                best_weights = self.get_all_params_values()
+                if rank == 0 and self.weights_file:
+                    with open(self.weights_file, 'wb') as f:
+                        pickle.dump(best_weights, f, protocol=2)
+            if rank == 0 and self.history_file:
+                with open(self.history_file, 'wb') as f:
+                    pickle.dump(self.train_history_, f, protocol=2)
+            if len(va) and best_epoch + self.patience < ep:
+                if self.verbose:
+                    print("Early stopping. Best valid loss was %.6f at epoch %d." % (best_valid, best_epoch))
+                if best_weights is not None:
+                    self.load_params_from(best_weights)
+                break
+        return self
+
+    def _array_batches(self, xs, y, dev):
+        """minibatch source of fit on host arrays: batches(index lists) yields the device tensors (in1..in4, y) of each
+        list, None for an empty one"""
+        import torch
         # the training set lives on the device when it fits (a minibatch is then one index_select per input instead of five
         # pageable host-to-device copies per step); otherwise minibatches are staged through page-locked buffers
         nbytes = sum(a.nbytes for a in xs) + y.nbytes
@@ -277,68 +357,28 @@ class Net(object):
                 torch.cuda.current_stream().synchronize()      # the staging buffers are reused by the next minibatch
                 return out
 
-        best_valid, best_train = np.inf, np.inf
-        best_epoch, best_weights = 0, None
-        first = len(self.train_history_)
-        bs = self.batch_size
-        n_epochs = epochs or self.max_epochs
-        grads = ctx.grad_tensor()
-        rng = np.random.RandomState(self._seed)
-        loss_buf = torch.zeros(1, dtype=torch.float32, device=dev)
-        for ep in range(first + 1, first + n_epochs + 1):
-            t0 = time.time()
-            losses, sizes = [], []
-            for s in range(0, len(tr), bs):
-                gidx = tr[s:s + bs]
-                lidx = parallel.shard_batch(gidx, rank, world)
-                if len(lidx):
-                    b = to_dev(lidx)
-                    ctx.train_forward_backward(*b, n_global=len(gidx), seed=int(rng.randint(1 << 62)) + rank, loss_out=loss_buf)
-                else:                      # a last partial batch smaller than the world size: contribute zeros
-                    grads.zero_()
-                    loss_buf.zero_()
-                if fused:
-                    ctx.allreduce_adam_step(lr=self.update_learning_rate)
-                    if world > 1:
-                        dist.all_reduce(loss_buf)
-                else:
-                    parallel.allreduce_gradients(grads, loss_buf)
-                    # the BN-statistics slots hold the SUM of the batch statistics of the ranks that had samples: rank r of
-                    # shard_batch has some iff r < len(gidx)
-                    ctx.adam_step(lr=self.update_learning_rate, stat_scale=1.0 / min(world, len(gidx)))
-                losses.append(loss_buf.clone())
-                sizes.append(len(gidx))
-            train_loss = float(np.average(torch.cat(losses).cpu().numpy(), weights=sizes)) if losses else float('nan')
-            vsum = torch.zeros(2, dtype=torch.float32, device=dev)
-            for s in range(0, len(va), bs):
-                vsum += ctx.eval_batch(*to_dev(va[s:s + bs]))
-            vs = vsum.cpu().numpy()
-            valid_loss = float(vs[0] / max(1, len(va)))
-            valid_acc = float(vs[1] / max(1, len(va)))
-            info = {'epoch': ep, 'train_loss': train_loss, 'valid_loss': valid_loss, 'valid_accuracy': valid_acc,
-                    'train_loss_best': train_loss < best_train, 'valid_loss_best': valid_loss < best_valid,
-                    'dur': time.time() - t0}
-            best_train = min(best_train, train_loss)
-            self.train_history_.append(info)
-            if self.verbose:
-                print("  %4d  train %.5f  valid %.5f  acc %.5f  %.2fs" % (ep, train_loss, valid_loss, valid_acc, info['dur']))
-            # on_epoch_finished: SaveWeights(only_best), SaveTrainingHistory, EarlyStopping (nets.py:154-156)
-            if valid_loss < best_valid or len(va) == 0:
-                best_valid, best_epoch = valid_loss, ep
-                best_weights = self.get_all_params_values()
-                if rank == 0 and self.weights_file:
-                    with open(self.weights_file, 'wb') as f:
-                        pickle.dump(best_weights, f, protocol=2)
-            if rank == 0 and self.history_file:
-                with open(self.history_file, 'wb') as f:
-                    pickle.dump(self.train_history_, f, protocol=2)
-            if len(va) and best_epoch + self.patience < ep:
-                if self.verbose:
-                    print("Early stopping. Best valid loss was %.6f at epoch %d." % (best_valid, best_epoch))
-                if best_weights is not None:
-                    self.load_params_from(best_weights)
-                break
-        return self
+        def batches(index_lists):
+            for idx in index_lists:
+                yield to_dev(idx) if len(idx) else None
+        return batches
+
+    def _scan_batches(self, scans, dev):
+        """minibatch source of fit on a ScanTrainingSet: one upload of all row indices of a pass (an epoch's training or
+        validation minibatches); every minibatch is then gathered from the scans on the device (sc_gather_samples, on
+        this net's context) out of a slice of that upload -- no host synchronise per step"""
+        import torch
+        ctx = self.ctx
+
+        def batches(index_lists):
+            flat = np.concatenate([np.asarray(i, dtype=np.int64) for i in index_lists]) if index_lists else np.zeros(0, np.int64)
+            if flat.size and (flat.min() < 0 or flat.max() >= len(scans)):
+                raise IndexError("fit: row index out of range [0, %d)" % len(scans))
+            d_idx = torch.from_numpy(flat).to(dev)
+            off = 0
+            for idx in index_lists:
+                yield scans.gather(d_idx[off:off + len(idx)], ctx=ctx) if len(idx) else None
+                off += len(idx)
+        return batches
 
 
 def build_model(weights_path, options):

@@ -58,12 +58,31 @@ def dataset_fingerprint(xs, y):
                      zlib.crc32(np.ascontiguousarray(xs[-1][::step]).tobytes())], dtype=np.int64)
 
 
+def scan_set_fingerprint(samples, atlas_rows, labels, volumes):
+    """int64 [5] of a ScanTrainingSet: size, CRCs of the sample table, the labels and the atlas rows, and one CRC over the
+    shape and a strided sample (about 4096 voxels) of every volume (CUDA tensors)"""
+    import zlib
+    import numpy as np
+    crc = 0
+    for v in volumes:
+        flat = v.reshape(-1)
+        crc = zlib.crc32(np.asarray(tuple(v.shape), np.int64).tobytes(), crc)
+        crc = zlib.crc32(flat[::max(1, flat.numel() // 4096)].cpu().numpy().tobytes(), crc)
+    return np.array([len(labels), zlib.crc32(np.ascontiguousarray(samples).tobytes()), zlib.crc32(np.ascontiguousarray(labels).tobytes()),
+                     zlib.crc32(np.ascontiguousarray(atlas_rows).tobytes()), crc], dtype=np.int64)
+
+
 def assert_same_dataset(xs, y, device=None):
     """Data-parallel fit shards every global minibatch by position, so all ranks must hold the same arrays in the same
     order.  Compares a fingerprint with rank 0's and raises on every rank if any rank differs."""
+    assert_same_fingerprint(dataset_fingerprint(xs, y), device)
+
+
+def assert_same_fingerprint(fingerprint, device=None):
+    """Raises on every rank unless every rank's int64 fingerprint equals rank 0's."""
     import torch
     import torch.distributed as dist
-    mine = torch.from_numpy(dataset_fingerprint(xs, y))
+    mine = torch.from_numpy(fingerprint)
     if device is not None and dist.get_backend() == "nccl":
         mine = mine.to(device)
     ref = mine.clone()

@@ -353,6 +353,20 @@ int sc_gather_center_labels(sc_ctx* ctx, const uint8_t* labels_dev, const int32_
   return launch_center_labels(ctx, labels_dev, dims, xyz_dev, n, y_dev, (cudaStream_t)stream);
 }
 
+int sc_gather_samples(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans, const int32_t* samples_dev, const float* atlas_rows_dev,
+                      const uint8_t* labels_dev, const int64_t* idx_dev, int64_t n, float* axial_dev, float* coronal_dev,
+                      float* saggital_dev, float* atlas_out_dev, uint8_t* y_out_dev, void* stream) {
+  SC_CHECK(ctx && n >= 0 && n_scans >= 0, SC_ERR_ARG, "sc_gather_samples: null context or negative count");
+  SC_CHECK(!atlas_out_dev || atlas_rows_dev, SC_ERR_ARG, "sc_gather_samples: atlas output requested without atlas rows");
+  SC_CHECK(!y_out_dev || labels_dev, SC_ERR_ARG, "sc_gather_samples: label output requested without labels");
+  if (n == 0) return SC_OK;
+  SC_CHECK(scans_dev && n_scans > 0 && samples_dev, SC_ERR_ARG, "sc_gather_samples: missing scan list or sample table");
+  SC_CHECK(((uintptr_t)samples_dev & 15) == 0, SC_ERR_ARG, "sc_gather_samples: sample table not 16-byte aligned");
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return launch_gather_samples(ctx, scans_dev, n_scans, samples_dev, atlas_rows_dev, labels_dev, idx_dev, n, axial_dev,
+                               coronal_dev, saggital_dev, atlas_out_dev, y_out_dev, (cudaStream_t)stream);
+}
+
 int sc_forward(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const float* in3_dev, const float* in4_dev,
                int64_t n, float* proba_dev, int32_t* label_dev, void* stream) {
   SC_TRY(fresh_weights(ctx, "sc_forward", (cudaStream_t)stream));

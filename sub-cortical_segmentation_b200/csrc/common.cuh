@@ -258,6 +258,9 @@ int launch_slab_compact(sc_ctx* ctx, const uint8_t* cand, const OutGeo& box, int
                         int32_t* cnt, int32_t* scratch, cudaStream_t st);
 int launch_center_labels(sc_ctx* ctx, const uint8_t* lab, const int32_t* dims, const int32_t* xyz, int64_t n,
                          uint8_t* y, cudaStream_t st);
+int launch_gather_samples(sc_ctx* ctx, const sc_scan* scans, int n_scans, const int32_t* samples, const float* atlas_rows,
+                          const uint8_t* labels, const int64_t* idx, int64_t n, float* ax, float* co, float* sa,
+                          float* atlas_out, uint8_t* y_out, cudaStream_t st);
 int launch_nonzero(sc_ctx* ctx, const void* vol, int elem_bytes, const int32_t* dims, int32_t* xyz,
                    int64_t capacity, int64_t* n_out_host, cudaStream_t st);
 int launch_dilate(sc_ctx* ctx, const uint8_t* mask, const int32_t* dims, int iterations, uint8_t* out, cudaStream_t st);

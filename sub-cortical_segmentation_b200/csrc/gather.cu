@@ -190,6 +190,75 @@ int launch_center_labels(sc_ctx* ctx, const uint8_t* lab, const int32_t* dims, c
   return SC_OK;
 }
 
+// ---- training minibatch from device-resident scans (sc_gather_samples) ---------------------------------------------
+// Rows of a shuffled training set come from random voxels of several volumes, so nothing is shared between neighbouring
+// samples (the np.nonzero-order fast paths of gather_patches_kernel never apply).  One warp per (sample, view), lane =
+// patch column j, a loop over the 32 patch rows i; every store is one full 128 B patch row.
+//   coronal  [dx][dz] at y, saggital [dy][dz] at x: the lanes read 32 consecutive z -> one 128 B line per row.
+//   axial    [dx][dy] at z: the lanes stride by Z (one 32 B sector per element, 32 KB of sector traffic per patch).
+// The warp of view 0 also passes the atlas row (lanes 0..14) and the label (lane 15) through.
+__global__ void __launch_bounds__(256) gather_samples_kernel(
+    const sc_scan* __restrict__ scans, int n_scans, const int32_t* __restrict__ samples, const float* __restrict__ atlas_rows,
+    const uint8_t* __restrict__ labels, const int64_t* __restrict__ idx, int64_t n, float* __restrict__ ax,
+    float* __restrict__ co, float* __restrict__ sa, float* __restrict__ atlas_out, uint8_t* __restrict__ y_out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t job = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (job >= n * 3) return;
+  const int64_t s = job / 3;
+  const int view = (int)(job - s * 3);
+  const int64_t r = idx ? __ldg(idx + s) : s;
+  if (view == 0) {
+    if (atlas_out && lane < 15) atlas_out[s * 15 + lane] = __ldg(atlas_rows + r * 15 + lane);
+    if (y_out && lane == 15) y_out[s] = __ldg(labels + r);
+  }
+  float* dst = view == 0 ? ax : view == 1 ? co : sa;
+  if (!dst) return;
+  const int4 row = __ldg(reinterpret_cast<const int4*>(samples) + r);     // scan, x, y, z
+  // an invalid scan index reads as an empty volume: zeros, never an out-of-bounds access
+  const bool scan_ok = (unsigned)row.x < (unsigned)n_scans;
+  const float* vol = nullptr;
+  int X = 0, Y = 0, Z = 0;
+  if (scan_ok) {
+    vol = scans[row.x].vol;
+    X = scans[row.x].dims[0]; Y = scans[row.x].dims[1]; Z = scans[row.x].dims[2];
+  }
+  const int64_t YZ = (int64_t)Y * Z;
+  // patch row i runs along axis (ci, di, si), column j along (cj, dj, sj); (cf, df, sf) is the fixed axis of the slice
+  int ci, di, cj, dj, cf, df;
+  int64_t si, sj, sf;
+  if (view == 0)      { ci = row.y; di = X; si = YZ; cj = row.z; dj = Y; sj = Z; cf = row.w; df = Z; sf = 1; }
+  else if (view == 1) { ci = row.y; di = X; si = YZ; cj = row.w; dj = Z; sj = 1; cf = row.z; df = Y; sf = Z; }
+  else                { ci = row.z; di = Y; si = Z;  cj = row.w; dj = Z; sj = 1; cf = row.y; df = X; sf = YZ; }
+  const int jj = cj - 16 + lane;
+  const bool jin = jj >= 0 && jj < dj && (unsigned)cf < (unsigned)df;
+  const int i0 = ci - 16, imax = di;
+  const float* src = vol + (int64_t)cf * sf + (int64_t)jj * sj + (int64_t)i0 * si;
+  float* out = dst + s * 1024 + lane;
+#pragma unroll 8
+  for (int i = 0; i < 32; ++i) {
+    const int ii = i0 + i;
+    float v = 0.f;
+    if (jin && ii >= 0 && ii < imax) v = __ldg(src);
+    __stcs(out, v);
+    src += si;
+    out += 32;
+  }
+}
+
+int launch_gather_samples(sc_ctx* ctx, const sc_scan* scans, int n_scans, const int32_t* samples, const float* atlas_rows,
+                          const uint8_t* labels, const int64_t* idx, int64_t n, float* ax, float* co, float* sa,
+                          float* atlas_out, uint8_t* y_out, cudaStream_t st) {
+  if (n == 0) return SC_OK;
+  const int64_t blocks = (n * 3 + 7) / 8;
+  SC_CHECK(blocks < (1ll << 31), SC_ERR_ARG, "sc_gather_samples: too many samples in one call");
+  ProfScope prof(ctx, PC_GATHER, st);
+  gather_samples_kernel<<<(unsigned)blocks, 256, 0, st>>>(scans, n_scans, samples, atlas_rows, labels, idx, n, ax, co, sa,
+                                                          atlas_out, y_out);
+  ctx->launches++;
+  SC_CUDA(cudaGetLastError());
+  return SC_OK;
+}
+
 // ---------------------------------------------------------------------------------------
 // Ordered stream compaction: count per 4096-element block, scan the block counts, emit.
 // ---------------------------------------------------------------------------------------
