@@ -92,7 +92,6 @@ constexpr int kH1 = 555;         // FC1 out (540) + atlas (15)
 constexpr int kH1Ld = 576;       // row stride (K of fc_2)
 constexpr int kH2 = 270;
 constexpr int kH2Ld = 272;
-constexpr int kH2LdTc = 320;     // tcgen05 dense path: h2 rows in the split layout, 5 k-blocks of 64 (the out_layer GEMM reads them)
 constexpr int kC5Ld = 64;        // conv5 output channels padded 60 -> 64 (NHWC)
 constexpr int kD1K = 9 * kC5Ld;  // 576: K of d1 as a 3x3 dilation-4 conv over conv5 output
 
@@ -162,8 +161,7 @@ struct sc_ctx {
   size_t derived_floats = 0;
   sc::BranchW br[3];
   sc::GemmW fc1, fc2;
-  sc::GemmW outl;                // out_layer 270 -> 15 as a K = 320, N = 16 GEMM (tcgen05 softmax epilogue)
-  float* out_w = nullptr;        // [270][16]
+  float* out_w = nullptr;        // [270][16] out_layer weights (fp32; SIMT kernel and the fused epilogue of fc_2)
   float* out_b = nullptr;        // [16]
   sc::Workspace ws;              // inference scratch (grow-only)
   sc::Workspace ws_train;        // staging of the host entry points, scan preparation, eval scratch
@@ -309,7 +307,7 @@ struct GemmProblem {
   const int32_t* rowvox = nullptr;
   const float* atlas = nullptr;            // tcgen05 pair kernel (FC1): write the atlas prior of every row (with the background
   OutGeo ageo;                             // fix of base.py:392-394) into columns 540..554 and zeros up to 575
-  const struct SoftmaxOut* sm = nullptr;   // tcgen05 back-end: softmax / argmax epilogue instead of the row store (out_layer)
+  const struct SoftmaxOut* sm = nullptr;   // tcgen05 back-end, fc_2 only: out_layer + softmax / argmax in the epilogue instead of the row store
   int a_swap = 0;       // tensor-map dimension order is (k, pixel, plane, line) instead of (k, pixel, line, plane)
 };
 int launch_gemm(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream_t st);
@@ -326,7 +324,7 @@ inline void gemm_problem_rows(GemmProblem& p, const float* A, int64_t lda, int k
 // rows of h2 -> softmax / argmax.  geo == nullptr: row m writes proba[m], label32[m].
 // geo != nullptr: row m is voxel (ix,iy,iz) of a box slab; results go to the volume-shaped
 // outputs (label8 / proba) at that voxel, skipped where mask[voxel] == 0.
-// out_layer + softmax fused into the tcgen05 GEMM epilogue (N = 16): where the results of row m go
+// out_layer + softmax fused into the epilogue of the tcgen05 fc_2 GEMM: where the results of row m go
 struct SoftmaxOut { float* proba; int32_t* label32; uint8_t* label8; const uint8_t* mask; OutGeo geo; int use_geo;
                     const int32_t* rowvox; };   // rowvox != nullptr: GEMM row m is the compacted candidate whose slab row is rowvox[m]
 int launch_out_softmax(sc_ctx* ctx, const float* h2, int64_t n, float* proba, int32_t* label32, uint8_t* label8,
@@ -434,6 +432,30 @@ int eval_batch(sc_ctx* ctx, const float* in1, const float* in2, const float* in3
                int64_t n, float* out2, cudaStream_t st);
 
 __device__ __forceinline__ float prelu(float x, float a) { return x > 0.f ? x : a * x; }
+// out_layer logits of one voxel (cnn_cort/nets.py:229-231) -> softmax in fp32; argmax on the float32 probabilities, first
+// maximum wins (np.argmax); the results of voxel o go to whichever outputs are set
+__device__ __forceinline__ void softmax_store(float (&z)[15], long long o, float* proba, int32_t* label32, uint8_t* label8) {
+  float mx = z[0];
+#pragma unroll
+  for (int c = 1; c < 15; ++c) mx = fmaxf(mx, z[c]);
+  float sum = 0.f;
+#pragma unroll
+  for (int c = 0; c < 15; ++c) { z[c] = expf(z[c] - mx); sum += z[c]; }
+  const float inv = 1.f / sum;
+  int best = 0;
+  float bp = z[0] * inv;
+#pragma unroll
+  for (int c = 0; c < 15; ++c) {
+    z[c] *= inv;
+    if (z[c] > bp) { bp = z[c]; best = c; }
+  }
+  if (proba) {
+#pragma unroll
+    for (int c = 0; c < 15; ++c) proba[o * 15 + c] = z[c];
+  }
+  if (label32) label32[o] = best;
+  if (label8) label8[o] = (uint8_t)best;
+}
 // split-precision store of 4 consecutive logical columns n..n+3 (n % 4 == 0) of one activation row
 __device__ __forceinline__ void store_split4(float* row, int n, float v0, float v1, float v2, float v3) {
   __nv_bfloat16* r = reinterpret_cast<__nv_bfloat16*>(row) + (n >> 6) * 128 + (n & 63);

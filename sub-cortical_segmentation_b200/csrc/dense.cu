@@ -371,8 +371,7 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
   const size_t rows_max = (size_t)slab * plane;
   const size_t feat_bytes = align256(rows_max * kFeatLd * sizeof(float));
   const size_t h1_bytes = align256(rows_max * kH1Ld * sizeof(float));
-  const int h2ld = tc ? kH2LdTc : kH2Ld;
-  const size_t h2_bytes = align256(rows_max * h2ld * sizeof(float));
+  const size_t h2_bytes = tc ? 0 : align256(rows_max * kH2Ld * sizeof(float));   // tensor-core mode: fc_2 feeds the out_layer in its epilogue
   // candidate compaction (tensor-core path with a mask): the FC head runs on the candidate rows of each slab only
   const int nslabs = (bx + slab - 1) / slab;
   bool compact = tc && cand != nullptr && ctx->tc_compact && nslabs <= 4096;
@@ -492,8 +491,6 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
   // ---- phase 2: d1 (x3) + FC head per slab of x-planes -------------------------------------
   int atlas_waited = 0;                                // chunked upload: chunks of x-planes this stream has already waited for
   OutGeo og = {b[0], b[2], b[4], by, bz, Y, Z};
-  // tensor-core mode: columns 272..319 of the split h2 rows are never written by fc_2 and must not hold NaN patterns
-  if (tc) SC_CUDA(cudaMemsetAsync(h2, 0, h2_bytes, st));
   for (int ix0 = 0; ix0 < bx; ix0 += slab) {
     const int nx = bx - ix0 < slab ? bx - ix0 : slab;
     const int64_t rows = (int64_t)nx * plane;
@@ -565,18 +562,16 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
     }
     SC_CUDA(cudaGetLastError());
     gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)rows_fc);
-    p.C = h2; p.ldc = h2ld; p.n_store = kH2Ld; p.out_split = tc ? 1 : 0;
     p.prof_cls = PC_GEMM_FC2;
-    SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->fc2, st) : launch_gemm(ctx, p, ctx->fc2, st));
     OutGeo og2 = og;
     og2.x0 = b[0] + ix0;
-    if (tc) {   // out_layer as a 16-column tcgen05 GEMM over the split h2 rows, softmax / argmax in its epilogue
+    if (tc) {   // fc_2 with the out_layer, softmax / argmax and the scatter into the volume in its epilogue
       SoftmaxOut smo = {proba_vol, nullptr, label_vol, cand, og2, 1, compact ? rowvox + slab_base : nullptr};
-      gemm_problem_rows(p, h2, h2ld, h2ld, (int)rows_fc);
-      p.C = nullptr; p.ldc = 0; p.n_store = 16; p.out_split = 0; p.sm = &smo;
-      p.prof_cls = PC_OUT;
-      SC_TRY(launch_gemm_tc(ctx, p, ctx->outl, st));
+      p.C = nullptr; p.ldc = 0; p.n_store = kH2Ld; p.sm = &smo;
+      SC_TRY(launch_gemm_tc(ctx, p, ctx->fc2, st));
     } else {
+      p.C = h2; p.ldc = kH2Ld; p.n_store = kH2Ld;
+      SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
       SC_TRY(launch_out_softmax(ctx, h2, rows, proba_vol, nullptr, label_vol, cand, &og2, st));
     }
   }

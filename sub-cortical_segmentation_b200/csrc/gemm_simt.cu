@@ -109,7 +109,7 @@ int launch_gemm(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream_t 
   return SC_OK;
 }
 
-// out_layer (270 -> 15) + softmax + argmax: one thread per voxel (each thread streams its own 1 088 B row
+// out_layer (270 -> 15) + softmax + argmax of the SIMT back-end (the tcgen05 back-end fuses them into fc_2): one thread per voxel (each thread streams its own 1 088 B row
 // through L1 with float4 loads; the 16 KB weight matrix is read from shared memory as warp-wide broadcasts).
 __global__ void __launch_bounds__(128) out_softmax_kernel(const float* __restrict__ h2, int64_t n,
                                                           const float* __restrict__ W, const float* __restrict__ b,
@@ -151,26 +151,7 @@ __global__ void __launch_bounds__(128) out_softmax_kernel(const float* __restric
       }
     }
   }
-  float mx = z[0];
-#pragma unroll
-  for (int c = 1; c < 15; ++c) mx = fmaxf(mx, z[c]);
-  float sum = 0.f;
-#pragma unroll
-  for (int c = 0; c < 15; ++c) { z[c] = expf(z[c] - mx); sum += z[c]; }
-  const float inv = 1.f / sum;
-  int best = 0;
-  float bp = z[0] * inv;
-#pragma unroll
-  for (int c = 0; c < 15; ++c) {
-    z[c] *= inv;
-    if (z[c] > bp) { bp = z[c]; best = c; }
-  }
-  if (proba) {
-#pragma unroll
-    for (int c = 0; c < 15; ++c) proba[o * 15 + c] = z[c];
-  }
-  if (label) label[o] = best;
-  if (label8) label8[o] = (uint8_t)best;
+  softmax_store(z, o, proba, label, label8);
 }
 
 int launch_out_softmax(sc_ctx* ctx, const float* h2, int64_t n, float* proba, int32_t* label, uint8_t* label8,

@@ -13,9 +13,9 @@
 //
 // Two kernels share this file:
 //   gemm_tc_pair_kernel        CTA pairs (cta_group::2, M = 256): tiles of >= 128 columns -- d1, FC1 (+ atlas prior
-//                              columns), fc_2, the dense layers of the training step: the hot ones
-//   gemm_tc_persistent_kernel  one persistent CTA per SM (M = 128): narrow layers -- the 16-column out_layer GEMM with the
-//                              softmax / argmax epilogue
+//                              columns), fc_2 (+ out_layer, softmax and argmax in its epilogue), the dense layers of the
+//                              training step: the hot ones
+//   gemm_tc_persistent_kernel  one persistent CTA per SM (M = 128): narrow layers
 // Both: warp 0 = TMA producer (per k block A hi, A lo as 4-D boxes of 64 bf16 x 128 pixels with the tap shift applied to
 // the pixel / line / plane coordinates and zero fill outside, W hi, W lo as 2-D boxes), warp 1 = converged MMA issue
 // (12 x tcgen05.mma K=16 per k block), the other warps = epilogue (tcgen05.ld -> scale / bias / PReLU -> plain fp32 or
@@ -67,9 +67,16 @@ struct TcArgs {
   const unsigned char* tile_on;   // pair kernel: tile t is computed only if tile_on[t] != 0 (row map: no candidate row in it)
   const float* atlas; // pair kernel: atlas prior volume [X][Y][Z][15] -> output columns 540..575 (see GemmProblem::atlas)
   OutGeo ageo;
-  int sm_on;          // persistent kernel, bn = 16: softmax / argmax epilogue (out_layer), results scattered through `sm`
-  SoftmaxOut sm;
+  SoftmaxOut sm;      // pair kernel, fc_2 with the out_layer epilogue (FUSED_OUT): where the softmax / argmax results go
+  const float* out_w; // FUSED_OUT: out_layer weights [270][16] and bias [16], fp32
+  const float* out_b;
 };
+
+// fused out_layer (FUSED_OUT): the 16 epilogue warps' store-transpose area is free and holds the out_layer weights (rows padded
+// to 272 with zeros: fc_2's last chunk ends at column 271), the bias, and the logit partials of column groups 1..3
+constexpr int kOutWFloats = kH2Ld * 16;
+constexpr int kOutPartFloats = 3 * 15 * TC_BM;          // [group - 1][class][row of the CTA]
+static_assert((kOutWFloats + 16 + kOutPartFloats) * 4 <= 16 * 2560, "fused out_layer scratch exceeds the store-transpose area");
 
 // ---------------------------------------------------------------------------------------------------
 // Persistent kernel: one CTA per SM walks the tile list (tile = blockIdx.x + i * gridDim.x).
@@ -226,61 +233,6 @@ gemm_tc_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid
       const int mw = m0 + q * 32;                       // first row of this warp
       uint8_t* stg = s_stage + (warp - 2) * 2560;
       uint8_t* mine = stg + lane * 80;
-      if (a.sm_on) {
-        // out_layer (cnn_cort/nets.py:229-231): 15 logits per row -> softmax; argmax on the float32 probabilities,
-        // first maximum wins (np.argmax).  One thread owns one row.
-        if (grp == 0) {
-          uint32_t rr[16];
-          const uint32_t taddr = tmem_base + b * 256 + ((uint32_t)(q * 32) << 16);
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-              : "=r"(rr[0]), "=r"(rr[1]), "=r"(rr[2]), "=r"(rr[3]), "=r"(rr[4]), "=r"(rr[5]), "=r"(rr[6]), "=r"(rr[7]), "=r"(rr[8]),
-                "=r"(rr[9]), "=r"(rr[10]), "=r"(rr[11]), "=r"(rr[12]), "=r"(rr[13]), "=r"(rr[14]), "=r"(rr[15])
-              : "r"(taddr));
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-          long long m = (long long)mw + lane;
-          bool ok = m < a.M;
-          if (ok && a.sm.rowvox) m = __ldg(a.sm.rowvox + m);      // compact row -> row of the dense slab
-          long long o = m;
-          if (ok && a.sm.use_geo) {
-            const long long plane = (long long)a.sm.geo.by * a.sm.geo.bz;
-            const int ix = (int)(m / plane);
-            const int rem = (int)(m - (long long)ix * plane);
-            const int iy = rem / a.sm.geo.bz, iz = rem - iy * a.sm.geo.bz;
-            o = ((long long)(a.sm.geo.x0 + ix) * a.sm.geo.Y + (a.sm.geo.y0 + iy)) * a.sm.geo.Z + (a.sm.geo.z0 + iz);
-            if (a.sm.mask && a.sm.mask[o] == 0) ok = false;
-          }
-          if (ok) {
-            float zz[15];
-#pragma unroll
-            for (int c = 0; c < 15; ++c) zz[c] = __uint_as_float(rr[c]) + cb[c];
-            float mx = zz[0];
-#pragma unroll
-            for (int c = 1; c < 15; ++c) mx = fmaxf(mx, zz[c]);
-            float sum = 0.f;
-#pragma unroll
-            for (int c = 0; c < 15; ++c) { zz[c] = expf(zz[c] - mx); sum += zz[c]; }
-            const float inv = 1.f / sum;
-            int best = 0;
-            float bp = zz[0] * inv;
-#pragma unroll
-            for (int c = 0; c < 15; ++c) {
-              zz[c] *= inv;
-              if (zz[c] > bp) { bp = zz[c]; best = c; }
-            }
-            if (a.sm.proba) {
-#pragma unroll
-              for (int c = 0; c < 15; ++c) a.sm.proba[o * 15 + c] = zz[c];
-            }
-            if (a.sm.label32) a.sm.label32[o] = best;
-            if (a.sm.label8) a.sm.label8[o] = (uint8_t)best;
-          }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[b]);
-        continue;
-      }
       for (int c0 = grp * 16; c0 < a.bn; c0 += 16 * G) {
         uint32_t rr[16];
         const uint32_t taddr = tmem_base + b * 256 + ((uint32_t)(q * 32) << 16) + (uint32_t)c0;
@@ -361,6 +313,7 @@ gemm_tc_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid
 //   * the leader's MMA warp issues tcgen05.mma.cta_group::2 (M = 256) and multicasts its commits to both CTAs
 //   * every CTA's epilogue warps drain their own TMEM half and arrive on the leader's tempty barrier (remote arrive)
 // ---------------------------------------------------------------------------------------------------
+template <bool FUSED_OUT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(576, 1)
 gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -382,7 +335,11 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();                 // position inside the CTA pair; rank 0 leads
   const int nepi = (blockDim.x >> 5) - 2;
-  const long long pair = (long long)(blockIdx.x >> 1), npairs = (long long)(gridDim.x >> 1);   // every pair walks the flat tile list
+  // every pair walks the flat tile list in work units of `per` consecutive tiles: one tile, or with the fused out_layer all n-tiles
+  // of a 256-row block, so that one CTA pair's epilogue sees every fc_2 output of its rows
+  const int pair = (int)(blockIdx.x >> 1), npairs = (int)(gridDim.x >> 1);   // (the host keeps the tile count below 2^31)
+  const int per = FUSED_OUT ? a.nt : 1;
+  const int units = (int)(a.num_tiles / per);
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < a.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
@@ -406,7 +363,9 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
       uint32_t it = 0;
       long long w_empty = 0;
       const long long tstart = a.dbg ? clock64() : 0;
-      for (long long t = pair; t < a.num_tiles; t += npairs) {
+      for (int u = pair; u < units; u += npairs)
+      for (int jt = 0; jt < per; ++jt) {
+        const int t = u * per + jt;
         if (a.tile_on && !a.tile_on[t]) continue;
         long long r = t;
         const int n_tile = (int)(r % a.nt); r /= a.nt;
@@ -446,7 +405,9 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
       uint32_t it = 0, ti = 0;
       long long w_full = 0, w_tempty = 0;
       const long long tstart = a.dbg ? clock64() : 0;
-      for (long long t = pair; t < a.num_tiles; t += npairs) {
+      for (int u = pair; u < units; u += npairs)
+      for (int jt = 0; jt < per; ++jt) {
+        const int t = u * per + jt;
         if (a.tile_on && !a.tile_on[t]) continue;
         const uint32_t b = ti & 1, buse = ti >> 1;
         const int bnj = min(a.bn, a.n_mma - (int)(t % a.nt) * a.bn);
@@ -501,9 +462,19 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
       cbw[a.bn + c] = ok ? __ldg(a.alpha + nn) : 1.f;
       cbw[2 * a.bn + c] = (a.scale && ok) ? __ldg(a.scale + nn) : 1.f;
     }
+    float* s_ow = reinterpret_cast<float*>(s_stage);    // FUSED_OUT: see kOutWFloats
+    float* s_ob = s_ow + kOutWFloats;
+    float* s_part = s_ob + 16;
+    if (FUSED_OUT) {
+      for (int i = threadIdx.x - 64; i < kOutWFloats + 16; i += epi_threads)
+        s_ow[i] = i < 270 * 16 ? __ldg(a.out_w + i) : (i >= kOutWFloats ? __ldg(a.out_b + i - kOutWFloats) : 0.f);
+    }
     asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
+    float logit[15];                                      // FUSED_OUT: this thread's share of its row's out_layer logits
     const long long tstart = a.dbg ? clock64() : 0;
-    for (long long t = pair; t < a.num_tiles; t += npairs) {
+    for (int u = pair; u < units; u += npairs)
+    for (int jt = 0; jt < per; ++jt) {
+      const int t = u * per + jt;
       if (a.tile_on && !a.tile_on[t]) continue;
       long long r = t;
       const int n_tile = (int)(r % a.nt); r /= a.nt;
@@ -521,6 +492,76 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
       const int mw = m0 + q * 32;
       uint8_t* stg = s_stage + (warp - 2) * 2560;
       uint8_t* mine = stg + lane * 80;
+      if (FUSED_OUT) {
+        // One 16-column chunk at a time: bias / PReLU, then the out_layer as fp32 FMAs into this thread's logit partials (the
+        // weight rows are broadcast reads).  Nothing is stored.  The accumulator goes back to the MMA warp after the last chunk;
+        // this epilogue is short next to the MMAs of the next tile, which run in the other accumulator meanwhile.
+        if (jt == 0) {
+#pragma unroll
+          for (int c = 0; c < 15; ++c) logit[c] = 0.f;
+        }
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          const int c0 = grp * 16 + i * 16 * G;
+          if (c0 >= a.bn || n0 + c0 >= a.n_store) continue;     // warp-uniform
+          uint32_t r[16];
+          tmem_ld16(r, tmem_base + b * 256 + ((uint32_t)(q * 32) << 16) + (uint32_t)c0);
+          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          const float4* w4 = reinterpret_cast<const float4*>(s_ow + (n0 + c0) * 16);
+#pragma unroll
+          for (int k = 0; k < 16; ++k) {
+            const float x = prelu(fmaf(__uint_as_float(r[k]), cb[2 * a.bn + c0 + k], cb[c0 + k]), cb[a.bn + c0 + k]);
+            const float4 w0 = w4[4 * k], w1 = w4[4 * k + 1], w2 = w4[4 * k + 2], w3 = w4[4 * k + 3];
+            logit[0] = fmaf(x, w0.x, logit[0]); logit[1] = fmaf(x, w0.y, logit[1]);
+            logit[2] = fmaf(x, w0.z, logit[2]); logit[3] = fmaf(x, w0.w, logit[3]);
+            logit[4] = fmaf(x, w1.x, logit[4]); logit[5] = fmaf(x, w1.y, logit[5]);
+            logit[6] = fmaf(x, w1.z, logit[6]); logit[7] = fmaf(x, w1.w, logit[7]);
+            logit[8] = fmaf(x, w2.x, logit[8]); logit[9] = fmaf(x, w2.y, logit[9]);
+            logit[10] = fmaf(x, w2.z, logit[10]); logit[11] = fmaf(x, w2.w, logit[11]);
+            logit[12] = fmaf(x, w3.x, logit[12]); logit[13] = fmaf(x, w3.y, logit[13]);
+            logit[14] = fmaf(x, w3.z, logit[14]);
+          }
+        }
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cta(&tempty[b], 0);
+        ++ti;
+        if (jt == per - 1) {
+          // the block's last n-tile: column groups 1..3 hand their logit partials to group 0 through shared memory; the second
+          // barrier keeps the next block's partials from overwriting these before group 0 has read them
+          const int crow = q * 32 + lane;
+          if (grp > 0) {
+#pragma unroll
+            for (int c = 0; c < 15; ++c) s_part[((grp - 1) * 15 + c) * TC_BM + crow] = logit[c];
+          }
+          asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
+          if (grp == 0) {
+#pragma unroll
+            for (int g = 0; g < 3; ++g)
+#pragma unroll
+              for (int c = 0; c < 15; ++c) logit[c] += s_part[(g * 15 + c) * TC_BM + crow];
+          }
+          asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
+          long long m = (long long)mw + lane;
+          bool ok = grp == 0 && m < a.M;
+          if (ok && a.sm.rowvox) m = __ldg(a.sm.rowvox + m);      // compact row -> row of the dense slab
+          long long o = m;
+          if (ok && a.sm.use_geo) {
+            const long long plane = (long long)a.sm.geo.by * a.sm.geo.bz;
+            const int ix = (int)(m / plane);
+            const int rem = (int)(m - (long long)ix * plane);
+            const int iy = rem / a.sm.geo.bz, iz = rem - iy * a.sm.geo.bz;
+            o = ((long long)(a.sm.geo.x0 + ix) * a.sm.geo.Y + (a.sm.geo.y0 + iy)) * a.sm.geo.Z + (a.sm.geo.z0 + iz);
+            if (a.sm.mask && a.sm.mask[o] == 0) ok = false;
+          }
+          if (ok) {
+#pragma unroll
+            for (int c = 0; c < 15; ++c) logit[c] += s_ob[c];
+            softmax_store(logit, o, a.sm.proba, a.sm.label32, a.sm.label8);
+          }
+        }
+        continue;
+      }
       // The warp's (up to three) 16-column chunks of the accumulator go to registers first; the accumulator is handed back
       // to the MMA warp right after that, so the arithmetic and the stores of this tile overlap the MMAs of the tile after next.
       uint32_t rr[3][16];
@@ -723,12 +764,13 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
   a.c_col0 = p.c_col0;
   a.nkb = p.ntaps * a.kpt;
   a.bn = pick_bn(p.n_store);
-  a.sm_on = 0;
+  a.out_w = ctx->out_w; a.out_b = ctx->out_b;
   a.atlas = p.atlas; a.ageo = p.ageo;
   a.rowmap = p.rowmap; a.rowvox = p.rowvox; a.crow_ld = 0; a.tile_on = nullptr;
-  if (p.sm) {
-    SC_CHECK(p.n_store == 16 && p.ntaps == 1, SC_ERR_ARG, "gemm_tc: the softmax epilogue needs a 16-column layer");
-    a.bn = 16; a.sm_on = 1; a.sm = *p.sm;
+  if (p.sm) {   // fc_2 with the out_layer, softmax and argmax in its epilogue
+    SC_CHECK(p.n_store == kH2Ld && p.ntaps == 1 && p.c_col0 == 0 && !p.out_split && !p.rowmap && !p.atlas && w.Npad == kH2Ld,
+             SC_ERR_ARG, "gemm_tc: the out_layer epilogue is for fc_2");
+    a.sm = *p.sm;
   }
   a.nt = (p.n_store + a.bn - 1) / a.bn;
   a.mt = (p.M + TC_BM - 1) / TC_BM;
@@ -745,8 +787,9 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
   }
   a.bias = w.bias; a.alpha = w.alpha; a.scale = w.scale; a.out_split = p.out_split;
   // CTA pairs (cta_group::2) for the wide streaming-weight tiles, the persistent single-CTA kernel for the narrow ones
-  const bool pair = a.bn >= 128 && a.bn % 16 == 0 && !p.sm;
+  const bool pair = a.bn >= 128 && a.bn % 16 == 0;
   SC_CHECK(!p.rowmap || pair, SC_ERR_ARG, "gemm_tc: the row map is implemented in the CTA-pair kernel");
+  SC_CHECK(!p.sm || pair, SC_ERR_ARG, "gemm_tc: the out_layer epilogue is implemented in the CTA-pair kernel");
   SC_CHECK(!p.atlas || (pair && p.c_col0 == 0 && p.n_store == 540 && w.Npad == 576), SC_ERR_ARG, "gemm_tc: the atlas epilogue is for FC1 in the CTA-pair kernel");
   const long long blocks = (long long)a.mt * a.nt * p.Y * p.Z;
   SC_CHECK(blocks < (1ll << 31), SC_ERR_ARG, "gemm_tc: grid too large");
@@ -802,7 +845,8 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
     SC_CHECK(r == CUDA_SUCCESS, SC_ERR_CUDA, "gemm_tc: cuTensorMapEncodeTiled(B) failed with %d", (int)r);
   }
   SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_persistent_kernel), 227 * 1024));
-  SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel), 227 * 1024));
+  SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel<false>), 227 * 1024));
+  SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel<true>), 227 * 1024));
   SC_CHECK(smem <= 227 * 1024, SC_ERR_ARG, "gemm_tc: shared memory budget exceeded (%zu)", smem);
   ProfScope prof(ctx, p.prof_cls, st);
   a.n_mma = a.nt * a.bn;
@@ -825,8 +869,10 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
     a.tile_on = ctx->tile_flags;
   }
   if (pair) {
-    long long pairs = a.num_tiles < ctx->sm_count / 2 ? a.num_tiles : ctx->sm_count / 2;
-    gemm_tc_pair_kernel<<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);   // __cluster_dims__(2,1,1)
+    const long long units = p.sm ? a.num_tiles / a.nt : a.num_tiles;   // work units of the pair kernel (see its tile walk)
+    const long long pairs = units < ctx->sm_count / 2 ? units : ctx->sm_count / 2;
+    if (p.sm) gemm_tc_pair_kernel<true><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);   // __cluster_dims__(2,1,1)
+    else gemm_tc_pair_kernel<false><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);
   } else {
     const unsigned grid = (unsigned)(blocks < ctx->sm_count ? blocks : ctx->sm_count);
     gemm_tc_persistent_kernel<<<grid, 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);

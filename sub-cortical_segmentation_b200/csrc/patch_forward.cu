@@ -5,7 +5,8 @@
 // memory (conv -> BN affine -> PReLU, 2x2 max-pools after conv2 and conv4, in that order:
 // trained PReLU slopes are negative or > 1, so pooling cannot move before the activation)
 // and emits the flattened 60x3x3 map (k = c*9 + h*3 + w).  d1 / FC1 / fc_2 then run as
-// GEMMs over the whole batch (gemm_simt.cu or gemm_tc.cu), out_layer+softmax last.
+// GEMMs over the whole batch (gemm_simt.cu or gemm_tc.cu), out_layer+softmax last (on the tensor cores: in
+// fc_2's epilogue).
 #include "common.cuh"
 
 namespace sc {
@@ -244,7 +245,7 @@ int forward_patches(sc_ctx* ctx, const float* in1, const float* in2, const float
                     float* proba, int32_t* label, cudaStream_t st) {
   const bool tc = ctx->gemm_backend == 1;
   const int64_t chunk = 32768, sub = 4096;      // head rows per pass / patches per tensor-core conv pass
-  const size_t row_floats = 3 * kFeatLd + kFeatLd + kH1Ld + kH2Ld;
+  const size_t row_floats = 3 * kFeatLd + kFeatLd + kH1Ld + (tc ? 0 : kH2Ld);   // tensor-core mode: no h2 rows (fused into fc_2)
   const int64_t cmax = n < chunk ? n : chunk;
   const size_t head_bytes = (size_t)cmax * row_floats * sizeof(float) + 1024;
   const size_t conv_bytes = tc ? branch_patches_tc_bytes(cmax < sub ? cmax : sub) : 0;
@@ -283,9 +284,15 @@ int forward_patches(sc_ctx* ctx, const float* in1, const float* in2, const float
     ctx->launches++;
     SC_CUDA(cudaGetLastError());
     gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)m);
-    p.C = h2; p.ldc = kH2Ld; p.n_store = kH2Ld; p.out_split = 0;
-    p.prof_cls = PC_GEMM_FC2;
-    SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->fc2, st) : launch_gemm(ctx, p, ctx->fc2, st));
+    p.n_store = kH2Ld; p.prof_cls = PC_GEMM_FC2;
+    if (tc) {   // fc_2 with the out_layer and softmax / argmax in its epilogue
+      SoftmaxOut smo = {proba ? proba + s * 15 : nullptr, label ? label + s : nullptr, nullptr, nullptr, OutGeo{}, 0, nullptr};
+      p.C = nullptr; p.ldc = 0; p.sm = &smo;
+      SC_TRY(launch_gemm_tc(ctx, p, ctx->fc2, st));
+      continue;
+    }
+    p.C = h2; p.ldc = kH2Ld;
+    SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
     SC_TRY(launch_out_softmax(ctx, h2, m, proba ? proba + s * 15 : nullptr, label ? label + s : nullptr, nullptr,
                               nullptr, nullptr, st));
   }

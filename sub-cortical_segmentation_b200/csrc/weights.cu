@@ -69,7 +69,7 @@ int derive_weights(sc_ctx* ctx, cudaStream_t st) {
 
   Arena A;
   struct BOff { size_t c1, conv[5], scale[5], shift[5], alpha[5], sw[5], swp[5]; GemmOff d1, d1d; } bo[3];
-  GemmOff fc1o, fc2o, outo;
+  GemmOff fc1o, fc2o;
   size_t outw, outb;
   for (int b = 0; b < 3; ++b) {
     const BranchOff& B = P.br[b];
@@ -151,10 +151,6 @@ int derive_weights(sc_ctx* ctx, cudaStream_t st) {
     A.host[fc2o.bias + n] = n < 270 ? h[P.fc2b + n] : 0.f;
     A.host[fc2o.alpha + n] = n < 270 ? h[P.a2 + n] : 1.f;
   }
-  outo = make_gemm(A, ctx->outl, 270, 15, kH2LdTc, 16);
-  for (int k = 0; k < 270; ++k)
-    for (int n = 0; n < 15; ++n) set_w(A, outo, ctx->outl, k, n, h[P.outW + k * 15 + n]);
-  for (int n = 0; n < 15; ++n) A.host[outo.bias + n] = h[P.outb + n];
   outw = A.alloc(270 * 16);
   outb = A.alloc(16);
   for (int k = 0; k < 270; ++k)
@@ -187,7 +183,6 @@ int derive_weights(sc_ctx* ctx, cudaStream_t st) {
   }
   bind(ctx->fc1, fc1o, base);
   bind(ctx->fc2, fc2o, base);
-  bind(ctx->outl, outo, base);
   ctx->out_w = base + outw;
   ctx->out_b = base + outb;
   return SC_OK;
