@@ -106,14 +106,25 @@ struct GemmW {      // one dense layer prepared for both GEMM back-ends
 };
 
 struct SweepW {     // one conv layer prepared for the strip-sweep tcgen05 kernel (conv_sweep.cu)
-  float* panels;    // [npanels][2*bn][64] bf16: rows 0..bn-1 = W hi, bn..2bn-1 = W lo; column block (gk & 3) of panel gk >> 2
-                    // holds k-step gk = tap * ksteps + ci / 16 (flipped taps, zero padded)
-  float* panels_pair;  // the same for the CTA-pair kernel: per panel the rows of rank 0 then rank 1, each W hi[bn/2] | W lo[bn/2]
+  float* panels;    // [npanels][6*bn][64] bf16: rows 0..3bn-1 = W hi stacked over the filter rows [W_ky2 | W_ky1 | W_ky0]
+                    // (bn rows each), 3bn..6bn-1 = W lo stacked alike; column block (gk & 3) of panel gk >> 2 holds
+                    // k-step gk = kx * ksteps + ci / 16 (flipped taps, zero padded)
+  float* panels_pair;  // the same for the CTA-pair kernel: per panel the rows of rank 0 then rank 1, each W hi | W lo of its
+                       // 1.5 bn stacked rows (rank 0: [W_ky2 | W_ky1[0, bn/2)], rank 1: [W_ky1[bn/2, bn) | W_ky0])
   float* scale;     // BN folded scale / shift and PReLU slope, padded to 64 with zeros
   float* shift;
   float* alpha;
-  int bn, ksteps, npanels;
+  int bn, ksteps, npanels;   // npanels = ceil(3 * ksteps / 4)
 };
+
+// bf16 element offsets of the hi part of weight (output channel o, filter row ky, column kx, input channel k) in the
+// plain and pair panels of SweepW; the lo parts lie 3 bn (plain) and 1.5 bn (pair) rows further
+__host__ __device__ inline void sweep_panel_pos(int o, int ky, int kx, int k, int ksteps, int bn, size_t& plain, size_t& pair) {
+  const int gk = kx * ksteps + (k >> 4), kk = (gk & 3) * 16 + (k & 15), panel = gk >> 2;
+  const int sr = (2 - ky) * bn + o, hb = 3 * bn / 2;   // stacked row; stacked rows per CTA of a pair
+  plain = ((size_t)panel * 6 * bn + sr) * 64 + kk;
+  pair = ((size_t)(panel * 2 + sr / hb) * 3 * bn + sr % hb) * 64 + kk;
+}
 
 struct Conv1Consts { float w[9 * 20]; float scale[20], shift[20], alpha[20]; };   // conv1 taps + folded BN + PReLU, passed by value
 

@@ -3,19 +3,31 @@
 //
 // Map layout ("wide rows"): all slices of a view lie side by side, position (row r, slice s, col c) is pixel
 // r * Pw + s * C1 + c with Pw = ns * C1.  A CTA owns a strip of 128 adjacent wide columns and sweeps down the rows:
-// every input row of the strip is TMA-loaded ONCE into a shared-memory ring and serves the three filter rows of
-// three consecutive output rows (the flattened one-tile-per-launch kernel loaded every row three times).  With
-// dilation d the rows r, r+d, r+2d interact, so a sweep runs over one residue class of rows (r = q + d*n).
+// every input row of the strip is TMA-loaded ONCE into a shared-memory ring.  With dilation d the rows r, r+d, r+2d
+// interact, so a sweep runs over one residue class of rows (r = q + d*n).
 //
 //   warp 0    TMA producer: one (128 + 2d)-pixel box per input row (two for the 256 B/pixel layout)
-//   warp 1    MMA issue, converged, compile-time unrolled: per output row 9 taps x KSTEPS x
-//             { xh * [wh | wl] (N = 2*bn),  xl * wh (N = bn) }  -- the bf16x3 split product as two MMAs;
+//   warp 1    MMA issue, converged, compile-time unrolled: ONE pass per input row.  Class row n feeds output rows
+//             n-2, n-1, n through filter rows 2, 1, 0, so the weights stack the three filter rows along N
+//             ([W_ky2 | W_ky1 | W_ky0], N = 3*bn) and per (kx, k-step) the bf16x3 split product is three MMAs
+//             xh*Wh, xh*Wl, xl*Wh into one D that spans the accumulators of output rows n-2 .. n;
 //             column taps are descriptor start offsets inside the row box, weights stay resident (k-step-packed panels)
 //   warps 2-17 epilogue (4 lane quarters x 4 column groups): TMEM -> BN scale/shift -> PReLU -> [fused 2x2 stride-1
 //             max-pool: horizontal neighbour by shuffle / a small exchange buffer, vertical neighbour = the previous
 //             row kept in registers] -> split bf16 hi|lo -> SWIZZLE_128B output tile in shared memory -> one TMA
 //             tensor store per row box (no per-thread global addressing; partial boxes are clipped by the TMA unit)
-// Two TMEM accumulators: the epilogue of row i overlaps the MMAs of row i+1.
+//
+// Accumulator ring: S slots of bn TMEM columns plus two spill slots, (S + 2) * bn <= 512.  A per-CTA input-row counter g
+// (not reset between items; it starts at 2) numbers the slots: input row g writes slots g-2, g-1, g, i.e. the physical
+// columns [p, p + 3) * bn with p = (g - 2) mod S, which never wrap: logical slot l < 2 is physical l + physical S + l.
+// An MMA writes its whole D, so no slot can start from zero inside a stacked MMA: every MMA accumulates, and the epilogue
+// clears a slot (both parts) after reading it; all slots are cleared once at the start.  Slot g is committed full after
+// input row g + 2, always.  An item of nrow output rows reads nrow + 2 input rows: its output rows are its first nrow
+// slots, the two before them (the previous item's two halo slots, or two leading slots) hold partial sums that the epilogue
+// clears and discards.  Output class row n always lands in slot (n + 2) mod S, so its summation order (one part or two)
+// does not depend on how the rows are cut into items or which items are skipped: an item whose first row does not follow
+// on from the previous one's slots jumps g ahead by d < S; the previous item's halo slots it does not share are committed
+// at once and it claims its own leading slots.  The slot barriers keep their phase parities per slot (bit masks).
 //
 // Pixel formats: F32CH: 128 B = 32 bf16 hi | 32 bf16 lo (20-channel maps); F64CH: 256 B = 64 hi | 64 lo.
 #include "tc_common.cuh"
@@ -23,10 +35,13 @@
 namespace sc {
 
 constexpr int SW_SLOT_HALF = 17408;   // bytes reserved per TMA box: (128 + 2*4) pixels x 128 B, 1024-aligned
+constexpr int SW_MAX_SLOTS = 14;      // accumulator slots (bn = 32); barriers of the largest ring fit SW_BAR_BYTES
+constexpr int SW_BAR_BYTES = 512;     // mbarriers + TMEM address slot
 
 struct SweepArgs {
   int Pw, R;              // wide-row pitch (pixels) and number of rows of the map geometry
-  int bn;                 // accumulator columns per half (output channels rounded up to 16)
+  int bn;                 // accumulator columns per output row (output channels rounded up to 16)
+  int S;                  // accumulator slots of the ring: (S + 2) * bn <= 512 TMEM columns
   int nstrips, strip_w;   // strips start every strip_w wide columns (128, or 128 - pool reach)
   int nseg, L;            // row segments per (strip, class); class rows per segment (output rows of an item)
   int n_items;
@@ -97,6 +112,63 @@ template <int CW>
 __device__ __forceinline__ void tmem_ld(uint32_t taddr, uint32_t (&r)[CW]) {
   if constexpr (CW == 16) tmem_ld16(taddr, r); else tmem_ld8(taddr, r);
 }
+template <int CW>
+__device__ __forceinline__ void tmem_zero(uint32_t taddr) {
+  if constexpr (CW == 16)
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1};"
+                 ::"r"(taddr), "r"(0u) : "memory");
+  else
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %1, %1, %1, %1, %1, %1, %1};" ::"r"(taddr), "r"(0u) : "memory");
+}
+// every accumulator column of this warp's lanes and column group starts at zero (the MMAs only ever accumulate)
+template <int CW>
+__device__ __forceinline__ void sweep_acc_clear(uint32_t tcol, int S, int bn) {
+  for (int j = 0; j < S + 2; ++j) tmem_zero<CW>(tcol + (uint32_t)(j * bn));
+  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+}
+// Epilogue side of the accumulator ring: wait for slot dj (phase parities: bit mask dph), read it into acc if `keep` (summing the
+// spill part of slots 0 and 1), clear it, hand it back to the MMA warp (aempty, of the leader CTA for PAIR), advance to the next slot.
+// tcol = TMEM address of this warp's lane quarter and first column; `real` = the warp's columns are computed ones.
+template <int CW, bool PAIR>
+__device__ __forceinline__ void sweep_drain(uint64_t* afull, uint64_t* aempty, uint32_t& dj, uint32_t& dph, int S, int bn,
+                                            uint32_t tcol, bool real, bool keep, int lane, float (&acc)[CW], bool timed,
+                                            uint32_t& w_wait) {
+  const long long c0 = timed ? clock64() : 0;
+  mbar_wait(&afull[dj], (dph >> dj) & 1u);
+  dph ^= 1u << dj;
+  if (timed) w_wait += (uint32_t)(clock64() - c0);
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  if (real) {
+    const uint32_t taddr = tcol + dj * (uint32_t)bn, tspill = taddr + (uint32_t)(S * bn);
+    const bool split = dj < 2;               // warp-uniform
+    if (keep) {
+#pragma unroll
+      for (int h = 0; h < CW; h += 8) {      // 8 columns at a time: the spill part costs no extra registers
+        uint32_t r1[8], r2[8];
+        tmem_ld8(taddr + h, r1);
+        if (split) tmem_ld8(tspill + h, r2);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+        for (int k = 0; k < 8; ++k) acc[h + k] = split ? __uint_as_float(r1[k]) + __uint_as_float(r2[k]) : __uint_as_float(r1[k]);
+      }
+    }
+    tmem_zero<CW>(taddr);
+    if (split) tmem_zero<CW>(tspill);
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncwarp();
+  if (lane == 0) {
+    if (PAIR) mbar_arrive_cta(&aempty[dj], 0); else mbar_arrive(&aempty[dj]);
+  }
+  if (++dj == (uint32_t)S) dj = 0;
+}
+// MMA side: wait until slot j's previous use has been drained (phase parities: bit mask eph)
+__device__ __forceinline__ void sweep_claim(uint64_t* aempty, uint32_t j, uint32_t& eph) {
+  mbar_wait(&aempty[j], ((eph >> j) & 1u) ^ 1u);
+  eph ^= 1u << j;
+}
+__device__ __forceinline__ uint32_t slot_back(uint32_t j, uint32_t k, int S) { return j >= k ? j - k : j + (uint32_t)S - k; }   // k <= 2
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* src, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
                ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2) : "memory");
@@ -116,7 +188,8 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
   constexpr int NBOX = LO64 ? 1 : 2;
   constexpr int SLOT = NBOX * SW_SLOT_HALF;
   constexpr int LO_OFF = LO64 ? 64 : SW_SLOT_HALF;
-  const int panel_bytes = 2 * a.bn * 128;
+  const int half_bytes = 3 * a.bn * 128;                               // W hi (or lo) rows of one panel, stacked filter rows
+  const int panel_bytes = 2 * half_bytes;
   const int w_bytes = a.npanels * panel_bytes;
   uint8_t* sW = smem;
   uint8_t* sRing = smem + w_bytes;
@@ -125,9 +198,9 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
   uint64_t* bars = reinterpret_cast<uint64_t*>(sOut + a.out_bufs * OB_BYTES);
   uint64_t* full = bars;
   uint64_t* empty = bars + a.stages;
-  uint64_t* tfull = bars + 2 * a.stages;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* wfull = tempty + 2;
+  uint64_t* afull = bars + 2 * a.stages;   // [S] accumulator slot complete (MMA commit)
+  uint64_t* aempty = afull + a.S;          // [S] accumulator slot read and cleared (16 epilogue warps)
+  uint64_t* wfull = aempty + a.S;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wfull + 1);
   float* s_const = reinterpret_cast<float*>(tmem_slot + 2);            // [scale 64 | shift 64 | alpha 64]
   float* s_xch = s_const + 192;                                        // [2 row parities][4 groups][4 quarters][2][16]
@@ -136,7 +209,7 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < a.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 16); }
+    for (int j = 0; j < a.S; ++j) { mbar_init(&afull[j], 1); mbar_init(&aempty[j], 16); }
     mbar_init(wfull, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -157,6 +230,14 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
+  // epilogue geometry: TMEM lane quarter, column group and the first accumulator column of this warp
+  const int q4 = warp & 3, ew = warp - 2, grp = ew >> 2, c0 = grp * CW;
+  const bool real = c0 < a.bn;             // groups beyond the computed columns only take part in the barriers
+  const uint32_t tcol = tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)c0;
+  if (warp >= 2 && real) sweep_acc_clear<CW>(tcol, a.S, a.bn);
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
   // item -> (strip, class q, segment); identical in every role
   auto decode = [&](int item, int& w0, int& q, int& n0, int& Lc) {
@@ -176,7 +257,7 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapW)) : "memory");
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapO)) : "memory");
       mbar_expect_tx(wfull, (uint32_t)w_bytes);
-      for (int p = 0; p < a.npanels; ++p) tma_load_2d(&mapW, wfull, sW + p * panel_bytes, 0, p * 2 * a.bn);
+      for (int p = 0; p < 2 * a.npanels; ++p) tma_load_2d(&mapW, wfull, sW + p * half_bytes, 0, p * 3 * a.bn);
       uint32_t g = 0;
       long long w_empty = 0;
       const long long tstart = a.dbg ? clock64() : 0;
@@ -204,83 +285,72 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
     __syncwarp();
   } else if (warp == 1) {
     const uint32_t leader = elect_one();
-    const uint32_t idesc1 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(a.bn >> 2) << 17) | ((uint32_t)(128 >> 4) << 24);  // N = 2*bn
-    const uint32_t idesc2 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(a.bn >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);  // N = bn
+    // D = F32, A = B = BF16, K-major, N = 3 * bn (stacked filter rows), M = 128
+    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(3 * a.bn >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
     mbar_wait(wfull, 0);
     const uint32_t w_lo = desc_lo(smem_u32(sW));
     const uint32_t ring_lo = desc_lo(smem_u32(sRing));
-    const uint32_t panel16 = (uint32_t)(panel_bytes >> 4);
-    uint32_t gs = 0, gph = 0, t = 0;           // ring slot / phase parity of the item's current first row
+    const uint32_t panel16 = (uint32_t)(panel_bytes >> 4), wl_off = (uint32_t)(half_bytes >> 4);
+    uint32_t rs = 0, rph = 0;                  // ring stage / phase parity of the next input row
+    uint32_t j = 2, eph = 0;                   // its accumulator slot g mod S (g starts at 2), slot phase parities
+    bool open = false;                         // the last computed item's halo slots await their commit
     long long w_full = 0, w_tempty = 0;
     const long long tstart = a.dbg ? clock64() : 0;
     for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
       int w0, q, n0, Lc;
       decode(item, w0, q, n0, Lc);
       if (Lc <= 0 || (a.item_on && !a.item_on[item])) continue;
-      const int nrow = Lc + (POOL == 1 ? 1 : 0);
-      for (int m = 0; m < nrow; ++m, ++t) {
-        const uint32_t b = t & 1;
+      const int nin = Lc + (POOL == 1 ? 1 : 0) + 2;
+      const uint32_t j0 = (uint32_t)(n0 + 2) % (uint32_t)a.S;     // slot of the item's first output row
+      const uint32_t d = open ? (j0 + (uint32_t)a.S - j) % (uint32_t)a.S : 2u;
+      if (d) {                                 // not following on: flush the unshared old halo slots, claim the new leading ones
+        if (open && leader) { umma_commit(&afull[slot_back(j, 2, a.S)]); if (d >= 2) umma_commit(&afull[slot_back(j, 1, a.S)]); }
+        if (d >= 2) sweep_claim(aempty, slot_back(j0, 2, a.S), eph);
+        sweep_claim(aempty, slot_back(j0, 1, a.S), eph);
+      }
+      j = j0; open = true;
+      for (int m = 0; m < nin; ++m) {
         long long c0 = a.dbg ? clock64() : 0;
-        mbar_wait(&tempty[b], ((t >> 1) & 1) ^ 1);
+        sweep_claim(aempty, j, eph);             // slot g: its previous use has been read and cleared
         if (a.dbg) { const long long c1 = clock64(); w_tempty += c1 - c0; c0 = c1; }
-        // ring slots / phase parities of the three input rows, advanced incrementally (no divisions on this path)
-        uint32_t sl[3], ss[3], sp[3];
-        ss[0] = gs; sp[0] = gph;
-#pragma unroll
-        for (int ky = 1; ky < 3; ++ky) {
-          const bool wrap = ss[ky - 1] + 1 == (uint32_t)a.stages;
-          ss[ky] = wrap ? 0u : ss[ky - 1] + 1;
-          sp[ky] = sp[ky - 1] ^ (wrap ? 1u : 0u);
-        }
-#pragma unroll
-        for (int ky = 0; ky < 3; ++ky) {
-          if (m == 0 || ky == 2) mbar_wait(&full[ss[ky]], sp[ky]);
-          sl[ky] = ring_lo + ss[ky] * (SLOT >> 4);
-        }
+        mbar_wait(&full[rs], rph);
         if (a.dbg) w_full += clock64() - c0;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t acc = tmem_base + b * 256;
+        const uint32_t p = slot_back(j, 2, a.S);                    // slots g-2 .. g = physical slots p .. p+2
+        const uint32_t acc = tmem_base + p * (uint32_t)a.bn;
+        const uint32_t sl = ring_lo + rs * (SLOT >> 4);
 #pragma unroll
-        for (int ky = 0; ky < 3; ++ky) {
+        for (int kx = 0; kx < 3; ++kx) {
 #pragma unroll
-          for (int kx = 0; kx < 3; ++kx) {
-#pragma unroll
-            for (int ks = 0; ks < KSTEPS; ++ks) {
-              const int gk = (ky * 3 + kx) * KSTEPS + ks;                    // compile-time after unrolling
-              const uint32_t a_hi = sl[ky] + (uint32_t)(kx * DIL * 8 + ks * 2);
-              const uint32_t a_lo = a_hi + (uint32_t)(LO_OFF >> 4);
-              const uint32_t bd = w_lo + (uint32_t)(gk >> 2) * panel16 + (uint32_t)((gk & 3) * 2);
-              sweep_mma(acc, a_hi, bd, idesc1, gk != 0, leader);
-              sweep_mma(acc, a_lo, bd, idesc2, 1, leader);
-            }
+          for (int ks = 0; ks < KSTEPS; ++ks) {
+            const int gk = kx * KSTEPS + ks;                            // compile-time after unrolling
+            const uint32_t a_hi = sl + (uint32_t)(kx * DIL * 8 + ks * 2);
+            const uint32_t a_lo = a_hi + (uint32_t)(LO_OFF >> 4);
+            const uint32_t wh = w_lo + (uint32_t)(gk >> 2) * panel16 + (uint32_t)((gk & 3) * 2);
+            sweep_mma(acc, a_lo, wh, idesc, 1, leader);
+            sweep_mma(acc, a_hi, wh + wl_off, idesc, 1, leader);
+            sweep_mma(acc, a_hi, wh, idesc, 1, leader);
           }
         }
         if (leader) {
-          umma_commit(&empty[ss[0]]);
-          if (m == nrow - 1) {
-            umma_commit(&empty[ss[1]]);
-            umma_commit(&empty[ss[2]]);
-          }
-          umma_commit(&tfull[b]);
+          umma_commit(&empty[rs]);
+          umma_commit(&afull[p]);                // slot g-2 has all three filter rows
         }
         __syncwarp();
-        gs = ss[1]; gph = sp[1];
-        if (m == nrow - 1) {                      // the two halo rows of the item are consumed as well
-          const bool wrap = ss[2] + 1 == (uint32_t)a.stages;
-          gs = wrap ? 0u : ss[2] + 1; gph = sp[2] ^ (wrap ? 1u : 0u);
-        }
+        if (++rs == (uint32_t)a.stages) { rs = 0; rph ^= 1; }
+        if (++j == (uint32_t)a.S) j = 0;
       }
     }
+    if (open && leader) {                        // the CTA's last two slots (halo rows) get no later input row
+      umma_commit(&afull[slot_back(j, 2, a.S)]);
+      umma_commit(&afull[slot_back(j, 1, a.S)]);
+    }
+    __syncwarp();
     if (a.dbg && leader) {
       a.dbg[blockIdx.x * 8 + 2] = (unsigned long long)w_full; a.dbg[blockIdx.x * 8 + 3] = (unsigned long long)w_tempty;
       a.dbg[blockIdx.x * 8 + 4] = (unsigned long long)(clock64() - tstart);
     }
   } else {
-    const int q4 = warp & 3;                 // TMEM lane quarter this warp may read
-    const int ew = warp - 2;                 // 0..15
-    const int grp = ew >> 2;                 // column group
-    const int c0 = grp * CW;                 // first accumulator column of this warp
-    const bool real = c0 < a.bn;             // groups beyond the computed columns only take part in the barriers
     const int px = q4 * 32 + lane;           // pixel inside the strip = row of the output tile
     const bool issuer = threadIdx.x == 64;
     // byte offsets of this thread's hi / lo pieces inside a tile (SWIZZLE_128B: 16 B chunk index ^= row & 7)
@@ -291,47 +361,48 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
     const uint32_t hi_chunk = (uint32_t)(c0 >> 3);
     const uint32_t lo_base = OUT32 ? 0u : 16384u, lo_chunk = OUT32 ? 4u + hi_chunk : hi_chunk;
     uint32_t t = 0, e = 0;                   // conv rows consumed, rows emitted
-    long long w_tfull = 0;
+    uint32_t dj = 0, dph = 0;                // accumulator slot to drain next, slot phase parities
+    uint32_t w_tfull = 0;
+    const bool timed = a.dbg != nullptr;
     const long long tstart = a.dbg ? clock64() : 0;
     constexpr bool STATS = POOL == 0 && DIL == 1;   // the instantiations the training forward uses
     float st_s[STATS ? CW : 1], st_q[STATS ? CW : 1];
 #pragma unroll
     for (int k = 0; k < (STATS ? CW : 1); ++k) st_s[k] = st_q[k] = 0.f;
+    float v[CW];
     for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
       int w0, q, n0, Lc;
       decode(item, w0, q, n0, Lc);
       if (Lc <= 0 || (a.item_on && !a.item_on[item])) continue;
       const int nrow = Lc + (POOL == 1 ? 1 : 0);
+      // halo slots of the previous item (dj = its first one) up to the new item's two leading ones, as the MMA warp jumps
+      const uint32_t j0 = (uint32_t)(n0 + 2) % (uint32_t)a.S;
+      const uint32_t d = (j0 + 2u * (uint32_t)a.S - 2u - dj) % (uint32_t)a.S;
+      if (t == 0 || d >= 3) {
+        if (t > 0)
+          for (int h = 0; h < 2; ++h) sweep_drain<CW, false>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
+        dj = slot_back(j0, 2, a.S);
+      } else {
+        for (uint32_t h = 0; h < d; ++h) sweep_drain<CW, false>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
+      }
+      for (int h = 0; h < 2; ++h) sweep_drain<CW, false>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
       float hprev[CW];
 #pragma unroll
       for (int k = 0; k < CW; ++k) hprev[k] = 0.f;
       for (int m = 0; m < nrow; ++m, ++t) {
-        const uint32_t b = t & 1;
-        const long long c0w = a.dbg ? clock64() : 0;
-        mbar_wait(&tfull[b], (t >> 1) & 1);
-        if (a.dbg) w_tfull += clock64() - c0w;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        float v[CW];
+        sweep_drain<CW, false>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, true, lane, v, timed, w_tfull);
         if (real) {
-          uint32_t r1[CW], r2[CW];
-          const uint32_t taddr = tmem_base + b * 256 + ((uint32_t)(q4 * 32) << 16) + (uint32_t)c0;
-          tmem_ld<CW>(taddr, r1);
-          tmem_ld<CW>(taddr + (uint32_t)a.bn, r2);
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
           for (int k4 = 0; k4 < CW / 4; ++k4) {
             const float4 sc_ = *reinterpret_cast<const float4*>(s_const + c0 + 4 * k4);
             const float4 sh = *reinterpret_cast<const float4*>(s_const + 64 + c0 + 4 * k4);
             const float4 al = *reinterpret_cast<const float4*>(s_const + 128 + c0 + 4 * k4);
-            v[4 * k4 + 0] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 0]) + __uint_as_float(r2[4 * k4 + 0]), sc_.x, sh.x), al.x);
-            v[4 * k4 + 1] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 1]) + __uint_as_float(r2[4 * k4 + 1]), sc_.y, sh.y), al.y);
-            v[4 * k4 + 2] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 2]) + __uint_as_float(r2[4 * k4 + 2]), sc_.z, sh.z), al.z);
-            v[4 * k4 + 3] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 3]) + __uint_as_float(r2[4 * k4 + 3]), sc_.w, sh.w), al.w);
+            v[4 * k4 + 0] = prelu(fmaf(v[4 * k4 + 0], sc_.x, sh.x), al.x);
+            v[4 * k4 + 1] = prelu(fmaf(v[4 * k4 + 1], sc_.y, sh.y), al.y);
+            v[4 * k4 + 2] = prelu(fmaf(v[4 * k4 + 2], sc_.z, sh.z), al.z);
+            v[4 * k4 + 3] = prelu(fmaf(v[4 * k4 + 3], sc_.w, sh.w), al.w);
           }
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[b]);
 
         int r_out = q + DIL * (n0 + m);
         if (POOL == 1) {
@@ -414,6 +485,8 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         ++e;
       }
     }
+    if (t > 0)                               // the last item's two halo slots
+      for (int h = 0; h < 2; ++h) sweep_drain<CW, false>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
     if (issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     if constexpr (STATS) {
       if (a.stats) sweep_stats_flush<CW>(st_s, st_q, s_xch, ew, c0, real, lane, a.stats);
@@ -434,11 +507,11 @@ conv_sweep_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
 // ---------------------------------------------------------------------------------------------------
 // CTA-pair variant (cta_group::2) for the 40-channel-input layers (conv4 + pool2, conv5), whose resident weights do
 // not leave room for a ring in one CTA.  A cluster of two CTAs sweeps two adjacent strips in lock-step:
-//   * every CTA loads its own strip's rows, but only HALF of the output channels' weights (N split across the pair)
+//   * every CTA loads its own strip's rows, but only HALF of the stacked weight rows (N split across the pair)
 //   * both producers signal the LEADER's full barrier; the leader's MMA warp issues tcgen05.mma.cta_group::2 (M = 256)
-//     -- the plain three-MMA split product xl*wh + xh*wl + xh*wh into ONE accumulator (the [wh | wl] column fusion would
-//     need asymmetric weight halves) -- and multicasts its commits to both CTAs
-//   * every CTA's epilogue drains its own 128 TMEM lanes and arrives remotely on the leader's accumulator-empty barrier
+//     in the stacked order of conv_sweep_kernel (D's first 1.5 bn columns take the leader's weight rows, the rest the
+//     peer's) and multicasts its commits to both CTAs
+//   * every CTA's epilogue drains its own 128 TMEM lanes and arrives remotely on the leader's accumulator-empty barriers
 // Input and output pixels are 256 B (64 hi | 64 lo); 4 column groups of 16.
 // ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void sweep_mma_2sm(uint32_t acc, uint32_t a_lo, uint32_t b_lo, uint32_t idesc, uint32_t accumulate, uint32_t elected) {
@@ -464,7 +537,7 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
   constexpr int BOX_BYTES = BOXPX * 128;
   constexpr int SLOT = 2 * SW_SLOT_HALF;
   constexpr int CW = 16;
-  const int panel_bytes = a.bn * 128;                                   // this CTA's half: bn/2 rows of W hi, bn/2 rows of W lo
+  const int panel_bytes = 3 * a.bn * 128;                               // this CTA's half: 1.5 bn stacked rows of W hi, then of W lo
   const int w_bytes = a.npanels * panel_bytes;
   uint8_t* sW = smem;
   uint8_t* sRing = smem + ((w_bytes + 1023) & ~1023);
@@ -473,9 +546,9 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
   uint64_t* bars = reinterpret_cast<uint64_t*>(sOut + a.out_bufs * OB_BYTES);
   uint64_t* full = bars;                        // leader only: both producers signal it
   uint64_t* empty = bars + a.stages;            // per CTA, arrived by the leader's multicast commit
-  uint64_t* tfull = bars + 2 * a.stages;        // per CTA
-  uint64_t* tempty = tfull + 2;                 // leader only: both CTAs' epilogue warps arrive
-  uint64_t* wfull = tempty + 2;                 // leader only: both CTAs' weight halves
+  uint64_t* afull = bars + 2 * a.stages;        // [S] per CTA, arrived by the leader's multicast commit
+  uint64_t* aempty = afull + a.S;               // [S] leader only: both CTAs' epilogue warps arrive
+  uint64_t* wfull = aempty + a.S;               // leader only: both CTAs' weight halves
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wfull + 1);
   float* s_const = reinterpret_cast<float*>(tmem_slot + 2);
   float* s_xch = s_const + 192;                 // pooled layers only
@@ -486,7 +559,7 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < a.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 32); }
+    for (int j = 0; j < a.S; ++j) { mbar_init(&afull[j], 1); mbar_init(&aempty[j], 32); }
     mbar_init(wfull, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -505,9 +578,16 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  cluster_sync_all();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
+  const int q4 = warp & 3, ew = warp - 2, grp = ew >> 2, c0 = grp * CW;
+  const bool real = c0 < a.bn;
+  const uint32_t tcol = tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)c0;
+  if (warp >= 2 && real) sweep_acc_clear<CW>(tcol, a.S, a.bn);
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  cluster_sync_all();                           // the leader's first MMAs write both CTAs' cleared accumulators
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
   // pair item -> (strip pair, class q, segment); this CTA's strip is 2 * strip_pair + rank
   const int nsp = (a.nstrips + 1) >> 1;
@@ -530,9 +610,11 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
       {
         const uint32_t lbar = smem_u32(wfull) & 0xFEFFFFFFu;            // the leader's barrier (peer bit cleared)
         if (rank == 0) mbar_expect_tx(wfull, (uint32_t)(2 * w_bytes));
-        for (int p = 0; p < a.npanels; ++p) tma_load_2d_2sm(&mapW, lbar, sW + p * panel_bytes, 0, (p * 2 + (int)rank) * a.bn);
+        for (int p = 0; p < a.npanels; ++p) tma_load_2d_2sm(&mapW, lbar, sW + p * panel_bytes, 0, (p * 2 + (int)rank) * 3 * a.bn);
       }
       uint32_t g = 0;
+      long long w_empty = 0;
+      const long long tstart = a.dbg ? clock64() : 0;
       for (int item = pair; item < a.n_items; item += npairs) {
         int w0, q, n0, Lc;
         decode(item, w0, q, n0, Lc);
@@ -540,7 +622,11 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
         const int nload = Lc + (POOL == 1 ? 1 : 0) + 2;
         for (int m = 0; m < nload; ++m, ++g) {
           const uint32_t s = g % a.stages, use = g / a.stages;
-          if (use > 0) mbar_wait(&empty[s], (use - 1) & 1);
+          if (use > 0) {
+            const long long c0w = a.dbg ? clock64() : 0;
+            mbar_wait(&empty[s], (use - 1) & 1);
+            if (a.dbg) w_empty += clock64() - c0w;
+          }
           const uint32_t lbar = smem_u32(&full[s]) & 0xFEFFFFFFu;
           if (rank == 0) mbar_expect_tx(&full[s], (uint32_t)(2 * 2 * BOX_BYTES));   // both CTAs' boxes land on it
           uint8_t* sp = sRing + s * SLOT;
@@ -549,81 +635,79 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
           tma_load_3d_2sm(&mapA, lbar, sp + SW_SLOT_HALF, 64, w0 + a.in_dx, r + a.in_dy);
         }
       }
+      if (a.dbg) { a.dbg[blockIdx.x * 8 + 0] = (unsigned long long)w_empty; a.dbg[blockIdx.x * 8 + 1] = (unsigned long long)(clock64() - tstart); }
     }
     __syncwarp();
   } else if (warp == 1) {
     if (rank == 0) {
       const uint32_t leader = elect_one();
-      // D = F32, A = B = BF16, K-major, N = bn (bn/2 weight rows from each CTA), M = 256
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(a.bn >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+      // D = F32, A = B = BF16, K-major, N = 3 * bn (1.5 bn stacked weight rows from each CTA), M = 256
+      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(3 * a.bn >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
       mbar_wait(wfull, 0);
       const uint32_t w_lo = desc_lo(smem_u32(sW));
       const uint32_t ring_lo = desc_lo(smem_u32(sRing));
       const uint32_t panel16 = (uint32_t)(panel_bytes >> 4);
-      const uint32_t wl_off = (uint32_t)((a.bn >> 1) * 128) >> 4;       // W lo rows follow the bn/2 W hi rows
-      uint32_t gs = 0, gph = 0, t = 0;
+      const uint32_t wl_off = (uint32_t)(3 * a.bn / 2 * 128) >> 4;   // W lo rows follow the 1.5 bn W hi rows
+      uint32_t rs = 0, rph = 0, j = 2, eph = 0;                      // as in conv_sweep_kernel
+      bool open = false;
+      long long w_full = 0, w_tempty = 0;
+      const long long tstart = a.dbg ? clock64() : 0;
       for (int item = pair; item < a.n_items; item += npairs) {
         int w0, q, n0, Lc;
         decode(item, w0, q, n0, Lc);
         if (Lc <= 0 || (a.item_on && !a.item_on[item])) continue;
-        const int nrow = Lc + (POOL == 1 ? 1 : 0);
-        for (int m = 0; m < nrow; ++m, ++t) {
-          const uint32_t b = t & 1;
-          mbar_wait(&tempty[b], ((t >> 1) & 1) ^ 1);
-          uint32_t sl[3], ss[3], sp[3];
-          ss[0] = gs; sp[0] = gph;
-#pragma unroll
-          for (int ky = 1; ky < 3; ++ky) {
-            const bool wrap = ss[ky - 1] + 1 == (uint32_t)a.stages;
-            ss[ky] = wrap ? 0u : ss[ky - 1] + 1;
-            sp[ky] = sp[ky - 1] ^ (wrap ? 1u : 0u);
-          }
-#pragma unroll
-          for (int ky = 0; ky < 3; ++ky) {
-            if (m == 0 || ky == 2) mbar_wait(&full[ss[ky]], sp[ky]);
-            sl[ky] = ring_lo + ss[ky] * (SLOT >> 4);
-          }
+        const int nin = Lc + (POOL == 1 ? 1 : 0) + 2;
+        const uint32_t j0 = (uint32_t)(n0 + 2) % (uint32_t)a.S;
+        const uint32_t d = open ? (j0 + (uint32_t)a.S - j) % (uint32_t)a.S : 2u;
+        if (d) {
+          if (open && leader) { umma_commit_2sm(&afull[slot_back(j, 2, a.S)]); if (d >= 2) umma_commit_2sm(&afull[slot_back(j, 1, a.S)]); }
+          if (d >= 2) sweep_claim(aempty, slot_back(j0, 2, a.S), eph);
+          sweep_claim(aempty, slot_back(j0, 1, a.S), eph);
+        }
+        j = j0; open = true;
+        for (int m = 0; m < nin; ++m) {
+          long long c0w = a.dbg ? clock64() : 0;
+          sweep_claim(aempty, j, eph);
+          if (a.dbg) { const long long c1 = clock64(); w_tempty += c1 - c0w; c0w = c1; }
+          mbar_wait(&full[rs], rph);
+          if (a.dbg) w_full += clock64() - c0w;
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          const uint32_t acc = tmem_base + b * 256;
+          const uint32_t p = slot_back(j, 2, a.S);
+          const uint32_t acc = tmem_base + p * (uint32_t)a.bn;
+          const uint32_t sl = ring_lo + rs * (SLOT >> 4);
 #pragma unroll
-          for (int ky = 0; ky < 3; ++ky) {
+          for (int kx = 0; kx < 3; ++kx) {
 #pragma unroll
-            for (int kx = 0; kx < 3; ++kx) {
-#pragma unroll
-              for (int ks = 0; ks < KSTEPS; ++ks) {
-                const int gk = (ky * 3 + kx) * KSTEPS + ks;
-                const uint32_t a_hi = sl[ky] + (uint32_t)(kx * DIL * 8 + ks * 2);
-                const uint32_t a_lo = a_hi + (uint32_t)(SW_SLOT_HALF >> 4);
-                const uint32_t wh = w_lo + (uint32_t)(gk >> 2) * panel16 + (uint32_t)((gk & 3) * 2);
-                sweep_mma_2sm(acc, a_lo, wh, idesc, gk != 0, leader);
-                sweep_mma_2sm(acc, a_hi, wh + wl_off, idesc, 1, leader);
-                sweep_mma_2sm(acc, a_hi, wh, idesc, 1, leader);
-              }
+            for (int ks = 0; ks < KSTEPS; ++ks) {
+              const int gk = kx * KSTEPS + ks;
+              const uint32_t a_hi = sl + (uint32_t)(kx * DIL * 8 + ks * 2);
+              const uint32_t a_lo = a_hi + (uint32_t)(SW_SLOT_HALF >> 4);
+              const uint32_t wh = w_lo + (uint32_t)(gk >> 2) * panel16 + (uint32_t)((gk & 3) * 2);
+              sweep_mma_2sm(acc, a_lo, wh, idesc, 1, leader);
+              sweep_mma_2sm(acc, a_hi, wh + wl_off, idesc, 1, leader);
+              sweep_mma_2sm(acc, a_hi, wh, idesc, 1, leader);
             }
           }
           if (leader) {
-            umma_commit_2sm(&empty[ss[0]]);
-            if (m == nrow - 1) {
-              umma_commit_2sm(&empty[ss[1]]);
-              umma_commit_2sm(&empty[ss[2]]);
-            }
-            umma_commit_2sm(&tfull[b]);
+            umma_commit_2sm(&empty[rs]);
+            umma_commit_2sm(&afull[p]);
           }
           __syncwarp();
-          gs = ss[1]; gph = sp[1];
-          if (m == nrow - 1) {
-            const bool wrap = ss[2] + 1 == (uint32_t)a.stages;
-            gs = wrap ? 0u : ss[2] + 1; gph = sp[2] ^ (wrap ? 1u : 0u);
-          }
+          if (++rs == (uint32_t)a.stages) { rs = 0; rph ^= 1; }
+          if (++j == (uint32_t)a.S) j = 0;
         }
+      }
+      if (open && leader) {
+        umma_commit_2sm(&afull[slot_back(j, 2, a.S)]);
+        umma_commit_2sm(&afull[slot_back(j, 1, a.S)]);
+      }
+      __syncwarp();
+      if (a.dbg && leader) {
+        a.dbg[blockIdx.x * 8 + 2] = (unsigned long long)w_full; a.dbg[blockIdx.x * 8 + 3] = (unsigned long long)w_tempty;
+        a.dbg[blockIdx.x * 8 + 4] = (unsigned long long)(clock64() - tstart);
       }
     }
   } else {
-    const int q4 = warp & 3;
-    const int ew = warp - 2;
-    const int grp = ew >> 2;
-    const int c0 = grp * CW;
-    const bool real = c0 < a.bn;
     const int px = q4 * 32 + lane;
     const bool issuer = threadIdx.x == 64;
     const int trow = POOL == 2 ? px >> 1 : px;
@@ -631,43 +715,48 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
     const uint32_t row_off = (uint32_t)trow * 128u;
     const uint32_t sw = (uint32_t)(trow & 7);
     const uint32_t hi_chunk = (uint32_t)(c0 >> 3);
-    uint32_t t = 0, e = 0;
+    uint32_t t = 0, e = 0, dj = 0, dph = 0;
+    uint32_t w_tfull = 0;
+    const bool timed = a.dbg != nullptr;
+    const long long tstart = a.dbg ? clock64() : 0;
     constexpr bool STATS = POOL == 0 && DIL == 1;
     float st_s[STATS ? CW : 1], st_q[STATS ? CW : 1];
 #pragma unroll
     for (int k = 0; k < (STATS ? CW : 1); ++k) st_s[k] = st_q[k] = 0.f;
+    float v[CW];
     for (int item = pair; item < a.n_items; item += npairs) {
       int w0, q, n0, Lc;
       decode(item, w0, q, n0, Lc);
       if (Lc <= 0 || (a.item_on && !a.item_on[item])) continue;
       const int nrow = Lc + (POOL == 1 ? 1 : 0);
+      // halo slots of the previous item (dj = its first one) up to the new item's two leading ones, as the MMA warp jumps
+      const uint32_t j0 = (uint32_t)(n0 + 2) % (uint32_t)a.S;
+      const uint32_t d = (j0 + 2u * (uint32_t)a.S - 2u - dj) % (uint32_t)a.S;
+      if (t == 0 || d >= 3) {
+        if (t > 0)
+          for (int h = 0; h < 2; ++h) sweep_drain<CW, true>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
+        dj = slot_back(j0, 2, a.S);
+      } else {
+        for (uint32_t h = 0; h < d; ++h) sweep_drain<CW, true>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
+      }
+      for (int h = 0; h < 2; ++h) sweep_drain<CW, true>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
       float hprev[CW];
 #pragma unroll
       for (int k = 0; k < CW; ++k) hprev[k] = 0.f;
       for (int m = 0; m < nrow; ++m, ++t) {
-        const uint32_t b = t & 1;
-        mbar_wait(&tfull[b], (t >> 1) & 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        float v[CW];
+        sweep_drain<CW, true>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, true, lane, v, timed, w_tfull);
         if (real) {
-          uint32_t r1[CW];
-          const uint32_t tb = tmem_base + b * 256 + ((uint32_t)(q4 * 32) << 16);
-          tmem_ld16(tb + (uint32_t)c0, r1);
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
           for (int k4 = 0; k4 < CW / 4; ++k4) {
             const float4 sc_ = *reinterpret_cast<const float4*>(s_const + c0 + 4 * k4);
             const float4 sh = *reinterpret_cast<const float4*>(s_const + 64 + c0 + 4 * k4);
             const float4 al = *reinterpret_cast<const float4*>(s_const + 128 + c0 + 4 * k4);
-            v[4 * k4 + 0] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 0]), sc_.x, sh.x), al.x);
-            v[4 * k4 + 1] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 1]), sc_.y, sh.y), al.y);
-            v[4 * k4 + 2] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 2]), sc_.z, sh.z), al.z);
-            v[4 * k4 + 3] = prelu(fmaf(__uint_as_float(r1[4 * k4 + 3]), sc_.w, sh.w), al.w);
+            v[4 * k4 + 0] = prelu(fmaf(v[4 * k4 + 0], sc_.x, sh.x), al.x);
+            v[4 * k4 + 1] = prelu(fmaf(v[4 * k4 + 1], sc_.y, sh.y), al.y);
+            v[4 * k4 + 2] = prelu(fmaf(v[4 * k4 + 2], sc_.z, sh.z), al.z);
+            v[4 * k4 + 3] = prelu(fmaf(v[4 * k4 + 3], sc_.w, sh.w), al.w);
           }
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cta(&tempty[b], 0);     // the leader's MMA warp owns the accumulator hand-off
 
         int r_out = q + DIL * (n0 + m);
         if (POOL == 1) {
@@ -748,9 +837,15 @@ conv_sweep_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_co
         ++e;
       }
     }
+    if (t > 0)
+      for (int h = 0; h < 2; ++h) sweep_drain<CW, true>(afull, aempty, dj, dph, a.S, a.bn, tcol, real, false, lane, v, timed, w_tfull);
     if (issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     if constexpr (STATS) {
       if (a.stats) sweep_stats_flush<CW>(st_s, st_q, s_xch, ew, c0, real, lane, a.stats);
+    }
+    if (a.dbg && threadIdx.x == 64) {
+      a.dbg[blockIdx.x * 8 + 5] = (unsigned long long)w_tfull; a.dbg[blockIdx.x * 8 + 6] = (unsigned long long)(clock64() - tstart);
+      a.dbg[blockIdx.x * 8 + 7] = t;
     }
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -998,19 +1093,22 @@ int launch_conv_sweep(sc_ctx* ctx, const SweepW& w, int layer, const float* in, 
   a.scale = w.scale; a.shift = w.shift; a.alpha = w.alpha;
   a.dbg = (ctx->tc_timing_cls == prof_cls) ? ctx->tc_timing_buf : nullptr;
   SC_CHECK(w.bn <= (out_fmt ? 32 : 64) && w.bn % 16 == 0, SC_ERR_ARG, "conv_sweep: bad channel geometry");
+  a.S = 512 / w.bn - 2;                                                 // accumulator slots + 2 spill slots fill the 512 TMEM columns
+  if (a.S > SW_MAX_SLOTS) a.S = SW_MAX_SLOTS;
   const int slot = (in_fmt ? 1 : 2) * SW_SLOT_HALF;                      // F32CH: one box per row (hi|lo in one 128 B pixel), F64CH: hi box + lo box
-  const int w_bytes = w.npanels * 2 * w.bn * 128;
+  const int w_bytes = w.npanels * 6 * w.bn * 128;
   const int ob_bytes = out_fmt ? 16384 : 32768;
-  const int fixed = 1024 + w_bytes + 256 /*barriers, tmem slot*/ + 192 * 4 + 2 * 4 * 4 * 2 * 16 * 4;
+  const int fixed = 1024 + w_bytes + SW_BAR_BYTES + 192 * 4 + 2 * 4 * 4 * 2 * 16 * 4;
+  // ring: one stage per input row in the MMAs, the others prefetch; two output tiles if that leaves >= 3 stages
   a.out_bufs = 2;
   a.stages = (227 * 1024 - fixed - 2 * ob_bytes) / slot;
-  if (a.stages < 4) {                                                   // short of shared memory: single output tile
+  if (a.stages < 3) {                                                   // short of shared memory: single output tile
     a.out_bufs = 1;
     a.stages = (227 * 1024 - fixed - ob_bytes) / slot;
   }
   if (a.stages > 8) a.stages = 8;
   const bool use_pair = w.ksteps >= 3 && !in_fmt && !out_fmt;          // >= 40 input channels: the resident weights need the CTA pair
-  SC_CHECK(use_pair || a.stages >= 3, SC_ERR_ARG, "conv_sweep: ring does not fit (layer %d)", layer);
+  SC_CHECK(use_pair || a.stages >= 2, SC_ERR_ARG, "conv_sweep: ring does not fit (layer %d)", layer);
   const size_t smem = (size_t)fixed + (size_t)a.stages * slot + (size_t)a.out_bufs * ob_bytes;
 
   CUtensorMap mapA, mapW, mapO;
@@ -1026,9 +1124,9 @@ int launch_conv_sweep(sc_ctx* ctx, const SweepW& w, int layer, const float* in, 
     SC_CHECK(r == CUDA_SUCCESS, SC_ERR_CUDA, "conv_sweep: cuTensorMapEncodeTiled(A) failed with %d (Pw %d R %d)", (int)r, Pw, R);
   }
   {
-    cuuint64_t dims[2] = {64, (cuuint64_t)w.npanels * 2 * w.bn};
+    cuuint64_t dims[2] = {64, (cuuint64_t)w.npanels * 6 * w.bn};
     cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)(2 * w.bn)};
+    cuuint32_t box[2] = {64, (cuuint32_t)(3 * w.bn)};                    // W hi or W lo rows of one panel (<= 192 rows)
     cuuint32_t es[2] = {1, 1};
     CUresult r = s->encode(&mapW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w.panels, dims, strides, box, es,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -1051,7 +1149,7 @@ int launch_conv_sweep(sc_ctx* ctx, const SweepW& w, int layer, const float* in, 
   }
   const bool i32 = in_fmt != 0, o32 = out_fmt != 0;
   if (use_pair) {
-    // ---- CTA pairs: half of the weights per CTA, ring of >= 4 rows ----
+    // ---- CTA pairs: half of the weights per CTA ----
     const int nsp = (a.nstrips + 1) / 2;
     const int pairs_max = ctx->sm_count / 2;
     nseg = (4 * pairs_max + nsp * dil - 1) / (nsp * dil);
@@ -1068,19 +1166,19 @@ int launch_conv_sweep(sc_ctx* ctx, const SweepW& w, int layer, const float* in, 
     nseg = (nq + L - 1) / L;
     a.L = L; a.nseg = nseg;
     a.n_items = nsp * dil * nseg;
-    const int wp_bytes = w.npanels * w.bn * 128;
-    const int fixed_p = 1024 + ((wp_bytes + 1023) & ~1023) + 256 + 192 * 4 + ((pool || stats) ? 2 * 4 * 4 * 2 * 16 * 4 : 0);
+    const int wp_bytes = w.npanels * 3 * w.bn * 128;
+    const int fixed_p = 1024 + ((wp_bytes + 1023) & ~1023) + SW_BAR_BYTES + 192 * 4 + ((pool || stats) ? 2 * 4 * 4 * 2 * 16 * 4 : 0);
     a.out_bufs = 2;
     a.stages = (227 * 1024 - fixed_p - 2 * ob_bytes) / slot;
-    if (a.stages < 4) { a.out_bufs = 1; a.stages = (227 * 1024 - fixed_p - ob_bytes) / slot; }
+    if (a.stages < 3) { a.out_bufs = 1; a.stages = (227 * 1024 - fixed_p - ob_bytes) / slot; }
     if (a.stages > 8) a.stages = 8;
-    SC_CHECK(a.stages >= 3, SC_ERR_ARG, "conv_sweep: pair ring does not fit (layer %d)", layer);
+    SC_CHECK(a.stages >= 2, SC_ERR_ARG, "conv_sweep: pair ring does not fit (layer %d)", layer);
     SC_CHECK(pool != 2 || (Pw % 2 == 0), SC_ERR_ARG, "conv_sweep: odd pitch with the stride-2 pool");
     const size_t smem_p = (size_t)fixed_p + (size_t)a.stages * slot + (size_t)a.out_bufs * ob_bytes;
     CUtensorMap mapWp;
-    cuuint64_t dims[2] = {64, (cuuint64_t)w.npanels * 2 * w.bn};
+    cuuint64_t dims[2] = {64, (cuuint64_t)w.npanels * 6 * w.bn};
     cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)w.bn};
+    cuuint32_t box[2] = {64, (cuuint32_t)(3 * w.bn)};
     cuuint32_t es[2] = {1, 1};
     CUresult r = s->encode(&mapWp, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w.panels_pair, dims, strides, box, es,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,

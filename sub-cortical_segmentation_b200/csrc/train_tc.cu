@@ -75,16 +75,15 @@ __global__ void derive_panels_kernel(const PanelJobs jobs) {
   // forward: true convolution -> correlation taps (tap 8 - t), rows = output channels, k = input channels
   // dgrad:   raw taps, rows = the layer's INPUT channels, k = its output channels
   const int o = dgrad ? ci : co, k = dgrad ? co : ci, tap = dgrad ? t : 8 - t;
-  const int gk = tap * ksteps + (k >> 4), kk = (gk & 3) * 16 + (k & 15), panel = gk >> 2;
   const __nv_bfloat16 hb16 = __float2bfloat16_rn(v);
   const uint16_t hi = __bfloat16_as_ushort(hb16);
   const uint16_t lo = __bfloat16_as_ushort(__float2bfloat16_rn(v - __bfloat162float(hb16)));
-  J.plain[((size_t)panel * 2 * bn + o) * 64 + kk] = hi;
-  J.plain[((size_t)panel * 2 * bn + bn + o) * 64 + kk] = lo;
-  const int hb = bn >> 1;
-  const size_t prow = ((size_t)panel * 2 + o / hb) * bn + o % hb;
-  J.pair[prow * 64 + kk] = hi;
-  J.pair[(prow + hb) * 64 + kk] = lo;
+  size_t ip, iq;
+  sweep_panel_pos(o, tap / 3, tap % 3, k, ksteps, bn, ip, iq);
+  J.plain[ip] = hi;
+  J.plain[ip + (size_t)3 * bn * 64] = lo;
+  J.pair[iq] = hi;
+  J.pair[iq + (size_t)3 * bn / 2 * 64] = lo;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1091,8 +1090,8 @@ static int ensure_train_panels(sc_ctx* ctx) {
   for (int l = 1; l < 5; ++l)
     for (int d = 0; d < 2; ++d) {
       const int kin = d ? kTL[l].cout : kTL[l].cin, nout = d ? kTL[l].cin : kTL[l].cout;
-      const int ksteps = (kin + 15) / 16, bn = pad16(nout), npanels = (9 * ksteps + 3) / 4;
-      total += 2 * (((size_t)npanels * 2 * bn * 64 * 2 + 1023) & ~(size_t)1023);
+      const int ksteps = (kin + 15) / 16, bn = pad16(nout), npanels = (3 * ksteps + 3) / 4;
+      total += 2 * (((size_t)npanels * 6 * bn * 64 * 2 + 1023) & ~(size_t)1023);
     }
   total *= 3;
   SC_CUDA(cudaMalloc(&ctx->train_panels, total));
@@ -1103,8 +1102,8 @@ static int ensure_train_panels(sc_ctx* ctx) {
       for (int d = 0; d < 2; ++d) {
         const int kin = d ? kTL[l].cout : kTL[l].cin, nout = d ? kTL[l].cin : kTL[l].cout;
         SweepW& S = ctx->train_sw[b][l][d];
-        S.ksteps = (kin + 15) / 16; S.bn = pad16(nout); S.npanels = (9 * S.ksteps + 3) / 4;
-        const size_t bytes = ((size_t)S.npanels * 2 * S.bn * 64 * 2 + 1023) & ~(size_t)1023;
+        S.ksteps = (kin + 15) / 16; S.bn = pad16(nout); S.npanels = (3 * S.ksteps + 3) / 4;
+        const size_t bytes = ((size_t)S.npanels * 6 * S.bn * 64 * 2 + 1023) & ~(size_t)1023;
         S.panels = reinterpret_cast<float*>(p); p += bytes;
         S.panels_pair = reinterpret_cast<float*>(p); p += bytes;
         S.scale = ctx->train_consts; S.shift = ctx->train_consts + kTrainZeros; S.alpha = ctx->train_consts;   // identity epilogue

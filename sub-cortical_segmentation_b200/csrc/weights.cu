@@ -88,26 +88,24 @@ int derive_weights(sc_ctx* ctx, cudaStream_t st) {
       bo[b].scale[l] = A.alloc(64);
       bo[b].shift[l] = A.alloc(64);
       bo[b].alpha[l] = A.alloc(64);
-      if (l > 0) {   // strip-sweep kernel: k-step-packed weight panels, W hi rows then W lo rows
+      if (l > 0) {   // strip-sweep kernel: k-step-packed weight panels, filter rows stacked, W hi rows then W lo rows
         SweepW& S = ctx->br[b].conv_sw[l];
-        S.ksteps = (ci_n + 15) / 16; S.bn = (co_n + 15) & ~15; S.npanels = (9 * S.ksteps + 3) / 4;
-        bo[b].sw[l] = A.alloc((size_t)S.npanels * 2 * S.bn * 32);
-        bo[b].swp[l] = A.alloc((size_t)S.npanels * 2 * S.bn * 32);
+        S.ksteps = (ci_n + 15) / 16; S.bn = (co_n + 15) & ~15; S.npanels = (3 * S.ksteps + 3) / 4;
+        bo[b].sw[l] = A.alloc((size_t)S.npanels * 6 * S.bn * 32);
+        bo[b].swp[l] = A.alloc((size_t)S.npanels * 6 * S.bn * 32);
         uint16_t* pw = reinterpret_cast<uint16_t*>(&A.host[bo[b].sw[l]]);
         uint16_t* pp = reinterpret_cast<uint16_t*>(&A.host[bo[b].swp[l]]);
-        const int hb = S.bn / 2;
         for (int co = 0; co < co_n; ++co)
           for (int ci = 0; ci < ci_n; ++ci)
             for (int t = 0; t < 9; ++t) {
               const float v = h[B.convW[l] + ((size_t)co * ci_n + ci) * 9 + (8 - t)];
-              const int gk = t * S.ksteps + ci / 16, kk = (gk & 3) * 16 + (ci & 15);
-              const uint16_t hi = bf16_rn(v);
-              pw[((size_t)(gk >> 2) * 2 * S.bn + co) * 64 + kk] = hi;
-              pw[((size_t)(gk >> 2) * 2 * S.bn + S.bn + co) * 64 + kk] = bf16_rn(v - bf16_to_float(hi));
-              // pair layout: rank = co / (bn/2) owns this output channel
-              const size_t prow = ((size_t)(gk >> 2) * 2 + co / hb) * S.bn + co % hb;
-              pp[prow * 64 + kk] = hi;
-              pp[(prow + hb) * 64 + kk] = bf16_rn(v - bf16_to_float(hi));
+              const uint16_t hi = bf16_rn(v), lo = bf16_rn(v - bf16_to_float(hi));
+              size_t ip, iq;
+              sweep_panel_pos(co, t / 3, t % 3, ci, S.ksteps, S.bn, ip, iq);
+              pw[ip] = hi;
+              pw[ip + (size_t)3 * S.bn * 64] = lo;
+              pp[iq] = hi;
+              pp[iq + (size_t)3 * S.bn / 2 * 64] = lo;
             }
       }
       for (int c = 0; c < co_n; ++c) {
