@@ -204,6 +204,24 @@ SC_API int sc_segment_volume_host(sc_ctx* ctx, const float* vol_host, const int3
 SC_API int sc_post_process(sc_ctx* ctx, const uint8_t* seg_dev, const uint8_t* mask_dev, const int32_t dims[3],
                     uint8_t* out_dev, void* stream);
 
+/* ---- evaluation against manual labels --------------------------------------------------
+ * replaces: the scipy / medpy-style host evaluation of a segmentation (binary_erosion surfaces, distance_transform_edt
+ * per structure and direction, np.percentile); the reference has none.  seg / ref: uint8 [X][Y][Z] label volumes with
+ * values 0..15, 15 counted as background (0) in both (as training does); seg_dev == ref_dev is allowed.  spacing: voxel
+ * size in mm along x, y, z (finite, > 0).  For each structure l = 1..14 (metrics_host[l - 1]), A = (seg == l),
+ * B = (ref == l): n_seg = |A|, n_ref = |B|, n_both = |A & B|; dice = 2 n_both / (n_seg + n_ref) (NaN when both are
+ * empty); volumes = counts x sx sy sz; with S(M) = the voxels of M having a 6-neighbour outside M or outside the volume and
+ * d_AB = for each voxel of S(A) the Euclidean distance in mm to the nearest voxel of S(B) (d_BA alike): hd_mm = max of both,
+ * hd95_mm = np.percentile(hstack(d_AB, d_BA), 95) (linear interpolation), assd_mm = (mean d_AB + mean d_BA) / 2, all three
+ * NaN when A or B is empty.  confusion_host (nullable) int64 [15][15]: [r][s] = voxels with reference class r and
+ * segmentation class s.  Synchronises the stream.  SC_ERR_ARG for NULL pointers, bad dims, a spacing that is not finite
+ * and > 0, or a label above 15 in either input (the message names it); outputs are untouched on an error. */
+typedef struct { int64_t n_seg, n_ref, n_both;
+                 double dice, vol_seg_mm3, vol_ref_mm3, hd_mm, hd95_mm, assd_mm; } sc_structure_metrics;  /* 72 bytes */
+SC_API int sc_evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg_dev, const uint8_t* ref_dev, const int32_t dims[3],
+                                    const double spacing[3], sc_structure_metrics* metrics_host /* [14], class l at l-1 */,
+                                    int64_t* confusion_host /* [15][15] or NULL */, void* stream);
+
 /* ---- scatter -------------------------------------------------------------------------
  * replaces: image[x,y,z] = y_pred and image_proba[x,y,z,c] = proba[:,c] (base.py:430-440) */
 SC_API int sc_scatter(sc_ctx* ctx, const int32_t* xyz_dev, int64_t n, const int32_t* label_dev,

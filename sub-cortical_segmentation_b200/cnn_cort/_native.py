@@ -19,6 +19,11 @@ DTYPE_CODES = {"u1": 1, "i1": 2, "u2": 3, "i2": 4, "u4": 5, "i4": 6, "f4": 7, "f
 SCAN_DTYPE = np.dtype([("vol", "<u8"), ("dims", "<i4", (3,)), ("reserved", "<i4")])
 assert SCAN_DTYPE.itemsize == 24
 
+# sc_structure_metrics of include/subcort_b200.h, one row per structure 1..14
+METRICS_DTYPE = np.dtype([("n_seg", "<i8"), ("n_ref", "<i8"), ("n_both", "<i8"), ("dice", "<f8"), ("vol_seg_mm3", "<f8"),
+                          ("vol_ref_mm3", "<f8"), ("hd_mm", "<f8"), ("hd95_mm", "<f8"), ("assd_mm", "<f8")])
+assert METRICS_DTYPE.itemsize == 72
+
 _lib = None
 
 
@@ -54,6 +59,7 @@ PROTOTYPES = {
     "sc_candidate_mask": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _p(_c_i32), _vp, _vp]),
     "sc_mask_bbox": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(_c_i32), _p(_c_i64), _vp]),
     "sc_post_process": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _vp, _vp]),
+    "sc_evaluate_segmentation": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _vp, _vp]),
     "sc_gather_patches": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, ctypes.c_int, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp]),
     "sc_gather_center_labels": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _c_i64, _vp, _vp]),
     "sc_gather_samples": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -265,6 +271,18 @@ class Context(object):
         out = torch.empty_like(seg)
         _check(self.lib.sc_post_process(self.h, _ptr(seg), _ptr(mask), _dims(seg.shape), _ptr(out), _stream()))
         return out
+
+    def evaluate_segmentation(self, seg, ref, spacing=(1.0, 1.0, 1.0), confusion=False):
+        """uint8 CUDA label volumes seg / ref [X,Y,Z] (0..15, 15 = background) -> (METRICS_DTYPE [14]: row l - 1 holds
+        structure l, confusion int64 [15, 15] [ref class][seg class] or None).  Synchronises (sc_evaluate_segmentation)."""
+        if tuple(seg.shape) != tuple(ref.shape) or seg.dim() != 3:
+            raise ValueError("seg and ref must be 3-D volumes of one shape, got %s and %s" % (tuple(seg.shape), tuple(ref.shape)))
+        out = np.zeros(14, METRICS_DTYPE)
+        conf = np.zeros((15, 15), np.int64) if confusion else None
+        sp = (ctypes.c_double * 3)(*[float(s) for s in spacing])
+        _check(self.lib.sc_evaluate_segmentation(self.h, _ptr(seg), _ptr(ref), _dims(seg.shape), sp, out.ctypes.data,
+                                                 None if conf is None else conf.ctypes.data, _stream()))
+        return out, conf
 
     def gather_patches(self, vol, xyz, atlas=None, bg_fix=True, views=(True, True, True)):
         import torch

@@ -340,6 +340,64 @@ def post_process_segmentation(image_folder, input_mask, device=None):
     return out.cpu().numpy().astype(input_mask.dtype)
 
 
+# ---------------------------------------------------------------------------------------------
+# evaluation against manual labels
+# ---------------------------------------------------------------------------------------------
+def _label_volume(a, name, device):
+    """label volume of any integer / float / bool dtype holding integral labels (numpy array or torch tensor) -> uint8
+    CUDA tensor.  Labels above 15 become 16, so that sc_evaluate_segmentation rejects them and names the input."""
+    import torch
+    if torch.is_tensor(a):
+        if a.dtype == torch.bool:
+            a = a.to(torch.uint8)
+        elif a.dtype != torch.uint8:
+            if a.is_floating_point() and not bool((a == torch.floor(a)).all()):
+                raise ValueError("%s holds non-integral labels" % name)
+            if bool((a < 0).any()):
+                raise ValueError("%s holds negative labels" % name)
+            a = a.clamp(max=16).to(torch.uint8)
+        return a.to('cuda:%d' % device).contiguous()
+    a = np.asarray(a)
+    if a.dtype != np.uint8:
+        if a.dtype.kind == 'f' and not np.array_equal(a, np.floor(a)):
+            raise ValueError("%s holds non-integral labels" % name)
+        if a.dtype.kind not in 'fiub':
+            raise TypeError("%s: unsupported label dtype %s" % (name, a.dtype))
+        if a.dtype.kind in 'fi' and a.size and a.min() < 0:
+            raise ValueError("%s holds negative labels" % name)
+        a = np.minimum(a, 16).astype(np.uint8)
+    return _dev(a, device)
+
+
+def evaluate_segmentation(seg, ref, spacing=(1.0, 1.0, 1.0), device=None):
+    """Score a segmentation against manual labels, on the device (sc_evaluate_segmentation).
+
+    seg, ref: [X, Y, Z] label volumes with values 0..15 (15 counts as background), as host arrays of any integer or float
+    dtype holding integral labels or as torch tensors; spacing: voxel size in mm along x, y, z.  Returns
+    ({l: {field: value}} for the structures l = 1..14, confusion int64 [15, 15] indexed [ref class][seg class]).  Fields:
+    n_seg, n_ref, n_both (voxel counts), dice (NaN when both are empty), vol_seg_mm3, vol_ref_mm3 and the surface distances
+    hd_mm, hd95_mm, assd_mm (NaN when either structure is empty); definitions in include/subcort_b200.h."""
+    ctx = get_context(device)
+    if tuple(seg.shape) != tuple(ref.shape) or len(seg.shape) != 3:
+        raise ValueError("seg and ref must be 3-D volumes of one shape, got %s and %s" % (tuple(seg.shape), tuple(ref.shape)))
+    d_seg = _label_volume(seg, 'seg', ctx.device)
+    d_ref = d_seg if ref is seg else _label_volume(ref, 'ref', ctx.device)
+    rows, confusion = ctx.evaluate_segmentation(d_seg, d_ref, spacing, confusion=True)
+    metrics = {l: {f: (int(rows[l - 1][f]) if f.startswith('n_') else float(rows[l - 1][f])) for f in rows.dtype.names}
+               for l in range(1, 15)}
+    return metrics, confusion
+
+
+def evaluate_scan(seg_path, ref_path, device=None):
+    """evaluate_segmentation of two NIfTI label files of one shape; the spacing is the reference's voxel size (the column
+    norms of its affine, as nifti.py writes them)."""
+    seg_nii, ref_nii = load_nii(seg_path), load_nii(ref_path)
+    if tuple(seg_nii.shape) != tuple(ref_nii.shape):
+        raise ValueError("%s and %s differ in shape: %s vs %s" % (seg_path, ref_path, seg_nii.shape, ref_nii.shape))
+    spacing = tuple(float(s) for s in np.sqrt((np.asarray(ref_nii.affine)[:3, :3] ** 2).sum(0)))
+    return evaluate_segmentation(seg_nii.get_data(), ref_nii.get_data(), spacing, device=device)
+
+
 def register_masks(input_mask):
     raise NotImplementedError("atlas registration (niftyreg reg_aladin / reg_f3d / reg_resample, base.py:483-551) "
                               "stays with the reference pipeline; it is outside the hot path rebuilt here")

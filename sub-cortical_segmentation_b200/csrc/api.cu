@@ -141,7 +141,7 @@ int sc_destroy(sc_ctx* ctx) {
   tc_destroy(ctx);
   fused_detach(ctx);
   cudaFree(ctx->params); cudaFree(ctx->grads); cudaFree(ctx->adam_m); cudaFree(ctx->adam_v);
-  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr);
+  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr); cudaFree(ctx->ws_eval.ptr);
   for (auto& g : ctx->train_graphs) cudaGraphExecDestroy(g.exec);
   for (int i = 0; i < 2; ++i) if (ctx->train_side[i]) cudaStreamDestroy(ctx->train_side[i]);
   for (int i = 0; i < 8; ++i) if (ctx->train_ev[i]) cudaEventDestroy(ctx->train_ev[i]);
@@ -227,7 +227,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -333,6 +333,17 @@ int sc_post_process(sc_ctx* ctx, const uint8_t* seg_dev, const uint8_t* mask_dev
   SC_TRY(check_dims(dims, "sc_post_process"));
   SC_CUDA(cudaSetDevice(ctx->device));
   return post_process(ctx, seg_dev, mask_dev, dims, out_dev, (cudaStream_t)stream);
+}
+
+int sc_evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg_dev, const uint8_t* ref_dev, const int32_t dims[3], const double spacing[3],
+                             sc_structure_metrics* metrics_host, int64_t* confusion_host, void* stream) {
+  SC_CHECK(ctx && seg_dev && ref_dev && spacing && metrics_host, SC_ERR_ARG, "sc_evaluate_segmentation: null argument");
+  SC_TRY(check_dims(dims, "sc_evaluate_segmentation"));
+  for (int i = 0; i < 3; ++i)
+    SC_CHECK(isfinite(spacing[i]) && spacing[i] > 0.0, SC_ERR_ARG, "sc_evaluate_segmentation: spacing[%d] = %g is not a finite positive number",
+             i, spacing[i]);
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return evaluate_segmentation(ctx, seg_dev, ref_dev, dims, spacing, metrics_host, confusion_host, (cudaStream_t)stream);
 }
 
 int sc_gather_patches(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], const float* atlas_dev, int bg_fix,

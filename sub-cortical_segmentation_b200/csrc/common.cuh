@@ -148,7 +148,7 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_COUNT
 };
 struct ProfEvent { int cls; cudaEvent_t a, b; };
 
@@ -177,6 +177,7 @@ struct sc_ctx {
   sc::Workspace ws;              // inference scratch (grow-only)
   sc::Workspace ws_train;        // staging of the host entry points, scan preparation, eval scratch
   sc::Workspace ws_fit;          // training step: staged inputs, saved activations, gradients of activations
+  sc::Workspace ws_eval;         // sc_evaluate_segmentation: distance fields, envelope stacks and distance lists of one class box
   // training step as a CUDA graph (one per (batch, global batch, injected masks) shape): the three branches run on
   // three captured streams; rebuilt when the arena moves
   struct TrainGraph { int n; long long n_global; int injected; int backend; void* arena; cudaGraphExec_t exec; int launches; };
@@ -286,6 +287,10 @@ int mask_bbox(sc_ctx* ctx, const uint8_t* mask, const int32_t* dims, int32_t* bo
 
 // postproc.cu : connected-component post-processing of a label volume
 int post_process(sc_ctx* ctx, const uint8_t* seg, const uint8_t* mask, const int32_t* dims, uint8_t* out, cudaStream_t st);
+
+// evaluate.cu : per-structure Dice, volumes and surface distances of a label volume against a reference
+int evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg, const uint8_t* ref, const int32_t* dims, const double* spacing,
+                          sc_structure_metrics* metrics, int64_t* confusion, cudaStream_t st);
 
 // weights.cu
 int derive_weights(sc_ctx* ctx, cudaStream_t st);

@@ -2,7 +2,10 @@
 """Example driver -- the Python 3 counterpart of the reference's train_model.py (same calls, same configuration.cfg
 keys); everything below the imports runs on the B200 kernels.
 
-    python train_model.py [configuration.cfg] [--train]
+    python train_model.py [configuration.cfg] [--train] [--evaluate]
+
+--evaluate scores each inference subject that has manual labels (<subject>/<roi_name>): per-structure Dice and
+surface distances of the segmentation test_scan wrote.
 """
 import configparser
 import os
@@ -11,7 +14,7 @@ import sys
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "sub-cortical_segmentation_b200"))
 
-from cnn_cort.base import generate_training_set, load_data, load_test_names, test_scan  # noqa: E402
+from cnn_cort.base import evaluate_scan, generate_training_set, load_data, load_test_names, test_scan  # noqa: E402
 from cnn_cort.load_options import load_options, print_options  # noqa: E402
 from cnn_cort.nets import build_model  # noqa: E402
 
@@ -39,6 +42,24 @@ def main():
     for t1, current_scan in zip(t1_test_paths, folder_names):
         t = test_scan(net, t1, options)
         print("    -->  tested subject :", current_scan, "(elapsed time:", t, "min.)")
+        if "--evaluate" in sys.argv:
+            print_evaluation(t1, options)
+
+
+def print_evaluation(t1_path, options):
+    """Score the segmentation test_scan wrote for one subject against its manual labels (<subject>/<roi_name>), if any."""
+    subject_dir = os.path.dirname(t1_path)
+    ref_path = os.path.join(subject_dir, options['roi_name'])
+    if not os.path.exists(ref_path):
+        return
+    out_name = 'out_subcortical_seg_prec.nii.gz' if options['post_process'] == 'True' else 'out_subcortical_rawseg.nii.gz'
+    metrics, _ = evaluate_scan(os.path.join(subject_dir, out_name), ref_path, device=options.get('device'))
+    print("    -->  %s vs %s" % (out_name, options['roi_name']))
+    print("         %9s %9s %9s %7s %9s %9s %9s" % ("structure", "n_seg", "n_ref", "dice", "hd_mm", "hd95_mm", "assd_mm"))
+    for l, m in metrics.items():
+        print("         %9d %9d %9d %7.4f %9.3f %9.3f %9.3f" % (l, m['n_seg'], m['n_ref'], m['dice'], m['hd_mm'], m['hd95_mm'], m['assd_mm']))
+    dice = [m['dice'] for m in metrics.values() if m['dice'] == m['dice']]
+    print("         mean dice %.4f over %d structures" % (sum(dice) / len(dice) if dice else float('nan'), len(dice)))
 
 
 if __name__ == "__main__":
