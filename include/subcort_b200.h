@@ -222,6 +222,51 @@ SC_API int sc_evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg_dev, const u
                                     const double spacing[3], sc_structure_metrics* metrics_host /* [14], class l at l-1 */,
                                     int64_t* confusion_host /* [15][15] or NULL */, void* stream);
 
+/* ---- atlas registration ---------------------------------------------------------------
+ * replaces: register_masks (base.py:483-551), i.e. niftyreg reg_aladin + reg_f3d + reg_resample, which map the template
+ * T1 and its 15 structure priors onto the subject.  Not bit-compatible with niftyreg; its structure and conventions:
+ *   - reference = the subject T1 (float32 [X][Y][Z]; its mask is the voxels != 0), floating = the template T1;
+ *   - *_vox2mm: row-major 4x4 voxel -> mm matrices (what cnn_cort/nifti.py returns as .affine);
+ *   - phi(x) = A [x; 1] + u(v) maps subject mm to template mm: A is the 3x4 top of `affine` (row-major 4x4, last row
+ *     0 0 0 1); u is a cubic B-spline displacement in template mm whose control point (i, j, k) sits at subject voxel
+ *     ((i-1) s, (j-1) s, (k-1) s), s = 5 voxels; grid [gx][gy][gz][3] float32 with g = floor((d - 1) / 5) + 4
+ *     (sc_ffd_grid_dims).  Because the control points hold template mm, d F(phi(x)) / d c_k = beta_k(x) grad F(phi(x));
+ *   - trilinear sampling in fp32 (in software); a point is inside the template when its voxel coordinate lies in [0, d-1]
+ *     on every axis; outside, warped values are 0 and the subject voxel does not count towards the similarity;
+ *   - NMI = (H_R + H_F) / H_RF, 64 bins, cubic B-spline Parzen windows on both axes; intensities mapped linearly to
+ *     [2, 61] from [min, max] over the subject's mask and over every template voxel;
+ *   - BE = mean over the interior control points of the squared second derivatives of u with respect to the grid
+ *     coordinates (cross terms doubled), analytic at the control points; the FFD maximises J = (1 - 0.001) NMI - 0.001 BE.
+ * sc_register_affine: A from the translation between the intensity centres of mass, then conjugate-gradient ascent of NMI
+ * on a 4-level pyramid (factors 8, 4, 2, 1; levels where either image would have a dim below 16 are skipped).
+ * sc_register_ffd: grid_dev (written) from a zero grid on a 3-level pyramid (factors 4, 2, 1; control points every 5
+ * voxels of each level, refined exactly by B-spline subdivision between levels) for the given affine.
+ * Deterministic: the same inputs give byte-identical results on every run.  Both synchronise the stream.
+ * SC_ERR_ARG: NULL pointers, a dim below 8, a singular or non-finite matrix, an empty reference mask or no overlap of the
+ * mask with the template (the message names the input). */
+SC_API int sc_ffd_grid_dims(const int32_t ref_dims[3], int32_t grid_dims_out[3]);
+SC_API int sc_register_affine(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16],
+                              const float* flo_dev, const int32_t flo_dims[3], const double flo_vox2mm[16], double affine_out[16],
+                              void* stream);
+SC_API int sc_register_ffd(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16],
+                           const float* flo_dev, const int32_t flo_dims[3], const double flo_vox2mm[16], const double affine[16],
+                           float* grid_dev, void* stream);
+/* replaces: reg_resample.  out_dev [X][Y][Z][channels] on the subject grid (ref_dims / ref_vox2mm) = the floating volume
+ * [fX][fY][fZ][channels] (channels 1 or 15, channels-last) sampled trilinearly at phi(x), 0 outside; grid_dev NULL = affine only. */
+SC_API int sc_warp_volume(sc_ctx* ctx, const float* flo_dev, const int32_t flo_dims[3], int channels, const double flo_vox2mm[16],
+                          const double affine[16], const float* grid_dev, const int32_t ref_dims[3], const double ref_vox2mm[16],
+                          float* out_dev, void* stream);
+/* the objective at full resolution for a fixed (affine, grid) (parity tests of the kernels, as sc_dense_layer is for the
+ * GEMMs): value_out = {NMI, BE, J} (BE = 0 and J = NMI when grid_dev is NULL); affine_grad_host[12] (nullable) = d NMI / d A
+ * for the 12 entries of the 3x4 top of `affine`, row-major; grid_grad_dev (nullable, needs grid_dev) = d J / d grid. */
+SC_API int sc_register_objective(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16],
+                                 const float* flo_dev, const int32_t flo_dims[3], const double flo_vox2mm[16], const double affine[16],
+                                 const float* grid_dev, double value_out[3], double* affine_grad_host, float* grid_grad_dev,
+                                 void* stream);
+/* the registered sub-cortical mask (base.py:540-551, quirk Q11): (sum of channels 0..12 of the warped priors [X][Y][Z][15]) > 0,
+ * dilated `iterations` times (sc_dilate_mask), as float32 0 / 1 [X][Y][Z]. */
+SC_API int sc_prior_mask(sc_ctx* ctx, const float* priors_dev, const int32_t dims[3], int iterations, float* mask_dev, void* stream);
+
 /* ---- scatter -------------------------------------------------------------------------
  * replaces: image[x,y,z] = y_pred and image_proba[x,y,z,c] = proba[:,c] (base.py:430-440) */
 SC_API int sc_scatter(sc_ctx* ctx, const int32_t* xyz_dev, int64_t n, const int32_t* label_dev,

@@ -60,6 +60,14 @@ PROTOTYPES = {
     "sc_mask_bbox": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(_c_i32), _p(_c_i64), _vp]),
     "sc_post_process": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _vp, _vp]),
     "sc_evaluate_segmentation": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _vp, _vp]),
+    "sc_ffd_grid_dims": (ctypes.c_int, [_p(_c_i32), _p(_c_i32)]),
+    "sc_register_affine": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _p(_c_i32), _p(ctypes.c_double), _p(ctypes.c_double), _vp]),
+    "sc_register_ffd": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _p(_c_i32), _p(ctypes.c_double), _p(ctypes.c_double), _vp, _vp]),
+    "sc_warp_volume": (ctypes.c_int, [_vp, _vp, _p(_c_i32), ctypes.c_int, _p(ctypes.c_double), _p(ctypes.c_double), _vp, _p(_c_i32),
+                                      _p(ctypes.c_double), _vp, _vp]),
+    "sc_register_objective": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _p(_c_i32), _p(ctypes.c_double),
+                                             _p(ctypes.c_double), _vp, _p(ctypes.c_double), _vp, _vp, _vp]),
+    "sc_prior_mask": (ctypes.c_int, [_vp, _vp, _p(_c_i32), ctypes.c_int, _vp, _vp]),
     "sc_gather_patches": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, ctypes.c_int, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp]),
     "sc_gather_center_labels": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _c_i64, _vp, _vp]),
     "sc_gather_samples": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -108,6 +116,11 @@ def _check(status):
 
 def _dims(shape):
     return (_c_i32 * 3)(*[int(s) for s in shape[:3]])
+
+
+def _mat(m):
+    """4x4 matrix -> row-major double[16]"""
+    return (ctypes.c_double * 16)(*[float(v) for v in np.asarray(m, np.float64).reshape(16)])
 
 
 def _ptr(t):
@@ -283,6 +296,57 @@ class Context(object):
         _check(self.lib.sc_evaluate_segmentation(self.h, _ptr(seg), _ptr(ref), _dims(seg.shape), sp, out.ctypes.data,
                                                  None if conf is None else conf.ctypes.data, _stream()))
         return out, conf
+
+    # -- atlas registration (include/subcort_b200.h) -----------------------------------------------
+    def ffd_grid_dims(self, ref_shape):
+        g = (_c_i32 * 3)()
+        _check(self.lib.sc_ffd_grid_dims(_dims(ref_shape), g))
+        return tuple(int(v) for v in g)
+
+    def register_affine(self, ref, ref_vox2mm, flo, flo_vox2mm):
+        """float32 CUDA volumes: subject T1 (reference) and template T1 (floating), 4x4 voxel -> mm matrices -> the 4x4
+        affine (subject mm -> template mm) as a numpy array.  Synchronises (sc_register_affine)."""
+        out = (ctypes.c_double * 16)()
+        _check(self.lib.sc_register_affine(self.h, _ptr(ref), _dims(ref.shape), _mat(ref_vox2mm), _ptr(flo), _dims(flo.shape),
+                                           _mat(flo_vox2mm), out, _stream()))
+        return np.array(out[:], np.float64).reshape(4, 4)
+
+    def register_ffd(self, ref, ref_vox2mm, flo, flo_vox2mm, affine):
+        """-> float32 CUDA control-point grid [gx, gy, gz, 3] (template mm) refining `affine` (sc_register_ffd)"""
+        import torch
+        grid = torch.empty(self.ffd_grid_dims(ref.shape) + (3,), dtype=torch.float32, device=ref.device)
+        _check(self.lib.sc_register_ffd(self.h, _ptr(ref), _dims(ref.shape), _mat(ref_vox2mm), _ptr(flo), _dims(flo.shape),
+                                        _mat(flo_vox2mm), _mat(affine), _ptr(grid), _stream()))
+        return grid
+
+    def warp_volume(self, flo, flo_vox2mm, affine, grid, ref_shape, ref_vox2mm, out=None):
+        """float32 CUDA volume [X,Y,Z] or [X,Y,Z,15] on the template grid -> the same on the subject grid through phi
+        (grid None: affine only), 0 outside (sc_warp_volume)"""
+        import torch
+        ch = 15 if flo.dim() == 4 else 1
+        shape = tuple(int(s) for s in ref_shape[:3]) + ((15,) if ch == 15 else ())
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=flo.device)
+        _check(self.lib.sc_warp_volume(self.h, _ptr(flo), _dims(flo.shape), ch, _mat(flo_vox2mm), _mat(affine), _ptr(grid),
+                                       _dims(shape), _mat(ref_vox2mm), _ptr(out), _stream()))
+        return out
+
+    def register_objective(self, ref, ref_vox2mm, flo, flo_vox2mm, affine, grid=None, want_grad=False):
+        """-> (NMI, BE, J, d NMI / d A [3, 4] or None, d J / d grid CUDA tensor or None) at full resolution"""
+        import torch
+        val = (ctypes.c_double * 3)()
+        ga = (ctypes.c_double * 12)() if want_grad else None
+        gg = torch.empty_like(grid) if want_grad and grid is not None else None
+        _check(self.lib.sc_register_objective(self.h, _ptr(ref), _dims(ref.shape), _mat(ref_vox2mm), _ptr(flo), _dims(flo.shape),
+                                              _mat(flo_vox2mm), _mat(affine), _ptr(grid), val, ga, _ptr(gg), _stream()))
+        return val[0], val[1], val[2], (np.array(ga[:]).reshape(3, 4) if want_grad else None), gg
+
+    def prior_mask(self, priors, iterations=5):
+        """float32 CUDA priors [X,Y,Z,15] -> float32 0/1 mask: channels 0..12 summing to > 0, dilated (sc_prior_mask)"""
+        import torch
+        out = torch.empty(tuple(priors.shape[:3]), dtype=torch.float32, device=priors.device)
+        _check(self.lib.sc_prior_mask(self.h, _ptr(priors), _dims(priors.shape), int(iterations), _ptr(out), _stream()))
+        return out
 
     def gather_patches(self, vol, xyz, atlas=None, bg_fix=True, views=(True, True, True)):
         import torch

@@ -9,8 +9,9 @@ exactly where the reference has them (outside the timed path).
 
 Deliberate deviations from reference quirks (SURVEY.md 5.6): Q1 prediction is not gated
 by ``debug``; Q2 ``speedup_segmentation`` is parsed as a boolean; Q10 one forward pass
-serves both labels and probabilities; registration (``register_masks``) is not rebuilt --
-the ``tmp/MNI_*`` files must exist.
+serves both labels and probabilities.  Registration (``register_masks``) runs on the device
+(affine + B-spline NMI registration instead of niftyreg's binaries) when the configuration names a
+template (``atlas_template`` / ``atlas_priors``); without one the ``tmp/MNI_*`` files must exist.
 """
 import os
 import random
@@ -110,6 +111,7 @@ def load_patch_batch(scan_name, options, datatype=np.float32):
     import torch
     ctx = get_context(options.get('device'))
     dir_name, name = os.path.split(scan_name)
+    _ensure_registered(scan_name, options)
     image = load_nii(scan_name).get_data()
     atlas_name = os.path.join(dir_name, 'tmp', 'MNI_sub_probabilities.nii.gz')
     _require_registered(atlas_name)
@@ -166,6 +168,20 @@ def _require_registered(atlas_name):
                       "implementation's scope -- create the tmp/MNI_* files with the reference pipeline" % atlas_name)
 
 
+_REGISTERED = ('MNI_sub_probabilities.nii.gz', 'MNI_subcortical_mask.nii.gz')
+
+
+def _ensure_registered(t1_path, options):
+    """register_masks for a subject whose tmp/MNI_* files are missing, when the configuration names a template; -> the
+    device-resident (priors, mask) it produced, or None (files present, or no template: the callers then raise)"""
+    tmp = os.path.join(os.path.dirname(t1_path), 'tmp')
+    if all(os.path.exists(os.path.join(tmp, n)) for n in _REGISTERED):
+        return None
+    if not (options.get('atlas_template') and options.get('atlas_priors')):
+        return None
+    return register_masks(t1_path, options)
+
+
 # ---------------------------------------------------------------------------------------------
 # inference
 # ---------------------------------------------------------------------------------------------
@@ -197,16 +213,22 @@ def test_scan(net, test_scan, options):
             else:
                 image[x, y, z] = net.predict(X)
     else:
-        atlas_name = os.path.join(image_path, 'tmp', 'MNI_sub_probabilities.nii.gz')
-        _require_registered(atlas_name)
-        atlas = nib.load(atlas_name, pinned=True).get_data()
-        crop_mask = None
-        if _crop_enabled(options):
-            crop_mask = nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
         timings = options.get('timings')
-        post_mask = None
-        if options['post_process'] == 'True':      # filtered on the device, before the label volume is downloaded
-            post_mask = crop_mask if crop_mask is not None else nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
+        registered = _ensure_registered(test_scan, options)
+        if registered is not None:                 # the priors and mask just registered stay on the device
+            atlas, mask = registered
+            crop_mask = mask if _crop_enabled(options) else None
+            post_mask = mask if options['post_process'] == 'True' else None
+        else:
+            atlas_name = os.path.join(image_path, 'tmp', 'MNI_sub_probabilities.nii.gz')
+            _require_registered(atlas_name)
+            atlas = nib.load(atlas_name, pinned=True).get_data()
+            crop_mask = None
+            if _crop_enabled(options):
+                crop_mask = nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
+            post_mask = None
+            if options['post_process'] == 'True':      # filtered on the device, before the label volume is downloaded
+                post_mask = crop_mask if crop_mask is not None else nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
         labels, image_proba, n_cand = segment_arrays(net.ctx, t1, atlas, crop_mask, want_proba, timings, post_mask=post_mask)
         if options['debug'] == 'True':
             print("    -->  num of samples to test:", n_cand)
@@ -228,19 +250,31 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
     number of candidates) out.  One upload per array (Fortran-ordered NIfTI arrays are reordered on the device), then
     normalisation over the non-zero voxels (numpy's result bit for bit), candidate mask (non-zero T1 voxels, or the
     registered mask dilated 10 times), its bounding box, the dense network pass and the scatter, all without the mask,
-    the normalised volume or the coordinates ever visiting the host; one download of the result."""
+    the normalised volume or the coordinates ever visiting the host; one download of the result.  atlas / crop_mask /
+    post_mask may also be CUDA tensors (float32 [X,Y,Z,15] C-ordered priors, [X,Y,Z] masks: what register_masks returns):
+    they are used in place."""
     import torch
     t0 = time.time()
     shape = tuple(int(s) for s in t1.shape[:3])
-    atlas = np.asarray(atlas)
-    if atlas.dtype != np.float32:          # a scaled NIfTI comes back as float64: the priors are consumed as float32 (base.py:388)
-        atlas = atlas.astype(np.float32, order='K')
+    on_device = torch.is_tensor(atlas)
+    if not on_device:
+        atlas = np.asarray(atlas)
+        if atlas.dtype != np.float32:      # a scaled NIfTI comes back as float64: the priors are consumed as float32 (base.py:388)
+            atlas = atlas.astype(np.float32, order='K')
     main = torch.cuda.current_stream()
     side = _side_stream(ctx.device)
     atlas_ready = torch.cuda.Event()
     d_atlas = None
 
+    def device_bytes(a):
+        """(C-ordered raw bytes on the device, dtype) of a host volume or a CUDA tensor"""
+        if torch.is_tensor(a):
+            return a.contiguous().view(-1).view(torch.uint8), np.dtype(str(a.dtype).replace('torch.', ''))
+        return ctx.upload_volume(a)
+
     def start_atlas_upload(box):
+        if on_device:
+            return atlas
         # The priors (94 % of the upload) are first needed by the FC head: they are uploaded and reordered on a side stream while
         # the convolution phase runs -- enqueued behind the host-synchronous steps that precede it, whose small device -> host
         # copies would otherwise queue up behind the gigabyte.  Crop mode reads the priors at the candidates only: just the
@@ -259,7 +293,7 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
     raw, dt = ctx.upload_volume(t1)
     vol, mean, std = ctx.normalise_volume(raw, dt, shape)
     if crop_mask is not None:
-        mraw, mdt = ctx.upload_volume(crop_mask)
+        mraw, mdt = device_bytes(crop_mask)
         cand = ctx.dilate_mask(ctx.candidate_mask(mraw, mdt, shape), 10)   # == ndimage.binary_dilation(mask, iterations=10)
     else:
         cand = ctx.candidate_mask(raw, dt, shape)                          # == image.astype('bool')
@@ -269,13 +303,14 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
     lab = torch.zeros(shape, dtype=torch.uint8, device=vol.device)
     prob = torch.zeros(shape + (15,), dtype=torch.float32, device=vol.device) if want_proba else None
     if box is not None:
-        ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob, atlas_ready=atlas_ready)
+        ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob,
+                           atlas_ready=None if on_device else atlas_ready)
     main.wait_stream(side)
     if post_mask is not None:        # post_process_segmentation (base.py:460-480) on the device-resident label volume
         if post_mask is crop_mask and crop_mask is not None:
             pm = ctx.candidate_mask(mraw, mdt, shape)
         else:
-            praw, pdt = ctx.upload_volume(post_mask)
+            praw, pdt = device_bytes(post_mask)
             pm = ctx.candidate_mask(praw, pdt, shape)
         lab = ctx.post_process(lab, pm)
     h_lab = _pinned_out('lab', shape, torch.uint8)
@@ -398,9 +433,71 @@ def evaluate_scan(seg_path, ref_path, device=None):
     return evaluate_segmentation(seg_nii.get_data(), ref_nii.get_data(), spacing, device=device)
 
 
-def register_masks(input_mask):
-    raise NotImplementedError("atlas registration (niftyreg reg_aladin / reg_f3d / reg_resample, base.py:483-551) "
-                              "stays with the reference pipeline; it is outside the hot path rebuilt here")
+# ---------------------------------------------------------------------------------------------
+# atlas registration
+# ---------------------------------------------------------------------------------------------
+def _cuda_f32(a, device):
+    import torch
+    if torch.is_tensor(a):
+        return a.to('cuda:%d' % device, torch.float32).contiguous()
+    return _dev(np.ascontiguousarray(a, dtype=np.float32), device)
+
+
+def register_arrays(ctx, t1, t1_affine, template, template_affine, priors):
+    """Map a template and its priors onto a subject on the device: affine then B-spline FFD registration of the template
+    T1 to the subject T1 (NMI; sc_register_affine / sc_register_ffd), the priors warped through the result
+    (sc_warp_volume) and the sub-cortical mask (sc_prior_mask: channels 0..12 summing to > 0, dilated 5 times).
+    t1 / template: [X,Y,Z] volumes (host arrays or tensors; zeros in t1 are outside the subject), priors [X,Y,Z,15] on the
+    template's grid, *_affine: 4x4 voxel -> mm.  -> CUDA tensors (affine float64 [4,4] subject mm -> template mm, grid
+    float32 [gx,gy,gz,3], priors float32 [X,Y,Z,15] on the subject's grid, mask float32 0/1 [X,Y,Z])."""
+    import torch
+    ref, flo = _cuda_f32(t1, ctx.device), _cuda_f32(template, ctx.device)
+    A = ctx.register_affine(ref, t1_affine, flo, template_affine)
+    grid = ctx.register_ffd(ref, t1_affine, flo, template_affine, A)
+    warped = ctx.warp_volume(_cuda_f32(priors, ctx.device), template_affine, A, grid, ref.shape, t1_affine)
+    mask = ctx.prior_mask(warped, 5)
+    return torch.from_numpy(A).to(ref.device), grid, warped, mask
+
+
+def register_masks(t1_path, options, timings=None):
+    """Register the configured template (options['atlas_template'], options['atlas_priors']) to the subject
+    <subject>/<t1> and write what the reference's niftyreg calls leave in <subject>/tmp/ (base.py:483-551), with the
+    subject's affine: transf.txt (4x4, subject mm -> template mm, the direction reg_aladin -aff writes),
+    rT1d_template.nii.gz (the warped template T1), MNI_sub_probabilities.nii.gz ([X,Y,Z,15] priors) and
+    MNI_subcortical_mask.nii.gz (float32 0/1).  Files that already exist are kept.  -> the device-resident
+    (priors, mask) CUDA tensors.  timings (dict, optional) receives register_s and write_s."""
+    template_path, priors_path = options.get('atlas_template'), options.get('atlas_priors')
+    if not (template_path and priors_path):
+        raise IOError("register_masks needs atlas_template and atlas_priors in the [database] section of the configuration")
+    t0 = time.time()
+    tmp = os.path.join(os.path.dirname(t1_path), 'tmp')
+    os.makedirs(tmp, exist_ok=True)
+    ctx = get_context(options.get('device'))
+    t1_nii, tpl_nii, pri_nii = load_nii(t1_path), load_nii(template_path), load_nii(priors_path)
+    if tuple(pri_nii.shape) != tuple(tpl_nii.shape[:3]) + (15,):
+        raise ValueError("%s: priors of shape %s do not match the template %s (expected [X,Y,Z,15])" % (
+            priors_path, tuple(pri_nii.shape), tuple(tpl_nii.shape)))
+    A, grid, priors, mask = register_arrays(ctx, t1_nii.get_data(), t1_nii.affine, tpl_nii.get_data(), tpl_nii.affine,
+                                            pri_nii.get_data())
+    import torch
+    torch.cuda.current_stream().synchronize()
+    t1_s = time.time()
+    aff = t1_nii.affine
+    out = {'transf.txt': None, 'rT1d_template.nii.gz': None, 'MNI_sub_probabilities.nii.gz': priors, 'MNI_subcortical_mask.nii.gz': mask}
+    for name, data in out.items():
+        path = os.path.join(tmp, name)
+        if os.path.exists(path):
+            continue
+        if name == 'transf.txt':
+            np.savetxt(path, A.cpu().numpy())
+        elif name == 'rT1d_template.nii.gz':
+            warped = ctx.warp_volume(_cuda_f32(tpl_nii.get_data(), ctx.device), tpl_nii.affine, A.cpu().numpy(), grid, priors.shape, aff)
+            nib.Nifti1Image(warped.cpu().numpy(), affine=aff).to_filename(path)
+        else:
+            nib.Nifti1Image(data.cpu().numpy(), affine=aff).to_filename(path)
+    if timings is not None:
+        timings.update({'register_s': t1_s - t0, 'write_s': time.time() - t1_s})
+    return priors, mask
 
 
 # ---------------------------------------------------------------------------------------------
@@ -409,10 +506,17 @@ def register_masks(input_mask):
 def load_data(options):
     """-> (x_axial, x_cor, x_sag, y_axial, x_atlas, names), lists indexed by subject.
     [base.py:11-37]"""
+    _register_folder(options['train_folder'], options)
     (x_axial, y_axial, x_cor, y_cor, x_sag, y_sag, x_atlas, names) = load_patches(
         dir_name=options['train_folder'], t1_name=options['t1_name'], mask_name=options['roi_name'],
         size=tuple(options['patch_size']), device=options.get('device'))
     return x_axial, x_cor, x_sag, y_axial, x_atlas, names
+
+
+def _register_folder(dir_name, options):
+    for subject in sorted(os.listdir(dir_name)):
+        if os.path.isdir(os.path.join(dir_name, subject)):
+            _ensure_registered(os.path.join(dir_name, subject, options['t1_name']), options)
 
 
 def load_patches(dir_name, mask_name, t1_name, size, seeds=None, balance_neg=True, device=None):
@@ -631,6 +735,7 @@ def load_scan_training_set(options, randomize=True, device=None):
         raise ValueError("only patch_size (32, 32) is implemented")
     ctx = get_context(options.get('device') if device is None else device)
     dir_name = options['train_folder']
+    _register_folder(dir_name, options)
     subjects = [f for f in sorted(os.listdir(dir_name)) if os.path.isdir(os.path.join(dir_name, f))]
     names, vols, samples, atlas_rows, labels = [], [], [], [], []
     for k, subject in enumerate(subjects):

@@ -48,6 +48,11 @@ def load_options(user_config):
     options['crop'] = g('model', 'speedup_segmentation').strip()
     options['crop_bool'] = _truthy(options['crop'])
     options['device'] = device_index(options['mode'])
+    # optional: the template T1 and its [X,Y,Z,15] priors (on the template's grid) that register_masks maps onto subjects
+    # whose tmp/ files are missing; without them such subjects are an error, as before
+    for key in ('atlas_template', 'atlas_priors'):
+        v = g('database', key, fallback='').strip()
+        options[key] = v or None
     return options
 
 

@@ -141,7 +141,7 @@ int sc_destroy(sc_ctx* ctx) {
   tc_destroy(ctx);
   fused_detach(ctx);
   cudaFree(ctx->params); cudaFree(ctx->grads); cudaFree(ctx->adam_m); cudaFree(ctx->adam_v);
-  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr); cudaFree(ctx->ws_eval.ptr);
+  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr); cudaFree(ctx->ws_eval.ptr); cudaFree(ctx->ws_reg.ptr);
   for (auto& g : ctx->train_graphs) cudaGraphExecDestroy(g.exec);
   for (int i = 0; i < 2; ++i) if (ctx->train_side[i]) cudaStreamDestroy(ctx->train_side[i]);
   for (int i = 0; i < 8; ++i) if (ctx->train_ev[i]) cudaEventDestroy(ctx->train_ev[i]);
@@ -150,6 +150,7 @@ int sc_destroy(sc_ctx* ctx) {
   for (auto& ev : ctx->prof_free) { cudaEventDestroy(ev.a); cudaEventDestroy(ev.b); }
   if (ctx->h_slab_cnt) { cudaFreeHost(ctx->h_slab_cnt); cudaEventDestroy(ctx->compact_ev); }
   cudaFree(ctx->tile_flags);
+  if (ctx->h_reg) cudaFreeHost(ctx->h_reg);
   for (int i = 0; i < 64; ++i) if (ctx->atlas_chunk_ev[i]) cudaEventDestroy(ctx->atlas_chunk_ev[i]);
   if (ctx->copy_stream) { cudaStreamDestroy(ctx->copy_stream); cudaEventDestroy(ctx->copy_ev[0]); cudaEventDestroy(ctx->copy_ev[1]); }
   delete ctx;
@@ -218,6 +219,10 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
     cudaMemcpy(&v, ctx->tc_timing_buf + i, sizeof(v), cudaMemcpyDeviceToHost);
     return (int64_t)v;
   }
+  if (!strncmp(key, "reg_iters:", 10)) {   // accepted steps per level of the last registration: 0..3 affine, 4..6 FFD
+    const int i = atoi(key + 10);
+    return i >= 0 && i < 8 ? ctx->reg_iters[i] : -1;
+  }
   if (!strcmp(key, "launches")) return ctx->launches;
   if (!strcmp(key, "gemm")) return ctx->gemm_backend;
   if (!strcmp(key, "adam_t")) return ctx->adam_t;
@@ -227,7 +232,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam", "evaluate"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate", "register"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -344,6 +349,97 @@ int sc_evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg_dev, const uint8_t*
              i, spacing[i]);
   SC_CUDA(cudaSetDevice(ctx->device));
   return evaluate_segmentation(ctx, seg_dev, ref_dev, dims, spacing, metrics_host, confusion_host, (cudaStream_t)stream);
+}
+
+// registration arguments: a volume of dims >= 8 and a finite, non-singular voxel -> mm matrix
+static int check_reg_volume(const void* dev, const int32_t* dims, const char* who, const char* name) {
+  SC_CHECK(dev != nullptr, SC_ERR_ARG, "%s: %s is NULL", who, name);
+  SC_CHECK(dims != nullptr, SC_ERR_ARG, "%s: %s dims are NULL", who, name);
+  for (int i = 0; i < 3; ++i)
+    SC_CHECK(dims[i] >= 8, SC_ERR_ARG, "%s: %s dims[%d] = %d is below 8", who, name, i, dims[i]);
+  SC_CHECK((int64_t)dims[0] * dims[1] * dims[2] < (1ll << 31), SC_ERR_ARG, "%s: %s volume too large", who, name);
+  return SC_OK;
+}
+static int check_matrix(const double* m, const char* who, const char* name) {
+  SC_CHECK(m != nullptr, SC_ERR_ARG, "%s: %s is NULL", who, name);
+  for (int i = 0; i < 16; ++i) SC_CHECK(isfinite(m[i]), SC_ERR_ARG, "%s: %s[%d] is not finite", who, name, i);
+  const double det = m[0] * (m[5] * m[10] - m[6] * m[9]) - m[1] * (m[4] * m[10] - m[6] * m[8]) + m[2] * (m[4] * m[9] - m[5] * m[8]);
+  SC_CHECK(fabs(det) > 1e-12, SC_ERR_ARG, "%s: %s is singular", who, name);
+  return SC_OK;
+}
+
+int sc_ffd_grid_dims(const int32_t ref_dims[3], int32_t grid_dims_out[3]) {
+  SC_CHECK(ref_dims && grid_dims_out, SC_ERR_ARG, "sc_ffd_grid_dims: null argument");
+  for (int i = 0; i < 3; ++i) SC_CHECK(ref_dims[i] >= 8, SC_ERR_ARG, "sc_ffd_grid_dims: ref_dims[%d] = %d is below 8", i, ref_dims[i]);
+  ffd_grid_dims(ref_dims, grid_dims_out);
+  return SC_OK;
+}
+
+int sc_register_affine(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16], const float* flo_dev,
+                       const int32_t flo_dims[3], const double flo_vox2mm[16], double affine_out[16], void* stream) {
+  const char* who = "sc_register_affine";
+  SC_CHECK(ctx && affine_out, SC_ERR_ARG, "%s: null context or affine_out", who);
+  SC_TRY(check_reg_volume(ref_dev, ref_dims, who, "ref_dev"));
+  SC_TRY(check_reg_volume(flo_dev, flo_dims, who, "flo_dev"));
+  SC_TRY(check_matrix(ref_vox2mm, who, "ref_vox2mm"));
+  SC_TRY(check_matrix(flo_vox2mm, who, "flo_vox2mm"));
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return register_affine(ctx, ref_dev, ref_dims, ref_vox2mm, flo_dev, flo_dims, flo_vox2mm, affine_out, (cudaStream_t)stream);
+}
+
+int sc_register_ffd(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16], const float* flo_dev,
+                    const int32_t flo_dims[3], const double flo_vox2mm[16], const double affine[16], float* grid_dev, void* stream) {
+  const char* who = "sc_register_ffd";
+  SC_CHECK(ctx && grid_dev, SC_ERR_ARG, "%s: null context or grid_dev", who);
+  SC_TRY(check_reg_volume(ref_dev, ref_dims, who, "ref_dev"));
+  SC_TRY(check_reg_volume(flo_dev, flo_dims, who, "flo_dev"));
+  SC_TRY(check_matrix(ref_vox2mm, who, "ref_vox2mm"));
+  SC_TRY(check_matrix(flo_vox2mm, who, "flo_vox2mm"));
+  SC_TRY(check_matrix(affine, who, "affine"));
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return register_ffd(ctx, ref_dev, ref_dims, ref_vox2mm, flo_dev, flo_dims, flo_vox2mm, affine, grid_dev, (cudaStream_t)stream);
+}
+
+int sc_warp_volume(sc_ctx* ctx, const float* flo_dev, const int32_t flo_dims[3], int channels, const double flo_vox2mm[16],
+                   const double affine[16], const float* grid_dev, const int32_t ref_dims[3], const double ref_vox2mm[16], float* out_dev,
+                   void* stream) {
+  const char* who = "sc_warp_volume";
+  SC_CHECK(ctx && out_dev, SC_ERR_ARG, "%s: null context or out_dev", who);
+  SC_CHECK(channels == 1 || channels == 15, SC_ERR_ARG, "%s: channels = %d (1 or 15)", who, channels);
+  SC_TRY(check_reg_volume(flo_dev, flo_dims, who, "flo_dev"));
+  SC_TRY(check_reg_volume(out_dev, ref_dims, who, "out_dev"));
+  SC_TRY(check_matrix(flo_vox2mm, who, "flo_vox2mm"));
+  SC_TRY(check_matrix(ref_vox2mm, who, "ref_vox2mm"));
+  SC_TRY(check_matrix(affine, who, "affine"));
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return warp_volume(ctx, flo_dev, flo_dims, channels, flo_vox2mm, affine, grid_dev, ref_dims, ref_vox2mm, out_dev, (cudaStream_t)stream);
+}
+
+int sc_register_objective(sc_ctx* ctx, const float* ref_dev, const int32_t ref_dims[3], const double ref_vox2mm[16], const float* flo_dev,
+                          const int32_t flo_dims[3], const double flo_vox2mm[16], const double affine[16], const float* grid_dev,
+                          double value_out[3], double* affine_grad_host, float* grid_grad_dev, void* stream) {
+  const char* who = "sc_register_objective";
+  SC_CHECK(ctx && value_out, SC_ERR_ARG, "%s: null context or value_out", who);
+  SC_CHECK(grid_dev || !grid_grad_dev, SC_ERR_ARG, "%s: grid_grad_dev needs grid_dev", who);
+  SC_TRY(check_reg_volume(ref_dev, ref_dims, who, "ref_dev"));
+  SC_TRY(check_reg_volume(flo_dev, flo_dims, who, "flo_dev"));
+  SC_TRY(check_matrix(ref_vox2mm, who, "ref_vox2mm"));
+  SC_TRY(check_matrix(flo_vox2mm, who, "flo_vox2mm"));
+  SC_TRY(check_matrix(affine, who, "affine"));
+  SC_CUDA(cudaSetDevice(ctx->device));
+  double ga[12];
+  SC_TRY(register_objective(ctx, ref_dev, ref_dims, ref_vox2mm, flo_dev, flo_dims, flo_vox2mm, affine, grid_dev, value_out,
+                            affine_grad_host ? ga : nullptr, grid_grad_dev, (cudaStream_t)stream));
+  if (affine_grad_host) memcpy(affine_grad_host, ga, sizeof(ga));   // uncentred: the objective's sums use c = 0
+  return SC_OK;
+}
+
+int sc_prior_mask(sc_ctx* ctx, const float* priors_dev, const int32_t dims[3], int iterations, float* mask_dev, void* stream) {
+  SC_CHECK(ctx && priors_dev && mask_dev, SC_ERR_ARG, "sc_prior_mask: null argument");
+  SC_CHECK(iterations >= 0, SC_ERR_ARG, "sc_prior_mask: iterations = %d is negative", iterations);
+  SC_TRY(check_dims(dims, "sc_prior_mask"));
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return prior_mask(ctx, priors_dev, dims, iterations, mask_dev, (cudaStream_t)stream);
 }
 
 int sc_gather_patches(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], const float* atlas_dev, int bg_fix,

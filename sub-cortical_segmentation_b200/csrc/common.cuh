@@ -148,7 +148,7 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_COUNT
 };
 struct ProfEvent { int cls; cudaEvent_t a, b; };
 
@@ -178,6 +178,9 @@ struct sc_ctx {
   sc::Workspace ws_train;        // staging of the host entry points, scan preparation, eval scratch
   sc::Workspace ws_fit;          // training step: staged inputs, saved activations, gradients of activations
   sc::Workspace ws_eval;         // sc_evaluate_segmentation: distance fields, envelope stacks and distance lists of one class box
+  sc::Workspace ws_reg;          // registration: pyramids, histogram, adjoint passes, control-point grids
+  double* h_reg = nullptr;       // pinned: the optimiser's per-trial read-backs
+  int reg_iters[8] = {};         // accepted steps of the last registration per level: affine 0..3, FFD 4..6
   // training step as a CUDA graph (one per (batch, global batch, injected masks) shape): the three branches run on
   // three captured streams; rebuilt when the arena moves
   struct TrainGraph { int n; long long n_global; int injected; int backend; void* arena; cudaGraphExec_t exec; int launches; };
@@ -291,6 +294,19 @@ int post_process(sc_ctx* ctx, const uint8_t* seg, const uint8_t* mask, const int
 // evaluate.cu : per-structure Dice, volumes and surface distances of a label volume against a reference
 int evaluate_segmentation(sc_ctx* ctx, const uint8_t* seg, const uint8_t* ref, const int32_t* dims, const double* spacing,
                           sc_structure_metrics* metrics, int64_t* confusion, cudaStream_t st);
+
+// register.cu : affine + B-spline FFD registration of the template to the subject (NMI), warps and the prior mask
+void ffd_grid_dims(const int32_t* ref_dims, int32_t* grid_dims);
+int register_affine(sc_ctx* ctx, const float* ref, const int32_t* rdims, const double* rv, const float* flo, const int32_t* fdims,
+                    const double* fv, double* affine_out, cudaStream_t st);
+int register_ffd(sc_ctx* ctx, const float* ref, const int32_t* rdims, const double* rv, const float* flo, const int32_t* fdims,
+                 const double* fv, const double* affine, float* grid_out, cudaStream_t st);
+int register_objective(sc_ctx* ctx, const float* ref, const int32_t* rdims, const double* rv, const float* flo, const int32_t* fdims,
+                       const double* fv, const double* affine, const float* grid, double* value, double* agrad, float* ggrad,
+                       cudaStream_t st);
+int warp_volume(sc_ctx* ctx, const float* flo, const int32_t* fdims, int channels, const double* fv, const double* affine, const float* grid,
+                const int32_t* rdims, const double* rv, float* out, cudaStream_t st);
+int prior_mask(sc_ctx* ctx, const float* priors, const int32_t* dims, int iterations, float* out, cudaStream_t st);
 
 // weights.cu
 int derive_weights(sc_ctx* ctx, cudaStream_t st);
