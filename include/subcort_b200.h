@@ -192,6 +192,23 @@ SC_API int sc_segment_volume(sc_ctx* ctx, const float* vol_dev, const int32_t di
  * cudaEvent_t recorded behind that upload here; the NEXT sc_segment_volume call makes its stream wait for the event right
  * before the FC head instead of the caller serialising upload and convolutions.  One-shot (cleared by that call). */
 SC_API int sc_atlas_ready_event(sc_ctx* ctx, void* cuda_event);
+/* Monte-Carlo dropout (Gal & Ghahramani 2016) over the same computation: `samples` (T) stochastic passes of the FC head
+ * with the dropout of training (p = 0.5, kept units x2) at *_l1drop, f1_drop and f2_drop; the convolutions run once.
+ * Pass t (0 <= t < T) keeps unit j of [3][540] l1drop (k = c*9 + h*3 + w) | [540] f1_drop | [540] f2_drop when
+ * hash3(seed, t * 2700 + j) & 1 (the training step's mask of sample t, csrc/common.cuh), ONE mask for every voxel; that
+ * is the deterministic head with the weight rows of the dropped inputs zeroed and the kept ones doubled.  Per voxel,
+ * with p_t the softmax of pass t (atlas background fix as above):
+ *   proba_vol   p = (1/T) sum_t p_t, float32 [X][Y][Z][15];   label_vol  the first arg-max of p, uint8 [X][Y][Z];
+ *   entropy_vol H = -sum_c p_c ln p_c in nats (0 ln 0 = 0), float32 [X][Y][Z];
+ *   mi_vol      max(0, H - (1/T) sum_t H(p_t)), the mutual information between prediction and weights (exactly 0 for T = 1).
+ * Outputs are written exactly where sc_segment_volume writes (the candidates inside the box); any may be NULL, not all.
+ * Deterministic: the same inputs and seed give byte-identical outputs.  sc_atlas_ready_event applies as above.
+ * SC_ERR_ARG, outputs untouched: samples outside [1, 1024], the SIMT back-end selected ("gemm" = 0), NULL inputs or
+ * all outputs NULL, bad dims, a box outside the volume.  The message names the argument. */
+SC_API int sc_segment_volume_mc(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], const float* atlas_dev,
+                                const int32_t* box, const uint8_t* cand_mask_dev, int samples, uint64_t seed,
+                                uint8_t* label_vol_dev, float* proba_vol_dev, float* entropy_vol_dev, float* mi_vol_dev,
+                                void* stream);
 /* host-buffer form: copies volume + atlas (+mask) in and the label (+proba) volume out. */
 SC_API int sc_segment_volume_host(sc_ctx* ctx, const float* vol_host, const int32_t dims[3],
                            const float* atlas_host, const int32_t* box, const uint8_t* cand_mask_host,

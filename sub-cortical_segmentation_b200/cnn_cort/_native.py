@@ -76,6 +76,8 @@ PROTOTYPES = {
     "sc_dense_layer": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _c_i64, _vp, ctypes.c_int, _vp]),
     "sc_forward_from_volume": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _vp, _c_i64, _vp, _vp, _vp]),
     "sc_segment_volume": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _p(_c_i32), _vp, _vp, _vp, _vp]),
+    "sc_segment_volume_mc": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _p(_c_i32), _vp, ctypes.c_int, ctypes.c_uint64, _vp, _vp,
+                                            _vp, _vp, _vp]),
     "sc_atlas_ready_event": (ctypes.c_int, [_vp, _vp]),
     "sc_segment_volume_host": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _p(_c_i32), _vp, _vp, _vp, _vp]),
     "sc_scatter": (ctypes.c_int, [_vp, _vp, _c_i64, _vp, _vp, _p(_c_i32), _vp, _vp, _vp]),
@@ -431,6 +433,17 @@ class Context(object):
             _check(self.lib.sc_atlas_ready_event(self.h, atlas_ready.cuda_event))
         _check(self.lib.sc_segment_volume(self.h, _ptr(vol), _dims(vol.shape), _ptr(atlas), cbox, _ptr(cand_mask),
                                           _ptr(label_vol), _ptr(proba_vol), _stream()))
+
+    def segment_volume_mc(self, vol, atlas, samples, seed=0, box=None, cand_mask=None, label_vol=None, proba_vol=None,
+                          entropy_vol=None, mi_vol=None, atlas_ready=None):
+        """Monte-Carlo dropout over segment_volume (sc_segment_volume_mc): `samples` passes of the FC head with the training
+        dropout masks drawn from `seed`; writes the arg-max and the mean of the passes' softmax, its entropy (nats) and the
+        mutual information into whichever of the four CUDA volumes are given, at the voxels segment_volume writes."""
+        cbox = (_c_i32 * 6)(*[int(b) for b in box]) if box is not None else None
+        if atlas_ready is not None:
+            _check(self.lib.sc_atlas_ready_event(self.h, atlas_ready.cuda_event))
+        _check(self.lib.sc_segment_volume_mc(self.h, _ptr(vol), _dims(vol.shape), _ptr(atlas), cbox, _ptr(cand_mask), int(samples),
+                                             int(seed), _ptr(label_vol), _ptr(proba_vol), _ptr(entropy_vol), _ptr(mi_vol), _stream()))
 
     def segment_volume_host(self, vol, atlas, box=None, cand_mask=None, want_proba=False, label_out=None):
         """numpy (or pinned torch CPU) in -> numpy uint8 label volume (+ float32 proba volume)."""

@@ -200,7 +200,11 @@ def test_scan(net, test_scan, options):
     t1_nii = nib.load(test_scan, pinned=(mode != 'patchwise'))
     t1 = t1_nii.get_data()
     want_proba = options['out_probabilities'] == 'True'
+    mc_samples = int(options.get('mc_samples', 0) or 0)
+    mc = {'samples': mc_samples, 'seed': int(options.get('mc_seed', 0) or 0)} if mc_samples > 0 else None
     if mode == 'patchwise':
+        if mc is not None:
+            raise ValueError("mc_samples = %d: Monte-Carlo dropout is implemented for the dense inference mode only" % mc_samples)
         image = np.zeros_like(t1)
         image_proba = np.zeros(t1_nii.shape + (15,)) if want_proba else None
         for batch_axial, batch_cor, batch_sag, atlas, centers in load_patch_batch(test_scan, options):
@@ -229,13 +233,16 @@ def test_scan(net, test_scan, options):
             post_mask = None
             if options['post_process'] == 'True':      # filtered on the device, before the label volume is downloaded
                 post_mask = crop_mask if crop_mask is not None else nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
-        labels, image_proba, n_cand = segment_arrays(net.ctx, t1, atlas, crop_mask, want_proba, timings, post_mask=post_mask)
+        labels, image_proba, n_cand = segment_arrays(net.ctx, t1, atlas, crop_mask, want_proba, timings, post_mask=post_mask, mc=mc)
         if options['debug'] == 'True':
             print("    -->  num of samples to test:", n_cand)
         image = labels.astype(t1.dtype)
 
     if want_proba:
         nib.Nifti1Image(image_proba, affine=t1_nii.affine).to_filename(os.path.join(image_path, 'out_subcortical_prob.nii.gz'))
+    if mc is not None:
+        for key, fname in (('entropy', 'out_subcortical_entropy.nii.gz'), ('mutual_info', 'out_subcortical_mi.nii.gz')):
+            nib.Nifti1Image(mc[key], affine=t1_nii.affine).to_filename(os.path.join(image_path, fname))
     if options['post_process'] == 'True':
         filtered = image if mode != 'patchwise' else post_process_segmentation(image_path, image, device=options.get('device'))
         nib.Nifti1Image(filtered, affine=t1_nii.affine).to_filename(os.path.join(image_path, 'out_subcortical_seg_prec.nii.gz'))
@@ -244,7 +251,7 @@ def test_scan(net, test_scan, options):
     return (time.time() - s_time) / 60.0
 
 
-def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=None, post_mask=None):
+def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=None, post_mask=None, mc=None):
     """The timed part of test_scan for one scan, device-resident from the first byte [base.py:357-372, 401-440]:
     raw T1 / atlas priors (/ registered mask) as host arrays in -> uint8 label volume (+ float32 [X,Y,Z,15] probabilities,
     number of candidates) out.  One upload per array (Fortran-ordered NIfTI arrays are reordered on the device), then
@@ -252,7 +259,11 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
     registered mask dilated 10 times), its bounding box, the dense network pass and the scatter, all without the mask,
     the normalised volume or the coordinates ever visiting the host; one download of the result.  atlas / crop_mask /
     post_mask may also be CUDA tensors (float32 [X,Y,Z,15] C-ordered priors, [X,Y,Z] masks: what register_masks returns):
-    they are used in place."""
+    they are used in place.
+
+    mc={'samples': T, 'seed': s}: Monte-Carlo dropout (sc_segment_volume_mc) -- the labels and probabilities are those of the
+    mean of T dropout passes, and on return the dict also holds 'entropy' (predictive entropy, nats) and 'mutual_info' as
+    float32 [X,Y,Z] host arrays, zero outside the candidates."""
     import torch
     t0 = time.time()
     shape = tuple(int(s) for s in t1.shape[:3])
@@ -302,9 +313,17 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
         d_atlas = start_atlas_upload(box if crop_mask is not None else None)
     lab = torch.zeros(shape, dtype=torch.uint8, device=vol.device)
     prob = torch.zeros(shape + (15,), dtype=torch.float32, device=vol.device) if want_proba else None
+    ent = mi = None
+    if mc is not None:
+        ent = torch.zeros(shape, dtype=torch.float32, device=vol.device)
+        mi = torch.zeros(shape, dtype=torch.float32, device=vol.device)
     if box is not None:
-        ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob,
-                           atlas_ready=None if on_device else atlas_ready)
+        ready = None if on_device else atlas_ready
+        if mc is None:
+            ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob, atlas_ready=ready)
+        else:
+            ctx.segment_volume_mc(vol, d_atlas, int(mc['samples']), int(mc.get('seed', 0)), box=box, cand_mask=cand, label_vol=lab,
+                                  proba_vol=prob, entropy_vol=ent, mi_vol=mi, atlas_ready=ready)
     main.wait_stream(side)
     if post_mask is not None:        # post_process_segmentation (base.py:460-480) on the device-resident label volume
         if post_mask is crop_mask and crop_mask is not None:
@@ -319,11 +338,36 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
     if want_proba:
         h_prob = _pinned_out('prob', shape + (15,), torch.float32)
         h_prob.copy_(prob, non_blocking=True)
+    if mc is not None:
+        mc['entropy'], mc['mutual_info'] = ent.cpu().numpy(), mi.cpu().numpy()
     torch.cuda.current_stream().synchronize()
     if timings is not None:
         timings.update({'hot_s': time.time() - t0, 'n_candidates': n_cand, 'mean_nz': mean, 'std_nz': std, 'box': box})
     # views of reusable page-locked buffers: valid until the next call
     return h_lab.numpy(), (h_prob.numpy() if want_proba else None), n_cand
+
+
+def structure_uncertainty(labels, entropy, mutual_info, device=None):
+    """Per-structure quality-control numbers of a Monte-Carlo dropout segmentation, on the device: for every label
+    l = 1..14 the voxel count of the predicted structure and the mean predictive entropy and mean mutual information
+    over its voxels (NaN for an empty structure).  labels [X,Y,Z] integral; entropy / mutual_info float [X,Y,Z]; host
+    arrays or torch tensors.  -> {l: {'voxels': int, 'entropy': float, 'mutual_info': float}}"""
+    import torch
+    ctx = get_context(device)
+    if not (tuple(labels.shape) == tuple(entropy.shape) == tuple(mutual_info.shape)) or len(labels.shape) != 3:
+        raise ValueError("labels, entropy and mutual_info must be 3-D volumes of one shape, got %s, %s and %s" % (
+            tuple(labels.shape), tuple(entropy.shape), tuple(mutual_info.shape)))
+    d = 'cuda:%d' % ctx.device
+    lab = _label_volume(labels, 'labels', ctx.device).view(-1).long()
+    stats = []
+    for v in (entropy, mutual_info):
+        t = v if torch.is_tensor(v) else torch.from_numpy(np.ascontiguousarray(v))
+        stats.append(torch.zeros(17, dtype=torch.float64, device=d).index_add_(0, lab, t.to(d, torch.float64).reshape(-1)))
+    count = torch.bincount(lab, minlength=17).cpu().numpy()
+    h, m = stats[0].cpu().numpy(), stats[1].cpu().numpy()
+    nan = float('nan')
+    return {l: {'voxels': int(count[l]), 'entropy': float(h[l] / count[l]) if count[l] else nan,
+                'mutual_info': float(m[l] / count[l]) if count[l] else nan} for l in range(1, 15)}
 
 
 _pinned_cache = {}

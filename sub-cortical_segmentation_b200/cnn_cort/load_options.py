@@ -53,6 +53,12 @@ def load_options(user_config):
     for key in ('atlas_template', 'atlas_priors'):
         v = g('database', key, fallback='').strip()
         options[key] = v or None
+    # optional: Monte-Carlo dropout passes of the dense inference (0 = off) and the seed of their masks
+    for key in ('mc_samples', 'mc_seed'):
+        v = user_config.getint('model', key, fallback=0)
+        if v < 0:
+            raise ValueError("[model] %s = %d must not be negative" % (key, v))
+        options[key] = v
     return options
 
 

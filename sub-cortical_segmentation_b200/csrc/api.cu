@@ -150,6 +150,7 @@ int sc_destroy(sc_ctx* ctx) {
   for (auto& ev : ctx->prof_free) { cudaEventDestroy(ev.a); cudaEventDestroy(ev.b); }
   if (ctx->h_slab_cnt) { cudaFreeHost(ctx->h_slab_cnt); cudaEventDestroy(ctx->compact_ev); }
   cudaFree(ctx->tile_flags);
+  cudaFree(ctx->mc_w);
   if (ctx->h_reg) cudaFreeHost(ctx->h_reg);
   for (int i = 0; i < 64; ++i) if (ctx->atlas_chunk_ev[i]) cudaEventDestroy(ctx->atlas_chunk_ev[i]);
   if (ctx->copy_stream) { cudaStreamDestroy(ctx->copy_stream); cudaEventDestroy(ctx->copy_ev[0]); cudaEventDestroy(ctx->copy_ev[1]); }
@@ -232,7 +233,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam", "evaluate", "register"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -545,6 +546,26 @@ int sc_segment_volume(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], 
   SC_CHECK(vol_dev && atlas_dev && (label_vol_dev || proba_vol_dev), SC_ERR_ARG, "sc_segment_volume: null argument");
   SC_TRY(check_dims(dims, "sc_segment_volume"));
   return segment_volume(ctx, vol_dev, dims, atlas_dev, box, cand_mask_dev, label_vol_dev, proba_vol_dev, (cudaStream_t)stream);
+}
+
+int sc_segment_volume_mc(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], const float* atlas_dev, const int32_t* box,
+                         const uint8_t* cand_mask_dev, int samples, uint64_t seed, uint8_t* label_vol_dev, float* proba_vol_dev,
+                         float* entropy_vol_dev, float* mi_vol_dev, void* stream) {
+  const char* who = "sc_segment_volume_mc";
+  SC_TRY(fresh_weights(ctx, who, (cudaStream_t)stream));
+  SC_CHECK(vol_dev, SC_ERR_ARG, "%s: vol_dev is NULL", who);
+  SC_CHECK(atlas_dev, SC_ERR_ARG, "%s: atlas_dev is NULL", who);
+  SC_CHECK(label_vol_dev || proba_vol_dev || entropy_vol_dev || mi_vol_dev, SC_ERR_ARG,
+           "%s: label_vol, proba_vol, entropy_vol and mi_vol are all NULL", who);
+  SC_CHECK(samples >= 1 && samples <= 1024, SC_ERR_ARG, "%s: samples = %d is outside [1, 1024]", who, samples);
+  SC_CHECK(ctx->gemm_backend == 1, SC_ERR_ARG, "%s: Monte-Carlo dropout runs on the tcgen05 back-end only (gemm = %d)", who,
+           ctx->gemm_backend);
+  SC_TRY(check_dims(dims, who));
+  if (box)
+    SC_CHECK(box[0] >= 0 && box[1] <= dims[0] && box[2] >= 0 && box[3] <= dims[1] && box[4] >= 0 && box[5] <= dims[2], SC_ERR_ARG,
+             "%s: box {%d,%d,%d,%d,%d,%d} outside the volume", who, box[0], box[1], box[2], box[3], box[4], box[5]);
+  const McArgs mc = {samples, seed, entropy_vol_dev, mi_vol_dev};
+  return segment_volume(ctx, vol_dev, dims, atlas_dev, box, cand_mask_dev, label_vol_dev, proba_vol_dev, (cudaStream_t)stream, &mc);
 }
 
 int sc_atlas_ready_event(sc_ctx* ctx, void* cuda_event) {

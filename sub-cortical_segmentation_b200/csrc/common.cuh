@@ -148,8 +148,18 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_COUNT
 };
+
+// counter-based random bits (splitmix64 finaliser): the dropout keep masks of the training step and of Monte-Carlo dropout
+__host__ __device__ inline uint32_t hash3(uint64_t seed, uint64_t idx) {
+  uint64_t z = seed + 0x9E3779B97F4A7C15ull * (idx + 1);
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return (uint32_t)((z ^ (z >> 31)) >> 16);
+}
+// keep bits per dropout pass: [3][540] *_l1drop (k = c*9 + h*3 + w) | [540] f1_drop | [540] f2_drop
+constexpr int kDropUnits = 2700;
 struct ProfEvent { int cls; cudaEvent_t a, b; };
 
 }  // namespace sc
@@ -210,6 +220,7 @@ struct sc_ctx {
   int tc_skip = 1;               // dense path with a sparse candidate mask: the conv sweeps skip the items no candidate needs
   int tc_compact = 1;            // dense path with a candidate mask: the FC head runs on the compacted candidate rows only
   int32_t* h_slab_cnt = nullptr; // pinned: candidates per slab
+  float* mc_w = nullptr;         // Monte-Carlo dropout: the row-masked split weights (w_nk) of d1 x3, FC1 and fc_2 for one pass
   unsigned char* tile_flags = nullptr;   // d1 with a row map: per-tile "has a candidate" flags (device, grow-only)
   size_t tile_flags_cap = 0;
   cudaEvent_t compact_ev = nullptr;
@@ -341,6 +352,10 @@ struct GemmProblem {
   OutGeo ageo;                             // fix of base.py:392-394) into columns 540..554 and zeros up to 575
   const struct SoftmaxOut* sm = nullptr;   // tcgen05 back-end, fc_2 only: out_layer + softmax / argmax in the epilogue instead of the row store
   int a_swap = 0;       // tensor-map dimension order is (k, pixel, plane, line) instead of (k, pixel, line, plane)
+  // with sm: Monte-Carlo dropout pass instead of the store -- row m adds {softmax p[0..14], sum_c p_c ln p_c} to
+  // mc_acc[m * 16 ..] (mc_first: stores instead of adding)
+  float* mc_acc = nullptr;
+  int mc_first = 0;
 };
 int launch_gemm(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream_t st);
 // plain [M][lda] row-major A, one tap: fills both the pointer form and the tensor-map form
@@ -415,8 +430,17 @@ int launch_conv1_patches(sc_ctx* ctx, const float* patches, int n, const float* 
 size_t branch_patches_tc_bytes(int64_t n);
 int branch_patches_tc(sc_ctx* ctx, int branch, const float* patches, int64_t n, float* scratch, float* feats /*[n][576] split*/,
                       cudaStream_t st);
+// Monte-Carlo dropout over the FC head (mc_dropout.cu): `samples` passes with the keep masks hash3(seed, t * 2700 + j)
+struct McArgs { int samples; uint64_t seed; float* entropy; float* mi; };
 int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const float* atlas, const int32_t* box,
-                   const uint8_t* cand, uint8_t* label_vol, float* proba_vol, cudaStream_t st);
+                   const uint8_t* cand, uint8_t* label_vol, float* proba_vol, cudaStream_t st, const McArgs* mc = nullptr);
+
+// mc_dropout.cu : the masked weights of one pass and the per-voxel statistics of a slab
+struct McWeights { GemmW d1[3], fc1, fc2; };
+int mc_prepare(sc_ctx* ctx, McWeights& w);
+int launch_mc_mask(sc_ctx* ctx, uint64_t seed, int t, cudaStream_t st);
+int launch_mc_finalize(sc_ctx* ctx, const float* acc, int64_t rows, int samples, const int32_t* rowvox, const OutGeo& geo,
+                       const uint8_t* mask, uint8_t* label, float* proba, float* entropy, float* mi, cudaStream_t st);
 
 // train_tc.cu : the convolutional part of the training step on the tensor cores (split-bf16 wide-row maps)
 constexpr float kBnEps = 1e-4f;
@@ -464,9 +488,9 @@ int eval_batch(sc_ctx* ctx, const float* in1, const float* in2, const float* in3
                int64_t n, float* out2, cudaStream_t st);
 
 __device__ __forceinline__ float prelu(float x, float a) { return x > 0.f ? x : a * x; }
-// out_layer logits of one voxel (cnn_cort/nets.py:229-231) -> softmax in fp32; argmax on the float32 probabilities, first
-// maximum wins (np.argmax); the results of voxel o go to whichever outputs are set
-__device__ __forceinline__ void softmax_store(float (&z)[15], long long o, float* proba, int32_t* label32, uint8_t* label8) {
+// out_layer logits of one voxel (cnn_cort/nets.py:229-231) -> softmax in fp32, in place; returns the argmax on the float32
+// probabilities, first maximum wins (np.argmax)
+__device__ __forceinline__ int softmax15(float (&z)[15]) {
   float mx = z[0];
 #pragma unroll
   for (int c = 1; c < 15; ++c) mx = fmaxf(mx, z[c]);
@@ -481,12 +505,25 @@ __device__ __forceinline__ void softmax_store(float (&z)[15], long long o, float
     z[c] *= inv;
     if (z[c] > bp) { bp = z[c]; best = c; }
   }
+  return best;
+}
+// the softmax / argmax of voxel o go to whichever outputs are set
+__device__ __forceinline__ void softmax_store(float (&z)[15], long long o, float* proba, int32_t* label32, uint8_t* label8) {
+  const int best = softmax15(z);
   if (proba) {
 #pragma unroll
     for (int c = 0; c < 15; ++c) proba[o * 15 + c] = z[c];
   }
   if (label32) label32[o] = best;
   if (label8) label8[o] = (uint8_t)best;
+}
+// sum_c p_c ln p_c with 0 ln 0 = 0 (minus the entropy in nats): Monte-Carlo dropout evaluates both the per-pass and the
+// predictive entropy with this one function, so that one pass gives a mutual information of exactly 0
+__device__ __forceinline__ float plogp15(const float (&p)[15]) {
+  float s = 0.f;
+#pragma unroll
+  for (int c = 0; c < 15; ++c) s = p[c] > 0.f ? fmaf(p[c], logf(p[c]), s) : s;
+  return s;
 }
 // split-precision store of 4 consecutive logical columns n..n+3 (n % 4 == 0) of one activation row
 __device__ __forceinline__ void store_split4(float* row, int n, float v0, float v1, float v2, float v3) {

@@ -320,7 +320,7 @@ __global__ void dense_atlas_kernel(const float* __restrict__ atlas, OutGeo g, in
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const float* atlas, const int32_t* box,
-                   const uint8_t* cand, uint8_t* label_vol, float* proba_vol, cudaStream_t st) {
+                   const uint8_t* cand, uint8_t* label_vol, float* proba_vol, cudaStream_t st, const McArgs* mc) {
   const int X = dims[0], Y = dims[1], Z = dims[2];
   int b[6] = {0, X, 0, Y, 0, Z};
   if (box) for (int i = 0; i < 6; ++i) b[i] = box[i];
@@ -329,6 +329,7 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
   if (bx <= 0 || by <= 0 || bz <= 0) return SC_OK;
   const int64_t YZ = (int64_t)Y * Z;
   const bool tc = ctx->gemm_backend == 1;
+  SC_CHECK(!mc || tc, SC_ERR_ARG, "segment_volume: Monte-Carlo dropout needs the tcgen05 back-end");
 
   ViewGeo vg[3];
   // axial: slices along z, rows x, cols y  (patch axes (dx, dy), base.py:291-292)
@@ -383,7 +384,8 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
   for (int v = 0; v < 3; ++v) { occ_off[v] = skip_bytes; skip_bytes += compact ? align256((size_t)vg[v].br * vg[v].ns * 4) : 0; }
   const size_t flags_off = skip_bytes;
   if (compact) skip_bytes += align256((size_t)1 << 20);
-  const size_t total = a5_bytes + scratch_bytes + feat_bytes + h1_bytes + h2_bytes + cmp_bytes + skip_bytes;
+  const size_t mc_bytes = mc ? align256(rows_max * 16 * sizeof(float)) : 0;   // Monte-Carlo dropout: 16 sums per FC row
+  const size_t total = a5_bytes + scratch_bytes + feat_bytes + h1_bytes + h2_bytes + cmp_bytes + mc_bytes + skip_bytes;
   SC_TRY(ensure_ws(ctx->ws, total));
   char* wsb = reinterpret_cast<char*>(ctx->ws.ptr);
   float* a5[3] = {reinterpret_cast<float*>(wsb + a5_off[0]), reinterpret_cast<float*>(wsb + a5_off[1]),
@@ -396,6 +398,7 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
   int32_t* rowvox = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(rowmap) + align256(nbox * 4));
   int32_t* cmp_scratch = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(rowvox) + align256(nbox * 4));
   int32_t* d_slab_cnt = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(cmp_scratch) + align256(cmp_blocks * 8 + 16));
+  float* mc_acc = reinterpret_cast<float*>(wsb + (total - skip_bytes - mc_bytes));
   char* skip_base = wsb + (total - skip_bytes);
   if (compact) {
     // enqueue the scan first: its (tiny) result is on the host long before phase 1 has been launched
@@ -490,6 +493,9 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
 
   // ---- phase 2: d1 (x3) + FC head per slab of x-planes -------------------------------------
   int atlas_waited = 0;                                // chunked upload: chunks of x-planes this stream has already waited for
+  const int passes = mc ? mc->samples : 1;
+  McWeights mcw;
+  if (mc) SC_TRY(mc_prepare(ctx, mcw));
   OutGeo og = {b[0], b[2], b[4], by, bz, Y, Z};
   for (int ix0 = 0; ix0 < bx; ix0 += slab) {
     const int nx = bx - ix0 < slab ? bx - ix0 : slab;
@@ -507,72 +513,83 @@ int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const flo
     const int64_t slab_base = (int64_t)ix0 * plane;
     const int64_t rows_fc = compact ? ctx->h_slab_cnt[ix0 / slab] : rows;      // rows of the FC head (compact: candidates only)
     if (rows_fc == 0) continue;
-    for (int v = 0; v < 3; ++v) {
-      const ViewGeo& g = vg[v];
-      const int64_t c5 = tc ? g.bc + 29 : g.bc + 8, r5 = tc ? g.br + 29 : g.br + 8;   // tensor-core mode: conv1 geometry (see phase 1)
+    // Monte-Carlo dropout: the FC head once per pass with the row-masked weights of that pass (mc_dropout.cu)
+    for (int pass = 0; pass < passes; ++pass) {
+      if (mc) SC_TRY(launch_mc_mask(ctx, mc->seed, pass, st));
+      for (int v = 0; v < 3; ++v) {
+        const ViewGeo& g = vg[v];
+        const int64_t c5 = tc ? g.bc + 29 : g.bc + 8, r5 = tc ? g.br + 29 : g.br + 8;   // tensor-core mode: conv1 geometry (see phase 1)
+        GemmProblem p;
+        p.lda = kC5Ld; p.a_ys = c5 * kC5Ld; p.a_zs = r5 * c5 * kC5Ld;
+        p.ntaps = 9; p.kc = kC5Ld;
+        for (int t = 0; t < 9; ++t) {
+          p.tap_off[t] = ((int64_t)(t / 3) * 4 * c5 + (t % 3) * 4) * kC5Ld;
+          p.tap_dx[t] = (t % 3) * 4; p.tap_dy[t] = (t / 3) * 4;
+        }
+        p.a_base = a5[v]; p.a_dims[0] = kC5Ld; p.a_dims[1] = c5; p.a_dims[2] = r5; p.a_dims[3] = g.ns;
+        p.a_strides[0] = kC5Ld; p.a_strides[1] = c5 * kC5Ld; p.a_strides[2] = r5 * c5 * kC5Ld;
+        p.a_swap = 0;
+        if (tc) {   // wide-row map: (k, col, slice, row) with strides (pixel, C1 pixels, ns * C1 pixels)
+          p.a_dims[2] = g.ns; p.a_dims[3] = r5;
+          p.a_strides[1] = c5 * kC5Ld; p.a_strides[2] = (int64_t)g.ns * c5 * kC5Ld;
+          p.a_swap = 1;
+        }
+        p.a_y0 = v == 2 ? 0 : ix0; p.a_z0 = v == 2 ? ix0 : 0;
+        p.ldc = 0; p.out_split = tc ? 1 : 0; p.c_col0 = v * 192; p.prof_cls = PC_GEMM_D1; p.k_used = 0;
+        p.n_store = 192;   // 180 features + 12 zero columns (zero weights / bias) per view
+        if (v == 0) {        // m = y, lines = x (slab), planes = z
+          p.A = a5[0] + (int64_t)ix0 * p.a_ys; p.M = by; p.Y = nx; p.Z = bz;
+          p.ldc = (int64_t)bz * kFeatLd; p.c_ys = plane * kFeatLd; p.c_zs = kFeatLd;
+        } else if (v == 1) { // m = z, lines = x (slab), planes = y
+          p.A = a5[1] + (int64_t)ix0 * p.a_ys; p.M = bz; p.Y = nx; p.Z = by;
+          p.ldc = kFeatLd; p.c_ys = plane * kFeatLd; p.c_zs = (int64_t)bz * kFeatLd;
+        } else {             // m = z, lines = y, planes = x (slab)
+          p.A = a5[2] + (int64_t)ix0 * p.a_zs; p.M = bz; p.Y = by; p.Z = nx;
+          p.ldc = kFeatLd; p.c_ys = (int64_t)bz * kFeatLd; p.c_zs = plane * kFeatLd;
+        }
+        p.C = feats;
+        if (compact) p.rowmap = rowmap + slab_base;      // dense row -> compact feature row (or skipped)
+        SC_TRY(tc ? launch_gemm_tc(ctx, p, mc ? mcw.d1[v] : ctx->br[v].d1_dense, st) : launch_gemm(ctx, p, ctx->br[v].d1_dense, st));
+      }
       GemmProblem p;
-      p.lda = kC5Ld; p.a_ys = c5 * kC5Ld; p.a_zs = r5 * c5 * kC5Ld;
-      p.ntaps = 9; p.kc = kC5Ld;
-      for (int t = 0; t < 9; ++t) {
-        p.tap_off[t] = ((int64_t)(t / 3) * 4 * c5 + (t % 3) * 4) * kC5Ld;
-        p.tap_dx[t] = (t % 3) * 4; p.tap_dy[t] = (t / 3) * 4;
+      SC_CHECK(rows < (1ll << 31), SC_ERR_ARG, "sc_segment_volume: chunk too large");
+      gemm_problem_rows(p, feats, kFeatLd, kFeatLd, (int)rows_fc);
+      p.C = h1; p.ldc = kH1Ld; p.n_store = 540; p.out_split = tc ? 1 : 0;
+      p.prof_cls = PC_GEMM_FC1;
+      const bool atlas_fused = tc;   // the CTA-pair kernel writes the atlas columns in its epilogue
+      if (ctx->atlas_ready && ctx->atlas_chunks == 0) {   // an atlas upload on a side stream (sc_atlas_ready_event): the priors are first
+        SC_CUDA(cudaStreamWaitEvent(st, ctx->atlas_ready, 0));   // read here, after the conv phase and the first slab's d1 launches
+        ctx->atlas_ready = nullptr;
       }
-      p.a_base = a5[v]; p.a_dims[0] = kC5Ld; p.a_dims[1] = c5; p.a_dims[2] = r5; p.a_dims[3] = g.ns;
-      p.a_strides[0] = kC5Ld; p.a_strides[1] = c5 * kC5Ld; p.a_strides[2] = r5 * c5 * kC5Ld;
-      p.a_swap = 0;
-      if (tc) {   // wide-row map: (k, col, slice, row) with strides (pixel, C1 pixels, ns * C1 pixels)
-        p.a_dims[2] = g.ns; p.a_dims[3] = r5;
-        p.a_strides[1] = c5 * kC5Ld; p.a_strides[2] = (int64_t)g.ns * c5 * kC5Ld;
-        p.a_swap = 1;
+      if (atlas_fused) { p.atlas = atlas; p.ageo = og; p.ageo.x0 = b[0] + ix0; if (compact) p.rowvox = rowvox + slab_base; }
+      SC_TRY(tc ? launch_gemm_tc(ctx, p, mc ? mcw.fc1 : ctx->fc1, st) : launch_gemm(ctx, p, ctx->fc1, st));
+      p.atlas = nullptr; p.rowvox = nullptr;
+      if (!atlas_fused) {  // after FC1: the tensor-core epilogue writes whole 16-column chunks (columns 540..543 as zeros)
+        ProfScope prof(ctx, PC_ATLAS, st);
+        dense_atlas_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(atlas, og, ix0, rows, h1, tc ? 1 : 0);
+        ctx->launches++;
       }
-      p.a_y0 = v == 2 ? 0 : ix0; p.a_z0 = v == 2 ? ix0 : 0;
-      p.ldc = 0; p.out_split = tc ? 1 : 0; p.c_col0 = v * 192; p.prof_cls = PC_GEMM_D1; p.k_used = 0;
-      p.n_store = 192;   // 180 features + 12 zero columns (zero weights / bias) per view
-      if (v == 0) {        // m = y, lines = x (slab), planes = z
-        p.A = a5[0] + (int64_t)ix0 * p.a_ys; p.M = by; p.Y = nx; p.Z = bz;
-        p.ldc = (int64_t)bz * kFeatLd; p.c_ys = plane * kFeatLd; p.c_zs = kFeatLd;
-      } else if (v == 1) { // m = z, lines = x (slab), planes = y
-        p.A = a5[1] + (int64_t)ix0 * p.a_ys; p.M = bz; p.Y = nx; p.Z = by;
-        p.ldc = kFeatLd; p.c_ys = plane * kFeatLd; p.c_zs = (int64_t)bz * kFeatLd;
-      } else {             // m = z, lines = y, planes = x (slab)
-        p.A = a5[2] + (int64_t)ix0 * p.a_zs; p.M = bz; p.Y = by; p.Z = nx;
-        p.ldc = kFeatLd; p.c_ys = (int64_t)bz * kFeatLd; p.c_zs = plane * kFeatLd;
+      SC_CUDA(cudaGetLastError());
+      gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)rows_fc);
+      p.prof_cls = PC_GEMM_FC2;
+      OutGeo og2 = og;
+      og2.x0 = b[0] + ix0;
+      if (tc) {   // fc_2 with the out_layer, softmax / argmax and the scatter into the volume in its epilogue
+        SoftmaxOut smo = {proba_vol, nullptr, label_vol, cand, og2, 1, compact ? rowvox + slab_base : nullptr};
+        p.C = nullptr; p.ldc = 0; p.n_store = kH2Ld; p.sm = &smo;
+        if (mc) { p.mc_acc = mc_acc; p.mc_first = pass == 0; }   // one Monte-Carlo pass: accumulate instead of the scatter
+        SC_TRY(launch_gemm_tc(ctx, p, mc ? mcw.fc2 : ctx->fc2, st));
+      } else {
+        p.C = h2; p.ldc = kH2Ld; p.n_store = kH2Ld;
+        SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
+        SC_TRY(launch_out_softmax(ctx, h2, rows, proba_vol, nullptr, label_vol, cand, &og2, st));
       }
-      p.C = feats;
-      if (compact) p.rowmap = rowmap + slab_base;      // dense row -> compact feature row (or skipped)
-      SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->br[v].d1_dense, st) : launch_gemm(ctx, p, ctx->br[v].d1_dense, st));
     }
-    GemmProblem p;
-    SC_CHECK(rows < (1ll << 31), SC_ERR_ARG, "sc_segment_volume: chunk too large");
-    gemm_problem_rows(p, feats, kFeatLd, kFeatLd, (int)rows_fc);
-    p.C = h1; p.ldc = kH1Ld; p.n_store = 540; p.out_split = tc ? 1 : 0;
-    p.prof_cls = PC_GEMM_FC1;
-    const bool atlas_fused = tc;   // the CTA-pair kernel writes the atlas columns in its epilogue
-    if (ctx->atlas_ready && ctx->atlas_chunks == 0) {   // an atlas upload on a side stream (sc_atlas_ready_event): the priors are first
-      SC_CUDA(cudaStreamWaitEvent(st, ctx->atlas_ready, 0));   // read here, after the conv phase and the first slab's d1 launches
-      ctx->atlas_ready = nullptr;
-    }
-    if (atlas_fused) { p.atlas = atlas; p.ageo = og; p.ageo.x0 = b[0] + ix0; if (compact) p.rowvox = rowvox + slab_base; }
-    SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->fc1, st) : launch_gemm(ctx, p, ctx->fc1, st));
-    p.atlas = nullptr; p.rowvox = nullptr;
-    if (!atlas_fused) {  // after FC1: the tensor-core epilogue writes whole 16-column chunks (columns 540..543 as zeros)
-      ProfScope prof(ctx, PC_ATLAS, st);
-      dense_atlas_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(atlas, og, ix0, rows, h1, tc ? 1 : 0);
-      ctx->launches++;
-    }
-    SC_CUDA(cudaGetLastError());
-    gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)rows_fc);
-    p.prof_cls = PC_GEMM_FC2;
-    OutGeo og2 = og;
-    og2.x0 = b[0] + ix0;
-    if (tc) {   // fc_2 with the out_layer, softmax / argmax and the scatter into the volume in its epilogue
-      SoftmaxOut smo = {proba_vol, nullptr, label_vol, cand, og2, 1, compact ? rowvox + slab_base : nullptr};
-      p.C = nullptr; p.ldc = 0; p.n_store = kH2Ld; p.sm = &smo;
-      SC_TRY(launch_gemm_tc(ctx, p, ctx->fc2, st));
-    } else {
-      p.C = h2; p.ldc = kH2Ld; p.n_store = kH2Ld;
-      SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
-      SC_TRY(launch_out_softmax(ctx, h2, rows, proba_vol, nullptr, label_vol, cand, &og2, st));
+    if (mc) {
+      OutGeo og3 = og;
+      og3.x0 = b[0] + ix0;
+      SC_TRY(launch_mc_finalize(ctx, mc_acc, rows_fc, mc->samples, compact ? rowvox + slab_base : nullptr, og3, cand, label_vol,
+                                proba_vol, mc->entropy, mc->mi, st));
     }
   }
   if (ctx->atlas_ready && ctx->atlas_chunks == 0) {     // no slab had a candidate: still join the upload before the caller goes on

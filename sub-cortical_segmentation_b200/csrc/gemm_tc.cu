@@ -70,6 +70,8 @@ struct TcArgs {
   SoftmaxOut sm;      // pair kernel, fc_2 with the out_layer epilogue (FUSED_OUT): where the softmax / argmax results go
   const float* out_w; // FUSED_OUT: out_layer weights [270][16] and bias [16], fp32
   const float* out_b;
+  float* mc_acc;      // MC_ACC: per-row Monte-Carlo dropout accumulator [M][16] (see GemmProblem::mc_acc)
+  int mc_first;
 };
 
 // fused out_layer (FUSED_OUT): the 16 epilogue warps' store-transpose area is free and holds the out_layer weights (rows padded
@@ -313,7 +315,9 @@ gemm_tc_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid
 //   * the leader's MMA warp issues tcgen05.mma.cta_group::2 (M = 256) and multicasts its commits to both CTAs
 //   * every CTA's epilogue warps drain their own TMEM half and arrive on the leader's tempty barrier (remote arrive)
 // ---------------------------------------------------------------------------------------------------
-template <bool FUSED_OUT>
+// MC_ACC (with FUSED_OUT): one Monte-Carlo dropout pass -- the softmax of row m and its sum_c p_c ln p_c are added to
+// mc_acc[m * 16 ..] (stored by the first pass) in pass order, instead of being scattered into the volume
+template <bool FUSED_OUT, bool MC_ACC = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(576, 1)
 gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -544,6 +548,27 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
           asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
           long long m = (long long)mw + lane;
           bool ok = grp == 0 && m < a.M;
+          if (MC_ACC) {
+            if (ok) {
+#pragma unroll
+              for (int c = 0; c < 15; ++c) logit[c] += s_ob[c];
+              softmax15(logit);
+              float4* acc = reinterpret_cast<float4*>(a.mc_acc + m * 16);
+              const float4 v[4] = {make_float4(logit[0], logit[1], logit[2], logit[3]), make_float4(logit[4], logit[5], logit[6], logit[7]),
+                                   make_float4(logit[8], logit[9], logit[10], logit[11]),
+                                   make_float4(logit[12], logit[13], logit[14], plogp15(logit))};
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                float4 r = v[i];
+                if (!a.mc_first) {
+                  const float4 o = acc[i];
+                  r.x += o.x; r.y += o.y; r.z += o.z; r.w += o.w;
+                }
+                acc[i] = r;
+              }
+            }
+            continue;
+          }
           if (ok && a.sm.rowvox) m = __ldg(a.sm.rowvox + m);      // compact row -> row of the dense slab
           long long o = m;
           if (ok && a.sm.use_geo) {
@@ -772,6 +797,8 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
              SC_ERR_ARG, "gemm_tc: the out_layer epilogue is for fc_2");
     a.sm = *p.sm;
   }
+  SC_CHECK(!p.mc_acc || p.sm, SC_ERR_ARG, "gemm_tc: the Monte-Carlo accumulator needs the out_layer epilogue");
+  a.mc_acc = p.mc_acc; a.mc_first = p.mc_first;
   a.nt = (p.n_store + a.bn - 1) / a.bn;
   a.mt = (p.M + TC_BM - 1) / TC_BM;
   a.Y = p.Y; a.M = p.M; a.npad = w.Npad;
@@ -847,6 +874,7 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
   SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_persistent_kernel), 227 * 1024));
   SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel<false>), 227 * 1024));
   SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel<true>), 227 * 1024));
+  if (p.mc_acc) SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(gemm_tc_pair_kernel<true, true>), 227 * 1024));
   SC_CHECK(smem <= 227 * 1024, SC_ERR_ARG, "gemm_tc: shared memory budget exceeded (%zu)", smem);
   ProfScope prof(ctx, p.prof_cls, st);
   a.n_mma = a.nt * a.bn;
@@ -871,7 +899,8 @@ int launch_gemm_tc(sc_ctx* ctx, const GemmProblem& p, const GemmW& w, cudaStream
   if (pair) {
     const long long units = p.sm ? a.num_tiles / a.nt : a.num_tiles;   // work units of the pair kernel (see its tile walk)
     const long long pairs = units < ctx->sm_count / 2 ? units : ctx->sm_count / 2;
-    if (p.sm) gemm_tc_pair_kernel<true><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);   // __cluster_dims__(2,1,1)
+    if (p.mc_acc) gemm_tc_pair_kernel<true, true><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);
+    else if (p.sm) gemm_tc_pair_kernel<true><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);   // __cluster_dims__(2,1,1)
     else gemm_tc_pair_kernel<false><<<(unsigned)(2 * pairs), 64 + 32 * a.epi_warps, smem, st>>>(mapA, mapB, a);
   } else {
     const unsigned grid = (unsigned)(blocks < ctx->sm_count ? blocks : ctx->sm_count);

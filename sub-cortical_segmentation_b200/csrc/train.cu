@@ -22,13 +22,6 @@ constexpr int kLd[5] = {32, 32, 16, 16, 8};     // row stride of the conv output
 constexpr int kInH[5] = {32, 30, 14, 12, 5};    // conv input size
 constexpr int kInLd[5] = {32, 32, 16, 16, 8};
 
-__host__ __device__ inline uint32_t hash3(uint64_t seed, uint64_t idx) {
-  uint64_t z = seed + 0x9E3779B97F4A7C15ull * (idx + 1);
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return (uint32_t)((z ^ (z >> 31)) >> 16);
-}
-
 // ---- parameter repacking ------------------------------------------------------------------------
 // fwd: out[ci][t][co] = W[co][ci][8-t] (true convolution -> correlation taps);  dgrad: out[co][t][ci] = W[co][ci][t]
 __global__ void repack_conv_kernel(const float* __restrict__ W, int cout, int cin, float* __restrict__ fwd, float* __restrict__ dgrad) {
