@@ -188,13 +188,12 @@ int sc_set_option(sc_ctx* ctx, const char* key, int64_t value) {
     ctx->train_graph_on = value != 0;
     return SC_OK;
   }
-  if (!strcmp(key, "train_fused_stats") || !strcmp(key, "train_wgrad_mn")) {     // captured graphs hold the launch sequence of the setting they were captured under
-    int& opt = !strcmp(key, "train_fused_stats") ? ctx->train_fused_stats : ctx->train_wgrad_mn;
-    if ((value != 0) != (opt != 0)) {
+  if (!strcmp(key, "train_fused_stats")) {     // captured graphs hold the launch sequence of the setting they were captured under
+    if ((value != 0) != (ctx->train_fused_stats != 0)) {
       for (auto& g : ctx->train_graphs) cudaGraphExecDestroy(g.exec);
       ctx->train_graphs.clear();
     }
-    opt = value != 0;
+    ctx->train_fused_stats = value != 0;
     return SC_OK;
   }
   if (!strcmp(key, "profile")) {

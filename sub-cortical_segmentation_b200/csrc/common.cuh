@@ -215,7 +215,6 @@ struct sc_ctx {
   void* tc_state = nullptr;      // tcgen05 back-end state (tensor-map encoder entry point)
   int tc_timing_cls = -1;        // ProfClass whose persistent launches record per-role wait cycles (debug)
   unsigned long long* tc_timing_buf = nullptr;   // [sm_count][8], overwritten by every instrumented launch
-  int train_wgrad_mn = 1;        // conv weight gradients from the pixel-major maps (MN-major operands) instead of planar transposed copies
   int train_fused_stats = 1;     // training forward: BatchNorm statistics accumulated in the sweep epilogues (off: a separate pass over the stored maps)
   int tc_skip = 1;               // dense path with a sparse candidate mask: the conv sweeps skip the items no candidate needs
   int tc_compact = 1;            // dense path with a candidate mask: the FC head runs on the compacted candidate rows only
@@ -445,13 +444,14 @@ int launch_mc_finalize(sc_ctx* ctx, const float* acc, int64_t rows, int samples,
 // train_tc.cu : the convolutional part of the training step on the tensor cores (split-bf16 wide-row maps)
 constexpr float kBnEps = 1e-4f;
 struct TcBranchBuf {
-  float* X[5]; float* A[5]; uint16_t* AT[5]; uint8_t* idx[5]; float* mean[5]; float* istd[5];
-  float* frame; float* dA; uint16_t* DT; float* dX0; double* sums;
+  float* X[5]; float* A[5]; uint8_t* idx[5]; float* mean[5]; float* istd[5];
+  float* frame; float* dA; double* sums;
+  float* wf0;     // conv1 taps [9][20] (repack_conv_kernel)
+  float* F5;      // flattened conv5 activation [n][540], l1drop applied: the input of d1
 };
 size_t tc_branch_bytes(int n);
 int tc_carve_branch(TcBranchBuf& T, char* base, int n);
-int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* patches, const float* wf0, int n, const uint8_t* masks,
-                      float* F5, cudaStream_t s);
+int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* patches, int n, const uint8_t* masks, cudaStream_t s);
 int tc_branch_backward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* patches, const float* dF5, int dF5_ld, const uint8_t* masks, int n,
                        cudaStream_t s);
 // train_dense.cu : the dense layers of the training step as split-bf16 tcgen05 GEMMs
@@ -471,7 +471,6 @@ int tdense_branch_forward(sc_ctx* ctx, int b, const TcDenseBuf& D, const float* 
 int tdense_head(sc_ctx* ctx, const TcDenseBuf& D, const float* in4, const uint8_t* y, int n, int64_t n_global, const uint8_t* masks, float* loss,
                 cudaStream_t s);
 int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const uint8_t* masks, cudaStream_t s);
-int launch_conv1_wgrad(sc_ctx* ctx, const float* patches, const float* dx_planar, int n, int zc, float* gW, cudaStream_t st);
 
 // fused_adam.cu
 int fused_export(sc_ctx* ctx, unsigned char* handles);

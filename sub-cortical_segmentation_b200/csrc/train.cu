@@ -619,227 +619,238 @@ struct Bump {
 
 static unsigned ew_grid(int64_t total) { return (unsigned)((total + 255) / 256 < 65535 * 8 ? (total + 255) / 256 : 65535 * 8); }
 
-// The step body.  Every pointer it touches lives in the context (staged inputs, arena, parameter / gradient buffers), every
-// scalar that changes from step to step is read from device memory (the dropout seed), so the same sequence of launches is
-// valid as a captured CUDA graph.  The three branches are independent between the patches and the concatenation (forward)
-// and after the gradient of the concatenation (backward): they run on three streams forked from / joined into `st`.
-struct StepBuf {
-  TcBranchBuf tc[3];
-  TcDenseBuf td;
-  struct BranchBuf {
+// ---- the step buffers: the staged batch, then the selected back-end's buffers
+struct SimtBuf {       // the exact-fp32 SIMT back-end (gemm = 0): planar fp32 maps and plain dense activations
+  struct Branch {
     float* X[5]; float* A[5]; uint8_t* idx[2]; float* mean[5]; float* istd[5];
     float* F5; float* Z1;
     float* wf[5]; float* wd[5];
     float *dZ1, *dF5, *dA, *dX, *dXpad;
     double* sums;
   } bb[3];
-  float *in[3], *in4; uint8_t* y;
   float *CAT, *ZF1, *CAT2, *ZF2, *H2, *ZO, *dZO, *dH2, *dZF2, *dCAT2, *dZF1, *dCAT;
+};
+struct StepBuf {
+  float *in[3], *in4; uint8_t* y;      // the caller's batch, staged
   uint8_t* masks;
   unsigned long long* seed;
   float* loss;
+  SimtBuf simt;                        // gemm = 0
+  TcBranchBuf tc[3];                   // gemm = 1
+  TcDenseBuf td;
 };
 
-static size_t carve_step(StepBuf& S, char* base, int n, bool tc) {
-  Bump B{base, 0};
+static void carve_simt(SimtBuf& M, Bump& B, int n) {
   for (int b = 0; b < 3; ++b) {
-    auto& bb = S.bb[b];
-    S.in[b] = B.take<float>((size_t)n * 1024);
+    auto& bb = M.bb[b];
     for (int l = 0; l < 5; ++l) {
-      // the tensor-core path keeps its activations in the split-bf16 maps of S.tc; the planar fp32 maps are the SIMT path's
-      bb.X[l] = tc ? nullptr : B.take<float>((size_t)n * kConvCout[l] * kH[l] * kLd[l]);
+      bb.X[l] = B.take<float>((size_t)n * kConvCout[l] * kH[l] * kLd[l]);
       const int oh = (l == 1 || l == 3) ? kH[l] / 2 : kH[l];
       const int old = (l == 1) ? 16 : (l == 3) ? 8 : kLd[l];
-      bb.A[l] = tc ? nullptr : B.take<float>((size_t)n * kConvCout[l] * oh * old);
+      bb.A[l] = B.take<float>((size_t)n * kConvCout[l] * oh * old);
       bb.mean[l] = B.take<float>(64); bb.istd[l] = B.take<float>(64);
       bb.wf[l] = B.take<float>((size_t)kConvCout[l] * kConvCin[l] * 9);
       bb.wd[l] = l > 0 ? B.take<float>((size_t)kConvCout[l] * kConvCin[l] * 9) : nullptr;
     }
-    bb.idx[0] = tc ? nullptr : B.take<uint8_t>((size_t)n * 20 * 14 * 16);
-    bb.idx[1] = tc ? nullptr : B.take<uint8_t>((size_t)n * 40 * 5 * 8);
+    bb.idx[0] = B.take<uint8_t>((size_t)n * 20 * 14 * 16);
+    bb.idx[1] = B.take<uint8_t>((size_t)n * 40 * 5 * 8);
     bb.F5 = B.take<float>((size_t)n * 540);
     bb.Z1 = B.take<float>((size_t)n * 180);
     bb.dZ1 = B.take<float>((size_t)n * 180);
     bb.dF5 = B.take<float>((size_t)n * 540);
-    bb.dA = tc ? nullptr : B.take<float>((size_t)n * 20 * 30 * 32);      // incoming activation gradient of the current layer
-    bb.dX = tc ? nullptr : B.take<float>((size_t)n * 20 * 30 * 32);      // compact conv-output gradient
-    bb.dXpad = tc ? nullptr : B.take<float>((size_t)n * 20 * 34 * 32);   // zero-padded copy for dgrad
+    bb.dA = B.take<float>((size_t)n * 20 * 30 * 32);      // incoming activation gradient of the current layer
+    bb.dX = B.take<float>((size_t)n * 20 * 30 * 32);      // compact conv-output gradient
+    bb.dXpad = B.take<float>((size_t)n * 20 * 34 * 32);   // zero-padded copy for dgrad
     bb.sums = B.take<double>(64 * 3);
-    if (tc) {
-      char* t = B.take<char>(tc_branch_bytes(n));
-      tc_carve_branch(S.tc[b], t, n);
-    }
   }
-  if (tc) {
-    char* t = B.take<char>(tdense_bytes(n));
-    tdense_carve(S.td, t, n);
-  }
+  M.CAT = B.take<float>((size_t)n * 540);     // [D1_ax | D1_cor | D1_sag], f1_drop applied
+  M.ZF1 = B.take<float>((size_t)n * 540);
+  M.CAT2 = B.take<float>((size_t)n * 555);    // [prelu(ZF1) with f2_drop | atlas]
+  M.ZF2 = B.take<float>((size_t)n * 270);
+  M.H2 = B.take<float>((size_t)n * 270);
+  M.ZO = B.take<float>((size_t)n * 15);
+  M.dZO = B.take<float>((size_t)n * 15);
+  M.dH2 = B.take<float>((size_t)n * 270);
+  M.dZF2 = B.take<float>((size_t)n * 270);
+  M.dCAT2 = B.take<float>((size_t)n * 555);
+  M.dZF1 = B.take<float>((size_t)n * 540);
+  M.dCAT = B.take<float>((size_t)n * 540);
+}
+
+static size_t carve_step(StepBuf& S, char* base, int n, bool tc) {
+  Bump B{base, 0};
+  for (int b = 0; b < 3; ++b) S.in[b] = B.take<float>((size_t)n * 1024);
   S.in4 = B.take<float>((size_t)n * 15);
   S.y = B.take<uint8_t>((size_t)n);
-  S.CAT = B.take<float>((size_t)n * 540);     // [D1_ax | D1_cor | D1_sag], f1_drop applied
-  S.ZF1 = B.take<float>((size_t)n * 540);
-  S.CAT2 = B.take<float>((size_t)n * 555);    // [prelu(ZF1) with f2_drop | atlas]
-  S.ZF2 = B.take<float>((size_t)n * 270);
-  S.H2 = B.take<float>((size_t)n * 270);
-  S.ZO = B.take<float>((size_t)n * 15);
-  S.dZO = B.take<float>((size_t)n * 15);
-  S.dH2 = B.take<float>((size_t)n * 270);
-  S.dZF2 = B.take<float>((size_t)n * 270);
-  S.dCAT2 = B.take<float>((size_t)n * 555);
-  S.dZF1 = B.take<float>((size_t)n * 540);
-  S.dCAT = B.take<float>((size_t)n * 540);
   S.masks = B.take<uint8_t>((size_t)n * 2700);
   S.seed = B.take<unsigned long long>(1);
   S.loss = B.take<float>(1);
+  if (tc) {
+    for (int b = 0; b < 3; ++b) tc_carve_branch(S.tc[b], B.take<char>(tc_branch_bytes(n)), n);
+    tdense_carve(S.td, B.take<char>(tdense_bytes(n)), n);
+  } else {
+    carve_simt(S.simt, B, n);
+  }
   return B.off;
 }
 
-int launch_conv1_wgrad(sc_ctx* ctx, const float* patches, const float* dx_planar, int n, int zc, float* gW, cudaStream_t st) {
-  ProfScope prof(ctx, PC_TRAIN_BWD, st);
-  conv_wgrad_kernel<<<dim3(20, 1, zc), 128, 0, st>>>(patches, 1, 32, 32, dx_planar, 20, 30, 30, 32, n, gW);
-  ctx->launches++;
-  SC_CUDA(cudaGetLastError());
-  return SC_OK;
-}
-
-static int train_body(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bool injected_masks, cudaStream_t st) {
-  const bool tc = ctx->gemm_backend == 1;
-  const ParamOff& O = ctx->off;
+// ---- SIMT back-end: conv1..conv5 with BatchNorm / PReLU / pools, d1 into CAT
+static int simt_branch_forward(sc_ctx* ctx, int b, const StepBuf& S, int n, cudaStream_t s) {
+  const BranchOff& Ob = ctx->off.br[b];
+  const auto& bb = S.simt.bb[b];
   float* P = ctx->params;
   float* G = ctx->grads;
   const float* ones = ctx->train_consts;
   const float* zeros = ctx->train_consts + kTrainZeros;
+  for (int l = 0; l < 5; ++l) {
+    const int co = kConvCout[l], ci = kConvCin[l];
+    repack_conv_kernel<<<(co * ci * 9 + 255) / 256, 256, 0, s>>>(P + Ob.convW[l], co, ci, bb.wf[l], bb.wd[l]);
+    ctx->launches++;
+    if (l == 0) {
+      SC_TRY(launch_conv1_patches(ctx, S.in[b], n, bb.wf[0], ones, zeros, ones, bb.X[0], s));
+    } else {
+      SC_TRY(train_conv(ctx, ci, co, bb.A[l - 1], kInH[l], kInLd[l], bb.X[l], kH[l], kLd[l], bb.wf[l], n, PC_TRAIN_FWD, s));
+    }
+    SC_CUDA(cudaMemsetAsync(bb.sums, 0, 64 * 3 * sizeof(double), s));
+    bn_stats_kernel<<<dim3(co, 32), 256, 0, s>>>(bb.X[l], n, co, kH[l], kH[l], kLd[l], bb.sums);
+    bn_finalize_kernel<<<1, 64, 0, s>>>(bb.sums, co, (double)n * kH[l] * kH[l], bb.mean[l], bb.istd[l], G + Ob.bn[l][2], G + Ob.bn[l][3]);
+    const int pool = (l == 1 || l == 3);
+    const int oh = pool ? kH[l] / 2 : kH[l];
+    const int old = (l == 1) ? 16 : (l == 3) ? 8 : kLd[l];
+    bn_act_kernel<<<ew_grid((int64_t)n * co * oh * oh), 256, 0, s>>>(bb.X[l], n, co, kH[l], kH[l], kLd[l], bb.mean[l], bb.istd[l],
+                                                                   P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], pool, bb.A[l], oh, oh, old,
+                                                                   pool ? bb.idx[l == 1 ? 0 : 1] : nullptr);
+    ctx->launches += 3;
+  }
+  flatten_drop_kernel<<<ew_grid((int64_t)n * 540), 256, 0, s>>>(bb.A[4], n, S.masks + b * 540, bb.F5);
+  SC_TRY((sgemm<false, false>(ctx, bb.F5, 540, P + Ob.d1W, 180, bb.Z1, 180, n, 180, 540, P + Ob.d1b, 0, PC_TRAIN_FWD, s)));
+  dense_act_kernel<<<ew_grid((int64_t)n * 180), 256, 0, s>>>(bb.Z1, n, 180, P + Ob.d1alpha, S.masks + 1620 + b * 180, 2700, S.simt.CAT, 540, b * 180);
+  ctx->launches += 2;
+  return SC_OK;
+}
+
+// FC1 -> fc_2 -> out_layer -> softmax cross-entropy, then the backward pass of the head down to dCAT
+static int simt_head(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, cudaStream_t st) {
+  const ParamOff& O = ctx->off;
+  const SimtBuf& M = S.simt;
+  float* P = ctx->params;
+  float* G = ctx->grads;
+  SC_TRY((sgemm<false, false>(ctx, M.CAT, 540, P + O.fc1W, 540, M.ZF1, 540, n, 540, 540, P + O.fc1b, 0, PC_TRAIN_FWD, st)));
+  dense_act_kernel<<<ew_grid((int64_t)n * 540), 256, 0, st>>>(M.ZF1, n, 540, P + O.a1, S.masks + 2160, 2700, M.CAT2, 555, 0);
+  SC_CUDA(cudaMemcpy2DAsync(M.CAT2 + 540, 555 * 4, S.in4, 15 * 4, 15 * 4, n, cudaMemcpyDeviceToDevice, st));
+  SC_TRY((sgemm<false, false>(ctx, M.CAT2, 555, P + O.fc2W, 270, M.ZF2, 270, n, 270, 555, P + O.fc2b, 0, PC_TRAIN_FWD, st)));
+  dense_act_kernel<<<ew_grid((int64_t)n * 270), 256, 0, st>>>(M.ZF2, n, 270, P + O.a2, nullptr, 0, M.H2, 270, 0);
+  SC_TRY((sgemm<false, false>(ctx, M.H2, 270, P + O.outW, 15, M.ZO, 15, n, 15, 270, P + O.outb, 0, PC_TRAIN_FWD, st)));
+  softmax_ce_kernel<<<(n + 127) / 128, 128, 0, st>>>(M.ZO, S.y, n, 1.f / (float)n_global, M.dZO, S.loss);
+  ctx->launches += 3;
+  // out layer
+  SC_TRY((sgemm<true, false>(ctx, M.H2, 270, M.dZO, 15, G + O.outW, 15, 270, 15, n, nullptr, 0, PC_TRAIN_BWD, st)));
+  colsum_kernel<<<dim3(1, 32), 32, 0, st>>>(M.dZO, n, 15, G + O.outb);
+  SC_TRY((sgemm<false, true>(ctx, M.dZO, 15, P + O.outW, 15, M.dH2, 270, n, 270, 15, nullptr, 0, PC_TRAIN_BWD, st)));
+  // fc_2
+  dense_act_bwd_kernel<<<dim3((270 + 31) / 32, 16), 256, 0, st>>>(M.dH2, 270, 0, M.ZF2, n, 270, P + O.a2, nullptr, 0, M.dZF2, G + O.a2, G + O.fc2b);
+  SC_TRY((sgemm<true, false>(ctx, M.CAT2, 555, M.dZF2, 270, G + O.fc2W, 270, 555, 270, n, nullptr, 0, PC_TRAIN_BWD, st)));
+  SC_TRY((sgemm<false, true>(ctx, M.dZF2, 270, P + O.fc2W, 270, M.dCAT2, 555, n, 555, 270, nullptr, 0, PC_TRAIN_BWD, st)));
+  // FC1 (dropout f2_drop sits on its activation)
+  dense_act_bwd_kernel<<<dim3((540 + 31) / 32, 16), 256, 0, st>>>(M.dCAT2, 555, 0, M.ZF1, n, 540, P + O.a1, S.masks + 2160, 2700, M.dZF1, G + O.a1, G + O.fc1b);
+  SC_TRY((sgemm<true, false>(ctx, M.CAT, 540, M.dZF1, 540, G + O.fc1W, 540, 540, 540, n, nullptr, 0, PC_TRAIN_BWD, st)));
+  SC_TRY((sgemm<false, true>(ctx, M.dZF1, 540, P + O.fc1W, 540, M.dCAT, 540, n, 540, 540, nullptr, 0, PC_TRAIN_BWD, st)));
+  ctx->launches += 3;
+  return SC_OK;
+}
+
+// d1 (dropout f1_drop sits on the concatenated d1 activations), then conv5..conv1
+static int simt_branch_backward(sc_ctx* ctx, int b, const StepBuf& S, int n, cudaStream_t s) {
+  const BranchOff& Ob = ctx->off.br[b];
+  const auto& bb = S.simt.bb[b];
+  float* P = ctx->params;
+  float* G = ctx->grads;
+  dense_act_bwd_kernel<<<dim3((180 + 31) / 32, 16), 256, 0, s>>>(S.simt.dCAT, 540, b * 180, bb.Z1, n, 180, P + Ob.d1alpha, S.masks + 1620 + b * 180, 2700,
+                                                                bb.dZ1, G + Ob.d1alpha, G + Ob.d1b);
+  SC_TRY((sgemm<true, false>(ctx, bb.F5, 540, bb.dZ1, 180, G + Ob.d1W, 180, 540, 180, n, nullptr, 0, PC_TRAIN_BWD, s)));
+  SC_TRY((sgemm<false, true>(ctx, bb.dZ1, 180, P + Ob.d1W, 180, bb.dF5, 540, n, 540, 180, nullptr, 0, PC_TRAIN_BWD, s)));
+  ctx->launches++;
+  unflatten_drop_kernel<<<ew_grid((int64_t)n * 540), 256, 0, s>>>(bb.dF5, n, S.masks + b * 540, bb.dA);
+  ctx->launches++;
+  for (int l = 4; l >= 0; --l) {
+    const int co = kConvCout[l], ci = kConvCin[l], H = kH[l], ld = kLd[l];
+    const int pool = (l == 1 || l == 3);
+    const int pld = (l == 1) ? 16 : 8;
+    const uint8_t* idx = pool ? bb.idx[l == 1 ? 0 : 1] : nullptr;
+    const double count = (double)n * H * H;
+    SC_CUDA(cudaMemsetAsync(bb.sums, 0, 64 * 3 * sizeof(double), s));
+    bn_bwd_reduce_kernel<<<dim3(co, 32), 256, 0, s>>>(bb.X[l], bb.dA, idx, n, co, H, H, ld, pool, pld, bb.mean[l], bb.istd[l],
+                                                      P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], bb.sums);
+    bn_bwd_params_kernel<<<1, 64, 0, s>>>(bb.sums, co, G + Ob.bn[l][0], G + Ob.bn[l][1], G + Ob.alpha[l]);
+    const int pld2 = kInLd[l];   // padded map has the size of this layer's input (H+4 >= inH, same row stride)
+    if (l > 0) SC_CUDA(cudaMemsetAsync(bb.dXpad, 0, (size_t)n * co * (H + 4) * pld2 * 4, s));
+    bn_bwd_dx_kernel<<<ew_grid((int64_t)n * co * H * H), 256, 0, s>>>(bb.X[l], bb.dA, idx, n, co, H, H, ld, pool, pld, bb.mean[l], bb.istd[l],
+                                                                     P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], bb.sums, count, bb.dX,
+                                                                     l > 0 ? bb.dXpad : nullptr, pld2);
+    // wgrad against this layer's input (the previous activation, or the patches for conv1)
+    const float* lin = l == 0 ? S.in[b] : bb.A[l - 1];
+    if (l == 0) {
+      int zc = n < 32 ? n : 32;
+      conv_wgrad_kernel<<<dim3(co, ci, zc), 128, 0, s>>>(lin, ci, kInH[l], kInLd[l], bb.dX, co, H, H, ld, n, G + Ob.convW[l]);
+      ctx->launches++;
+    } else if (co == 20) {
+      SC_TRY(launch_wgrad_tiled<20>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
+    } else if (co == 40) {
+      SC_TRY(launch_wgrad_tiled<40>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
+    } else {
+      SC_TRY(launch_wgrad_tiled<60>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
+    }
+    ctx->launches += 3;
+    if (l > 0) {
+      // dgrad: d(input) = valid conv of the zero-padded dx with the raw taps, channel roles swapped
+      SC_TRY(train_conv(ctx, co, ci, bb.dXpad, H + 4, pld2, bb.dA, kInH[l], kInLd[l], bb.wd[l], n, PC_TRAIN_BWD, s));
+    }
+  }
+  return SC_OK;
+}
+
+// ---- tcgen05 back-end: the split-bf16 conv maps of train_tc.cu and the dense layers of train_dense.cu
+static int tcgen05_branch_forward(sc_ctx* ctx, int b, const StepBuf& S, int n, cudaStream_t s) {
+  const TcBranchBuf& T = S.tc[b];
+  repack_conv_kernel<<<1, 256, 0, s>>>(ctx->params + ctx->off.br[b].convW[0], 20, 1, T.wf0, nullptr);
+  ctx->launches++;
+  SC_TRY(tc_branch_forward(ctx, b, T, S.in[b], n, S.masks, s));
+  return tdense_branch_forward(ctx, b, S.td, T.F5, n, S.masks, s);
+}
+
+static int tcgen05_branch_backward(sc_ctx* ctx, int b, const StepBuf& S, int n, cudaStream_t s) {
+  SC_TRY(tdense_branch_backward(ctx, b, S.td, n, S.masks, s));
+  return tc_branch_backward(ctx, b, S.tc[b], S.in[b], S.td.dF5[b], 576, S.masks, n, s);
+}
+
+// The step body.  Every pointer it touches lives in the context (staged inputs, arena, parameter / gradient buffers), every
+// scalar that changes from step to step is read from device memory (the dropout seed), so the same sequence of launches is
+// valid as a captured CUDA graph.  The three branches are independent between the patches and the concatenation (forward)
+// and after the gradient of the concatenation (backward): they run on three streams forked from / joined into `st`.
+static int train_body(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bool injected_masks, cudaStream_t st) {
+  const bool tc = ctx->gemm_backend == 1;
   cudaStream_t sb[3] = {st, ctx->train_side[0], ctx->train_side[1]};
   cudaEvent_t* ev = ctx->train_ev;
 
-  SC_CUDA(cudaMemsetAsync(G, 0, sizeof(float) * SC_PARAM_FLOATS, st));
+  SC_CUDA(cudaMemsetAsync(ctx->grads, 0, sizeof(float) * SC_PARAM_FLOATS, st));
   SC_CUDA(cudaMemsetAsync(S.loss, 0, sizeof(float), st));
   if (!injected_masks) { make_masks_kernel<<<ew_grid((int64_t)n * 2700), 256, 0, st>>>(S.masks, (int64_t)n * 2700, S.seed); ctx->launches++; }
-  if (tc) SC_CUDA(cudaMemsetAsync(S.td.zero_begin, 0, S.td.zero_bytes, st));
   SC_CUDA(cudaEventRecord(ev[0], st));
   for (int b = 1; b < 3; ++b) SC_CUDA(cudaStreamWaitEvent(sb[b], ev[0], 0));
 
-  // ================= forward =================
+  // forward of the branches, then the head (forward and backward) on `st`
   for (int b = 0; b < 3; ++b) {
-    const BranchOff& Ob = O.br[b];
-    const auto& bb = S.bb[b];
-    cudaStream_t s = sb[b];
-    if (tc) {   // conv1..conv5 with their BatchNorm / PReLU / pools on the split-bf16 maps (train_tc.cu)
-      repack_conv_kernel<<<1, 256, 0, s>>>(P + Ob.convW[0], 20, 1, bb.wf[0], nullptr);
-      ctx->launches++;
-      SC_TRY(tc_branch_forward(ctx, b, S.tc[b], S.in[b], bb.wf[0], n, S.masks, bb.F5, s));
-    }
-    for (int l = 0; l < 5 && !tc; ++l) {
-      const int co = kConvCout[l], ci = kConvCin[l];
-      repack_conv_kernel<<<(co * ci * 9 + 255) / 256, 256, 0, s>>>(P + Ob.convW[l], co, ci, bb.wf[l], bb.wd[l]);
-      ctx->launches++;
-      if (l == 0) {
-        SC_TRY(launch_conv1_patches(ctx, S.in[b], n, bb.wf[0], ones, zeros, ones, bb.X[0], s));
-      } else {
-        SC_TRY(train_conv(ctx, ci, co, bb.A[l - 1], kInH[l], kInLd[l], bb.X[l], kH[l], kLd[l], bb.wf[l], n, PC_TRAIN_FWD, s));
-      }
-      SC_CUDA(cudaMemsetAsync(bb.sums, 0, 64 * 3 * sizeof(double), s));
-      bn_stats_kernel<<<dim3(co, 32), 256, 0, s>>>(bb.X[l], n, co, kH[l], kH[l], kLd[l], bb.sums);
-      bn_finalize_kernel<<<1, 64, 0, s>>>(bb.sums, co, (double)n * kH[l] * kH[l], bb.mean[l], bb.istd[l], G + Ob.bn[l][2], G + Ob.bn[l][3]);
-      const int pool = (l == 1 || l == 3);
-      const int oh = pool ? kH[l] / 2 : kH[l];
-      const int old = (l == 1) ? 16 : (l == 3) ? 8 : kLd[l];
-      bn_act_kernel<<<ew_grid((int64_t)n * co * oh * oh), 256, 0, s>>>(bb.X[l], n, co, kH[l], kH[l], kLd[l], bb.mean[l], bb.istd[l],
-                                                                     P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], pool, bb.A[l], oh, oh, old,
-                                                                     pool ? bb.idx[l == 1 ? 0 : 1] : nullptr);
-      ctx->launches += 3;
-    }
-    if (tc) {
-      SC_TRY(tdense_branch_forward(ctx, b, S.td, bb.F5, n, S.masks, s));
-    } else {
-      flatten_drop_kernel<<<ew_grid((int64_t)n * 540), 256, 0, s>>>(bb.A[4], n, S.masks + b * 540, bb.F5);
-      SC_TRY((sgemm<false, false>(ctx, bb.F5, 540, P + Ob.d1W, 180, bb.Z1, 180, n, 180, 540, P + Ob.d1b, 0, PC_TRAIN_FWD, s)));
-      dense_act_kernel<<<ew_grid((int64_t)n * 180), 256, 0, s>>>(bb.Z1, n, 180, P + Ob.d1alpha, S.masks + 1620 + b * 180, 2700, S.CAT, 540, b * 180);
-      ctx->launches += 2;
-    }
-    if (b > 0) { SC_CUDA(cudaEventRecord(ev[b], s)); SC_CUDA(cudaStreamWaitEvent(st, ev[b], 0)); }
+    SC_TRY(tc ? tcgen05_branch_forward(ctx, b, S, n, sb[b]) : simt_branch_forward(ctx, b, S, n, sb[b]));
+    if (b > 0) { SC_CUDA(cudaEventRecord(ev[b], sb[b])); SC_CUDA(cudaStreamWaitEvent(st, ev[b], 0)); }
   }
-  if (tc) SC_TRY(tdense_head(ctx, S.td, S.in4, S.y, n, n_global, S.masks, S.loss, st));
-  if (!tc) {
-  SC_TRY((sgemm<false, false>(ctx, S.CAT, 540, P + O.fc1W, 540, S.ZF1, 540, n, 540, 540, P + O.fc1b, 0, PC_TRAIN_FWD, st)));
-  dense_act_kernel<<<ew_grid((int64_t)n * 540), 256, 0, st>>>(S.ZF1, n, 540, P + O.a1, S.masks + 2160, 2700, S.CAT2, 555, 0);
-  SC_CUDA(cudaMemcpy2DAsync(S.CAT2 + 540, 555 * 4, S.in4, 15 * 4, 15 * 4, n, cudaMemcpyDeviceToDevice, st));
-  SC_TRY((sgemm<false, false>(ctx, S.CAT2, 555, P + O.fc2W, 270, S.ZF2, 270, n, 270, 555, P + O.fc2b, 0, PC_TRAIN_FWD, st)));
-  dense_act_kernel<<<ew_grid((int64_t)n * 270), 256, 0, st>>>(S.ZF2, n, 270, P + O.a2, nullptr, 0, S.H2, 270, 0);
-  SC_TRY((sgemm<false, false>(ctx, S.H2, 270, P + O.outW, 15, S.ZO, 15, n, 15, 270, P + O.outb, 0, PC_TRAIN_FWD, st)));
-  softmax_ce_kernel<<<(n + 127) / 128, 128, 0, st>>>(S.ZO, S.y, n, 1.f / (float)n_global, S.dZO, S.loss);
-  ctx->launches += 3;
-
-  // ================= backward =================
-  // out layer
-  SC_TRY((sgemm<true, false>(ctx, S.H2, 270, S.dZO, 15, G + O.outW, 15, 270, 15, n, nullptr, 0, PC_TRAIN_BWD, st)));
-  colsum_kernel<<<dim3(1, 32), 32, 0, st>>>(S.dZO, n, 15, G + O.outb);
-  SC_TRY((sgemm<false, true>(ctx, S.dZO, 15, P + O.outW, 15, S.dH2, 270, n, 270, 15, nullptr, 0, PC_TRAIN_BWD, st)));
-  // fc_2
-  dense_act_bwd_kernel<<<dim3((270 + 31) / 32, 16), 256, 0, st>>>(S.dH2, 270, 0, S.ZF2, n, 270, P + O.a2, nullptr, 0, S.dZF2, G + O.a2, G + O.fc2b);
-  SC_TRY((sgemm<true, false>(ctx, S.CAT2, 555, S.dZF2, 270, G + O.fc2W, 270, 555, 270, n, nullptr, 0, PC_TRAIN_BWD, st)));
-  SC_TRY((sgemm<false, true>(ctx, S.dZF2, 270, P + O.fc2W, 270, S.dCAT2, 555, n, 555, 270, nullptr, 0, PC_TRAIN_BWD, st)));
-  // FC1 (dropout f2_drop sits on its activation)
-  dense_act_bwd_kernel<<<dim3((540 + 31) / 32, 16), 256, 0, st>>>(S.dCAT2, 555, 0, S.ZF1, n, 540, P + O.a1, S.masks + 2160, 2700, S.dZF1, G + O.a1, G + O.fc1b);
-  SC_TRY((sgemm<true, false>(ctx, S.CAT, 540, S.dZF1, 540, G + O.fc1W, 540, 540, 540, n, nullptr, 0, PC_TRAIN_BWD, st)));
-  SC_TRY((sgemm<false, true>(ctx, S.dZF1, 540, P + O.fc1W, 540, S.dCAT, 540, n, 540, 540, nullptr, 0, PC_TRAIN_BWD, st)));
-  ctx->launches += 3;
-  }
+  SC_TRY(tc ? tdense_head(ctx, S.td, S.in4, S.y, n, n_global, S.masks, S.loss, st) : simt_head(ctx, S, n, n_global, st));
   SC_CUDA(cudaEventRecord(ev[3], st));
   for (int b = 1; b < 3; ++b) SC_CUDA(cudaStreamWaitEvent(sb[b], ev[3], 0));
 
+  // backward of the branches
   for (int b = 0; b < 3; ++b) {
-    const BranchOff& Ob = O.br[b];
-    const auto& bb = S.bb[b];
-    cudaStream_t s = sb[b];
-    // d1 (dropout f1_drop sits on the concatenated d1 activations)
-    if (tc) {
-      SC_TRY(tdense_branch_backward(ctx, b, S.td, n, S.masks, s));
-      SC_TRY(tc_branch_backward(ctx, b, S.tc[b], S.in[b], S.td.dF5[b], 576, S.masks, n, s));
-    } else {
-      dense_act_bwd_kernel<<<dim3((180 + 31) / 32, 16), 256, 0, s>>>(S.dCAT, 540, b * 180, bb.Z1, n, 180, P + Ob.d1alpha, S.masks + 1620 + b * 180, 2700,
-                                                                    bb.dZ1, G + Ob.d1alpha, G + Ob.d1b);
-      SC_TRY((sgemm<true, false>(ctx, bb.F5, 540, bb.dZ1, 180, G + Ob.d1W, 180, 540, 180, n, nullptr, 0, PC_TRAIN_BWD, s)));
-      SC_TRY((sgemm<false, true>(ctx, bb.dZ1, 180, P + Ob.d1W, 180, bb.dF5, 540, n, 540, 180, nullptr, 0, PC_TRAIN_BWD, s)));
-      ctx->launches++;
-      unflatten_drop_kernel<<<ew_grid((int64_t)n * 540), 256, 0, s>>>(bb.dF5, n, S.masks + b * 540, bb.dA);
-      ctx->launches++;
-    }
-    for (int l = 4; l >= 0 && !tc; --l) {
-      const int co = kConvCout[l], ci = kConvCin[l], H = kH[l], ld = kLd[l];
-      const int pool = (l == 1 || l == 3);
-      const int pld = (l == 1) ? 16 : 8;
-      const uint8_t* idx = pool ? bb.idx[l == 1 ? 0 : 1] : nullptr;
-      const double count = (double)n * H * H;
-      SC_CUDA(cudaMemsetAsync(bb.sums, 0, 64 * 3 * sizeof(double), s));
-      bn_bwd_reduce_kernel<<<dim3(co, 32), 256, 0, s>>>(bb.X[l], bb.dA, idx, n, co, H, H, ld, pool, pld, bb.mean[l], bb.istd[l],
-                                                        P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], bb.sums);
-      bn_bwd_params_kernel<<<1, 64, 0, s>>>(bb.sums, co, G + Ob.bn[l][0], G + Ob.bn[l][1], G + Ob.alpha[l]);
-      const int pld2 = kInLd[l];   // padded map has the size of this layer's input (H+4 >= inH, same row stride)
-      if (l > 0) SC_CUDA(cudaMemsetAsync(bb.dXpad, 0, (size_t)n * co * (H + 4) * pld2 * 4, s));
-      bn_bwd_dx_kernel<<<ew_grid((int64_t)n * co * H * H), 256, 0, s>>>(bb.X[l], bb.dA, idx, n, co, H, H, ld, pool, pld, bb.mean[l], bb.istd[l],
-                                                                       P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], bb.sums, count, bb.dX,
-                                                                       l > 0 ? bb.dXpad : nullptr, pld2);
-      // wgrad against this layer's input (the previous activation, or the patches for conv1)
-      const float* lin = l == 0 ? S.in[b] : bb.A[l - 1];
-      if (l == 0) {
-        int zc = n < 32 ? n : 32;
-        conv_wgrad_kernel<<<dim3(co, ci, zc), 128, 0, s>>>(lin, ci, kInH[l], kInLd[l], bb.dX, co, H, H, ld, n, G + Ob.convW[l]);
-        ctx->launches++;
-      } else if (co == 20) {
-        SC_TRY(launch_wgrad_tiled<20>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
-      } else if (co == 40) {
-        SC_TRY(launch_wgrad_tiled<40>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
-      } else {
-        SC_TRY(launch_wgrad_tiled<60>(ctx, lin, ci, kInH[l], kInLd[l], bb.dX, H, ld, n, G + Ob.convW[l], s));
-      }
-      ctx->launches += 3;
-      if (l > 0) {
-        // dgrad: d(input) = valid conv of the zero-padded dx with the raw taps, channel roles swapped
-        SC_TRY(train_conv(ctx, co, ci, bb.dXpad, H + 4, pld2, bb.dA, kInH[l], kInLd[l], bb.wd[l], n, PC_TRAIN_BWD, s));
-      }
-    }
-    if (b > 0) { SC_CUDA(cudaEventRecord(ev[3 + b], s)); SC_CUDA(cudaStreamWaitEvent(st, ev[3 + b], 0)); }
+    SC_TRY(tc ? tcgen05_branch_backward(ctx, b, S, n, sb[b]) : simt_branch_backward(ctx, b, S, n, sb[b]));
+    if (b > 0) { SC_CUDA(cudaEventRecord(ev[3 + b], sb[b])); SC_CUDA(cudaStreamWaitEvent(st, ev[3 + b], 0)); }
   }
   SC_CUDA(cudaGetLastError());
   return SC_OK;
@@ -873,6 +884,8 @@ int train_forward_backward(sc_ctx* ctx, const float* in1, const float* in2, cons
   if (masks_in) SC_CUDA(cudaMemcpyAsync(S.masks, masks_in, (size_t)n * 2700, cudaMemcpyDeviceToDevice, st));
   const unsigned long long seed_h = seed;
   SC_CUDA(cudaMemcpyAsync(S.seed, &seed_h, sizeof(seed_h), cudaMemcpyHostToDevice, st));   // pageable source: staged before the call returns
+  // the split dense operands of the tcgen05 step: the step writes their valid entries only, the K padding must read as zero
+  if (tc) SC_CUDA(cudaMemsetAsync(S.td.zero_begin, 0, S.td.zero_bytes, st));
 
   const bool use_graph = ctx->train_graph_on && !ctx->profile && !(tc && ctx->ar_hook);   // the sync-BN hook runs host code between kernels
   if (!use_graph) {

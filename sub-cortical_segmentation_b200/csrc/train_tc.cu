@@ -10,11 +10,7 @@
 //       wgrad    conv2..conv5   = wgrad_mn_kernel below: an implicit GEMM whose K dimension is the PIXEL axis
 //                                 (gW[tap][ci][co] = sum_p A[p + shift(tap)][ci] * dX[p][co]) with both operands MN-major, read
 //                                 straight from the pixel-major maps (a TMA box of a map IS the canonical MN-major operand; a tap
-//                                 is a shift of the outer TMA coordinate / a row-shifted descriptor start).  Its predecessor
-//                                 wgrad_tc_kernel (sc_set_option "train_wgrad_mn" = 0) reads K-major operands from channel-major
-//                                 ("planar transposed") bf16 hi/lo copies that the element-wise kernels then write next to the
-//                                 pixel-major maps -- the gradient three times, shifted by 0, 1 and 2 pixels, because a filter
-//                                 COLUMN would be a 2-byte shift of the innermost TMA coordinate, which must stay 16-byte aligned
+//                                 is a shift of the outer TMA coordinate / a row-shifted descriptor start)
 //   * every product is the bf16x3 split (xl*wh + xh*wl + xh*wh, fp32 accumulate in TMEM), like inference
 //   * BatchNorm statistics / activation / pooling and their backward passes are element-wise kernels over the split maps
 // conv1 (K = 9) stays on CUDA cores.  The dense layers are in train_dense.cu.
@@ -229,8 +225,7 @@ __device__ __forceinline__ void bn_moments_cta(const double* __restrict__ sums, 
 
 // ---------------------------------------------------------------------------------------------------------------
 // y = (x - mean) * gamma * istd + beta; a = prelu(y); optional 2x2 / 2 max-pool with arg-max record.
-// Writes the activation map (pixel-major split, the next conv's input) and its planar transposed copy
-// AT[2 * CP][Npix] (rows 0..CP-1 hi, CP..2CP-1 lo: the wgrad operand), zeros outside the valid region.
+// Writes the activation map (pixel-major split: the next conv's input and the wgrad operand), zeros outside the valid region.
 // One CTA = 64 consecutive positions of the OUTPUT map x all channel chunks.
 // ---------------------------------------------------------------------------------------------------------------
 template <int FMT>
@@ -241,9 +236,8 @@ __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 5 : 2) tbn_act_ker
                                                                   const float* __restrict__ gamma, const float* __restrict__ beta,
                                                                   const float* __restrict__ alpha, int pool,
                                                                   float* __restrict__ A, int oR, int oPitch, int oH,
-                                                                  uint8_t* __restrict__ idx, uint16_t* __restrict__ AT, int CP) {
+                                                                  uint8_t* __restrict__ idx) {
   constexpr int NCH = FMT / 8;
-  __shared__ uint16_t tile[2][FMT][66];
   __shared__ float s_mu[64], s_is[64];
   if (cnt) count = *cnt;
   bn_moments_cta(sums, count, C, s_mu, s_is, mean, istd, g_mean_slot, g_istd_slot);
@@ -293,32 +287,6 @@ __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 5 : 2) tbn_act_ker
     uint4 h, l;
     split8(a, h, l);
     store8<FMT>(A, q, chunk, h, l);
-    if (AT) {
-      const uint32_t hh[4] = {h.x, h.y, h.z, h.w}, ll[4] = {l.x, l.y, l.z, l.w};
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        tile[0][chunk * 8 + 2 * k][px] = (uint16_t)(hh[k] & 0xffffu); tile[0][chunk * 8 + 2 * k + 1][px] = (uint16_t)(hh[k] >> 16);
-        tile[1][chunk * 8 + 2 * k][px] = (uint16_t)(ll[k] & 0xffffu); tile[1][chunk * 8 + 2 * k + 1][px] = (uint16_t)(ll[k] >> 16);
-      }
-    }
-  } else if (AT) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { tile[0][chunk * 8 + k][px] = 0; tile[1][chunk * 8 + k][px] = 0; }
-  }
-  if (!AT) return;       // the MN-major wgrad reads the pixel-major map itself: no planar transposed copy
-  __syncthreads();
-  {
-    // rows of 64 positions (128 B) per channel: one warp per row, lane = two positions
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-    const int64_t q0 = (int64_t)blockIdx.x * 64;
-    for (int row = warp; row < 2 * CP; row += nw) {
-      const int half = row / CP, ch = row - half * CP;
-      const int64_t qa = q0 + 2 * lane;
-      if (qa < npix) {   // npix is even
-        const uint32_t v = (uint32_t)tile[half][ch][2 * lane] | ((uint32_t)tile[half][ch][2 * lane + 1] << 16);
-        *reinterpret_cast<uint32_t*>(AT + (int64_t)row * npix + qa) = v;
-      }
-    }
   }
 }
 
@@ -445,12 +413,9 @@ __global__ void tbn_bwd_params_kernel(const double* __restrict__ sums, int C, fl
   bn_publish_grads(sums, C, gbeta, ggamma, galpha);
 }
 
-// pass 2 over ALL positions of the conv-output map (64 consecutive positions per CTA):
-//   frame   (l >= 1): dx as a split map of the same geometry, zeros outside the valid region = the dgrad sweep's input
-//                     (the sweep reads it with a window offset of (-2, -2): full correlation, zero fill by the TMA unit)
-//   DT      (l >= 1): three planar transposed copies [3][2 * CP][Npix], copy k shifted right by k positions
-//                     (DT_k[p] = dx[p - k]), zeros outside the valid region = the wgrad operand of filter column k
-//   planar  (l == 0): fp32 [n][C][H][ld] for the CUDA-core conv1 wgrad
+// pass 2 over ALL positions of the conv-output map (64 consecutive positions per CTA), conv2..conv5: dx as a split map of the same
+// geometry, zeros outside the valid region = the wgrad operand and the dgrad sweep's input (the sweep reads it with a window
+// offset of (-2, -2): full correlation, zero fill by the TMA unit)
 template <int FMT, int DFMT>
 __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 6 : 3) tbn_bwd_dx_kernel(const float* __restrict__ X, const float* __restrict__ dA, const uint8_t* __restrict__ idx,
                                                                      const float* __restrict__ dF5, int dF5_ld, const uint8_t* __restrict__ mask,
@@ -460,12 +425,10 @@ __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 6 : 3) tbn_bwd_dx_
                                                                      const float* __restrict__ alpha, const double* __restrict__ sums, double count,
                                                                      const double* __restrict__ cnt,
                                                                      float* __restrict__ gbeta, float* __restrict__ ggamma, float* __restrict__ galpha,
-                                                                     float* __restrict__ frame, uint16_t* __restrict__ DT, int CP,
-                                                                     float* __restrict__ planar, int pld) {
+                                                                     float* __restrict__ frame) {
   constexpr int NCH = FMT / 8;
   if (cnt) count = *cnt;
   bn_publish_grads(sums, C, gbeta, ggamma, galpha);
-  __shared__ uint16_t tile[2][FMT][68];     // columns 0..63: this CTA's positions; 64, 65: the two positions to their left
   // per-channel constants once per CTA: the two double divisions per channel cost more than the rest of a thread's work (issuing the
   // map loads before this barrier was tried: the longer live ranges cost more occupancy than the overlap gains)
   __shared__ float s_k[64][5];              // mean, istd, gamma, beta, alpha
@@ -479,18 +442,16 @@ __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 6 : 3) tbn_bwd_dx_
     s_m[ch][1] = on ? (float)(sums[ch * 3 + 1] / count) : 0.f;
   }
   __syncthreads();
-  const int chunk = threadIdx.x % NCH, px = threadIdx.x / NCH;
-  const int64_t npix = (int64_t)R * Pw;
-  const int64_t q0 = (int64_t)blockIdx.x * 64;
-  // dx of position q (zeros outside the valid region / the map) -> returns whether q is a valid position of this chunk
-  auto point = [&](int64_t q, float (&dx)[8], int& r, int& s, int& c) {
+  const int chunk = threadIdx.x % NCH;
+  const int64_t q = (int64_t)blockIdx.x * 64 + threadIdx.x / NCH;
+  if (q >= (int64_t)R * Pw) return;
+  const int c = (int)(q % pitch);
+  const int s = (int)((q / pitch) % n);
+  const int r = (int)(q / Pw);
+  float dx[8];
 #pragma unroll
-    for (int k = 0; k < 8; ++k) dx[k] = 0.f;
-    if (q < 0 || q >= npix) return false;
-    c = (int)(q % pitch);
-    s = (int)((q / pitch) % n);
-    r = (int)(q / Pw);
-    if (!(r < H && c < H && chunk * 8 < C)) return false;
+  for (int k = 0; k < 8; ++k) dx[k] = 0.f;
+  if (r < H && c < H && chunk * 8 < C) {
     float x[8], g[8];
     bwd_point<FMT, DFMT>(X, dA, idx, dF5, dF5_ld, mask, n, C, Pw, pitch, pool, dPw, dPitch, r, s, c, chunk, x, g);
 #pragma unroll
@@ -504,57 +465,10 @@ __global__ void __launch_bounds__(64 * (FMT / 8), FMT == 32 ? 6 : 3) tbn_bwd_dx_
         dx[k] = ga * is * (dy - s_m[ch][0] - xh * s_m[ch][1]);
       }
     }
-    return true;
-  };
-  auto to_tile = [&](const uint4& h, const uint4& l, int col) {
-    const uint32_t hh[4] = {h.x, h.y, h.z, h.w}, ll[4] = {l.x, l.y, l.z, l.w};
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      tile[0][chunk * 8 + 2 * k][col] = (uint16_t)(hh[k] & 0xffffu); tile[0][chunk * 8 + 2 * k + 1][col] = (uint16_t)(hh[k] >> 16);
-      tile[1][chunk * 8 + 2 * k][col] = (uint16_t)(ll[k] & 0xffffu); tile[1][chunk * 8 + 2 * k + 1][col] = (uint16_t)(ll[k] >> 16);
-    }
-  };
-  const int64_t q = q0 + px;
-  float dx[8];
-  int r = 0, s = 0, c = 0;
-  const bool valid = point(q, dx, r, s, c);
-  if (planar) {
-    if (valid) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        const int ch = chunk * 8 + k;
-        if (ch < C) planar[(((int64_t)s * C + ch) * H + r) * pld + c] = dx[k];
-      }
-    }
-    return;
   }
   uint4 h, l;
   split8(dx, h, l);
-  if (q < npix) store8<FMT>(frame, q, chunk, h, l);
-  if (!DT) return;       // wgrad reads the pixel-major frame itself (wgrad_mn_kernel): no planar copies
-  to_tile(h, l, px);
-  if (px < 2) {          // the shifted copies of this CTA's 64 positions start one / two positions to the left: recompute those two
-    float dh[8];
-    int r2, s2, c2;
-    point(q0 - 2 + px, dh, r2, s2, c2);
-    uint4 h2, l2;
-    split8(dh, h2, l2);
-    to_tile(h2, l2, 64 + px);
-  }
-  __syncthreads();
-  // DT_k[p] = dx[p - k]: every copy is written as whole aligned 128 B rows (two positions per lane)
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  const int64_t qa = q0 + 2 * lane;
-  if (qa < npix) {     // npix is even
-    for (int row = warp; row < 2 * CP; row += nw) {
-      const int half = row / CP, ch = row - half * CP;
-      const uint16_t* t = tile[half][ch];
-      const uint32_t m2 = lane ? t[2 * lane - 2] : t[64], m1 = lane ? t[2 * lane - 1] : t[65], v0 = t[2 * lane], v1 = t[2 * lane + 1];
-      *reinterpret_cast<uint32_t*>(DT + (int64_t)row * npix + qa) = v0 | (v1 << 16);
-      *reinterpret_cast<uint32_t*>(DT + ((int64_t)2 * CP + row) * npix + qa) = m1 | (v0 << 16);
-      *reinterpret_cast<uint32_t*>(DT + ((int64_t)4 * CP + row) * npix + qa) = m2 | (m1 << 16);
-    }
-  }
+  store8<FMT>(frame, q, chunk, h, l);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -637,191 +551,7 @@ __global__ void __launch_bounds__(256, 2) tbn_bwd_conv1_kernel(const float* __re
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// wgrad on the tensor cores.  With p' = p + tx:
-//   gW[ty][tx][ci][co] = sum_p A[ci][p + ty*Pw + tx] * dX[co][p] = sum_p' A[ci][p' + ty*Pw] * DT_tx[co][p']
-//   A operand (M): the three row-shifted windows of the planar input map, stacked: 3 x CIN8 <= 120 rows of one M = 128 tile
-//   B operand (N): the three column-shifted copies DT_tx of the planar output gradient stacked, 3 x NCO rows: ONE MMA per
-//                   k-step and split term produces all three filter columns (the A tile is fetched once instead of thrice)
-//   K: 64 pixels per stage; the CTAs split the pixel range (split-K) and add their partial sums atomically
-// warp 0: TMA producer (12 boxes per stage), warp 1: MMA issue (3 accumulators x 4 k-steps x 3 split products), warps 2-5: epilogue
-// ---------------------------------------------------------------------------------------------------------------
-static inline int pad8(int c) { return (c + 7) & ~7; }
-static inline int pad16(int c) { return (c + 15) & ~15; }
-
-struct WgradArgs {
-  int cin, cout, cin8, nco;      // real channels, input rows per window (multiple of 8), gradient rows per copy in shared memory (multiple of 16)
-  int co8;                       // gradient rows per copy as stored / loaded (multiple of 8): the rows [co8, nco) of a slot are never
-                                 // written and only feed accumulator columns nobody reads
-  int Pw;                        // wide-row pitch in pixels: filter row = shift by Pw
-  int nkb;                       // 64-pixel blocks to reduce over
-  int stages;
-  float* gW;                     // [cout][cin][3][3] master-layout gradient (accumulated atomically)
-};
-
-__global__ void __launch_bounds__(192, 1)
-wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapD, const WgradArgs a) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  const int a_half = 3 * a.cin8 * 128;                    // bytes of the stacked hi (or lo) windows
-  const int d_one = a.nco * 128, d_half = 3 * d_one;      // one shifted copy; the three hi (or lo) copies
-  const int stage_bytes = 2 * a_half + 2 * d_half;        // (the M = 128 tile of the lo windows reads on into the gradient boxes)
-  const int tx_bytes = 2 * a_half + 2 * 3 * a.co8 * 128;  // bytes the TMA unit actually delivers per stage
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + a.stages * stage_bytes);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + a.stages;
-  uint64_t* done = bars + 2 * a.stages;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(done + 1);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // this CTA's share of the pixel blocks
-  const int per = (a.nkb + gridDim.x - 1) / gridDim.x;
-  const int kb0 = blockIdx.x * per, kb1 = min(a.nkb, kb0 + per);
-  const int nk = kb1 - kb0;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < a.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    mbar_init(done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(256) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (nk > 0) {
-    if (warp == 0) {
-      if (lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapA)) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&mapD)) : "memory");
-        for (int i = 0; i < nk; ++i) {
-          const int s = i % a.stages, use = i / a.stages;
-          if (use > 0) mbar_wait(&empty[s], (use - 1) & 1);
-          mbar_expect_tx(&full[s], (uint32_t)tx_bytes);
-          uint8_t* sp = smem + s * stage_bytes;
-          const int p0 = (kb0 + i) * 64;
-#pragma unroll 1
-          for (int t = 0; t < 3; ++t) {
-            tma_load_2d(&mapA, &full[s], sp + t * a.cin8 * 128, p0 + t * a.Pw, 0);                 // window of filter row t, hi rows
-            tma_load_2d(&mapA, &full[s], sp + a_half + t * a.cin8 * 128, p0 + t * a.Pw, a.cin8);   // lo rows
-            tma_load_2d(&mapD, &full[s], sp + 2 * a_half + t * d_one, p0, t * 2 * a.co8);          // copy shifted by t, hi rows
-            tma_load_2d(&mapD, &full[s], sp + 2 * a_half + d_half + t * d_one, p0, t * 2 * a.co8 + a.co8);
-          }
-        }
-      }
-      __syncwarp();
-    } else if (warp == 1) {
-      const uint32_t leader = elect_one();
-      // D = F32, A = B = BF16, both K-major, N = 3 * nco (the three shifted copies are adjacent row blocks), M = 128
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)((3 * a.nco) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-      for (int i = 0; i < nk; ++i) {
-        const int s = i % a.stages;
-        mbar_wait(&full[s], (i / a.stages) & 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t sp = smem_u32(smem + s * stage_bytes);
-        const uint64_t ah = umma_desc(sp), al = umma_desc(sp + a_half);
-        const uint64_t dh = umma_desc(sp + 2 * a_half), dl = umma_desc(sp + 2 * a_half + d_half);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const uint64_t o = (uint64_t)(j * 2);
-          umma_bf16_elect(tmem_base, al + o, dh + o, idesc, (i | j) != 0, leader);
-          umma_bf16_elect(tmem_base, ah + o, dl + o, idesc, 1, leader);
-          umma_bf16_elect(tmem_base, ah + o, dh + o, idesc, 1, leader);
-        }
-        if (leader) umma_commit(&empty[s]);
-        __syncwarp();
-      }
-      if (leader) umma_commit(done);
-      __syncwarp();
-    } else {
-      const int q = warp & 3;      // TMEM lane quarter this warp may read
-      mbar_wait(done, 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const int row = q * 32 + lane;
-      const int ty = row / a.cin8, ci = row - ty * a.cin8;
-      const bool on = ty < 3 && ci < a.cin;
-      for (int tx = 0; tx < 3; ++tx) {
-        for (int c0 = 0; c0 < a.nco; c0 += 16) {
-          uint32_t rr[16];
-          const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(tx * a.nco + c0);
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-              : "=r"(rr[0]), "=r"(rr[1]), "=r"(rr[2]), "=r"(rr[3]), "=r"(rr[4]), "=r"(rr[5]), "=r"(rr[6]), "=r"(rr[7]), "=r"(rr[8]),
-                "=r"(rr[9]), "=r"(rr[10]), "=r"(rr[11]), "=r"(rr[12]), "=r"(rr[13]), "=r"(rr[14]), "=r"(rr[15])
-              : "r"(taddr));
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-          if (on) {
-#pragma unroll
-            for (int k = 0; k < 16; ++k) {
-              const int co = c0 + k;
-              // tap t of the correlation = element 8 - t of the (true-convolution) filter
-              if (co < a.cout) atomicAdd(a.gW + ((int64_t)co * a.cin + ci) * 9 + (8 - (ty * 3 + tx)), __uint_as_float(rr[k]));
-            }
-          }
-        }
-      }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    }
-  }
-  __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256) : "memory");
-  }
-}
-
-static int launch_wgrad_tc(sc_ctx* ctx, const uint16_t* AT, const uint16_t* DT, int cin, int cout, int cin8, int nco, int Pw, int64_t npix,
-                           int rows_valid, float* gW, cudaStream_t st) {
-  TcState* s = reinterpret_cast<TcState*>(ctx->tc_state);
-  SC_CHECK(s != nullptr, SC_ERR_UNSUPPORTED, "tcgen05 back-end not initialised");
-  SC_CHECK(npix % 8 == 0 && Pw % 8 == 0 && npix < (1ll << 31), SC_ERR_ARG, "wgrad_tc: bad map size");
-  SC_CHECK(3 * cin8 <= 128 && nco <= 64 && nco % 16 == 0 && cin8 % 8 == 0, SC_ERR_ARG, "wgrad_tc: bad channel geometry");
-  WgradArgs a;
-  a.cin = cin; a.cout = cout; a.cin8 = cin8; a.nco = nco; a.Pw = Pw; a.gW = gW;
-  a.co8 = pad8(cout);
-  a.nkb = (int)(((int64_t)rows_valid * Pw + 2 + 63) / 64);  // the (shifted) gradient is zero beyond its valid rows
-  const int stage_bytes = 2 * 3 * cin8 * 128 + 2 * 3 * nco * 128;
-  a.stages = (227 * 1024 - 2048) / stage_bytes;
-  if (a.stages > 6) a.stages = 6;
-  SC_CHECK(a.stages >= 2, SC_ERR_ARG, "wgrad_tc: stage does not fit (%d bytes)", stage_bytes);
-  const size_t smem = 1024 + (size_t)a.stages * stage_bytes + (2 * a.stages + 1) * 8 + 16;
-  CUtensorMap mapA, mapD;
-  {
-    cuuint64_t dims[2] = {(cuuint64_t)npix, (cuuint64_t)(2 * cin8)};
-    cuuint64_t strides[1] = {(cuuint64_t)npix * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)cin8};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = s->encode(&mapA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<uint16_t*>(AT), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    SC_CHECK(r == CUDA_SUCCESS, SC_ERR_CUDA, "wgrad_tc: cuTensorMapEncodeTiled(A) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[2] = {(cuuint64_t)npix, (cuuint64_t)(3 * 2 * a.co8)};
-    cuuint64_t strides[1] = {(cuuint64_t)npix * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)a.co8};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = s->encode(&mapD, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<uint16_t*>(DT), dims, strides, box, es,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    SC_CHECK(r == CUDA_SUCCESS, SC_ERR_CUDA, "wgrad_tc: cuTensorMapEncodeTiled(D) failed with %d", (int)r);
-  }
-  SC_TRY(ensure_smem_attr(ctx, reinterpret_cast<const void*>(wgrad_tc_kernel), 227 * 1024));
-  // at least ~6 pixel blocks per CTA: the epilogue (up to 120 x 3 x 60 atomics per CTA) must not dominate
-  int grid = (a.nkb + 5) / 6;
-  if (grid > ctx->sm_count) grid = ctx->sm_count;
-  if (grid < 1) grid = 1;
-  ProfScope prof(ctx, PC_TRAIN_BWD, st);
-  wgrad_tc_kernel<<<grid, 192, smem, st>>>(mapA, mapD, a);
-  ctx->launches++;
-  SC_CUDA(cudaGetLastError());
-  return SC_OK;
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// wgrad straight from the PIXEL-major split maps (no planar copies): both operands MN-major.
+// wgrad straight from the PIXEL-major split maps: both operands MN-major.
 //   gW[ty][tx][ci][co] = sum_p A[p + ty*Pw + tx][ci] * dX[p][co]
 // A TMA box of 64 bf16 x 64 pixels of a split map is, in shared memory, 64 K-rows (pixels) of 128 B holding 64 "MN" elements:
 // exactly the canonical MN-major SWIZZLE_128B operand (8-row groups 1024 B apart = SBO; further 64-element MN chunks LBO apart).
@@ -1036,7 +766,6 @@ size_t tc_branch_bytes(int n) {
     if (l < 4) {
       const size_t opx = (size_t)L.oR * n * L.oPitch;
       b += al(opx * L.fmt * 4);                                    // A_l
-      b += al(opx * 2 * pad8(L.cout) * 2);                         // A_l planar transposed (hi | lo)
       if (L.pool) b += al(opx * (L.fmt / 8) * 2);                  // arg-max record
     }
     b += 2 * 1024;                                                 // mean, istd
@@ -1044,8 +773,7 @@ size_t tc_branch_bytes(int n) {
   const size_t big32 = (size_t)30 * n * 32 * 128, big64 = (size_t)15 * n * 16 * 256;
   const size_t big = big32 > big64 ? big32 : big64;
   b += 2 * al(big);                                                // frame, dA
-  b += al((size_t)30 * n * 32 * 3 * 2 * 32 * 2);                   // DT: three shifted copies (largest: conv2, 3 x 2 x 32 rows)
-  b += al((size_t)n * 20 * 30 * 32 * 4);                           // planar fp32 dX of conv1
+  b += al(180 * 4) + al((size_t)n * 540 * 4);                      // conv1 taps, F5
   b += al(10 * kSumsStride * 8) + 1024 * 4;                        // BatchNorm reduction buffers
   return b;
 }
@@ -1060,10 +788,9 @@ int tc_carve_branch(TcBranchBuf& T, char* base, int n) {
     if (l < 4) {
       const size_t opx = (size_t)L.oR * n * L.oPitch;
       T.A[l] = reinterpret_cast<float*>(take(opx * L.fmt * 4));
-      T.AT[l] = reinterpret_cast<uint16_t*>(take(opx * 2 * pad8(L.cout) * 2));
       T.idx[l] = L.pool ? reinterpret_cast<uint8_t*>(take(opx * (L.fmt / 8) * 2)) : nullptr;
     } else {
-      T.A[l] = nullptr; T.AT[l] = nullptr; T.idx[l] = nullptr;
+      T.A[l] = nullptr; T.idx[l] = nullptr;
     }
     T.mean[l] = reinterpret_cast<float*>(take(256));
     T.istd[l] = reinterpret_cast<float*>(take(256));
@@ -1072,11 +799,13 @@ int tc_carve_branch(TcBranchBuf& T, char* base, int n) {
   const size_t big = big32 > big64 ? big32 : big64;
   T.frame = reinterpret_cast<float*>(take(big));
   T.dA = reinterpret_cast<float*>(take(big));
-  T.DT = reinterpret_cast<uint16_t*>(take((size_t)30 * n * 32 * 3 * 2 * 32 * 2));
-  T.dX0 = reinterpret_cast<float*>(take((size_t)n * 20 * 30 * 32 * 4));
+  T.wf0 = reinterpret_cast<float*>(take(180 * 4));
+  T.F5 = reinterpret_cast<float*>(take((size_t)n * 540 * 4));
   T.sums = reinterpret_cast<double*>(take(10 * kSumsStride * 8));   // per layer, forward (l) and backward (5 + l): [64][3] sums + the count slot
   return (int)0;
 }
+
+static inline int pad16(int c) { return (c + 15) & ~15; }
 
 static unsigned cap_grid(sc_ctx* ctx, int64_t blocks, int per_sm) {
   const int64_t cap = (int64_t)ctx->sm_count * per_sm;
@@ -1113,8 +842,7 @@ static int ensure_train_panels(sc_ctx* ctx) {
 
 int tc_train_prepare(sc_ctx* ctx) { return ensure_train_panels(ctx); }
 
-int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* patches, const float* wf0, int n, const uint8_t* masks,
-                      float* F5, cudaStream_t s) {
+int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* patches, int n, const uint8_t* masks, cudaStream_t s) {
   SC_TRY(ensure_train_panels(ctx));
   const ParamOff& O = ctx->off;
   const BranchOff& Ob = O.br[b];
@@ -1143,7 +871,7 @@ int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* pat
     if (l == 0) {
       {
         ProfScope prof(ctx, PC_TRAIN_FWD, s);
-        tconv1_kernel<<<cap_grid(ctx, ((int64_t)30 * n * 32 + 255) / 256, 8), 256, 0, s>>>(patches, n, wf0, T.X[0]);
+        tconv1_kernel<<<cap_grid(ctx, ((int64_t)30 * n * 32 + 255) / 256, 8), 256, 0, s>>>(patches, n, T.wf0, T.X[0]);
       }
       tbn_stats_kernel<32><<<cap_grid(ctx, (vpix + 63) / 64 / 4 + 1, 2), 256, 0, s>>>(T.X[l], n, L.cout, L.H, Pw, L.pitch, sums);
       ctx->launches += 2;
@@ -1170,16 +898,14 @@ int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* pat
       const unsigned grid = (unsigned)((opix + 63) / 64);
       if (L.fmt == 32)
         tbn_act_kernel<32><<<grid, 256, 0, s>>>(T.X[l], n, L.cout, Pw, L.pitch, sums, (double)vpix, cnt, T.mean[l], T.istd[l], G + Ob.bn[l][2], G + Ob.bn[l][3],
-                                                P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], L.pool, T.A[l], L.oR, L.oPitch, L.oH, T.idx[l], ctx->train_wgrad_mn ? nullptr : T.AT[l],
-                                                pad8(L.cout));
+                                                P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], L.pool, T.A[l], L.oR, L.oPitch, L.oH, T.idx[l]);
       else
         tbn_act_kernel<64><<<grid, 512, 0, s>>>(T.X[l], n, L.cout, Pw, L.pitch, sums, (double)vpix, cnt, T.mean[l], T.istd[l], G + Ob.bn[l][2], G + Ob.bn[l][3],
-                                                P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], L.pool, T.A[l], L.oR, L.oPitch, L.oH, T.idx[l], ctx->train_wgrad_mn ? nullptr : T.AT[l],
-                                                pad8(L.cout));
+                                                P + Ob.bn[l][1], P + Ob.bn[l][0], P + Ob.alpha[l], L.pool, T.A[l], L.oR, L.oPitch, L.oH, T.idx[l]);
     } else {
       tact5_flatten_kernel<<<(unsigned)(((int64_t)n * 540 + 255) / 256), 256, 0, s>>>(T.X[4], n, sums, (double)vpix, cnt, T.mean[4], T.istd[4], G + Ob.bn[4][2],
                                                                                      G + Ob.bn[4][3], P + Ob.bn[4][1], P + Ob.bn[4][0], P + Ob.alpha[4],
-                                                                                     masks + b * 540, F5);
+                                                                                     masks + b * 540, T.F5);
     }
     ctx->launches++;
   }
@@ -1189,7 +915,7 @@ int tc_branch_forward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* pat
 
 template <int FMT, int DFMT>
 static int bwd_layer(sc_ctx* ctx, int b, int l, const TcBranchBuf& T, const float* dA, const float* dF5, int dF5_ld, const uint8_t* mask, int n,
-                     int dPw, int dPitch, float* frame, uint16_t* DT, float* planar, cudaStream_t s) {
+                     int dPw, int dPitch, cudaStream_t s) {
   const TLayer& L = kTL[l];
   const BranchOff& Ob = ctx->off.br[b];
   float* P = ctx->params;
@@ -1208,7 +934,7 @@ static int bwd_layer(sc_ctx* ctx, int b, int l, const TcBranchBuf& T, const floa
   const int64_t npix = (int64_t)L.R * Pw;
   tbn_bwd_dx_kernel<FMT, DFMT><<<(unsigned)((npix + 63) / 64), 64 * NCH, 0, s>>>(
       T.X[l], dA, T.idx[l], dF5, dF5_ld, mask, n, L.cout, L.H, L.R, Pw, L.pitch, L.pool, dPw, dPitch, T.mean[l], T.istd[l], P + Ob.bn[l][1], P + Ob.bn[l][0],
-      P + Ob.alpha[l], sums, (double)vpix, cnt, hook ? nullptr : G + Ob.bn[l][0], G + Ob.bn[l][1], G + Ob.alpha[l], frame, DT, pad8(L.cout), planar, 32);
+      P + Ob.alpha[l], sums, (double)vpix, cnt, hook ? nullptr : G + Ob.bn[l][0], G + Ob.bn[l][1], G + Ob.alpha[l], T.frame);
   ctx->launches += 2;
   SC_CUDA(cudaGetLastError());
   return SC_OK;
@@ -1219,16 +945,15 @@ int tc_branch_backward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* pa
                        cudaStream_t s) {
   const BranchOff& Ob = ctx->off.br[b];
   float* G = ctx->grads;
-  uint16_t* DT = ctx->train_wgrad_mn ? nullptr : T.DT;     // the MN-major wgrad reads the frame itself: no planar gradient copies
   for (int l = 4; l >= 0; --l) {
     const TLayer& L = kTL[l];
     const int Pw = n * L.pitch;
     // the incoming gradient: conv5 <- dF5; pooled layers <- the dgrad output at the pooled geometry; others same geometry
     const int dPw = L.pool ? n * L.oPitch : Pw, dPitch = L.pool ? L.oPitch : L.pitch;
-    if (l == 4) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, nullptr, dF5, dF5_ld, masks + b * 540, n, dPw, dPitch, T.frame, DT, nullptr, s)));
-    else if (l == 3) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, T.frame, DT, nullptr, s)));
-    else if (l == 2) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, T.frame, DT, nullptr, s)));
-    else if (l == 1) SC_TRY((bwd_layer<32, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, T.frame, DT, nullptr, s)));
+    if (l == 4) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, nullptr, dF5, dF5_ld, masks + b * 540, n, dPw, dPitch, s)));
+    else if (l == 3) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, s)));
+    else if (l == 2) SC_TRY((bwd_layer<64, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, s)));
+    else if (l == 1) SC_TRY((bwd_layer<32, 64>(ctx, b, l, T, T.dA, nullptr, 0, nullptr, n, dPw, dPitch, s)));
     else {
       // conv1: reduction pass, then dx and the weight gradient in one fused pass (no dgrad below conv1)
       float* P = ctx->params;
@@ -1251,8 +976,7 @@ int tc_branch_backward(sc_ctx* ctx, int b, const TcBranchBuf& T, const float* pa
     }
     const TLayer& Li = kTL[l - 1];
     const int64_t npix = (int64_t)L.R * Pw;
-    if (ctx->train_wgrad_mn) SC_TRY(launch_wgrad_mn(ctx, T.A[l - 1], Li.fmt, T.frame, L.fmt, L.cin, L.cout, Pw, npix, L.H, G + Ob.convW[l], s));
-    else SC_TRY(launch_wgrad_tc(ctx, T.AT[l - 1], T.DT, L.cin, L.cout, pad8(L.cin), pad16(L.cout), Pw, npix, L.H, G + Ob.convW[l], s));
+    SC_TRY(launch_wgrad_mn(ctx, T.A[l - 1], Li.fmt, T.frame, L.fmt, L.cin, L.cout, Pw, npix, L.H, G + Ob.convW[l], s));
     // dgrad: the gradient of this layer's input = sweep over the zero-framed dx with the raw taps; valid Li.oH x Li.oH
     SC_TRY(launch_conv_sweep(ctx, ctx->train_sw[b][l][1], l, T.frame, L.fmt == 32 ? 1 : 0, T.dA, (l == 1) ? 1 : 0, Pw, L.R, Li.oH, 1, 0,
                              PC_TRAIN_BWD, s, -2, -2));
