@@ -337,6 +337,41 @@ SC_API int sc_set_allreduce_hook(sc_ctx* ctx, sc_allreduce_fn fn, void* user);
 SC_API int sc_eval_batch(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const float* in3_dev,
                   const float* in4_dev, const uint8_t* y_dev, int64_t n, float* out2_dev, void* stream);
 
+/* ---- fine-tuning on a new domain: frozen trunk, cached trunk features, head-only steps ------------------------------
+ * Supervised domain adaptation as in Kushibar et al. (Sci. Rep. 2019): keep the convolutional layers, retrain the fully
+ * connected part on a few labelled target-domain samples.
+ *   trunk = every <view>_ch_conv1..5 (W), <view>_ch_conv1..5_bn (beta, gamma, mean, inv_std) and <view>_ch_prelu1..5 array of
+ *           the three views; head = every other array (d1 x3, FC1, fc_2, out_layer and their PReLUs).
+ * The trunk is evaluated in deterministic mode, with the STORED BatchNorm statistics: a sample's features then do not depend
+ * on its minibatch (so they are computed once and cached), and the batch statistics of a single target image cannot shift the
+ * frozen layers.  This deliberately differs from a training-mode forward pass with frozen weights.  The head trains with the
+ * semantics of sc_train_forward_backward: dropout p = .5 at *_l1drop (on the cached features), f1_drop and f2_drop with the same
+ * [n][2700] mask layout and the same hash3(seed, i) masks, softmax cross-entropy divided by n_global, Lasagne Adam.
+ * Feature rows (public layout): float32 [N][3][540]; per view, entry k = c*9 + h*3 + w is the flattened conv5 activation after
+ * BatchNorm and PReLU, i.e. the input of <view>_d1 before dropout.
+ * All four calls return SC_ERR_ARG with the SIMT back-end selected ("gemm" = 0; sc_freeze_trunk(ctx, 0) excepted), for NULL
+ * required pointers and for bad sizes; the message names the argument. */
+/* trunk of the three views on [n][1][32][32] patches (the tensor-core patchwise trunk of sc_forward) -> feats_dev [n][3][540]. */
+SC_API int sc_trunk_features(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const float* in3_dev, int64_t n,
+                             float* feats_dev, void* stream);
+/* One training step of the head on rows r = idx_dev[i] (r = i when idx_dev is NULL), i < n <= 16384, of a feature table
+ * feats_dev [N][3][540] with the atlas rows atlas_rows_dev [N][15] and labels labels_dev [N] (uint8 0..14) that a training set
+ * holds on the device.  n_global, seed, drop_masks_dev and loss_dev as for sc_train_forward_backward (the masks are per batch
+ * entry i).  Gradients land in the context's gradient buffer; every trunk entry of it, the BatchNorm-statistics slots included,
+ * is exactly 0 afterwards.  Indices are device data and are not range-checked (0 <= idx[i] < N is the caller's to guarantee).
+ * Captured as a CUDA graph per (n, n_global, injected masks, tables, idx NULL or not) like the full step ("train_graph"). */
+SC_API int sc_head_train_forward_backward(sc_ctx* ctx, const float* feats_dev, const float* atlas_rows_dev, const uint8_t* labels_dev,
+                                          const int64_t* idx_dev, int64_t n, int64_t n_global, uint64_t seed,
+                                          const uint8_t* drop_masks_dev, float* loss_dev, void* stream);
+/* deterministic head on the same rows (the validation pass of fine-tuning): out2_dev = {sum of -log p[y], number of correct
+ * arg-max}, as sc_eval_batch reports for the patches the features came from. */
+SC_API int sc_head_eval_batch(sc_ctx* ctx, const float* feats_dev, const float* atlas_rows_dev, const uint8_t* labels_dev,
+                              const int64_t* idx_dev, int64_t n, float* out2_dev, void* stream);
+/* frozen != 0: sc_adam_step and sc_allreduce_adam_step leave every trunk entry untouched (parameter, Adam moments, BatchNorm
+ * running statistics), and sc_train_forward_backward returns SC_ERR_STATE; 0 restores the default.  Inference is unaffected.
+ * Synchronises the device. */
+SC_API int sc_freeze_trunk(sc_ctx* ctx, int frozen);
+
 #ifdef __cplusplus
 }
 #endif

@@ -91,7 +91,13 @@ PROTOTYPES = {
     "sc_allreduce_adam_step": (ctypes.c_int, [_vp, _c_f, _c_f, _c_f, _c_f, _vp]),
     "sc_set_allreduce_hook": (ctypes.c_int, [_vp, _vp, _vp]),
     "sc_eval_batch": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp]),
+    "sc_trunk_features": (ctypes.c_int, [_vp, _vp, _vp, _vp, _c_i64, _vp, _vp]),
+    "sc_head_train_forward_backward": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, ctypes.c_uint64, _vp, _vp, _vp]),
+    "sc_head_eval_batch": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp]),
+    "sc_freeze_trunk": (ctypes.c_int, [_vp, ctypes.c_int]),
 }
+# sc_trunk_features: float32 per sample and view, the flattened conv5 activation (k = c*9 + h*3 + w)
+TRUNK_FEATURES = (3, 540)
 
 
 def load_library():
@@ -556,6 +562,42 @@ class Context(object):
         out = torch.zeros(2, dtype=torch.float32, device=in1.device)
         _check(self.lib.sc_eval_batch(self.h, _ptr(in1), _ptr(in2), _ptr(in3), _ptr(in4), _ptr(y), in1.shape[0], _ptr(out), _stream()))
         return out
+
+    # -- fine-tuning on cached trunk features (include/subcort_b200.h) ------------------------------
+    def trunk_features(self, in1, in2, in3, out=None):
+        """[n,1,32,32] CUDA patches of the three views -> float32 CUDA tensor [n, 3, 540] (or `out`, rows written in place):
+        the frozen trunk in deterministic mode, per view the flattened conv5 activation (sc_trunk_features)"""
+        import torch
+        n = in1.shape[0]
+        if out is None:
+            out = torch.empty((n,) + TRUNK_FEATURES, dtype=torch.float32, device=in1.device)
+        _check(self.lib.sc_trunk_features(self.h, _ptr(in1), _ptr(in2), _ptr(in3), n, _ptr(out), _stream()))
+        return out
+
+    def head_train_forward_backward(self, feats, atlas_rows, labels, idx=None, n=None, n_global=None, seed=0, drop_masks=None,
+                                    loss_out=None):
+        """one head-only training step on rows idx (CUDA int64, trusted; None: rows 0..n-1) of the feature table `feats`
+        [N, 3, 540] with its atlas rows [N, 15] and labels [N] (sc_head_train_forward_backward)"""
+        import torch
+        if n is None:
+            n = idx.shape[0] if idx is not None else feats.shape[0]
+        loss = loss_out if loss_out is not None else torch.zeros(1, dtype=torch.float32, device=feats.device)
+        _check(self.lib.sc_head_train_forward_backward(self.h, _ptr(feats), _ptr(atlas_rows), _ptr(labels), _ptr(idx), int(n),
+                                                       int(n_global or n), int(seed), _ptr(drop_masks), _ptr(loss), _stream()))
+        return loss
+
+    def head_eval_batch(self, feats, atlas_rows, labels, idx=None, n=None):
+        """deterministic head on rows idx of the feature table -> CUDA {sum of -log p[y], correct count} (sc_head_eval_batch)"""
+        import torch
+        if n is None:
+            n = idx.shape[0] if idx is not None else feats.shape[0]
+        out = torch.zeros(2, dtype=torch.float32, device=feats.device)
+        _check(self.lib.sc_head_eval_batch(self.h, _ptr(feats), _ptr(atlas_rows), _ptr(labels), _ptr(idx), int(n), _ptr(out), _stream()))
+        return out
+
+    def freeze_trunk(self, frozen=True):
+        """while frozen the Adam steps leave the trunk untouched and train_forward_backward raises (sc_freeze_trunk)"""
+        _check(self.lib.sc_freeze_trunk(self.h, int(bool(frozen))))
 
 
 class _CudaArrayHolder(object):

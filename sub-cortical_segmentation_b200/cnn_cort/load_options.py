@@ -59,6 +59,12 @@ def load_options(user_config):
         if v < 0:
             raise ValueError("[model] %s = %d must not be negative" % (key, v))
         options[key] = v
+    # optional: fine-tune the head of a trained experiment's weights (nets/<fine_tune_from>/) on this experiment's training set
+    # with the convolutional trunk frozen (Net.fine_tune) instead of training from scratch; off when absent or empty
+    v = g('model', 'fine_tune_from', fallback='').strip()
+    options['fine_tune_from'] = v or None
+    if options['fine_tune_from'] == options['experiment']:
+        raise ValueError("[model] fine_tune_from = %s names this experiment: its weights would be overwritten" % v)
     return options
 
 

@@ -261,14 +261,38 @@ class Net(object):
         if fused:
             ctx.fused_attach()
         batches = self._scan_batches(X, dev) if scans else self._array_batches(xs, y, dev)
+        grads = ctx.grad_tensor()
+        rng = np.random.RandomState(self._seed)
 
+        def step(gidx, b, loss_buf):
+            if b is not None:
+                ctx.train_forward_backward(*b, n_global=len(gidx), seed=int(rng.randint(1 << 62)) + rank, loss_out=loss_buf)
+            else:                      # a last partial batch smaller than the world size: contribute zeros
+                grads.zero_()
+                loss_buf.zero_()
+            if fused:
+                ctx.allreduce_adam_step(lr=self.update_learning_rate)
+                if world > 1:
+                    dist.all_reduce(loss_buf)
+            else:
+                parallel.allreduce_gradients(grads, loss_buf)
+                # the BN-statistics slots hold the SUM of the batch statistics of the ranks that had samples: rank r of
+                # shard_batch has some iff r < len(gidx)
+                ctx.adam_step(lr=self.update_learning_rate, stat_scale=1.0 / min(world, len(gidx)))
+
+        return self._epoch_loop(tr, va, batches, step, lambda b: ctx.eval_batch(*b), dev, epochs, rank, world)
+
+    def _epoch_loop(self, tr, va, batches, step, evaluate, dev, epochs, rank=0, world=1):
+        """nolearn's epoch loop over the training rows tr and validation rows va: minibatches of batch_size rows, this rank's
+        share of each (shard_batch); batches(index lists) yields each list's minibatch (None for an empty one),
+        step(global rows, minibatch, loss buffer) trains on it, evaluate(minibatch) -> CUDA {sum of -log p[y], correct}.
+        History, best-weight checkpoint, history file and early stopping as nolearn's handlers (nets.py:154-156)."""
+        import torch
         best_valid, best_train = np.inf, np.inf
         best_epoch, best_weights = 0, None
         first = len(self.train_history_)
         bs = self.batch_size
         n_epochs = epochs or self.max_epochs
-        grads = ctx.grad_tensor()
-        rng = np.random.RandomState(self._seed)
         loss_buf = torch.zeros(1, dtype=torch.float32, device=dev)
         steps = [tr[s:s + bs] for s in range(0, len(tr), bs)]
         local_steps = [parallel.shard_batch(gidx, rank, world) for gidx in steps]
@@ -277,26 +301,13 @@ class Net(object):
             t0 = time.time()
             losses, sizes = [], []
             for gidx, b in zip(steps, batches(local_steps)):
-                if b is not None:
-                    ctx.train_forward_backward(*b, n_global=len(gidx), seed=int(rng.randint(1 << 62)) + rank, loss_out=loss_buf)
-                else:                      # a last partial batch smaller than the world size: contribute zeros
-                    grads.zero_()
-                    loss_buf.zero_()
-                if fused:
-                    ctx.allreduce_adam_step(lr=self.update_learning_rate)
-                    if world > 1:
-                        dist.all_reduce(loss_buf)
-                else:
-                    parallel.allreduce_gradients(grads, loss_buf)
-                    # the BN-statistics slots hold the SUM of the batch statistics of the ranks that had samples: rank r of
-                    # shard_batch has some iff r < len(gidx)
-                    ctx.adam_step(lr=self.update_learning_rate, stat_scale=1.0 / min(world, len(gidx)))
+                step(gidx, b, loss_buf)
                 losses.append(loss_buf.clone())
                 sizes.append(len(gidx))
             train_loss = float(np.average(torch.cat(losses).cpu().numpy(), weights=sizes)) if losses else float('nan')
             vsum = torch.zeros(2, dtype=torch.float32, device=dev)
             for b in batches(valid_steps):
-                vsum += ctx.eval_batch(*b)
+                vsum += evaluate(b)
             vs = vsum.cpu().numpy()
             valid_loss = float(vs[0] / max(1, len(va)))
             valid_acc = float(vs[1] / max(1, len(va)))
@@ -324,6 +335,81 @@ class Net(object):
                     self.load_params_from(best_weights)
                 break
         return self
+
+    # -- fine-tuning on a new domain (Kushibar et al., Sci. Rep. 2019) ------------------------------
+    def fine_tune(self, X, y=None, epochs=None):
+        """Retrain the head on a few labelled target-domain samples with the convolutional trunk frozen.
+
+        X: a base.ScanTrainingSet, or the {'in1', 'in2', 'in3', 'in4'} arrays fit takes with labels y.  The trunk (conv1..conv5
+        with BatchNorm and PReLU, all three views) runs ONCE per sample, in deterministic mode with its stored BatchNorm
+        statistics, into a device table of 3 x 540 float32 features per sample (6 480 B); every step then trains d1 x3, FC1,
+        fc_2 and out_layer from those rows with the training dropout, loss and Adam of fit.  The optimiser is reset, and
+        the trunk -- parameters, Adam moments and BatchNorm running statistics -- stays exactly as it was.  Same epoch loop,
+        history, checkpoint, history file and early stopping as fit.  Single device only."""
+        import torch
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise RuntimeError("fine_tune: data-parallel fine-tuning is not supported (world size %d)" % dist.get_world_size())
+        ctx = self.ctx
+        dev = torch.device('cuda', self.device)
+        feats, atlas, labels, y = self._feature_table(X, y, dev)
+        tr, va = self.train_split.indices(y)
+
+        def batches(index_lists):   # one upload of the pass's row indices; each minibatch is a slice of it
+            flat = np.concatenate([np.asarray(i, dtype=np.int64) for i in index_lists]) if index_lists else np.zeros(0, np.int64)
+            d_idx = torch.from_numpy(flat).to(dev)
+            off = 0
+            for idx in index_lists:
+                yield d_idx[off:off + len(idx)] if len(idx) else None
+                off += len(idx)
+
+        rng = np.random.RandomState(self._seed)
+
+        def step(gidx, idx, loss_buf):
+            ctx.head_train_forward_backward(feats, atlas, labels, idx=idx, seed=int(rng.randint(1 << 62)), loss_out=loss_buf)
+            ctx.adam_step(lr=self.update_learning_rate)
+
+        ctx.reset_optimizer()
+        ctx.freeze_trunk(True)
+        try:
+            return self._epoch_loop(tr, va, batches, step, lambda idx: ctx.head_eval_batch(feats, atlas, labels, idx=idx), dev,
+                                    epochs)
+        finally:
+            ctx.freeze_trunk(False)
+
+    def _feature_table(self, X, y, dev, chunk=16384):
+        """-> (trunk features [N, 3, 540], atlas rows [N, 15], labels [N] uint8 as CUDA tensors, host labels)"""
+        import torch
+        ctx = self.ctx
+        scans = hasattr(X, 'gather')
+        if scans:
+            if y is not None:
+                raise ValueError("fine_tune: a ScanTrainingSet carries its own labels; call fine_tune(scans) without y")
+            y = X.y
+        else:
+            y = np.asarray(y).astype(np.uint8)
+        if y.size and int(y.max()) > 14:
+            raise ValueError("fine_tune: labels must be in 0..14 (generate_training_set maps the boundary label 15 to 0, base.py:89)")
+        n = len(y)
+        need = n * 3 * 540 * 4
+        free_b = torch.cuda.mem_get_info(dev)[0]
+        if need > free_b:
+            raise MemoryError("fine_tune: the trunk feature table of %d samples needs %.2f GB of device memory, %.2f GB are free"
+                              % (n, need / 1e9, free_b / 1e9))
+        feats = torch.empty((n, 3, 540), dtype=torch.float32, device=dev)
+        if scans:
+            atlas, labels = X.atlas, X.labels
+            for s in range(0, n, chunk):
+                in1, in2, in3, _, _ = X.gather(np.arange(s, min(n, s + chunk)), ctx=ctx)
+                ctx.trunk_features(in1, in2, in3, out=feats[s:s + len(in1)])
+        else:
+            xs = [np.ascontiguousarray(X[k], dtype=np.float32) for k in ('in1', 'in2', 'in3')]
+            atlas = torch.from_numpy(np.ascontiguousarray(X['in4'], dtype=np.float32)).to(dev)
+            labels = torch.from_numpy(np.ascontiguousarray(y)).to(dev)
+            for s in range(0, n, chunk):
+                ins = [torch.from_numpy(a[s:s + chunk]).to(dev) for a in xs]
+                ctx.trunk_features(*ins, out=feats[s:s + len(ins[0])])
+        return feats, atlas, labels, y
 
     def _array_batches(self, xs, y, dev):
         """minibatch source of fit on host arrays: batches(index lists) yields the device tensors (in1..in4, y) of each

@@ -164,14 +164,22 @@ def make_registration_pair(subject_shape=(128, 128, 128), template_shape=None, s
 
 
 def write_subject(root, name, shape=(256, 256, 256), seed=1234, with_labels=False, t1_name="T1.nii.gz",
-                  roi_name="gt_15_classes.nii.gz", zoom=1.0, t1_dtype=np.float32):
+                  roi_name="gt_15_classes.nii.gz", zoom=1.0, t1_dtype=np.float32, contrast=None):
+    """contrast: None, or per-label mean intensities {label: value} (or a sequence indexed by label 0..15) added to the T1
+    inside each labelled structure, so that the image carries its structures; two tables make two "scanner" domains.  None
+    writes exactly what it always did."""
     d = os.path.join(root, name)
     os.makedirs(os.path.join(d, "tmp"), exist_ok=True)
     aff = np.diag([zoom, zoom, zoom, 1.0])
     t1 = make_t1(shape, seed)
+    atlas, _, _ = make_atlas(shape, seed)
+    if contrast is not None:
+        table = np.zeros(16, np.float32)
+        for l, v in (contrast.items() if isinstance(contrast, dict) else enumerate(contrast)):
+            table[int(l)] = v
+        t1 = (t1 + table[make_labels(atlas)]).astype(t1.dtype)
     if np.dtype(t1_dtype).kind in "iu":       # scanner-style integer intensities (the usual on-disk type of a T1)
         t1 = np.rint(t1).astype(t1_dtype)
-    atlas, _, _ = make_atlas(shape, seed)
     nifti.Nifti1Image(t1, aff).to_filename(os.path.join(d, t1_name))
     nifti.Nifti1Image(atlas, aff).to_filename(os.path.join(d, "tmp", "MNI_sub_probabilities.nii.gz"))
     nifti.Nifti1Image(make_mask(atlas), aff).to_filename(os.path.join(d, "tmp", "MNI_subcortical_mask.nii.gz"))

@@ -112,14 +112,7 @@ int sc_create(int device, sc_ctx** out) {
   SC_CUDA(cudaMemset(ctx->grads, 0, pb));
   SC_CUDA(cudaMemset(ctx->adam_m, 0, pb));
   SC_CUDA(cudaMemset(ctx->adam_v, 0, pb));
-  {
-    std::vector<uint8_t> t(SC_PARAM_FLOATS, 1);
-    for (int b = 0; b < 3; ++b)
-      for (int l = 0; l < 5; ++l)
-        for (int k = 2; k < 4; ++k)
-          for (int c = 0; c < kConvCout[l]; ++c) t[ctx->off.br[b].bn[l][k] + c] = 0;  // BN mean / inv_std are state
-    SC_CUDA(cudaMemcpy(ctx->trainable, t.data(), SC_PARAM_FLOATS, cudaMemcpyHostToDevice));
-  }
+  SC_TRY(freeze_trunk(ctx, false));   // BN mean / inv_std are state, every other entry trains
   SC_CUDA(cudaMalloc(&ctx->d_count, sizeof(int64_t)));
   SC_CUDA(cudaMallocHost(&ctx->h_count, sizeof(int64_t)));
   // the tcgen05 / TMA back-end is the product: a box on which it cannot be brought up is an error, never a silent
@@ -232,7 +225,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc", "head"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -715,6 +708,7 @@ int sc_train_forward_backward(sc_ctx* ctx, const float* in1_dev, const float* in
                               const float* in4_dev, const uint8_t* y_dev, int64_t n, int64_t n_global, uint64_t seed,
                               const uint8_t* drop_masks_dev, float* loss_dev, void* stream) {
   SC_TRY(need_weights(ctx, "sc_train_forward_backward"));
+  SC_CHECK(!ctx->trunk_frozen, SC_ERR_STATE, "sc_train_forward_backward: the trunk is frozen (sc_freeze_trunk); use sc_head_train_forward_backward");
   SC_CHECK(n > 0 && n_global >= n, SC_ERR_ARG, "sc_train_forward_backward: bad batch size");
   SC_CHECK(in1_dev && in2_dev && in3_dev && in4_dev && y_dev && loss_dev, SC_ERR_ARG, "sc_train_forward_backward: null argument");
   return train_forward_backward(ctx, in1_dev, in2_dev, in3_dev, in4_dev, y_dev, n, n_global, seed, drop_masks_dev,
@@ -772,6 +766,65 @@ int sc_eval_batch(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const
   SC_TRY(fresh_weights(ctx, "sc_eval_batch", (cudaStream_t)stream));
   SC_CHECK(n > 0 && in1_dev && in2_dev && in3_dev && in4_dev && y_dev && out2_dev, SC_ERR_ARG, "sc_eval_batch: bad argument");
   return eval_batch(ctx, in1_dev, in2_dev, in3_dev, in4_dev, y_dev, n, out2_dev, (cudaStream_t)stream);
+}
+
+// ---- fine-tuning the head on cached trunk features
+static int check_tc(sc_ctx* ctx, const char* who) {
+  SC_CHECK(ctx->gemm_backend == 1, SC_ERR_ARG, "%s: runs on the tcgen05 back-end only (gemm = %d)", who, ctx->gemm_backend);
+  return SC_OK;
+}
+
+int sc_trunk_features(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const float* in3_dev, int64_t n, float* feats_dev,
+                      void* stream) {
+  const char* who = "sc_trunk_features";
+  SC_TRY(fresh_weights(ctx, who, (cudaStream_t)stream));
+  SC_TRY(check_tc(ctx, who));
+  SC_CHECK(in1_dev, SC_ERR_ARG, "%s: in1_dev is NULL", who);
+  SC_CHECK(in2_dev, SC_ERR_ARG, "%s: in2_dev is NULL", who);
+  SC_CHECK(in3_dev, SC_ERR_ARG, "%s: in3_dev is NULL", who);
+  SC_CHECK(feats_dev, SC_ERR_ARG, "%s: feats_dev is NULL", who);
+  SC_CHECK(n > 0, SC_ERR_ARG, "%s: n = %lld must be positive", who, (long long)n);
+  return trunk_features(ctx, in1_dev, in2_dev, in3_dev, n, feats_dev, (cudaStream_t)stream);
+}
+
+static int check_head_tables(const float* feats, const float* atlas_rows, const uint8_t* labels, int64_t n, int64_t n_max, const char* who) {
+  SC_CHECK(feats, SC_ERR_ARG, "%s: feats_dev is NULL", who);
+  SC_CHECK(atlas_rows, SC_ERR_ARG, "%s: atlas_rows_dev is NULL", who);
+  SC_CHECK(labels, SC_ERR_ARG, "%s: labels_dev is NULL", who);
+  SC_CHECK(n > 0 && n <= n_max, SC_ERR_ARG, "%s: n = %lld is outside [1, %lld]", who, (long long)n, (long long)n_max);
+  return SC_OK;
+}
+
+int sc_head_train_forward_backward(sc_ctx* ctx, const float* feats_dev, const float* atlas_rows_dev, const uint8_t* labels_dev,
+                                   const int64_t* idx_dev, int64_t n, int64_t n_global, uint64_t seed, const uint8_t* drop_masks_dev,
+                                   float* loss_dev, void* stream) {
+  const char* who = "sc_head_train_forward_backward";
+  SC_TRY(need_weights(ctx, who));
+  SC_TRY(check_tc(ctx, who));
+  SC_TRY(check_head_tables(feats_dev, atlas_rows_dev, labels_dev, n, 16384, who));
+  SC_CHECK(loss_dev, SC_ERR_ARG, "%s: loss_dev is NULL", who);
+  SC_CHECK(n_global >= n, SC_ERR_ARG, "%s: n_global = %lld is below n = %lld", who, (long long)n_global, (long long)n);
+  return head_train_forward_backward(ctx, feats_dev, atlas_rows_dev, labels_dev, idx_dev, n, n_global, seed, drop_masks_dev, loss_dev,
+                                     (cudaStream_t)stream);
+}
+
+int sc_head_eval_batch(sc_ctx* ctx, const float* feats_dev, const float* atlas_rows_dev, const uint8_t* labels_dev, const int64_t* idx_dev,
+                       int64_t n, float* out2_dev, void* stream) {
+  const char* who = "sc_head_eval_batch";
+  SC_TRY(fresh_weights(ctx, who, (cudaStream_t)stream));
+  SC_TRY(check_tc(ctx, who));
+  SC_TRY(check_head_tables(feats_dev, atlas_rows_dev, labels_dev, n, 1ll << 31, who));
+  SC_CHECK(out2_dev, SC_ERR_ARG, "%s: out2_dev is NULL", who);
+  return head_eval_batch(ctx, feats_dev, atlas_rows_dev, labels_dev, idx_dev, n, out2_dev, (cudaStream_t)stream);
+}
+
+int sc_freeze_trunk(sc_ctx* ctx, int frozen) {
+  const char* who = "sc_freeze_trunk";
+  SC_CHECK(ctx, SC_ERR_ARG, "%s: null context", who);
+  if (frozen) SC_TRY(check_tc(ctx, who));     // unfreezing is always allowed
+  SC_CUDA(cudaSetDevice(ctx->device));
+  SC_CUDA(cudaDeviceSynchronize());           // an Adam step in flight still reads the old map
+  return freeze_trunk(ctx, frozen != 0);
 }
 
 }  // extern "C"

@@ -148,7 +148,7 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_HEAD, PC_COUNT
 };
 
 // counter-based random bits (splitmix64 finaliser): the dropout keep masks of the training step and of Monte-Carlo dropout
@@ -176,7 +176,8 @@ struct sc_ctx {
   float* grads = nullptr;        // same layout
   float* adam_m = nullptr;
   float* adam_v = nullptr;
-  uint8_t* trainable = nullptr;  // 1 where the entry is trainable
+  uint8_t* trainable = nullptr;  // per entry: 1 Adam, 0 BatchNorm running statistic, 2 frozen (sc_freeze_trunk: untouched)
+  bool trunk_frozen = false;     // sc_freeze_trunk: the trunk entries of `trainable` are 2
   int64_t adam_t = 0;
   float* derived = nullptr;      // arena for the derived layouts
   size_t derived_floats = 0;
@@ -192,8 +193,10 @@ struct sc_ctx {
   double* h_reg = nullptr;       // pinned: the optimiser's per-trial read-backs
   int reg_iters[8] = {};         // accepted steps of the last registration per level: affine 0..3, FFD 4..6
   // training step as a CUDA graph (one per (batch, global batch, injected masks) shape): the three branches run on
-  // three captured streams; rebuilt when the arena moves
-  struct TrainGraph { int n; long long n_global; int injected; int backend; void* arena; cudaGraphExec_t exec; int launches; };
+  // three captured streams; rebuilt when the arena moves.  The head-only step of fine-tuning (tables != nullptr) is keyed
+  // on its feature / atlas / label tables and on whether an index list selects the rows.
+  struct TrainGraph { int n; long long n_global; int injected; int backend; void* arena; cudaGraphExec_t exec; int launches;
+                      const void* tables[3]; int has_idx; };
   std::vector<TrainGraph> train_graphs;
   cudaStream_t train_side[2] = {nullptr, nullptr};
   cudaEvent_t train_ev[8] = {};
@@ -414,6 +417,10 @@ int launch_branch_patches(sc_ctx* ctx, int branch, const float* patches, int64_t
                           cudaStream_t st);
 int forward_patches(sc_ctx* ctx, const float* in1, const float* in2, const float* in3, const float* in4, int64_t n,
                     float* proba, int32_t* label, cudaStream_t st);
+// deterministic FC1 -> atlas -> fc_2 -> out_layer / softmax of m feature rows [m][576] (d1 outputs, 192 columns per view);
+// h1 [m][576] and (SIMT back-end) h2 [m][272] are scratch; proba [m][15] / label [m] may be NULL
+int head_rows(sc_ctx* ctx, const float* feats, const float* in4, int64_t m, float* h1, float* h2, float* proba, int32_t* label,
+              cudaStream_t st);
 
 // dense.cu
 struct ConvArgs {
@@ -429,6 +436,9 @@ int launch_conv1_patches(sc_ctx* ctx, const float* patches, int n, const float* 
 size_t branch_patches_tc_bytes(int64_t n);
 int branch_patches_tc(sc_ctx* ctx, int branch, const float* patches, int64_t n, float* scratch, float* feats /*[n][576] split*/,
                       cudaStream_t st);
+// conv1..conv5 of one view (stored BatchNorm statistics) on n patches -> *c5_out, inside scratch: the wide-row split conv5 map
+// [7][n][8] of 256 B pixels (64 bf16 hi | 64 bf16 lo channel slots), valid in rows 0..2 / columns 0..2 of every patch
+int branch_trunk_tc(sc_ctx* ctx, int branch, const float* patches, int64_t n, float* scratch, float** c5_out, cudaStream_t st);
 // Monte-Carlo dropout over the FC head (mc_dropout.cu): `samples` passes with the keep masks hash3(seed, t * 2700 + j)
 struct McArgs { int samples; uint64_t seed; float* entropy; float* mi; };
 int segment_volume(sc_ctx* ctx, const float* vol, const int32_t* dims, const float* atlas, const int32_t* box,
@@ -467,10 +477,30 @@ int tc_train_prepare(sc_ctx* ctx);      // persistent buffers: allocated outside
 int tdense_prepare(sc_ctx* ctx);
 size_t tdense_bytes(int n);
 void tdense_carve(TcDenseBuf& D, char* base, int n);
+// F5 == nullptr: the caller has already written d1's A operand (D.F5s[b] / D.F5T[b], dropout applied)
 int tdense_branch_forward(sc_ctx* ctx, int b, const TcDenseBuf& D, const float* F5, int n, const uint8_t* masks, cudaStream_t s);
 int tdense_head(sc_ctx* ctx, const TcDenseBuf& D, const float* in4, const uint8_t* y, int n, int64_t n_global, const uint8_t* masks, float* loss,
                 cudaStream_t s);
-int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const uint8_t* masks, cudaStream_t s);
+// dgrad = false: no gradient of d1's input (the head-only step of fine-tuning, whose trunk is frozen)
+int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const uint8_t* masks, bool dgrad, cudaStream_t s);
+
+// fine_tune.cu : fine-tuning the head on cached trunk features (feature rows [N][3][540] float32, k = c*9 + h*3 + w per view)
+constexpr int kTrunkFeat = 3 * 540;
+struct HeadGather {
+  const float* feats; const float* atlas_rows; const uint8_t* labels;   // the tables [N][1620], [N][15], [N]
+  const int64_t* idx; int64_t row0;   // row of batch entry m: idx[m], or row0 + m when idx is NULL
+  int n;
+  const uint8_t* masks;               // [n][2700] keep masks (l1drop of view b at b*540), NULL: none
+  float* F5s[3];                      // d1's A operand per view: split rows [n][576] (columns 540..575 written as zeros)
+  float* F5T[3];                      // and transposed split [576][npad] (NULL: not written)
+  int npad;
+  float* in4; uint8_t* y;             // the batch's atlas rows [n][15] and labels [n]
+};
+int launch_head_gather(sc_ctx* ctx, const HeadGather& g, cudaStream_t st);
+int trunk_features(sc_ctx* ctx, const float* in1, const float* in2, const float* in3, int64_t n, float* feats, cudaStream_t st);
+int head_eval_batch(sc_ctx* ctx, const float* feats, const float* atlas_rows, const uint8_t* labels, const int64_t* idx, int64_t n,
+                    float* out2, cudaStream_t st);
+int freeze_trunk(sc_ctx* ctx, bool frozen);   // writes the trainable map (also its initial state, from sc_create)
 
 // fused_adam.cu
 int fused_export(sc_ctx* ctx, unsigned char* handles);
@@ -485,6 +515,10 @@ int train_forward_backward(sc_ctx* ctx, const float* in1, const float* in2, cons
 int adam_step(sc_ctx* ctx, float lr, float b1, float b2, float eps, float gscale, float sscale, cudaStream_t st);
 int eval_batch(sc_ctx* ctx, const float* in1, const float* in2, const float* in3, const float* in4, const uint8_t* y,
                int64_t n, float* out2, cudaStream_t st);
+// out2 += {sum of -log p[y], number of correct arg-max} over n softmax rows
+int launch_eval_reduce(sc_ctx* ctx, const float* proba, const uint8_t* y, int64_t n, float* out2, cudaStream_t st);
+int head_train_forward_backward(sc_ctx* ctx, const float* feats, const float* atlas_rows, const uint8_t* labels, const int64_t* idx,
+                                int64_t n, int64_t n_global, uint64_t seed, const uint8_t* masks, float* loss, cudaStream_t st);
 
 __device__ __forceinline__ float prelu(float x, float a) { return x > 0.f ? x : a * x; }
 // out_layer logits of one voxel (cnn_cort/nets.py:229-231) -> softmax in fp32, in place; returns the argmax on the float32

@@ -227,7 +227,7 @@ size_t branch_patches_tc_bytes(int64_t n) {
   return (size_t)n * ((960 + 240) * 32 + (240 + 56 + 56) * 64) * sizeof(float) + 5 * 256;
 }
 
-int branch_patches_tc(sc_ctx* ctx, int b, const float* patches, int64_t n, float* scratch, float* feats, cudaStream_t st) {
+int branch_trunk_tc(sc_ctx* ctx, int b, const float* patches, int64_t n, float* scratch, float** c5_out, cudaStream_t st) {
   const BranchW& W = ctx->br[b];
   auto carve = [&](float*& cur, size_t floats) { float* p = cur; cur += (floats + 63) & ~(size_t)63; return p; };
   float* cur = scratch;
@@ -245,6 +245,13 @@ int branch_patches_tc(sc_ctx* ctx, int b, const float* patches, int64_t n, float
   SC_TRY(launch_conv_sweep(ctx, W.conv_sw[2], 2, p1, 1, c3, 0, (int)(n * 16), 15, 12, 1, 0, PC_CONV3, st));   // conv3
   SC_TRY(launch_conv_sweep(ctx, W.conv_sw[3], 3, c3, 0, p2, 0, (int)(n * 16), 15, 10, 1, 2, PC_CONV4, st));   // conv4 + pool2 -> [7][n][8]
   SC_TRY(launch_conv_sweep(ctx, W.conv_sw[4], 4, p2, 0, c5, 0, (int)(n * 8), 7, 3, 1, 0, PC_CONV5, st));     // conv5
+  *c5_out = c5;
+  return SC_OK;
+}
+
+int branch_patches_tc(sc_ctx* ctx, int b, const float* patches, int64_t n, float* scratch, float* feats, cudaStream_t st) {
+  float* c5 = nullptr;
+  SC_TRY(branch_trunk_tc(ctx, b, patches, n, scratch, &c5, st));
   // d1: rows = patches; tap (ty, tx) of the 3x3 conv5 map is tensor-map coordinate (k, patch, tx, ty); K = tap*64 + c
   GemmProblem p;
   p.A = c5; p.lda = 8 * kC5Ld; p.a_ys = 0; p.a_zs = 0;
@@ -258,7 +265,7 @@ int branch_patches_tc(sc_ctx* ctx, int b, const float* patches, int64_t n, float
   p.a_y0 = p.a_z0 = 0;
   p.C = feats; p.ldc = kFeatLd; p.c_ys = p.c_zs = 0; p.M = (int)n; p.Y = p.Z = 1;
   p.n_store = 192; p.c_col0 = b * 192; p.out_split = 1; p.prof_cls = PC_GEMM_D1;
-  SC_TRY(launch_gemm_tc(ctx, p, W.d1_dense, st));
+  SC_TRY(launch_gemm_tc(ctx, p, ctx->br[b].d1_dense, st));
   SC_CUDA(cudaGetLastError());
   return SC_OK;
 }

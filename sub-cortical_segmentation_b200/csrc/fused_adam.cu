@@ -51,13 +51,16 @@ __global__ void __launch_bounds__(512) allreduce_adam_kernel(PeerTable T, int ra
     for (int p = 0; p < world; ++p) g += ld_peer(T.grads[p] + i);
     float np_;
     const float pi = T.params[rank][i];
-    if (trainable[i]) {
+    const uint8_t t = trainable[i];
+    if (t == 1) {
       const float mi = b1 * m[i] + (1.f - b1) * g;
       const float vi = b2 * v[i] + (1.f - b2) * g * g;
       m[i] = mi; v[i] = vi;
       np_ = pi - a_t * mi / (sqrtf(vi) + eps);
-    } else {
+    } else if (t == 0) {
       np_ = 0.9f * pi + 0.1f * (g * sscale);                 // BN running mean / inv_std: average of the ranks' batch statistics
+    } else {
+      np_ = pi;                                              // 2: frozen (sc_freeze_trunk)
     }
     for (int p = 0; p < world; ++p) T.params[p][i] = np_;
   }

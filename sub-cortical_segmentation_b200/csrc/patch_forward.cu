@@ -274,29 +274,33 @@ int forward_patches(sc_ctx* ctx, const float* in1, const float* in2, const float
       p.n_store = 192; p.out_split = 0; p.prof_cls = PC_GEMM_D1;
       SC_TRY(launch_gemm(ctx, p, ctx->br[b].d1, st));
     }
-    GemmProblem p;
-    gemm_problem_rows(p, feats, kFeatLd, kFeatLd, (int)m);
-    p.C = h1; p.ldc = kH1Ld; p.n_store = 540; p.out_split = tc ? 1 : 0;
-    p.prof_cls = PC_GEMM_FC1;
-    SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->fc1, st) : launch_gemm(ctx, p, ctx->fc1, st));
-    { ProfScope prof(ctx, PC_ATLAS, st);   // after FC1 (whose epilogue may zero columns 540..543)
-      atlas_rows_kernel<<<(unsigned)((m * 9 + 255) / 256), 256, 0, st>>>(in4 + s * 15, m, h1, tc ? 1 : 0); }
-    ctx->launches++;
-    SC_CUDA(cudaGetLastError());
-    gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)m);
-    p.n_store = kH2Ld; p.prof_cls = PC_GEMM_FC2;
-    if (tc) {   // fc_2 with the out_layer and softmax / argmax in its epilogue
-      SoftmaxOut smo = {proba ? proba + s * 15 : nullptr, label ? label + s : nullptr, nullptr, nullptr, OutGeo{}, 0, nullptr};
-      p.C = nullptr; p.ldc = 0; p.sm = &smo;
-      SC_TRY(launch_gemm_tc(ctx, p, ctx->fc2, st));
-      continue;
-    }
-    p.C = h2; p.ldc = kH2Ld;
-    SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
-    SC_TRY(launch_out_softmax(ctx, h2, m, proba ? proba + s * 15 : nullptr, label ? label + s : nullptr, nullptr,
-                              nullptr, nullptr, st));
+    SC_TRY(head_rows(ctx, feats, in4 + s * 15, m, h1, h2, proba ? proba + s * 15 : nullptr, label ? label + s : nullptr, st));
   }
   return SC_OK;
+}
+
+int head_rows(sc_ctx* ctx, const float* feats, const float* in4, int64_t m, float* h1, float* h2, float* proba, int32_t* label,
+              cudaStream_t st) {
+  const bool tc = ctx->gemm_backend == 1;
+  GemmProblem p;
+  gemm_problem_rows(p, feats, kFeatLd, kFeatLd, (int)m);
+  p.C = h1; p.ldc = kH1Ld; p.n_store = 540; p.out_split = tc ? 1 : 0;
+  p.prof_cls = PC_GEMM_FC1;
+  SC_TRY(tc ? launch_gemm_tc(ctx, p, ctx->fc1, st) : launch_gemm(ctx, p, ctx->fc1, st));
+  { ProfScope prof(ctx, PC_ATLAS, st);   // after FC1 (whose epilogue may zero columns 540..543)
+    atlas_rows_kernel<<<(unsigned)((m * 9 + 255) / 256), 256, 0, st>>>(in4, m, h1, tc ? 1 : 0); }
+  ctx->launches++;
+  SC_CUDA(cudaGetLastError());
+  gemm_problem_rows(p, h1, kH1Ld, kH1Ld, (int)m);
+  p.n_store = kH2Ld; p.prof_cls = PC_GEMM_FC2;
+  if (tc) {   // fc_2 with the out_layer and softmax / argmax in its epilogue
+    SoftmaxOut smo = {proba, label, nullptr, nullptr, OutGeo{}, 0, nullptr};
+    p.C = nullptr; p.ldc = 0; p.sm = &smo;
+    return launch_gemm_tc(ctx, p, ctx->fc2, st);
+  }
+  p.C = h2; p.ldc = kH2Ld;
+  SC_TRY(launch_gemm(ctx, p, ctx->fc2, st));
+  return launch_out_softmax(ctx, h2, m, proba, label, nullptr, nullptr, nullptr, st);
 }
 
 }  // namespace sc

@@ -583,15 +583,16 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
                             float sscale) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  if (trainable[i]) {
+  const uint8_t t = trainable[i];
+  if (t == 1) {
     const float gi = g[i] * gscale;
     const float mi = b1 * m[i] + (1.f - b1) * gi;
     const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
     m[i] = mi; v[i] = vi;
     p[i] = p[i] - a_t * mi / (sqrtf(vi) + eps);
-  } else {
+  } else if (t == 0) {
     p[i] = 0.9f * p[i] + 0.1f * (g[i] * sscale);   // BN running mean / inv_std (Lasagne alpha = 0.1)
-  }
+  }                                                 // 2: frozen (sc_freeze_trunk), parameter and moments untouched
 }
 
 int adam_step(sc_ctx* ctx, float lr, float b1, float b2, float eps, float gscale, float sscale, cudaStream_t st) {
@@ -631,10 +632,12 @@ struct SimtBuf {       // the exact-fp32 SIMT back-end (gemm = 0): planar fp32 m
   float *CAT, *ZF1, *CAT2, *ZF2, *H2, *ZO, *dZO, *dH2, *dZF2, *dCAT2, *dZF1, *dCAT;
 };
 struct StepBuf {
-  float *in[3], *in4; uint8_t* y;      // the caller's batch, staged
+  float *in[3], *in4; uint8_t* y;      // the caller's batch, staged (the head-only step: in4 / y gathered from its tables)
   uint8_t* masks;
   unsigned long long* seed;
   float* loss;
+  int64_t* idx;                        // head-only step: the staged row indices (unused without an index list)
+  const HeadGather* head = nullptr;    // head-only step of fine-tuning: gather of cached trunk features, no convolutions
   SimtBuf simt;                        // gemm = 0
   TcBranchBuf tc[3];                   // gemm = 1
   TcDenseBuf td;
@@ -677,16 +680,20 @@ static void carve_simt(SimtBuf& M, Bump& B, int n) {
   M.dCAT = B.take<float>((size_t)n * 540);
 }
 
-static size_t carve_step(StepBuf& S, char* base, int n, bool tc) {
+// head: the head-only step (tensor cores only) keeps no patches and no conv maps
+static size_t carve_step(StepBuf& S, char* base, int n, bool tc, bool head = false) {
   Bump B{base, 0};
-  for (int b = 0; b < 3; ++b) S.in[b] = B.take<float>((size_t)n * 1024);
+  if (!head)
+    for (int b = 0; b < 3; ++b) S.in[b] = B.take<float>((size_t)n * 1024);
   S.in4 = B.take<float>((size_t)n * 15);
   S.y = B.take<uint8_t>((size_t)n);
   S.masks = B.take<uint8_t>((size_t)n * 2700);
   S.seed = B.take<unsigned long long>(1);
   S.loss = B.take<float>(1);
+  if (head) S.idx = B.take<int64_t>((size_t)n);
   if (tc) {
-    for (int b = 0; b < 3; ++b) tc_carve_branch(S.tc[b], B.take<char>(tc_branch_bytes(n)), n);
+    if (!head)
+      for (int b = 0; b < 3; ++b) tc_carve_branch(S.tc[b], B.take<char>(tc_branch_bytes(n)), n);
     tdense_carve(S.td, B.take<char>(tdense_bytes(n)), n);
   } else {
     carve_simt(S.simt, B, n);
@@ -819,7 +826,7 @@ static int tcgen05_branch_forward(sc_ctx* ctx, int b, const StepBuf& S, int n, c
 }
 
 static int tcgen05_branch_backward(sc_ctx* ctx, int b, const StepBuf& S, int n, cudaStream_t s) {
-  SC_TRY(tdense_branch_backward(ctx, b, S.td, n, S.masks, s));
+  SC_TRY(tdense_branch_backward(ctx, b, S.td, n, S.masks, true, s));
   return tc_branch_backward(ctx, b, S.tc[b], S.in[b], S.td.dF5[b], 576, S.masks, n, s);
 }
 
@@ -827,6 +834,8 @@ static int tcgen05_branch_backward(sc_ctx* ctx, int b, const StepBuf& S, int n, 
 // scalar that changes from step to step is read from device memory (the dropout seed), so the same sequence of launches is
 // valid as a captured CUDA graph.  The three branches are independent between the patches and the concatenation (forward)
 // and after the gradient of the concatenation (backward): they run on three streams forked from / joined into `st`.
+// With S.head (fine-tuning) the branches start at d1: one gather writes d1's operands from the cached trunk features, and
+// the backward pass stops at d1's weight gradients.  Every trunk entry of the gradient buffer then stays 0.
 static int train_body(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bool injected_masks, cudaStream_t st) {
   const bool tc = ctx->gemm_backend == 1;
   cudaStream_t sb[3] = {st, ctx->train_side[0], ctx->train_side[1]};
@@ -835,12 +844,14 @@ static int train_body(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bo
   SC_CUDA(cudaMemsetAsync(ctx->grads, 0, sizeof(float) * SC_PARAM_FLOATS, st));
   SC_CUDA(cudaMemsetAsync(S.loss, 0, sizeof(float), st));
   if (!injected_masks) { make_masks_kernel<<<ew_grid((int64_t)n * 2700), 256, 0, st>>>(S.masks, (int64_t)n * 2700, S.seed); ctx->launches++; }
+  if (S.head) SC_TRY(launch_head_gather(ctx, *S.head, st));
   SC_CUDA(cudaEventRecord(ev[0], st));
   for (int b = 1; b < 3; ++b) SC_CUDA(cudaStreamWaitEvent(sb[b], ev[0], 0));
 
   // forward of the branches, then the head (forward and backward) on `st`
   for (int b = 0; b < 3; ++b) {
-    SC_TRY(tc ? tcgen05_branch_forward(ctx, b, S, n, sb[b]) : simt_branch_forward(ctx, b, S, n, sb[b]));
+    if (S.head) SC_TRY(tdense_branch_forward(ctx, b, S.td, nullptr, n, S.masks, sb[b]));
+    else SC_TRY(tc ? tcgen05_branch_forward(ctx, b, S, n, sb[b]) : simt_branch_forward(ctx, b, S, n, sb[b]));
     if (b > 0) { SC_CUDA(cudaEventRecord(ev[b], sb[b])); SC_CUDA(cudaStreamWaitEvent(st, ev[b], 0)); }
   }
   SC_TRY(tc ? tdense_head(ctx, S.td, S.in4, S.y, n, n_global, S.masks, S.loss, st) : simt_head(ctx, S, n, n_global, st));
@@ -849,10 +860,75 @@ static int train_body(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bo
 
   // backward of the branches
   for (int b = 0; b < 3; ++b) {
-    SC_TRY(tc ? tcgen05_branch_backward(ctx, b, S, n, sb[b]) : simt_branch_backward(ctx, b, S, n, sb[b]));
+    if (S.head) SC_TRY(tdense_branch_backward(ctx, b, S.td, n, S.masks, false, sb[b]));
+    else SC_TRY(tc ? tcgen05_branch_backward(ctx, b, S, n, sb[b]) : simt_branch_backward(ctx, b, S, n, sb[b]));
     if (b > 0) { SC_CUDA(cudaEventRecord(ev[3 + b], sb[b])); SC_CUDA(cudaStreamWaitEvent(st, ev[3 + b], 0)); }
   }
   SC_CUDA(cudaGetLastError());
+  return SC_OK;
+}
+
+// the step's persistent resources (allocated outside any stream capture)
+static int step_prepare(sc_ctx* ctx, bool tc, bool head) {
+  if (!ctx->train_consts) {
+    SC_CUDA(cudaMalloc(&ctx->train_consts, 2 * kTrainZeros * sizeof(float)));
+    std::vector<float> h1(2 * kTrainZeros);
+    for (int i = 0; i < 2 * kTrainZeros; ++i) h1[i] = i < kTrainZeros ? 1.f : 0.f;
+    SC_CUDA(cudaMemcpy(ctx->train_consts, h1.data(), h1.size() * sizeof(float), cudaMemcpyHostToDevice));
+  }
+  if (!ctx->train_side[0]) {
+    for (int i = 0; i < 2; ++i) SC_CUDA(cudaStreamCreateWithFlags(&ctx->train_side[i], cudaStreamNonBlocking));
+    for (int i = 0; i < 8; ++i) SC_CUDA(cudaEventCreateWithFlags(&ctx->train_ev[i], cudaEventDisableTiming));
+  }
+  if (tc && !head) SC_TRY(tc_train_prepare(ctx));
+  if (tc) SC_TRY(tdense_prepare(ctx));
+  return SC_OK;
+}
+
+// train_body on `st`, kernel by kernel or as the captured graph of its shape
+static int run_step(sc_ctx* ctx, const StepBuf& S, int n, int64_t n_global, bool injected, cudaStream_t st) {
+  const bool tc = ctx->gemm_backend == 1;
+  const bool use_graph = ctx->train_graph_on && !ctx->profile && !(tc && ctx->ar_hook && !S.head);   // the sync-BN hook runs host code between kernels
+  if (!use_graph) return train_body(ctx, S, n, n_global, injected, st);
+  sc_ctx::TrainGraph key = {n, (long long)n_global, injected ? 1 : 0, ctx->gemm_backend, ctx->ws_fit.ptr, nullptr, 0,
+                            {nullptr, nullptr, nullptr}, 0};
+  if (S.head) {
+    key.tables[0] = S.head->feats; key.tables[1] = S.head->atlas_rows; key.tables[2] = S.head->labels;
+    key.has_idx = S.head->idx != nullptr;
+  }
+  sc_ctx::TrainGraph* g = nullptr;
+  for (auto& e : ctx->train_graphs)
+    if (e.n == key.n && e.n_global == key.n_global && e.injected == key.injected && e.backend == key.backend && e.arena == key.arena &&
+        e.tables[0] == key.tables[0] && e.tables[1] == key.tables[1] && e.tables[2] == key.tables[2] && e.has_idx == key.has_idx) g = &e;
+  if (!g) {
+    // a moved arena invalidates every captured address
+    for (size_t i = 0; i < ctx->train_graphs.size();) {
+      if (ctx->train_graphs[i].arena != ctx->ws_fit.ptr) { cudaGraphExecDestroy(ctx->train_graphs[i].exec); ctx->train_graphs.erase(ctx->train_graphs.begin() + i); }
+      else ++i;
+    }
+    if (ctx->train_graphs.size() >= 8) { cudaGraphExecDestroy(ctx->train_graphs[0].exec); ctx->train_graphs.erase(ctx->train_graphs.begin()); }
+    cudaStream_t cap;
+    SC_CUDA(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));   // capture on a private stream: `st` may be the legacy default stream
+    const int64_t l0 = ctx->launches;
+    SC_CUDA(cudaStreamBeginCapture(cap, cudaStreamCaptureModeRelaxed));
+    const int bs = train_body(ctx, S, n, n_global, injected, cap);
+    cudaGraph_t graph = nullptr;
+    const cudaError_t ce = cudaStreamEndCapture(cap, &graph);
+    cudaStreamDestroy(cap);
+    const int launches = (int)(ctx->launches - l0);
+    ctx->launches = l0;
+    if (bs != SC_OK) { if (graph) cudaGraphDestroy(graph); return bs; }
+    SC_CUDA(ce);
+    cudaGraphExec_t exec = nullptr;
+    const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
+    cudaGraphDestroy(graph);
+    SC_CUDA(ie);
+    key.exec = exec; key.launches = launches;
+    ctx->train_graphs.push_back(key);
+    g = &ctx->train_graphs.back();
+  }
+  SC_CUDA(cudaGraphLaunch(g->exec, st));
+  ctx->launches += g->launches;
   return SC_OK;
 }
 
@@ -865,17 +941,7 @@ int train_forward_backward(sc_ctx* ctx, const float* in1, const float* in2, cons
   const size_t need = carve_step(S, nullptr, n, tc);
   SC_TRY(ensure_ws(ctx->ws_fit, need + 4096));
   carve_step(S, reinterpret_cast<char*>(ctx->ws_fit.ptr), n, tc);
-  if (!ctx->train_consts) {
-    SC_CUDA(cudaMalloc(&ctx->train_consts, 2 * kTrainZeros * sizeof(float)));
-    std::vector<float> h1(2 * kTrainZeros);
-    for (int i = 0; i < 2 * kTrainZeros; ++i) h1[i] = i < kTrainZeros ? 1.f : 0.f;
-    SC_CUDA(cudaMemcpy(ctx->train_consts, h1.data(), h1.size() * sizeof(float), cudaMemcpyHostToDevice));
-  }
-  if (!ctx->train_side[0]) {
-    for (int i = 0; i < 2; ++i) SC_CUDA(cudaStreamCreateWithFlags(&ctx->train_side[i], cudaStreamNonBlocking));
-    for (int i = 0; i < 8; ++i) SC_CUDA(cudaEventCreateWithFlags(&ctx->train_ev[i], cudaEventDisableTiming));
-  }
-  if (tc) { SC_TRY(tc_train_prepare(ctx)); SC_TRY(tdense_prepare(ctx)); }
+  SC_TRY(step_prepare(ctx, tc, false));
   // stage the caller's batch into the arena: the step itself only ever sees context-owned addresses
   const float* ins[3] = {in1, in2, in3};
   for (int b = 0; b < 3; ++b) SC_CUDA(cudaMemcpyAsync(S.in[b], ins[b], (size_t)n * 4096, cudaMemcpyDeviceToDevice, st));
@@ -886,44 +952,34 @@ int train_forward_backward(sc_ctx* ctx, const float* in1, const float* in2, cons
   SC_CUDA(cudaMemcpyAsync(S.seed, &seed_h, sizeof(seed_h), cudaMemcpyHostToDevice, st));   // pageable source: staged before the call returns
   // the split dense operands of the tcgen05 step: the step writes their valid entries only, the K padding must read as zero
   if (tc) SC_CUDA(cudaMemsetAsync(S.td.zero_begin, 0, S.td.zero_bytes, st));
+  SC_TRY(run_step(ctx, S, n, n_global, masks_in != nullptr, st));
+  SC_CUDA(cudaMemcpyAsync(loss, S.loss, sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return SC_OK;
+}
 
-  const bool use_graph = ctx->train_graph_on && !ctx->profile && !(tc && ctx->ar_hook);   // the sync-BN hook runs host code between kernels
-  if (!use_graph) {
-    SC_TRY(train_body(ctx, S, n, n_global, masks_in != nullptr, st));
-  } else {
-    sc_ctx::TrainGraph* g = nullptr;
-    for (auto& e : ctx->train_graphs)
-      if (e.n == n && e.n_global == (long long)n_global && e.injected == (masks_in ? 1 : 0) && e.backend == ctx->gemm_backend &&
-          e.arena == ctx->ws_fit.ptr) g = &e;
-    if (!g) {
-      // a moved arena invalidates every captured address
-      for (size_t i = 0; i < ctx->train_graphs.size();) {
-        if (ctx->train_graphs[i].arena != ctx->ws_fit.ptr) { cudaGraphExecDestroy(ctx->train_graphs[i].exec); ctx->train_graphs.erase(ctx->train_graphs.begin() + i); }
-        else ++i;
-      }
-      if (ctx->train_graphs.size() >= 8) { cudaGraphExecDestroy(ctx->train_graphs[0].exec); ctx->train_graphs.erase(ctx->train_graphs.begin()); }
-      cudaStream_t cap;
-      SC_CUDA(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));   // capture on a private stream: `st` may be the legacy default stream
-      const int64_t l0 = ctx->launches;
-      SC_CUDA(cudaStreamBeginCapture(cap, cudaStreamCaptureModeRelaxed));
-      const int bs = train_body(ctx, S, n, n_global, masks_in != nullptr, cap);
-      cudaGraph_t graph = nullptr;
-      const cudaError_t ce = cudaStreamEndCapture(cap, &graph);
-      cudaStreamDestroy(cap);
-      const int launches = (int)(ctx->launches - l0);
-      ctx->launches = l0;
-      if (bs != SC_OK) { if (graph) cudaGraphDestroy(graph); return bs; }
-      SC_CUDA(ce);
-      cudaGraphExec_t exec = nullptr;
-      const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
-      cudaGraphDestroy(graph);
-      SC_CUDA(ie);
-      ctx->train_graphs.push_back({n, (long long)n_global, masks_in ? 1 : 0, ctx->gemm_backend, ctx->ws_fit.ptr, exec, launches});
-      g = &ctx->train_graphs.back();
-    }
-    SC_CUDA(cudaGraphLaunch(g->exec, st));
-    ctx->launches += g->launches;
-  }
+// fine-tuning: one training step of the head (d1 x3, FC1, fc_2, out_layer) on rows idx[0..n) of a table of cached trunk
+// features; the same dropout masks, loss and gradients as train_forward_backward with a trunk evaluated in deterministic mode
+int head_train_forward_backward(sc_ctx* ctx, const float* feats, const float* atlas_rows, const uint8_t* labels, const int64_t* idx,
+                                int64_t n64, int64_t n_global, uint64_t seed, const uint8_t* masks_in, float* loss, cudaStream_t st) {
+  const int n = (int)n64;
+  StepBuf S;
+  const size_t need = carve_step(S, nullptr, n, true, true);
+  SC_TRY(ensure_ws(ctx->ws_fit, need + 4096));
+  carve_step(S, reinterpret_cast<char*>(ctx->ws_fit.ptr), n, true, true);
+  SC_TRY(step_prepare(ctx, true, true));
+  HeadGather g;
+  g.feats = feats; g.atlas_rows = atlas_rows; g.labels = labels;
+  g.idx = idx ? S.idx : nullptr; g.row0 = 0; g.n = n; g.masks = S.masks;
+  for (int b = 0; b < 3; ++b) { g.F5s[b] = S.td.F5s[b]; g.F5T[b] = S.td.F5T[b]; }
+  g.npad = S.td.npad; g.in4 = S.in4; g.y = S.y;
+  S.head = &g;
+  // per-step values: the index slice, the injected masks and the seed are staged into the arena (the tables are in the graph key)
+  if (idx) SC_CUDA(cudaMemcpyAsync(S.idx, idx, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+  if (masks_in) SC_CUDA(cudaMemcpyAsync(S.masks, masks_in, (size_t)n * 2700, cudaMemcpyDeviceToDevice, st));
+  const unsigned long long seed_h = seed;
+  SC_CUDA(cudaMemcpyAsync(S.seed, &seed_h, sizeof(seed_h), cudaMemcpyHostToDevice, st));   // pageable source: staged before the call returns
+  SC_CUDA(cudaMemsetAsync(S.td.zero_begin, 0, S.td.zero_bytes, st));
+  SC_TRY(run_step(ctx, S, n, n_global, masks_in != nullptr, st));
   SC_CUDA(cudaMemcpyAsync(loss, S.loss, sizeof(float), cudaMemcpyDeviceToDevice, st));
   return SC_OK;
 }
@@ -950,6 +1006,10 @@ int eval_batch(sc_ctx* ctx, const float* in1, const float* in2, const float* in3
   float* proba = reinterpret_cast<float*>(ctx->ws_train.ptr);
   SC_TRY(forward_patches(ctx, in1, in2, in3, in4, n, proba, nullptr, st));
   SC_CUDA(cudaMemsetAsync(out2, 0, 2 * sizeof(float), st));
+  return launch_eval_reduce(ctx, proba, y, n, out2, st);
+}
+
+int launch_eval_reduce(sc_ctx* ctx, const float* proba, const uint8_t* y, int64_t n, float* out2, cudaStream_t st) {
   eval_reduce_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(proba, y, (int)n, out2);
   ctx->launches++;
   SC_CUDA(cudaGetLastError());

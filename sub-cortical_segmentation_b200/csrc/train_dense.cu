@@ -258,11 +258,12 @@ int tdense_split(sc_ctx* ctx, const float* in, int ld_in, int n, int N, const fl
   return SC_OK;
 }
 
-// d1 of branch b, forward: F5 (plain [n][540], dropout applied) -> CAT columns b*180.. (PReLU + f1_drop)
+// d1 of branch b, forward: F5 (plain [n][540], dropout applied) -> CAT columns b*180.. (PReLU + f1_drop).  F5 == nullptr: the
+// split operands D.F5s[b] / D.F5T[b] are already written (the head-only step gathers them from cached trunk features)
 int tdense_branch_forward(sc_ctx* ctx, int b, const TcDenseBuf& D, const float* F5, int n, const uint8_t* masks, cudaStream_t s) {
   const BranchOff& Ob = ctx->off.br[b];
   SC_TRY(tdense_derive(ctx, b, s));
-  SC_TRY(tdense_split(ctx, F5, 540, n, 540, nullptr, nullptr, D.F5s[b], 576, 0, D.F5T[b], D.npad, s));
+  if (F5) SC_TRY(tdense_split(ctx, F5, 540, n, 540, nullptr, nullptr, D.F5s[b], 576, 0, D.F5T[b], D.npad, s));
   SC_TRY(tgemm(ctx, D.F5s[b], n, 576, ctx->train_dw[b].wnk, 180, 192, ctx->train_dw[b].bias, D.Z1[b], 192, 180, PC_TRAIN_FWD, s));
   SC_TRY(tdense_split(ctx, D.Z1[b], 192, n, 180, ctx->params + Ob.d1alpha, masks + 1620 + b * 180, D.CATs, 576, b * 180, D.CATT, D.npad, s));
   return SC_OK;
@@ -306,8 +307,8 @@ int tdense_head(sc_ctx* ctx, const TcDenseBuf& D, const float* in4, const uint8_
   return SC_OK;
 }
 
-// d1 of branch b, backward: dCAT columns b*180.. -> gradients of d1 and dF5 (plain [n][576], columns 0..539)
-int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const uint8_t* masks, cudaStream_t s) {
+// d1 of branch b, backward: dCAT columns b*180.. -> gradients of d1 and (dgrad) dF5 (plain [n][576], columns 0..539)
+int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const uint8_t* masks, bool dgrad, cudaStream_t s) {
   const BranchOff& Ob = ctx->off.br[b];
   float* P = ctx->params;
   float* G = ctx->grads;
@@ -315,7 +316,8 @@ int tdense_branch_backward(sc_ctx* ctx, int b, const TcDenseBuf& D, int n, const
                                                   D.dZ1s[b], 192, D.dZ1T[b], D.npad, G + Ob.d1alpha, G + Ob.d1b);
   SC_TRY(tgemm(ctx, D.F5T[b], 540, D.npad, D.dZ1T[b], 180, 192, ctx->train_consts + kTrainZeros, D.gW1[b], 192, 180, PC_TRAIN_BWD, s));
   tcopy_grad_kernel<<<g256(540 * 180), 256, 0, s>>>(D.gW1[b], 192, 540, 180, G + Ob.d1W);
-  SC_TRY(tgemm(ctx, D.dZ1s[b], n, 192, ctx->train_dw[b].wkn, 540, 576, ctx->train_consts + kTrainZeros, D.dF5[b], 576, 540, PC_TRAIN_BWD, s));
+  if (dgrad)
+    SC_TRY(tgemm(ctx, D.dZ1s[b], n, 192, ctx->train_dw[b].wkn, 540, 576, ctx->train_consts + kTrainZeros, D.dF5[b], 576, 540, PC_TRAIN_BWD, s));
   ctx->launches += 2;
   SC_CUDA(cudaGetLastError());
   return SC_OK;

@@ -4,6 +4,9 @@ keys); everything below the imports runs on the B200 kernels.
 
     python train_model.py [configuration.cfg] [--train] [--evaluate]
 
+--train with [model] fine_tune_from = <experiment> fine-tunes the head of nets/<experiment>/<experiment>.pkl on the training
+folder (frozen convolutional trunk, Net.fine_tune) instead of training from scratch.
+
 --evaluate scores each inference subject that has manual labels (<subject>/<roi_name>): per-structure Dice and
 surface distances of the segmentation test_scan wrote, and with [model] mc_samples > 0 the mean Monte-Carlo dropout entropy
 inside each predicted structure.
@@ -15,8 +18,8 @@ import sys
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "sub-cortical_segmentation_b200"))
 
-from cnn_cort.base import (evaluate_scan, generate_training_set, load_data, load_test_names, structure_uncertainty,  # noqa: E402
-                           test_scan)
+from cnn_cort.base import (evaluate_scan, generate_training_set, load_data, load_scan_training_set, load_test_names,  # noqa: E402
+                           structure_uncertainty, test_scan)
 from cnn_cort.nifti import load as load_nii  # noqa: E402
 from cnn_cort.load_options import load_options, print_options  # noqa: E402
 from cnn_cort.nets import build_model  # noqa: E402
@@ -32,7 +35,15 @@ def main():
     print_options(options)
     weights_path = os.path.join(os.getcwd(), "nets")
 
-    if "--train" in sys.argv:
+    if "--train" in sys.argv and options['fine_tune_from']:
+        # supervised domain adaptation: start from another experiment's weights, retrain the head on this training set with the
+        # convolutional trunk frozen; the best weights land in nets/<name>/<name>.pkl as after fit
+        net = build_model(weights_path, dict(options, load_weights='False'))
+        src = os.path.join(weights_path, options['fine_tune_from'], options['fine_tune_from'] + '.pkl')
+        print("    --> fine-tuning the head of", src)
+        net.load_params_from(src)
+        net.fine_tune(load_scan_training_set(options))
+    elif "--train" in sys.argv:
         x_axial, x_cor, x_sag, y, x_atlas, names = load_data(options)
         x_train_axial, x_train_cor, x_train_sag, x_train_atlas, y_train = generate_training_set(
             x_axial, x_cor, x_sag, x_atlas, y, options)
