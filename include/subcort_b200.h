@@ -284,6 +284,32 @@ SC_API int sc_register_objective(sc_ctx* ctx, const float* ref_dev, const int32_
  * dilated `iterations` times (sc_dilate_mask), as float32 0 / 1 [X][Y][Z]. */
 SC_API int sc_prior_mask(sc_ctx* ctx, const float* priors_dev, const int32_t dims[3], int iterations, float* mask_dev, void* stream);
 
+/* ---- resampling to the network's grid ------------------------------------------------
+ * The network is defined in voxels (32-voxel patches, 3x3 taps) and its weights were trained on 1 mm isotropic images; with
+ * [model] resample_mm the dense path runs on an isotropic grid of that voxel size and maps its output back to the scan's grid.
+ * Per axis independently: the native grid has n voxels, the target grid m (cnn_cort/base.py:resample_dims), r = n / m; the
+ * target grid keeps the native array axes and covers the same field of view (affine: native . [[diag(r), (r - 1) / 2], [0, 1]]).
+ *   sc_resample_volume: native -> target.  Target index j sits at native coordinate x_j = (j + 0.5) r - 0.5; with h = max(r, 1)
+ *     and w_ij = max(0, 1 - |i - x_j| / h) for 0 <= i < n, out_j = sum_i w_ij v_i / sum_i w_ij; the 3-D result is the separable
+ *     product of the three 1-D filters.  r > 1: antialiasing triangle filter; r < 1: linear interpolation with the edge value
+ *     held; r = 1: the identity, bit for bit.  Equal to torch's interpolate(mode='bilinear', antialias=True, align_corners=False)
+ *     per pair of axes.  in_dev [X][Y][Z][channels] and out_dev [m0][m1][m2][channels] float32, channels-last, channels 1 or 15,
+ *     filtered per channel.  The weights are convex: priors stay in [0, 1] and their per-voxel sum is kept.
+ *   sc_map_proba_back: target -> native.  Native voxel v sits at target y = (v + 0.5) / r - 0.5 per axis, clamped to [0, m - 1];
+ *     of its 8 trilinear neighbours those with non-zero weight and cand_dev != 0 are kept and their weights renormalised; the
+ *     native probability vector is the weighted mean of their proba_dev rows [m0*m1*m2][15], the label its first arg-max.  A
+ *     native voxel is written (label_dev uint8 [X][Y][Z], proba_out_dev float32 [X][Y][Z][15] when not NULL) only if it has at
+ *     least one such neighbour and native_mask_dev (uint8 [X][Y][Z], NULL = every voxel) is non-zero there; every other voxel
+ *     keeps what the outputs held.
+ * Both accumulate in fp32 in a fixed order without atomics (the same inputs give byte-identical outputs); intermediates and the
+ * per-axis weight tables live in the context.  SC_ERR_ARG, outputs untouched, for NULL required pointers, a dim below 1,
+ * channels not 1 or 15 and an output that is its input; the message names the argument. */
+SC_API int sc_resample_volume(sc_ctx* ctx, const float* in_dev, const int32_t in_dims[3], int channels, const int32_t out_dims[3],
+                              float* out_dev, void* stream);
+SC_API int sc_map_proba_back(sc_ctx* ctx, const float* proba_dev, const uint8_t* cand_dev, const int32_t target_dims[3],
+                             const uint8_t* native_mask_dev, const int32_t native_dims[3], uint8_t* label_dev, float* proba_out_dev,
+                             void* stream);
+
 /* ---- scatter -------------------------------------------------------------------------
  * replaces: image[x,y,z] = y_pred and image_proba[x,y,z,c] = proba[:,c] (base.py:430-440) */
 SC_API int sc_scatter(sc_ctx* ctx, const int32_t* xyz_dev, int64_t n, const int32_t* label_dev,

@@ -68,6 +68,8 @@ PROTOTYPES = {
     "sc_register_objective": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _p(ctypes.c_double), _vp, _p(_c_i32), _p(ctypes.c_double),
                                              _p(ctypes.c_double), _vp, _p(ctypes.c_double), _vp, _vp, _vp]),
     "sc_prior_mask": (ctypes.c_int, [_vp, _vp, _p(_c_i32), ctypes.c_int, _vp, _vp]),
+    "sc_resample_volume": (ctypes.c_int, [_vp, _vp, _p(_c_i32), ctypes.c_int, _p(_c_i32), _vp, _vp]),
+    "sc_map_proba_back": (ctypes.c_int, [_vp, _vp, _vp, _p(_c_i32), _vp, _p(_c_i32), _vp, _vp, _vp]),
     "sc_gather_patches": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, ctypes.c_int, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp]),
     "sc_gather_center_labels": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _c_i64, _vp, _vp]),
     "sc_gather_samples": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -355,6 +357,33 @@ class Context(object):
         out = torch.empty(tuple(priors.shape[:3]), dtype=torch.float32, device=priors.device)
         _check(self.lib.sc_prior_mask(self.h, _ptr(priors), _dims(priors.shape), int(iterations), _ptr(out), _stream()))
         return out
+
+    # -- resampling to the network's grid (include/subcort_b200.h) ------------------------------------
+    def resample_volume(self, vol, out_shape, out=None):
+        """float32 CUDA volume [X,Y,Z] or [X,Y,Z,15] -> the same on the grid of out_shape (3 dims) covering the same field of
+        view: separable triangle filter (antialiased when shrinking, linear when growing), the identity on an unchanged axis
+        (sc_resample_volume)"""
+        import torch
+        ch = int(vol.shape[3]) if vol.dim() == 4 else 1
+        shape = tuple(int(s) for s in out_shape[:3]) + ((ch,) if vol.dim() == 4 else ())
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=vol.device)
+        _check(self.lib.sc_resample_volume(self.h, _ptr(vol), _dims(vol.shape), ch, _dims(shape), _ptr(out), _stream()))
+        return out
+
+    def map_proba_back(self, proba, cand, native_shape, native_mask=None, want_proba=False, label_out=None, proba_out=None):
+        """target-grid probabilities (float32 CUDA [m0,m1,m2,15]) and candidates (uint8 [m0,m1,m2]) -> (uint8 labels [X,Y,Z],
+        float32 probabilities [X,Y,Z,15] or None) on the native grid: trilinear mean over the candidate neighbours, first arg-max
+        (sc_map_proba_back).  Voxels without a candidate neighbour, or outside native_mask, keep the outputs' contents (zeros
+        unless label_out / proba_out are given)."""
+        import torch
+        shape = tuple(int(s) for s in native_shape[:3])
+        label = label_out if label_out is not None else torch.zeros(shape, dtype=torch.uint8, device=proba.device)
+        if proba_out is None and want_proba:
+            proba_out = torch.zeros(shape + (15,), dtype=torch.float32, device=proba.device)
+        _check(self.lib.sc_map_proba_back(self.h, _ptr(proba), _ptr(cand), _dims(proba.shape), _ptr(native_mask), _dims(shape),
+                                          _ptr(label), _ptr(proba_out), _stream()))
+        return label, proba_out
 
     def gather_patches(self, vol, xyz, atlas=None, bg_fix=True, views=(True, True, True)):
         import torch

@@ -202,6 +202,10 @@ def test_scan(net, test_scan, options):
     want_proba = options['out_probabilities'] == 'True'
     mc_samples = int(options.get('mc_samples', 0) or 0)
     mc = {'samples': mc_samples, 'seed': int(options.get('mc_seed', 0) or 0)} if mc_samples > 0 else None
+    resample_mm = options.get('resample_mm')
+    if resample_mm is not None and (mode == 'patchwise' or mc is not None):
+        raise ValueError("resample_mm = %g is implemented for the dense inference mode without Monte-Carlo dropout only "
+                         "(inference = %s, mc_samples = %d)" % (resample_mm, mode, mc_samples))
     if mode == 'patchwise':
         if mc is not None:
             raise ValueError("mc_samples = %d: Monte-Carlo dropout is implemented for the dense inference mode only" % mc_samples)
@@ -233,7 +237,8 @@ def test_scan(net, test_scan, options):
             post_mask = None
             if options['post_process'] == 'True':      # filtered on the device, before the label volume is downloaded
                 post_mask = crop_mask if crop_mask is not None else nib.load(os.path.join(image_path, 'tmp', 'MNI_subcortical_mask.nii.gz'), pinned=True).get_data()
-        labels, image_proba, n_cand = segment_arrays(net.ctx, t1, atlas, crop_mask, want_proba, timings, post_mask=post_mask, mc=mc)
+        labels, image_proba, n_cand = segment_arrays(net.ctx, t1, atlas, crop_mask, want_proba, timings, post_mask=post_mask, mc=mc,
+                                                     spacing=voxel_spacing(t1_nii.affine), resample_mm=resample_mm)
         if options['debug'] == 'True':
             print("    -->  num of samples to test:", n_cand)
         image = labels.astype(t1.dtype)
@@ -251,7 +256,8 @@ def test_scan(net, test_scan, options):
     return (time.time() - s_time) / 60.0
 
 
-def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=None, post_mask=None, mc=None):
+def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=None, post_mask=None, mc=None, spacing=None,
+                   resample_mm=None):
     """The timed part of test_scan for one scan, device-resident from the first byte [base.py:357-372, 401-440]:
     raw T1 / atlas priors (/ registered mask) as host arrays in -> uint8 label volume (+ float32 [X,Y,Z,15] probabilities,
     number of candidates) out.  One upload per array (Fortran-ordered NIfTI arrays are reordered on the device), then
@@ -263,10 +269,23 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
 
     mc={'samples': T, 'seed': s}: Monte-Carlo dropout (sc_segment_volume_mc) -- the labels and probabilities are those of the
     mean of T dropout passes, and on return the dict also holds 'entropy' (predictive entropy, nats) and 'mutual_info' as
-    float32 [X,Y,Z] host arrays, zero outside the candidates."""
+    float32 [X,Y,Z] host arrays, zero outside the candidates.
+
+    resample_mm (with spacing, the scan's voxel size in mm along x, y, z): the network runs on the isotropic grid of that voxel
+    size (resample_dims) and its output is mapped back (_segment_resampled); labels and probabilities keep the scan's grid.  When
+    the target grid equals the scan's, this is the path without resampling, launch for launch."""
     import torch
     t0 = time.time()
     shape = tuple(int(s) for s in t1.shape[:3])
+    tshape = None
+    if resample_mm is not None:
+        if spacing is None:
+            raise ValueError("segment_arrays: resample_mm needs the scan's voxel spacing")
+        tshape, _ = resample_dims(shape, spacing, resample_mm)
+        if tshape == shape:
+            tshape = None
+        elif mc is not None:
+            raise ValueError("segment_arrays: Monte-Carlo dropout is not implemented with resample_mm")
     on_device = torch.is_tensor(atlas)
     if not on_device:
         atlas = np.asarray(atlas)
@@ -302,29 +321,33 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
 
     # T1 first: copies of one direction are served in issue order, and the convolution phase only waits for the T1 volume
     raw, dt = ctx.upload_volume(t1)
-    vol, mean, std = ctx.normalise_volume(raw, dt, shape)
-    if crop_mask is not None:
-        mraw, mdt = device_bytes(crop_mask)
-        cand = ctx.dilate_mask(ctx.candidate_mask(mraw, mdt, shape), 10)   # == ndimage.binary_dilation(mask, iterations=10)
+    if tshape is not None:
+        mraw, mdt = device_bytes(crop_mask) if crop_mask is not None else (None, None)
+        lab, prob, box, n_cand, mean, std = _segment_resampled(ctx, raw, dt, shape, tshape, atlas, mraw, mdt, want_proba)
     else:
-        cand = ctx.candidate_mask(raw, dt, shape)                          # == image.astype('bool')
-    box, n_cand = ctx.mask_bbox(cand)
-    if box is not None:
-        d_atlas = start_atlas_upload(box if crop_mask is not None else None)
-    lab = torch.zeros(shape, dtype=torch.uint8, device=vol.device)
-    prob = torch.zeros(shape + (15,), dtype=torch.float32, device=vol.device) if want_proba else None
-    ent = mi = None
-    if mc is not None:
-        ent = torch.zeros(shape, dtype=torch.float32, device=vol.device)
-        mi = torch.zeros(shape, dtype=torch.float32, device=vol.device)
-    if box is not None:
-        ready = None if on_device else atlas_ready
-        if mc is None:
-            ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob, atlas_ready=ready)
+        vol, mean, std = ctx.normalise_volume(raw, dt, shape)
+        if crop_mask is not None:
+            mraw, mdt = device_bytes(crop_mask)
+            cand = ctx.dilate_mask(ctx.candidate_mask(mraw, mdt, shape), 10)   # == ndimage.binary_dilation(mask, iterations=10)
         else:
-            ctx.segment_volume_mc(vol, d_atlas, int(mc['samples']), int(mc.get('seed', 0)), box=box, cand_mask=cand, label_vol=lab,
-                                  proba_vol=prob, entropy_vol=ent, mi_vol=mi, atlas_ready=ready)
-    main.wait_stream(side)
+            cand = ctx.candidate_mask(raw, dt, shape)                          # == image.astype('bool')
+        box, n_cand = ctx.mask_bbox(cand)
+        if box is not None:
+            d_atlas = start_atlas_upload(box if crop_mask is not None else None)
+        lab = torch.zeros(shape, dtype=torch.uint8, device=vol.device)
+        prob = torch.zeros(shape + (15,), dtype=torch.float32, device=vol.device) if want_proba else None
+        ent = mi = None
+        if mc is not None:
+            ent = torch.zeros(shape, dtype=torch.float32, device=vol.device)
+            mi = torch.zeros(shape, dtype=torch.float32, device=vol.device)
+        if box is not None:
+            ready = None if on_device else atlas_ready
+            if mc is None:
+                ctx.segment_volume(vol, d_atlas, box=box, cand_mask=cand, label_vol=lab, proba_vol=prob, atlas_ready=ready)
+            else:
+                ctx.segment_volume_mc(vol, d_atlas, int(mc['samples']), int(mc.get('seed', 0)), box=box, cand_mask=cand, label_vol=lab,
+                                      proba_vol=prob, entropy_vol=ent, mi_vol=mi, atlas_ready=ready)
+        main.wait_stream(side)
     if post_mask is not None:        # post_process_segmentation (base.py:460-480) on the device-resident label volume
         if post_mask is crop_mask and crop_mask is not None:
             pm = ctx.candidate_mask(mraw, mdt, shape)
@@ -345,6 +368,67 @@ def segment_arrays(ctx, t1, atlas, crop_mask=None, want_proba=False, timings=Non
         timings.update({'hot_s': time.time() - t0, 'n_candidates': n_cand, 'mean_nz': mean, 'std_nz': std, 'box': box})
     # views of reusable page-locked buffers: valid until the next call
     return h_lab.numpy(), (h_prob.numpy() if want_proba else None), n_cand
+
+
+def _torch_dtype(dt):
+    import torch
+    return torch.from_numpy(np.zeros(1, dt)).dtype
+
+
+def _segment_resampled(ctx, raw, dt, shape, tshape, atlas, mraw, mdt, want_proba):
+    """The dense pass of segment_arrays on the target grid tshape: the raw T1 bytes (and the registered mask's, mraw; None without
+    crop) of the native grid `shape` are resampled (sc_resample_volume), normalised over the non-zero resampled voxels, and the
+    candidates taken there (non-zero resampled T1, or the resampled mask > 0 dilated 10 times: 10 mm at 1 mm, as the reference's
+    10 voxels meant); the full priors are resampled too.  The target probabilities are mapped back (sc_map_proba_back) with the
+    non-zero native T1 voxels as the native mask (none in crop mode).  -> native (labels, probabilities or None), target box,
+    target candidates, mean_nz, std_nz."""
+    import torch
+    rs = ctx.resample_volume(raw.view(_torch_dtype(dt)).view(shape).to(torch.float32), tshape)
+    rs_bytes = rs.view(-1).view(torch.uint8)
+    vol, mean, std = ctx.normalise_volume(rs_bytes, np.float32, tshape)
+    if mraw is not None:
+        rm = ctx.resample_volume(mraw.view(_torch_dtype(mdt)).view(shape).to(torch.float32), tshape)
+        cand = ctx.dilate_mask(ctx.candidate_mask(rm.view(-1).view(torch.uint8), np.float32, tshape), 10)
+    else:
+        cand = ctx.candidate_mask(rs_bytes, np.float32, tshape)
+    box, n_cand = ctx.mask_bbox(cand)
+    lab = torch.zeros(shape, dtype=torch.uint8, device=vol.device)
+    prob = torch.zeros(shape + (15,), dtype=torch.float32, device=vol.device) if want_proba else None
+    if box is not None:
+        if torch.is_tensor(atlas):
+            d_atlas = atlas.to(vol.device, torch.float32).contiguous()
+        else:
+            d_atlas, _ = ctx.upload_volume(atlas, channels=15)
+            d_atlas = d_atlas.view(torch.float32).view(shape + (15,))
+        t_atlas = ctx.resample_volume(d_atlas, tshape)
+        del d_atlas
+        t_lab = torch.zeros(tshape, dtype=torch.uint8, device=vol.device)
+        t_prob = torch.zeros(tuple(tshape) + (15,), dtype=torch.float32, device=vol.device)
+        ctx.segment_volume(vol, t_atlas, box=box, cand_mask=cand, label_vol=t_lab, proba_vol=t_prob)
+        nmask = ctx.candidate_mask(raw, dt, shape) if mraw is None else None
+        ctx.map_proba_back(t_prob, cand, shape, native_mask=nmask, label_out=lab, proba_out=prob)
+    return lab, prob, box, n_cand, mean, std
+
+
+def voxel_spacing(affine):
+    """voxel size in mm along the three array axes: the column norms of a 4x4 voxel -> mm affine"""
+    return tuple(float(s) for s in np.sqrt((np.asarray(affine)[:3, :3] ** 2).sum(0)))
+
+
+def resample_dims(shape, spacing, resample_mm):
+    """The network's grid for a scan of `shape` voxels of `spacing` mm: per axis m = max(1, floor(n s / t + 0.5)) voxels for
+    t = resample_mm, with the native array axes kept and the same field of view, so the target voxel is r = n / m native voxels
+    (exactly t mm only where n s / t is an integer).  -> (target shape, r per axis)"""
+    t = float(resample_mm)
+    dims = tuple(max(1, int(np.floor(int(n) * float(s) / t + 0.5))) for n, s in zip(shape[:3], spacing))
+    return dims, tuple(int(n) / float(m) for n, m in zip(shape[:3], dims))
+
+
+def nearest_index(n, m):
+    """native index of each of the m target voxels of an axis of n native voxels, nearest neighbour: clamp(floor(x_j + 0.5))
+    with x_j = (j + 0.5) n / m - 0.5"""
+    x = (np.arange(m) + 0.5) * (float(n) / m) - 0.5
+    return np.clip(np.floor(x + 0.5), 0, n - 1).astype(np.int64)
 
 
 def structure_uncertainty(labels, entropy, mutual_info, device=None):
@@ -473,7 +557,7 @@ def evaluate_scan(seg_path, ref_path, device=None):
     seg_nii, ref_nii = load_nii(seg_path), load_nii(ref_path)
     if tuple(seg_nii.shape) != tuple(ref_nii.shape):
         raise ValueError("%s and %s differ in shape: %s vs %s" % (seg_path, ref_path, seg_nii.shape, ref_nii.shape))
-    spacing = tuple(float(s) for s in np.sqrt((np.asarray(ref_nii.affine)[:3, :3] ** 2).sum(0)))
+    spacing = voxel_spacing(ref_nii.affine)
     return evaluate_segmentation(seg_nii.get_data(), ref_nii.get_data(), spacing, device=device)
 
 
@@ -550,6 +634,8 @@ def register_masks(t1_path, options, timings=None):
 def load_data(options):
     """-> (x_axial, x_cor, x_sag, y_axial, x_atlas, names), lists indexed by subject.
     [base.py:11-37]"""
+    if options.get('resample_mm') is not None:
+        raise ValueError("load_data: resample_mm is implemented for the device-resident training set only (load_scan_training_set)")
     _register_folder(options['train_folder'], options)
     (x_axial, y_axial, x_cor, y_cor, x_sag, y_sag, x_atlas, names) = load_patches(
         dir_name=options['train_folder'], t1_name=options['t1_name'], mask_name=options['roi_name'],
@@ -774,25 +860,52 @@ def load_scan_training_set(options, randomize=True, device=None):
     (base.py:153-181), the atlas rows without background fix (quirk Q4), labels with 15 -> 0; subjects concatenated,
     then one permutation drawn as generate_training_set draws it.  Only the normalised T1 volumes stay on the device;
     the atlas rows and labels are picked from the host arrays the NIfTI reader returns (an upload of the 15-channel
-    priors would move 60 B per voxel to read 60 B per sample)."""
+    priors would move 60 B per voxel to read 60 B per sample).
+
+    options['resample_mm'] (optional): a subject whose grid differs from the network's (resample_dims) is resampled first, as
+    segment_arrays does at inference: the T1 on the device, then the train-path normalisation; the labels by nearest neighbour
+    (nearest_index); the atlas rows from the priors resampled on the device.  T1, labels and priors must then have one shape."""
     if tuple(options['patch_size']) != (32, 32):
         raise ValueError("only patch_size (32, 32) is implemented")
     ctx = get_context(options.get('device') if device is None else device)
     dir_name = options['train_folder']
     _register_folder(dir_name, options)
     subjects = [f for f in sorted(os.listdir(dir_name)) if os.path.isdir(os.path.join(dir_name, f))]
+    resample_mm = options.get('resample_mm')
     names, vols, samples, atlas_rows, labels = [], [], [], [], []
     for k, subject in enumerate(subjects):
         image_name = os.path.join(dir_name, subject, options['t1_name'])
         atlas_name = os.path.join(dir_name, subject, 'tmp', 'MNI_sub_probabilities.nii.gz')
         _require_registered(atlas_name)
-        vols.append(_dev(_train_normalise(load_nii(image_name).get_data()), ctx.device, np.float32))
+        t1_nii = load_nii(image_name)
         mask = load_nii(os.path.join(dir_name, subject, options['roi_name'])).get_data()
-        cen = _training_centres(mask, ctx.device)
-        x, y, z = cen[:, 0], cen[:, 1], cen[:, 2]
-        lab = mask[x, y, z].astype(np.uint8)
+        tshape = None
+        if resample_mm is not None:
+            shape = tuple(int(s) for s in t1_nii.shape[:3])
+            tshape, _ = resample_dims(shape, voxel_spacing(t1_nii.affine), resample_mm)
+            tshape = None if tshape == shape else tshape
+        if tshape is None:
+            vols.append(_dev(_train_normalise(t1_nii.get_data()), ctx.device, np.float32))
+            cen = _training_centres(mask, ctx.device)
+            x, y, z = cen[:, 0], cen[:, 1], cen[:, 2]
+            lab = mask[x, y, z].astype(np.uint8)
+            atlas_rows.append(np.asarray(load_nii(atlas_name).get_data()[x, y, z], dtype=np.float32))
+        else:
+            priors = load_nii(atlas_name).get_data()
+            if tuple(mask.shape[:3]) != shape or tuple(priors.shape) != shape + (15,):
+                raise ValueError("%s: T1 %s, labels %s and priors %s must share one grid to be resampled" % (
+                    subject, shape, tuple(mask.shape), tuple(priors.shape)))
+            t1 = ctx.resample_volume(_cuda_f32(t1_nii.get_data(), ctx.device), tshape).cpu().numpy()
+            vols.append(_dev(_train_normalise(t1), ctx.device, np.float32))
+            mask = np.asarray(mask)[np.ix_(*[nearest_index(n, m) for n, m in zip(shape, tshape)])]
+            cen = _training_centres(mask, ctx.device)
+            x, y, z = cen[:, 0], cen[:, 1], cen[:, 2]
+            lab = mask[x, y, z].astype(np.uint8)
+            rp = ctx.resample_volume(_cuda_f32(priors, ctx.device), tshape)
+            idx = _dev(cen.astype(np.int64), ctx.device)
+            atlas_rows.append(rp[idx[:, 0], idx[:, 1], idx[:, 2]].cpu().numpy())
+            del rp
         lab[lab == 15] = 0
-        atlas_rows.append(np.asarray(load_nii(atlas_name).get_data()[x, y, z], dtype=np.float32))
         samples.append(np.concatenate([np.full((len(cen), 1), k, np.int32), cen], axis=1))
         labels.append(lab)
         names.append(image_name)

@@ -10,6 +10,7 @@ Differences, all deliberate (SURVEY.md 5.6):
   ``speedup_segmentation = False`` still cropped there (quirk Q2); here it does not.
 """
 import configparser
+import math
 
 
 def _truthy(s):
@@ -65,7 +66,22 @@ def load_options(user_config):
     options['fine_tune_from'] = v or None
     if options['fine_tune_from'] == options['experiment']:
         raise ValueError("[model] fine_tune_from = %s names this experiment: its weights would be overwritten" % v)
+    # optional: the isotropic voxel size (mm) the network runs on; the scan is resampled to it and the outputs mapped back to
+    # the scan's grid (base.segment_arrays).  Off when absent or empty
+    v = g('model', 'resample_mm', fallback='').strip()
+    options['resample_mm'] = parse_resample_mm(v) if v else None
     return options
+
+
+def parse_resample_mm(v):
+    """a finite voxel size > 0 in mm, else ValueError"""
+    try:
+        mm = float(v)
+    except (TypeError, ValueError):
+        raise ValueError("[model] resample_mm = %r is not a number" % (v,))
+    if not math.isfinite(mm) or mm <= 0:
+        raise ValueError("[model] resample_mm = %r must be a finite number > 0" % (v,))
+    return mm
 
 
 def device_index(mode):

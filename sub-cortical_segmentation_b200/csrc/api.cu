@@ -134,7 +134,7 @@ int sc_destroy(sc_ctx* ctx) {
   tc_destroy(ctx);
   fused_detach(ctx);
   cudaFree(ctx->params); cudaFree(ctx->grads); cudaFree(ctx->adam_m); cudaFree(ctx->adam_v);
-  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr); cudaFree(ctx->ws_eval.ptr); cudaFree(ctx->ws_reg.ptr);
+  cudaFree(ctx->trainable); cudaFree(ctx->derived); cudaFree(ctx->ws.ptr); cudaFree(ctx->ws_train.ptr); cudaFree(ctx->ws_fit.ptr); cudaFree(ctx->ws_eval.ptr); cudaFree(ctx->ws_reg.ptr); cudaFree(ctx->ws_resample.ptr);
   for (auto& g : ctx->train_graphs) cudaGraphExecDestroy(g.exec);
   for (int i = 0; i < 2; ++i) if (ctx->train_side[i]) cudaStreamDestroy(ctx->train_side[i]);
   for (int i = 0; i < 8; ++i) if (ctx->train_ev[i]) cudaEventDestroy(ctx->train_ev[i]);
@@ -225,7 +225,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc", "head"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc", "head", "resample"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -433,6 +433,43 @@ int sc_prior_mask(sc_ctx* ctx, const float* priors_dev, const int32_t dims[3], i
   SC_TRY(check_dims(dims, "sc_prior_mask"));
   SC_CUDA(cudaSetDevice(ctx->device));
   return prior_mask(ctx, priors_dev, dims, iterations, mask_dev, (cudaStream_t)stream);
+}
+
+// resampling: every dim >= 1 and a volume the 32-bit voxel indices of the other calls can address
+static int check_grid(const int32_t* dims, const char* who, const char* name) {
+  SC_CHECK(dims != nullptr, SC_ERR_ARG, "%s: %s is NULL", who, name);
+  for (int i = 0; i < 3; ++i) SC_CHECK(dims[i] >= 1, SC_ERR_ARG, "%s: %s[%d] = %d is below 1", who, name, i, dims[i]);
+  SC_CHECK((int64_t)dims[0] * dims[1] * dims[2] < (1ll << 31), SC_ERR_ARG, "%s: %s volume too large", who, name);
+  return SC_OK;
+}
+
+int sc_resample_volume(sc_ctx* ctx, const float* in_dev, const int32_t in_dims[3], int channels, const int32_t out_dims[3], float* out_dev,
+                       void* stream) {
+  const char* who = "sc_resample_volume";
+  SC_CHECK(ctx, SC_ERR_ARG, "%s: ctx is NULL", who);
+  SC_CHECK(in_dev, SC_ERR_ARG, "%s: in_dev is NULL", who);
+  SC_CHECK(out_dev, SC_ERR_ARG, "%s: out_dev is NULL", who);
+  SC_CHECK(channels == 1 || channels == 15, SC_ERR_ARG, "%s: channels = %d (1 or 15)", who, channels);
+  SC_TRY(check_grid(in_dims, who, "in_dims"));
+  SC_TRY(check_grid(out_dims, who, "out_dims"));
+  SC_CHECK(out_dev != in_dev, SC_ERR_ARG, "%s: out_dev == in_dev (not in place)", who);
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return resample_volume(ctx, in_dev, in_dims, channels, out_dims, out_dev, (cudaStream_t)stream);
+}
+
+int sc_map_proba_back(sc_ctx* ctx, const float* proba_dev, const uint8_t* cand_dev, const int32_t target_dims[3], const uint8_t* native_mask_dev,
+                      const int32_t native_dims[3], uint8_t* label_dev, float* proba_out_dev, void* stream) {
+  const char* who = "sc_map_proba_back";
+  SC_CHECK(ctx, SC_ERR_ARG, "%s: ctx is NULL", who);
+  SC_CHECK(proba_dev, SC_ERR_ARG, "%s: proba_dev is NULL", who);
+  SC_CHECK(cand_dev, SC_ERR_ARG, "%s: cand_dev is NULL", who);
+  SC_CHECK(label_dev, SC_ERR_ARG, "%s: label_dev is NULL", who);
+  SC_TRY(check_grid(target_dims, who, "target_dims"));
+  SC_TRY(check_grid(native_dims, who, "native_dims"));
+  SC_CHECK(proba_out_dev != proba_dev, SC_ERR_ARG, "%s: proba_out_dev == proba_dev (not in place)", who);
+  SC_CHECK(label_dev != cand_dev, SC_ERR_ARG, "%s: label_dev == cand_dev (not in place)", who);
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return map_proba_back(ctx, proba_dev, cand_dev, target_dims, native_mask_dev, native_dims, label_dev, proba_out_dev, (cudaStream_t)stream);
 }
 
 int sc_gather_patches(sc_ctx* ctx, const float* vol_dev, const int32_t dims[3], const float* atlas_dev, int bg_fix,

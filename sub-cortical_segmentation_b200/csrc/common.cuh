@@ -148,7 +148,7 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_HEAD, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_HEAD, PC_RESAMPLE, PC_COUNT
 };
 
 // counter-based random bits (splitmix64 finaliser): the dropout keep masks of the training step and of Monte-Carlo dropout
@@ -190,6 +190,7 @@ struct sc_ctx {
   sc::Workspace ws_fit;          // training step: staged inputs, saved activations, gradients of activations
   sc::Workspace ws_eval;         // sc_evaluate_segmentation: distance fields, envelope stacks and distance lists of one class box
   sc::Workspace ws_reg;          // registration: pyramids, histogram, adjoint passes, control-point grids
+  sc::Workspace ws_resample;     // resampling: per-axis tables and the intermediates between the axis passes
   double* h_reg = nullptr;       // pinned: the optimiser's per-trial read-backs
   int reg_iters[8] = {};         // accepted steps of the last registration per level: affine 0..3, FFD 4..6
   // training step as a CUDA graph (one per (batch, global batch, injected masks) shape): the three branches run on
@@ -320,6 +321,12 @@ int register_objective(sc_ctx* ctx, const float* ref, const int32_t* rdims, cons
 int warp_volume(sc_ctx* ctx, const float* flo, const int32_t* fdims, int channels, const double* fv, const double* affine, const float* grid,
                 const int32_t* rdims, const double* rv, float* out, cudaStream_t st);
 int prior_mask(sc_ctx* ctx, const float* priors, const int32_t* dims, int iterations, float* out, cudaStream_t st);
+
+// resample.cu : native grid <-> the network's isotropic grid (separable triangle filter; trilinear back-mapping of probabilities)
+int resample_volume(sc_ctx* ctx, const float* in, const int32_t* in_dims, int channels, const int32_t* out_dims, float* out,
+                    cudaStream_t st);
+int map_proba_back(sc_ctx* ctx, const float* proba, const uint8_t* cand, const int32_t* tdims, const uint8_t* nmask,
+                   const int32_t* ndims, uint8_t* label, float* pout, cudaStream_t st);
 
 // weights.cu
 int derive_weights(sc_ctx* ctx, cudaStream_t st);

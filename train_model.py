@@ -6,6 +6,8 @@ keys); everything below the imports runs on the B200 kernels.
 
 --train with [model] fine_tune_from = <experiment> fine-tunes the head of nets/<experiment>/<experiment>.pkl on the training
 folder (frozen convolutional trunk, Net.fine_tune) instead of training from scratch.
+With [model] resample_mm set, training runs on the device-resident set resampled to that isotropic grid, as test_scan
+segments.
 
 --evaluate scores each inference subject that has manual labels (<subject>/<roi_name>): per-structure Dice and
 surface distances of the segmentation test_scan wrote, and with [model] mc_samples > 0 the mean Monte-Carlo dropout entropy
@@ -43,6 +45,10 @@ def main():
         print("    --> fine-tuning the head of", src)
         net.load_params_from(src)
         net.fine_tune(load_scan_training_set(options))
+    elif "--train" in sys.argv and options['resample_mm'] is not None:
+        # on the network's grid: the device-resident set resamples every subject as test_scan does (load_data cannot)
+        net = build_model(weights_path, options)
+        net.fit(load_scan_training_set(options))
     elif "--train" in sys.argv:
         x_axial, x_cor, x_sag, y, x_atlas, names = load_data(options)
         x_train_axial, x_train_cor, x_train_sag, x_train_atlas, y_train = generate_training_set(
