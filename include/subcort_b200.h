@@ -154,6 +154,43 @@ SC_API int sc_gather_samples(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans,
                       const float* atlas_rows_dev, const uint8_t* labels_dev, const int64_t* idx_dev, int64_t n,
                       float* axial_dev, float* coronal_dev, float* saggital_dev, float* atlas_out_dev,
                       uint8_t* y_out_dev, void* stream);
+/* Training-time augmentation in the same gather: every sample's three patches are resampled through one random 3-D similarity
+ * about its centre voxel, then given a random contrast, brightness and Gaussian noise.  Arguments, outputs, NULL rules and trust
+ * rules are those of sc_gather_samples; atlas_out and y_out are its rows unchanged, which stays correct because the transform
+ * keeps the centre voxel fixed.
+ *   Random numbers are keyed by (seed, epoch, table row r = idx[i]), never by the batch position i, so a shuffled minibatch, a
+ *   validation fold or a data-parallel shard sees the same transform for the same row: with s_e = seed ^ (epoch *
+ *   0xD1B54A32D192ED03) (uint64, wrapping) and u(k) = (hash3(s_e, r * 8192 + k) + 0.5) * 2^-32 in (0, 1) (hash3 of
+ *   csrc/common.cuh):
+ *     rotation axis  k = (sqrt(1 - z^2) cos(2 pi u(1)), sqrt(1 - z^2) sin(2 pi u(1)), z), z = 2 u(0) - 1 (uniform on the sphere);
+ *     angle          theta = rotation_deg * (2 u(2) - 1) degrees;          scale  s = (1 + scale)^(2 u(3) - 1);
+ *     contrast       a = 1 + intensity * (2 u(4) - 1);                     brightness  b = intensity * (2 u(5) - 1);
+ *     noise          pixel (view v, row i, column j): g = sqrt(-2 ln u(n)) cos(2 pi u(n + 1)), n = 1024 + 2 (v * 1024 + i * 32 + j).
+ *   Geometry: M = s R(k, theta), R by Rodrigues' formula, evaluated in double and rounded to float per entry.  Pixel (i, j) of a
+ *   view sits at the voxel-index offset o = (i - 16) e_row + (j - 16) e_col from the centre c, with the axes of get_patches
+ *   (axial: rows x, columns y; coronal: rows x, columns z; saggital: rows y, columns z), and samples the scan at
+ *   p = c + (i - 16) M e_row + (j - 16) M e_col (float).  The transform acts in voxel-index space, which is isotropic in mm
+ *   when the scans are on the [model] resample_mm grid.
+ *   Value: trilinear interpolation at p of the zero-extended volume (a corner voxel outside the scan contributes 0: the
+ *   continuous form of get_patches's zero fill), float accumulation in a fixed corner order; out = a * value + b + noise * g for
+ *   every pixel, the zero fill included.  No atomics: the same arguments give byte-identical outputs.
+ *   With all four ranges 0 the outputs equal those of sc_gather_samples: M = I exactly, p is the integer voxel, a = 1, b = 0.
+ *   No mirroring: the 14 structures are seven left / right pairs (Kushibar et al. 2018), and a mirrored patch would need its
+ *   label and its prior channels swapped to the other side's; that is not done here.
+ * SC_ERR_ARG, outputs untouched, in addition to the checks of sc_gather_samples: aug NULL, a non-finite range, rotation_deg
+ * outside [0, 180], scale or noise below 0, intensity outside [0, 1).  The message names the entry point and the field. */
+typedef struct {
+  float rotation_deg;   /* max rotation angle in degrees, [0, 180] */
+  float scale;          /* isotropic scale range sigma_s >= 0: s in [1 / (1 + sigma_s), 1 + sigma_s] */
+  float intensity;      /* contrast / brightness range sigma_i in [0, 1) */
+  float noise;          /* std of the additive Gaussian noise, >= 0 (normalised intensity units) */
+  uint64_t seed;
+  int64_t epoch;
+} sc_augment;           /* 32 bytes */
+SC_API int sc_gather_samples_augmented(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans, const int32_t* samples_dev,
+                                       const float* atlas_rows_dev, const uint8_t* labels_dev, const int64_t* idx_dev, int64_t n,
+                                       const sc_augment* aug, float* axial_dev, float* coronal_dev, float* saggital_dev,
+                                       float* atlas_out_dev, uint8_t* y_out_dev, void* stream);
 
 /* ---- network forward (patchwise) -----------------------------------------------------
  * replaces: net.predict_proba / net.predict on {'in1','in2','in3','in4'}

@@ -24,6 +24,16 @@ METRICS_DTYPE = np.dtype([("n_seg", "<i8"), ("n_ref", "<i8"), ("n_both", "<i8"),
                           ("vol_ref_mm3", "<f8"), ("hd_mm", "<f8"), ("hd95_mm", "<f8"), ("assd_mm", "<f8")])
 assert METRICS_DTYPE.itemsize == 72
 
+
+
+class Augment(ctypes.Structure):
+    """sc_augment of include/subcort_b200.h"""
+    _fields_ = [("rotation_deg", ctypes.c_float), ("scale", ctypes.c_float), ("intensity", ctypes.c_float),
+                ("noise", ctypes.c_float), ("seed", ctypes.c_uint64), ("epoch", ctypes.c_int64)]
+
+
+assert ctypes.sizeof(Augment) == 32
+
 _lib = None
 
 
@@ -73,6 +83,8 @@ PROTOTYPES = {
     "sc_gather_patches": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, ctypes.c_int, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp]),
     "sc_gather_center_labels": (ctypes.c_int, [_vp, _vp, _p(_c_i32), _vp, _c_i64, _vp, _vp]),
     "sc_gather_samples": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "sc_gather_samples_augmented": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, _vp, _vp, _vp, _c_i64, _p(Augment), _vp, _vp, _vp, _vp,
+                                                   _vp, _vp]),
     "sc_forward": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp]),
     "sc_forward_host": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _vp, _vp, _vp]),
     "sc_dense_layer": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _c_i64, _vp, ctypes.c_int, _vp]),
@@ -411,10 +423,12 @@ class Context(object):
         return torch.from_numpy(t.view(np.uint8)).to("cuda:%d" % self.device)
 
     def gather_samples(self, table, n_scans, samples, atlas_rows=None, labels=None, idx=None, n=None,
-                       views=(True, True, True), want_atlas=True, want_y=True):
+                       views=(True, True, True), want_atlas=True, want_y=True, augment=None):
         """Rows idx (None: the first n rows) of a device sample table (int32 [N,4] scan, x, y, z) ->
         (axial, coronal, saggital [n,1,32,32] float32, atlas [n,15] float32, y [n] uint8); outputs not asked for, or
-        whose source is None, are None (sc_gather_samples)."""
+        whose source is None, are None (sc_gather_samples).  augment: None, or a dict of the sc_augment fields
+        (rotation_deg, scale, intensity, noise, seed, epoch; absent ones 0): the patches are gathered through that
+        sample's random transform (sc_gather_samples_augmented)."""
         import torch
         if n is None:
             n = idx.shape[0] if idx is not None else samples.shape[0]
@@ -422,9 +436,16 @@ class Context(object):
         outs = [torch.empty((n, 1, 32, 32), dtype=torch.float32, device=d) if v else None for v in views]
         at = torch.empty((n, 15), dtype=torch.float32, device=d) if want_atlas and atlas_rows is not None else None
         y = torch.empty((n,), dtype=torch.uint8, device=d) if want_y and labels is not None else None
-        _check(self.lib.sc_gather_samples(self.h, _ptr(table), int(n_scans), _ptr(samples), _ptr(atlas_rows), _ptr(labels),
-                                          _ptr(idx), int(n), _ptr(outs[0]), _ptr(outs[1]), _ptr(outs[2]), _ptr(at), _ptr(y),
-                                          _stream()))
+        common = (self.h, _ptr(table), int(n_scans), _ptr(samples), _ptr(atlas_rows), _ptr(labels), _ptr(idx), int(n))
+        outputs = (_ptr(outs[0]), _ptr(outs[1]), _ptr(outs[2]), _ptr(at), _ptr(y), _stream())
+        if augment is None:
+            _check(self.lib.sc_gather_samples(*(common + outputs)))
+        else:
+            unknown = set(augment) - {f for f, _ in Augment._fields_}
+            if unknown:
+                raise ValueError("augment: unknown field(s) %s" % sorted(unknown))
+            aug = Augment(**{k: (int(v) if k in ("seed", "epoch") else float(v)) for k, v in augment.items()})
+            _check(self.lib.sc_gather_samples_augmented(*(common + (ctypes.byref(aug),) + outputs)))
         return outs[0], outs[1], outs[2], at, y
 
     # -- network ------------------------------------------------------------------------------

@@ -825,10 +825,13 @@ class ScanTrainingSet(object):
         ts = self.volumes + [self.table, self.samples, self.atlas, self.labels]
         return int(sum(t.numel() * t.element_size() for t in ts))
 
-    def gather(self, idx=None, ctx=None):
+    def gather(self, idx=None, ctx=None, augment=None, epoch=None):
         """-> (in1, in2, in3, in4, y): axial / coronal / saggital [n, 1, 32, 32] float32, atlas [n, 15] float32 and
         labels [n] uint8 CUDA tensors of rows idx (host integer array, CUDA int64 tensor, or None for every row).  A host
-        idx is range-checked; a device idx is trusted.  ctx: the sc_ctx to launch on (default: the data layer's)."""
+        idx is range-checked; a device idx is trusted.  ctx: the sc_ctx to launch on (default: the data layer's).
+        augment: None, or options['augment'] ({rotation_deg, scale, intensity, noise, seed}): the patches of each row go
+        through that row's random transform of epoch `epoch` (default 0; sc_gather_samples_augmented); atlas rows and labels
+        are unchanged."""
         import torch
         n = None
         if idx is None:
@@ -838,8 +841,10 @@ class ScanTrainingSet(object):
             if idx.size and (idx.min() < 0 or idx.max() >= len(self)):
                 raise IndexError("row index out of range [0, %d)" % len(self))
             idx = _dev(idx, self.ctx.device)
+        if augment is not None:
+            augment = dict(augment, epoch=int(epoch or 0))
         return (ctx or self.ctx).gather_samples(self.table, len(self.volumes), self.samples, self.atlas, self.labels,
-                                                idx=idx, n=n)
+                                                idx=idx, n=n, augment=augment)
 
     def to_arrays(self, chunk=32768):
         """(x_axial, x_cor, x_sag, x_atlas, y) host arrays: what generate_training_set returns for the same seeds."""

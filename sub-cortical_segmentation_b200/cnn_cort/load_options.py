@@ -70,7 +70,43 @@ def load_options(user_config):
     # the scan's grid (base.segment_arrays).  Off when absent or empty
     v = g('model', 'resample_mm', fallback='').strip()
     options['resample_mm'] = parse_resample_mm(v) if v else None
+    # optional: training-time augmentation of the device-resident training set (Net.fit / Net.fine_tune on a ScanTrainingSet):
+    # per sample a random rotation and scale about the centre voxel, contrast, brightness and Gaussian noise.  Off (None) when
+    # every range is absent or 0
+    options['augment'] = parse_augment({key: g('model', 'augment_' + key, fallback='').strip() for key in AUGMENT_KEYS})
     return options
+
+
+# [model] augment_<key>: (lowest value, highest value, highest value allowed itself) of each range, the sc_augment contract
+AUGMENT_RANGES = {'rotation_deg': (0.0, 180.0, True), 'scale': (0.0, math.inf, False), 'intensity': (0.0, 1.0, False),
+                  'noise': (0.0, math.inf, False)}
+AUGMENT_KEYS = tuple(AUGMENT_RANGES) + ('seed',)
+
+
+def parse_augment(values):
+    """{rotation_deg, scale, intensity, noise, seed: string or ''} -> the augmentation dict, or None when every range is 0
+    or absent; a value that is not a number, not finite or out of its range raises ValueError"""
+    aug = {}
+    for key, (lo, hi, hi_ok) in AUGMENT_RANGES.items():
+        v = values.get(key, '')
+        try:
+            x = float(v) if v != '' else 0.0
+        except (TypeError, ValueError):
+            raise ValueError("[model] augment_%s = %r is not a number" % (key, v))
+        if not math.isfinite(x) or x < lo or x > hi or (x == hi and not hi_ok):
+            raise ValueError("[model] augment_%s = %r must be finite and in [%g, %g%s" % (key, v, lo, hi, ']' if hi_ok else ')'))
+        aug[key] = x
+    v = values.get('seed', '')
+    try:
+        seed = int(v) if v != '' else 0
+    except (TypeError, ValueError):
+        raise ValueError("[model] augment_seed = %r is not an integer" % (v,))
+    if not 0 <= seed < 1 << 64:
+        raise ValueError("[model] augment_seed = %r must be in [0, 2^64)" % (v,))
+    if not any(aug.values()):
+        return None
+    aug['seed'] = seed
+    return aug
 
 
 def parse_resample_mm(v):

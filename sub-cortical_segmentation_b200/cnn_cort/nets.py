@@ -25,6 +25,7 @@ from . import _native
 from . import parallel
 
 BRANCHES = ('axial', 'coronal', 'saggital')   # reference spelling, nets.py:202
+FEATURE_CHUNK = 16384                         # samples per trunk-feature pass of fine_tune
 _CONV = ((1, 20), (20, 20), (20, 40), (40, 40), (40, 60))
 
 
@@ -221,7 +222,9 @@ class Net(object):
     # -- training (nolearn epoch loop: nets.py:233-246) ---------------------------------------
     def fit(self, X, y=None, epochs=None):
         """nolearn's fit on X = {'in1', 'in2', 'in3', 'in4'} arrays with labels y, or on a base.ScanTrainingSet (y
-        omitted), whose minibatches are gathered on the device from the scans.  Same epoch loop either way."""
+        omitted), whose minibatches are gathered on the device from the scans.  Same epoch loop either way.
+        With options['augment'] (ScanTrainingSet only) every training minibatch of epoch ep is gathered through the rows'
+        random transforms of that epoch; validation minibatches never are."""
         import torch
         import torch.distributed as dist
         ctx = self.ctx
@@ -229,6 +232,9 @@ class Net(object):
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         rank = dist.get_rank() if world > 1 else 0
         scans = hasattr(X, 'gather')
+        augment = self.options.get('augment')
+        if augment is not None and not scans:
+            raise ValueError("fit: augmentation needs a ScanTrainingSet (arrays hold patches that are already cut)")
         if scans:
             if y is not None:
                 raise ValueError("fit: a ScanTrainingSet carries its own labels; call fit(scans) without y")
@@ -280,12 +286,17 @@ class Net(object):
                 # shard_batch has some iff r < len(gidx)
                 ctx.adam_step(lr=self.update_learning_rate, stat_scale=1.0 / min(world, len(gidx)))
 
-        return self._epoch_loop(tr, va, batches, step, lambda b: ctx.eval_batch(*b), dev, epochs, rank, world)
+        train_batches = None
+        if scans and augment is not None:
+            train_batches = lambda index_lists, ep: batches(index_lists, augment, ep)   # noqa: E731
+        return self._epoch_loop(tr, va, batches, step, lambda b: ctx.eval_batch(*b), dev, epochs, rank, world, train_batches)
 
-    def _epoch_loop(self, tr, va, batches, step, evaluate, dev, epochs, rank=0, world=1):
+    def _epoch_loop(self, tr, va, batches, step, evaluate, dev, epochs, rank=0, world=1, train_batches=None):
         """nolearn's epoch loop over the training rows tr and validation rows va: minibatches of batch_size rows, this rank's
         share of each (shard_batch); batches(index lists) yields each list's minibatch (None for an empty one),
         step(global rows, minibatch, loss buffer) trains on it, evaluate(minibatch) -> CUDA {sum of -log p[y], correct}.
+        train_batches(index lists, epoch), when given, replaces batches for the training minibatches of each epoch; the epoch
+        number continues across calls (the history's length), so a resumed run never repeats an epoch's number.
         History, best-weight checkpoint, history file and early stopping as nolearn's handlers (nets.py:154-156)."""
         import torch
         best_valid, best_train = np.inf, np.inf
@@ -300,7 +311,7 @@ class Net(object):
         for ep in range(first + 1, first + n_epochs + 1):
             t0 = time.time()
             losses, sizes = [], []
-            for gidx, b in zip(steps, batches(local_steps)):
+            for gidx, b in zip(steps, batches(local_steps) if train_batches is None else train_batches(local_steps, ep)):
                 step(gidx, b, loss_buf)
                 losses.append(loss_buf.clone())
                 sizes.append(len(gidx))
@@ -345,13 +356,18 @@ class Net(object):
         statistics, into a device table of 3 x 540 float32 features per sample (6 480 B); every step then trains d1 x3, FC1,
         fc_2 and out_layer from those rows with the training dropout, loss and Adam of fit.  The optimiser is reset, and
         the trunk -- parameters, Adam moments and BatchNorm running statistics -- stays exactly as it was.  Same epoch loop,
-        history, checkpoint, history file and early stopping as fit.  Single device only."""
+        history, checkpoint, history file and early stopping as fit.  Single device only.
+        With options['augment'] (ScanTrainingSet only) the table rows of the training split are rebuilt at the start of every
+        epoch from that epoch's augmented gather (what fit would feed the frozen trunk); the validation rows stay unaugmented."""
         import torch
         import torch.distributed as dist
         if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
             raise RuntimeError("fine_tune: data-parallel fine-tuning is not supported (world size %d)" % dist.get_world_size())
         ctx = self.ctx
         dev = torch.device('cuda', self.device)
+        augment = self.options.get('augment')
+        if augment is not None and not hasattr(X, 'gather'):
+            raise ValueError("fine_tune: augmentation needs a ScanTrainingSet (arrays hold patches that are already cut)")
         feats, atlas, labels, y = self._feature_table(X, y, dev)
         tr, va = self.train_split.indices(y)
 
@@ -363,6 +379,17 @@ class Net(object):
                 yield d_idx[off:off + len(idx)] if len(idx) else None
                 off += len(idx)
 
+        train_batches = None
+        if augment is not None:
+            d_tr = torch.from_numpy(np.asarray(tr, dtype=np.int64)).to(dev)
+
+            def train_batches(index_lists, ep):
+                for s in range(0, len(tr), FEATURE_CHUNK):     # the training rows' features of this epoch's transforms
+                    rows = d_tr[s:s + FEATURE_CHUNK]
+                    in1, in2, in3, _, _ = X.gather(rows, ctx=ctx, augment=augment, epoch=ep)
+                    feats.index_copy_(0, rows, ctx.trunk_features(in1, in2, in3))
+                return batches(index_lists)
+
         rng = np.random.RandomState(self._seed)
 
         def step(gidx, idx, loss_buf):
@@ -373,11 +400,11 @@ class Net(object):
         ctx.freeze_trunk(True)
         try:
             return self._epoch_loop(tr, va, batches, step, lambda idx: ctx.head_eval_batch(feats, atlas, labels, idx=idx), dev,
-                                    epochs)
+                                    epochs, train_batches=train_batches)
         finally:
             ctx.freeze_trunk(False)
 
-    def _feature_table(self, X, y, dev, chunk=16384):
+    def _feature_table(self, X, y, dev, chunk=FEATURE_CHUNK):
         """-> (trunk features [N, 3, 540], atlas rows [N, 15], labels [N] uint8 as CUDA tensors, host labels)"""
         import torch
         ctx = self.ctx
@@ -451,18 +478,19 @@ class Net(object):
     def _scan_batches(self, scans, dev):
         """minibatch source of fit on a ScanTrainingSet: one upload of all row indices of a pass (an epoch's training or
         validation minibatches); every minibatch is then gathered from the scans on the device (sc_gather_samples, on
-        this net's context) out of a slice of that upload -- no host synchronise per step"""
+        this net's context) out of a slice of that upload -- no host synchronise per step.  batches(index lists, augment,
+        epoch) gathers through the rows' random transforms of that epoch (sc_gather_samples_augmented)."""
         import torch
         ctx = self.ctx
 
-        def batches(index_lists):
+        def batches(index_lists, augment=None, epoch=None):
             flat = np.concatenate([np.asarray(i, dtype=np.int64) for i in index_lists]) if index_lists else np.zeros(0, np.int64)
             if flat.size and (flat.min() < 0 or flat.max() >= len(scans)):
                 raise IndexError("fit: row index out of range [0, %d)" % len(scans))
             d_idx = torch.from_numpy(flat).to(dev)
             off = 0
             for idx in index_lists:
-                yield scans.gather(d_idx[off:off + len(idx)], ctx=ctx) if len(idx) else None
+                yield scans.gather(d_idx[off:off + len(idx)], ctx=ctx, augment=augment, epoch=epoch) if len(idx) else None
                 off += len(idx)
         return batches
 

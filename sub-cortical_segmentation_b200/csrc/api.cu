@@ -225,7 +225,7 @@ int64_t sc_get_counter(sc_ctx* ctx, const char* key) {
 
 static const char* kProfNames[PC_COUNT] = {"gather", "nonzero", "scatter", "patch_branch", "conv1", "conv2", "conv3",
                                            "conv4", "conv5", "gemm_d1", "gemm_fc1", "gemm_fc2", "atlas", "out_softmax", "pool",
-                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc", "head", "resample"};
+                                           "train_fwd", "train_bwd", "adam", "evaluate", "register", "mc", "head", "resample", "augment"};
 }  // extern "C"
 namespace sc { const char* prof_class_name(int cls) { return cls >= 0 && cls < PC_COUNT ? kProfNames[cls] : "subcort"; } }
 extern "C" {
@@ -502,6 +502,29 @@ int sc_gather_samples(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans, const 
   SC_CUDA(cudaSetDevice(ctx->device));
   return launch_gather_samples(ctx, scans_dev, n_scans, samples_dev, atlas_rows_dev, labels_dev, idx_dev, n, axial_dev,
                                coronal_dev, saggital_dev, atlas_out_dev, y_out_dev, (cudaStream_t)stream);
+}
+
+int sc_gather_samples_augmented(sc_ctx* ctx, const sc_scan* scans_dev, int n_scans, const int32_t* samples_dev,
+                                const float* atlas_rows_dev, const uint8_t* labels_dev, const int64_t* idx_dev, int64_t n,
+                                const sc_augment* aug, float* axial_dev, float* coronal_dev, float* saggital_dev,
+                                float* atlas_out_dev, uint8_t* y_out_dev, void* stream) {
+  const char* who = "sc_gather_samples_augmented";
+  SC_CHECK(ctx && n >= 0 && n_scans >= 0, SC_ERR_ARG, "%s: null context or negative count", who);
+  SC_CHECK(aug, SC_ERR_ARG, "%s: aug is NULL", who);
+  SC_CHECK(isfinite(aug->rotation_deg) && aug->rotation_deg >= 0.f && aug->rotation_deg <= 180.f, SC_ERR_ARG,
+           "%s: aug->rotation_deg = %g (finite, in [0, 180])", who, aug->rotation_deg);
+  SC_CHECK(isfinite(aug->scale) && aug->scale >= 0.f, SC_ERR_ARG, "%s: aug->scale = %g (finite, >= 0)", who, aug->scale);
+  SC_CHECK(isfinite(aug->intensity) && aug->intensity >= 0.f && aug->intensity < 1.f, SC_ERR_ARG,
+           "%s: aug->intensity = %g (in [0, 1))", who, aug->intensity);
+  SC_CHECK(isfinite(aug->noise) && aug->noise >= 0.f, SC_ERR_ARG, "%s: aug->noise = %g (finite, >= 0)", who, aug->noise);
+  SC_CHECK(!atlas_out_dev || atlas_rows_dev, SC_ERR_ARG, "%s: atlas output requested without atlas rows", who);
+  SC_CHECK(!y_out_dev || labels_dev, SC_ERR_ARG, "%s: label output requested without labels", who);
+  if (n == 0) return SC_OK;
+  SC_CHECK(scans_dev && n_scans > 0 && samples_dev, SC_ERR_ARG, "%s: missing scan list or sample table", who);
+  SC_CHECK(((uintptr_t)samples_dev & 15) == 0, SC_ERR_ARG, "%s: sample table not 16-byte aligned", who);
+  SC_CUDA(cudaSetDevice(ctx->device));
+  return launch_gather_samples_augmented(ctx, scans_dev, n_scans, samples_dev, atlas_rows_dev, labels_dev, idx_dev, n, *aug,
+                                         axial_dev, coronal_dev, saggital_dev, atlas_out_dev, y_out_dev, (cudaStream_t)stream);
 }
 
 int sc_forward(sc_ctx* ctx, const float* in1_dev, const float* in2_dev, const float* in3_dev, const float* in4_dev,

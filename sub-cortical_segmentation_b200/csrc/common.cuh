@@ -148,7 +148,7 @@ struct Workspace {
 // per-kernel-class timing with CUDA events on the launching stream (sc_set_option "profile")
 enum ProfClass {
   PC_GATHER = 0, PC_NONZERO, PC_SCATTER, PC_PATCH_BRANCH, PC_CONV1, PC_CONV2, PC_CONV3, PC_CONV4, PC_CONV5,
-  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_HEAD, PC_RESAMPLE, PC_COUNT
+  PC_GEMM_D1, PC_GEMM_FC1, PC_GEMM_FC2, PC_ATLAS, PC_OUT, PC_POOL, PC_TRAIN_FWD, PC_TRAIN_BWD, PC_ADAM, PC_EVALUATE, PC_REGISTER, PC_MC, PC_HEAD, PC_RESAMPLE, PC_AUGMENT, PC_COUNT
 };
 
 // counter-based random bits (splitmix64 finaliser): the dropout keep masks of the training step and of Monte-Carlo dropout
@@ -288,6 +288,10 @@ int launch_center_labels(sc_ctx* ctx, const uint8_t* lab, const int32_t* dims, c
 int launch_gather_samples(sc_ctx* ctx, const sc_scan* scans, int n_scans, const int32_t* samples, const float* atlas_rows,
                           const uint8_t* labels, const int64_t* idx, int64_t n, float* ax, float* co, float* sa,
                           float* atlas_out, uint8_t* y_out, cudaStream_t st);
+// augment.cu : the same gather through a random similarity per sample, with contrast, brightness and noise (sc_gather_samples_augmented)
+int launch_gather_samples_augmented(sc_ctx* ctx, const sc_scan* scans, int n_scans, const int32_t* samples, const float* atlas_rows,
+                                    const uint8_t* labels, const int64_t* idx, int64_t n, const sc_augment& aug, float* ax, float* co,
+                                    float* sa, float* atlas_out, uint8_t* y_out, cudaStream_t st);
 int launch_nonzero(sc_ctx* ctx, const void* vol, int elem_bytes, const int32_t* dims, int32_t* xyz,
                    int64_t capacity, int64_t* n_out_host, cudaStream_t st);
 int launch_dilate(sc_ctx* ctx, const uint8_t* mask, const int32_t* dims, int iterations, uint8_t* out, cudaStream_t st);

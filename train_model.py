@@ -7,7 +7,8 @@ keys); everything below the imports runs on the B200 kernels.
 --train with [model] fine_tune_from = <experiment> fine-tunes the head of nets/<experiment>/<experiment>.pkl on the training
 folder (frozen convolutional trunk, Net.fine_tune) instead of training from scratch.
 With [model] resample_mm set, training runs on the device-resident set resampled to that isotropic grid, as test_scan
-segments.
+segments.  With [model] augment_* ranges set, training runs on the device-resident set too, and every training minibatch is
+gathered through random per-sample rotations, scales, contrast, brightness and noise.
 
 --evaluate scores each inference subject that has manual labels (<subject>/<roi_name>): per-structure Dice and
 surface distances of the segmentation test_scan wrote, and with [model] mc_samples > 0 the mean Monte-Carlo dropout entropy
@@ -45,8 +46,9 @@ def main():
         print("    --> fine-tuning the head of", src)
         net.load_params_from(src)
         net.fine_tune(load_scan_training_set(options))
-    elif "--train" in sys.argv and options['resample_mm'] is not None:
-        # on the network's grid: the device-resident set resamples every subject as test_scan does (load_data cannot)
+    elif "--train" in sys.argv and (options['resample_mm'] is not None or options['augment'] is not None):
+        # on the network's grid: the device-resident set resamples every subject as test_scan does (load_data cannot); the
+        # augmented gather cuts every minibatch from the scans (the patch arrays of load_data are already cut)
         net = build_model(weights_path, options)
         net.fit(load_scan_training_set(options))
     elif "--train" in sys.argv:
